@@ -3,9 +3,12 @@
 (MC samples x data rows) / s, beside the reference algorithm's CPU path on the same box.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload bnn|logreg|svgd|vae]
+                    [--dump-outputs DIR]
 
 One "step" = one ELBO + pathwise-gradient evaluation (loss and d loss/d every variational parameter)
-of the workload on synthetic data.  Workloads (SURVEY.md §8d):
+of the workload on synthetic data.  --dump-outputs DIR writes what the last timed step returned (loss and
+gradients; for svgd also the particle gradients and the SVGD direction) as DIR/<name>.npy, so that two builds
+can be compared output for output: the inputs depend only on the arguments.  Workloads (SURVEY.md §8d):
   bnn     C3  MNIST-shaped BNN 784-100-10, minibatch 1024, 256 MC samples per GPU     (default; the
               config BASELINE.json's north_star quotes its target on)
   logreg  C2  Bayesian logistic regression, 10^6 rows x 128 features, 1024 MC samples
@@ -19,6 +22,8 @@ import subprocess
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True          # the benchmark leaves the tree it runs from as it found it
 
 # stdout carries exactly ONE JSON line.  NCCL prints its version banner to stdout on the multi-GPU boxes, so file descriptor 1 is
 # pointed at stderr for the whole run and the result line is written to a private duplicate of the original stdout.
@@ -420,6 +425,23 @@ def api_e2e(dev):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """arrays: name -> device tensor.  Written as float64 when computed in fp64, float32 otherwise."""
+    host = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        host[name] = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(path, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------
 # our arm
 # ---------------------------------------------------------------------------------------------
@@ -463,6 +485,12 @@ def main_ours(args):
             gflat.zero_()
             return cu.bnn_elbo_fwd_bwd(Xd, yd, mvars, r, data_ready=data_ready)
 
+        def outputs():
+            out = {}
+            for n, v in zip(names, mvars):
+                out["grad_%s_loc" % n], out["grad_%s_scale" % n] = v.dmu.view(shapes[n]), v.drho.view(shapes[n])
+            return out
+
         # the product's training loop replays ONE captured iteration (brancher_b200/inference._fused_loop): the same here --
         # the evaluation is captured once, its Philox offset lives in device memory and is bumped inside the graph
         offset_dev = torch.zeros(1, dtype=torch.int64, device=dev)
@@ -502,6 +530,14 @@ def main_ours(args):
             r = cu.sample_range(S_total, seed=args.seed, offset=it)
             gflat.zero_()
             return cu.vae_elbo_fwd_bwd(Xd, net, r, row0=rank * B, B_total=B * world, add_constant=(rank == 0))
+
+        def outputs():
+            layers = (["enc.%d" % i for i in range(len(net.enc))] + ["enc_mean", "enc_sd"] +
+                      ["dec.%d" % i for i in range(len(net.dec))] + ["dec_out"])
+            out = {}
+            for n, (gW, gb) in zip(layers, net.grads):
+                out["grad_%s.W" % n], out["grad_%s.b" % n] = gW, gb
+            return out
     elif wl == "ar1":
         # MC samples sharded (pointless at this size, SURVEY 8e: shown for completeness); all-reduce of 43 gradients + loss
         from brancher_b200 import lowering
@@ -528,6 +564,9 @@ def main_ours(args):
             loss, g = cu.dag_elbo_fwd_bwd(ops, ops.numel() // 24, Pg.n_slots, pvec, Xd, plan.n_rows, None, len(Pg.eps_names), r)
             gflat[:pvec.numel()] = g
             return loss
+
+        def outputs():
+            return {"grad_params": gflat[:pvec.numel()]}         # the program's parameters in table order
     elif wl == "svgd":
         # particles sharded over ranks (weak scaling: n particles per rank), data replicated; the pairwise stage needs
         # all particles: all-gather theta and G (2 MB each per rank), every rank computes its rows of K and the update
@@ -549,12 +588,12 @@ def main_ours(args):
         gflat = torch.zeros(4, device=dev)
         theta_all = torch.empty((n_total, F), device=dev)
         G_all = torch.empty((n_total, F), device=dev)
-        svgd_out = [None, None]
+        svgd_out = [None, None, None]         # direction, variant, particle gradients
         S_total = n_total
 
         def device_step(it, Xd=X, yd=y):
             loss, G = cu.linear_particles_loss_grad(Xd, yd, cu.BERNOULLI, theta_local, 1, pl, ps)
-            svgd_out[1] = cu.last_variant()
+            svgd_out[1], svgd_out[2] = cu.last_variant(), G
             if world > 1 and not os.environ.get("BRN_BENCH_SVGD_REPLICATED"):
                 # all-gather of (theta, G), then the median selection sharded by rows: 5 small NCCL collectives
                 svgd_out[0], _ = distributed.svgd_direction_sharded(theta_local, G)
@@ -568,6 +607,9 @@ def main_ours(args):
                 svgd_out[0], _ = cu.svgd_direction(th, gg, row0=rank * n_local, rows=n_local)
             svgd_out[1] += " (K4a) + %s (K4b)" % cu.last_variant()
             return loss
+
+        def outputs():
+            return {"particle_grad": svgd_out[2], "direction": svgd_out[0]}
     else:
         rows = cfg["N"]
         Xh, yh, params = synth_logreg(cfg, seed=rank)
@@ -595,6 +637,9 @@ def main_ours(args):
             gflat.zero_()
             # rows are sharded: every rank holds the same samples; prior/entropy counted once (rank 0)
             return cu.linear_elbo_fwd_bwd(Xd, yd, cu.BERNOULLI, w, 1, r, with_prior=(rank == 0), prepared=prepared)
+
+        def outputs():
+            return {"grad_weights_loc": w.dmu.view(1, -1), "grad_weights_scale": w.drho.view(1, -1)}
 
     def reduce_partials(loss):
         """all-reduce [grads | loss_hi, loss_lo] across ranks IN PLACE: one NCCL collective on the flat gradient
@@ -687,7 +732,8 @@ def main_ours(args):
             dist.barrier()
             torch.cuda.synchronize()
 
-    def timed(fn, steps, warmup, profile=False):
+    def timed(fn, steps, warmup, profile=False, last=None):
+        """last: optional list whose element 0 receives what the last timed step returned"""
         for i in range(warmup):
             fn(i)
         barrier()
@@ -698,8 +744,10 @@ def main_ours(args):
         for i in range(steps):
             flush.fill_(float(i))                   # L2 flush between timed iterations (not timed)
             evs[i][0].record()
-            fn(warmup + i)
+            res = fn(warmup + i)
             evs[i][1].record()
+        if last is not None:
+            last[0] = res
         barrier()
         launches = cu.launch_count() - l0
         stages = {}
@@ -750,7 +798,10 @@ def main_ours(args):
     # the library (10 records per C3 step) cost ~29 us per step when they sit in that region (measured, profiles/r1z_*), so the
     # stage split and the dominant kernel's duration come from a second, equally long pass with the events enabled; its own
     # total normalises the shares.
-    ms, launches, _ = timed(graph_step or step, args.steps, args.warmup, profile=False)
+    last_loss = [None]
+    ms, launches, _ = timed(graph_step or step, args.steps, args.warmup, profile=False, last=last_loss)
+    if args.dump_outputs and rank == 0:          # before the later passes overwrite the gradient buffers
+        dump_outputs(args.dump_outputs, dict(outputs(), loss=last_loss[0].reshape(())))
     if graph_step:
         launches = launches_per_graph * args.steps
     ms_prof, _, stages = timed(step, args.steps, 1, profile=True)
@@ -841,14 +892,20 @@ def main_ours(args):
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=1000)
+    ap.add_argument("--steps", type=int, default=1000, help="timed steps of the headline measurement")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="bnn", choices=sorted(WORKLOADS))
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-api", action="store_true", help="skip the perform_inference (API-level) timing block")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and gradients of the last timed step as DIR/<name>.npy (--impl ours)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
     if a.impl == "reference":
         main_reference(a)
