@@ -26,7 +26,9 @@ struct LinearArgs {
     double* ll_cols;                 // optional [S]: per-sample log-likelihood sums (K6), += ; loss may then be NULL
 };
 
-template <int LIK>   // 0: Bernoulli/Binomial(1) with float y, 1: Categorical with int32 labels
+// 0: Bernoulli/Binomial(1) with float y, 1: Categorical with int32 labels, 2: Gaussian residuals with float y (C == 1): d = r =
+// y - l and ll_cols[s] += sum r^2 (loss unused; the noise scale is applied per sample afterwards, linreg_finish_kernel)
+template <int LIK>
 __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
     extern __shared__ __align__(16) float sm[];
     float (*Xs)[LN_LD] = reinterpret_cast<float (*)[LN_LD]>(sm);                       // [row][f]
@@ -57,7 +59,7 @@ __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) acc2[i][j] = 0.f;
     double ll_thread = 0.0;
-    double llc[8];                   // LIK == 0 with ll_cols: this thread's 8 columns, summed over its rows and tiles
+    double llc[8];                   // LIK == 0 / 2 with ll_cols: this thread's 8 columns, summed over its rows and tiles
 #pragma unroll
     for (int j = 0; j < 8; ++j) llc[j] = 0.0;
     __shared__ double llcol_s[LN_T];  // LIK == 1 with ll_cols: per sample of the tile
@@ -85,7 +87,7 @@ __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
         if (t < LN_T) {
             float v = 0.f;
             if (r0 + t < a.N) {
-                if (LIK == 0) v = reinterpret_cast<const float*>(a.y)[r0 + t];
+                if (LIK != 1) v = reinterpret_cast<const float*>(a.y)[r0 + t];
                 else v = __int_as_float(reinterpret_cast<const int32_t*>(a.y)[r0 + t]);
             }
             ys[t] = v;
@@ -122,7 +124,25 @@ __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
 
         // ---- phase 2: log-likelihood and d ll / d logit
         float ll_tile = 0.f;
-        if (LIK == 0) {
+        if (LIK == 2) {
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+                int row = (i < 4 ? ty * 4 + i : 64 + ty * 4 + (i - 4));
+                bool rv = r0 + row < a.N;
+                float yv = ys[row];
+                float d[8];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    int col = (j < 4 ? tx * 4 + j : 64 + tx * 4 + (j - 4));
+                    bool ok = rv && col < ncols && (j0 + col) < J;
+                    d[j] = ok ? yv - acc[i][j] : 0.f;
+                    if (a.ll_cols) llc[j] += (double)(d[j] * d[j]);
+                }
+                *reinterpret_cast<float4*>(&Ls[row][tx * 4]) = make_float4(d[0], d[1], d[2], d[3]);
+                *reinterpret_cast<float4*>(&Ls[row][64 + tx * 4]) = make_float4(d[4], d[5], d[6], d[7]);
+            }
+            __syncthreads();
+        } else if (LIK == 0) {
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
                 int row = (i < 4 ? ty * 4 + i : 64 + ty * 4 + (i - 4));
@@ -204,7 +224,7 @@ __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
 
     // ---- flush
     if (a.ll_cols) {
-        if (LIK == 0) {
+        if (LIK != 1) {
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
                 const int col = (j < 4 ? tx * 4 + j : 64 + tx * 4 + (j - 4));
@@ -371,6 +391,9 @@ static int launch_linear_fused(const float* X, const void* y, int likelihood, in
     if (likelihood == 0) {
         BRN_CUDA_OK(cudaFuncSetAttribute(linear_fused_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         linear_fused_kernel<0><<<grid, 256, smem, stream>>>(a);
+    } else if (likelihood == 2) {
+        BRN_CUDA_OK(cudaFuncSetAttribute(linear_fused_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        linear_fused_kernel<2><<<grid, 256, smem, stream>>>(a);
     } else {
         BRN_CUDA_OK(cudaFuncSetAttribute(linear_fused_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         linear_fused_kernel<1><<<grid, 256, smem, stream>>>(a);
@@ -627,4 +650,182 @@ extern "C" int brn_linear_elbo_fwd_bwd_px(const float* X, const void* px, const 
     }
     StageTimer st3("linear.reduce_finalize", stream);
     return launch_mf_reduce_finalize(*w, eps, numel, ws.dW, numel, ws.stats, *r, with_prior, loss, stream);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Bayesian linear regression: y_b ~ Normal(w_s . x_b, sigma_s) (see include/brancher_cuda.h, brn_linreg_elbo_fwd_bwd).
+// The kernels that read X never see sigma: they produce G_s = sum_b r_sb x_b and R_s = sum_b r_sb^2 per sample, and
+// linreg_finish_kernel applies the noise scale, so both noise modes share one pass over X and sigma_s costs nothing there.
+// ---------------------------------------------------------------------------------------------
+namespace brn {
+
+struct LinregWorkspace {
+    float *eps, *W, *dW, *stats;
+    double* R;                 // [S] sums of squared residuals
+    LinearFlashBuffers flash;
+    size_t bytes;
+    LinregWorkspace(void* base, int S, int64_t N, int F, bool flash_path, int sms) {
+        WorkspaceCarver take(base);
+        eps = take((size_t)S * F);
+        W = take((size_t)S * F);
+        dW = take((size_t)S * F);
+        stats = take(4 * (size_t)((F + 3) / 4 * 4));
+        R = reinterpret_cast<double*>(take(2 * (size_t)S));
+        flash = LinearFlashBuffers();
+        if (flash_path) {
+            flash.carve(take, S, F, sms);
+            flash.Xh = reinterpret_cast<__half*>(take(((size_t)N * F + 1) / 2));
+            flash.Xl = reinterpret_cast<__half*>(take(((size_t)N * F + 1) / 2));
+        }
+        bytes = take.off;
+    }
+};
+
+// the one-pass kernel where the Bernoulli evaluation of the same shape takes it; there is no staged-GEMM-pair variant
+static bool linreg_use_flash(const float* X, int64_t N, int F, int S) {
+    return linear_use_tc(0, N, F, 1, S) && linear_flash_ok(X, N, F, S);
+}
+
+// One thread per element (s, f) of the per-sample gradient rows: dW_s *= 1 / sigma_s^2 in place.  The thread of f == 0 also owns
+// sample s's scalar terms, all scaled by 1 / S_total (the partial contract of brn_mf_normal_prior_entropy, so sharded samples
+// sum to the unsharded result):
+//   ll_s = -R_s / (2 sigma_s^2) - N log sigma_s - N log sqrt(2 pi)
+// and, for the LogNormal latent (u_s = m + softplus(rho) e_s, sigma_s = exp(u_s)), d ll_s / d u_s = R_s / sigma_s^2 - N chained to
+// (m, rho), with log p(nu_s) = NORMAL_LP(log nu_s; a, b) - log nu_s and H[q(nu)] = H_Normal(softplus(rho)) + m composed as the
+// scalar-DAG family composes them (tied: a = m, b = softplus(rho), differentiated through both the sample and the prior, where
+// the terms cancel in closed form as in the mean-field finalisation).
+__global__ void __launch_bounds__(256)
+linreg_finish_kernel(float* __restrict__ dW, const double* __restrict__ R, int F, int64_t N, brn_mf_var nu, int has_nu,
+                     const float* __restrict__ noise_scale, brn_sample_range r, int with_prior, double* __restrict__ loss) {
+    __shared__ double red[32];
+    __shared__ float red_m[32], red_s[32];
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t total = (int64_t)r.s_local * F;
+    double elbo = 0.0;
+    float gm = 0.f, gs = 0.f;            // d ELBO_s / d m, d ELBO_s / d softplus(rho) of the noise latent
+    if (i < total) {
+        const int s = (int)(i / F);
+        float sigma, e = 0.f, m = 0.f, sg = 1.f;
+        if (has_nu) {
+            e = nu.eps ? nu.eps[s] : philox_normal1(r.seed, philox_offset(r), nu.var_id, (uint32_t)(r.s0 + s), 0);
+            m = nu.mu[0];
+            sg = softplusf(nu.rho[0]);
+            sigma = expf(__fmaf_rn(e, sg, m));
+        } else {
+            sigma = *noise_scale;
+        }
+        dW[i] *= 1.0f / (sigma * sigma);
+        if (i % F == 0) {
+            const double sd = sigma, inv_s2 = 1.0 / (sd * sd), Rs = R[s];
+            elbo = -0.5 * Rs * inv_s2 - (double)N * (log(sd) + (double)BRN_HALF_LOG_2PI);
+            if (has_nu) {
+                const float gu = (float)(Rs * inv_s2 - (double)N);
+                gm = gu;
+                gs = gu * e;
+                if (with_prior) {
+                    const float lx = logf(sigma);                      // LOG(EXP(u)): the sample's log as the DAG evaluates it
+                    const float a = nu.tied ? m : nu.prior_loc[0], b = nu.tied ? sg : nu.prior_scale[0];
+                    const float dd = lx - a, ib2 = 1.0f / (b * b);
+                    const float lp = -0.5f * dd * dd * ib2 - logf(b) - BRN_HALF_LOG_2PI - lx;
+                    const float ent = 0.5f + BRN_HALF_LOG_2PI + logf(sg) + m;
+                    elbo += (double)lp + (double)ent;
+                    if (nu.tied) {
+                        // log p = -e^2/2 - log sg - c - u with a = m, b = sg: d/dm = -1, d/dsg = -1/sg - e; with the entropy's
+                        // +1, +1/sg the (m, sg) gradient of prior + entropy is (0, -e) exactly
+                        gs -= e;
+                    } else {
+                        const float gpu = -dd * ib2 - 1.0f;            // d log p / d u
+                        gm += gpu + 1.0f;
+                        gs += gpu * e + 1.0f / sg;
+                    }
+                }
+            }
+        }
+    }
+    const double tot = block_sum<double>(elbo, red);
+    if (threadIdx.x == 0 && tot != 0.0) atomicAdd(loss, -tot / (double)r.s_total);
+    if (has_nu) {
+        const float tm = block_sum<float>(gm, red_m), ts = block_sum<float>(gs, red_s);
+        if (threadIdx.x == 0) {
+            const float inv_S = 1.0f / (float)r.s_total;
+            atomicAdd(nu.dmu, -tm * inv_S);
+            atomicAdd(nu.drho, -ts * inv_S * sigmoidf(nu.rho[0]));
+        }
+    }
+}
+
+}  // namespace brn
+
+extern "C" size_t brn_linreg_workspace_bytes(int64_t N, int F, int s_local) {
+    if (N < 0 || F <= 0 || s_local < 0) return 0;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    // sized for the one-pass kernel whenever a call of this shape may take it (X's alignment is not known here)
+    return LinregWorkspace(nullptr, s_local, N, F, linreg_use_flash(nullptr, N, F, s_local), sms).bytes;
+}
+
+extern "C" int brn_linreg_elbo_fwd_bwd(const float* X, const void* px, const float* y, int64_t N, int F, const brn_mf_var* w,
+                                       const brn_mf_var* nu, const float* noise_scale, const brn_sample_range* r,
+                                       void* workspace, size_t workspace_bytes, int with_prior, double* loss, void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    BRN_CHECK_ARG(w && r && loss, "brn_linreg_elbo_fwd_bwd: NULL pointer");
+    BRN_CHECK_ARG(N >= 0 && F > 0, "brn_linreg_elbo_fwd_bwd: bad shape N=%lld F=%d", (long long)N, F);
+    BRN_CHECK_ARG(N == 0 || (X && y), "brn_linreg_elbo_fwd_bwd: NULL data pointer");
+    BRN_CHECK_ARG(F <= LN_T, "brn_linreg_elbo_fwd_bwd: F=%d exceeds the supported maximum %d", F, LN_T);
+    BRN_CHECK_ARG(!px || (linear_prepared_x_bytes(N, F) > 0 && (reinterpret_cast<uintptr_t>(px) & 255) == 0),
+                  "brn_linreg_elbo_fwd_bwd: a prepared X does not exist for N=%lld F=%d, or px is not 256-byte aligned", (long long)N, F);
+    BRN_CHECK_ARG((nu == nullptr) != (noise_scale == nullptr),
+                  "brn_linreg_elbo_fwd_bwd: give exactly one of nu (LogNormal noise latent) and noise_scale (fixed noise)");
+    BRN_CHECK_ARG(r->s_local >= 0 && r->s_total > 0 && r->s0 >= 0 && r->s0 + r->s_local <= r->s_total,
+                  "bad sample range s0=%d s_local=%d s_total=%d", r->s0, r->s_local, r->s_total);
+    BRN_CHECK_ARG(w->numel == F, "w->numel=%lld, expected F=%d", (long long)w->numel, F);
+    BRN_CHECK_ARG(w->mu && w->rho && w->dmu && w->drho, "w: NULL parameter pointer");
+    BRN_CHECK_ARG(!with_prior || w->tied || (w->prior_loc && w->prior_scale), "w: prior_loc/prior_scale required when not tied");
+    if (nu) {
+        BRN_CHECK_ARG(nu->numel == 1, "nu->numel=%lld, the noise latent is a scalar", (long long)nu->numel);
+        BRN_CHECK_ARG(nu->mu && nu->rho && nu->dmu && nu->drho, "nu: NULL parameter pointer");
+        BRN_CHECK_ARG(!with_prior || nu->tied || (nu->prior_loc && nu->prior_scale), "nu: prior_loc/prior_scale required when not tied");
+    }
+    const int S = r->s_local;
+    if (S == 0) return 0;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const bool use_flash = N > 0 && linreg_use_flash(X, N, F, S);
+    LinregWorkspace ws(workspace, S, N, F, use_flash, sms);
+    BRN_CHECK_ARG(workspace && workspace_bytes >= ws.bytes, "workspace too small: %zu < %zu", workspace_bytes, ws.bytes);
+    set_variant(use_flash ? "tcgen05-flash" : "simt");
+
+    const float* eps = w->eps;
+    {
+        StageTimer st("linreg.sample_weights", stream);
+        if (!eps) {
+            if (int e = launch_philox_fill(ws.eps, F, F, w->var_id, *r, stream)) return e;
+            eps = ws.eps;
+        }
+        if (int e = launch_sample_weights(w->mu, w->rho, eps, F, ws.W, F, F, S, stream)) return e;
+        BRN_CUDA_OK(cudaMemsetAsync(ws.R, 0, sizeof(double) * (size_t)S, stream));
+        if (!use_flash) BRN_CUDA_OK(cudaMemsetAsync(ws.dW, 0, sizeof(float) * (size_t)S * F, stream));
+    }
+    if (use_flash) {
+        StageTimer st("linreg.fused", stream);
+        if (int e = launch_linear_flash(X, px, y, N, F, S, ws.W, ws.dW, 0.f, nullptr, ws.flash, stream, ws.R)) return e;
+        const int64_t tot = (int64_t)S * F;
+        sum_slices_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(ws.flash.part, ws.flash.groups, tot, tot, ws.dW);
+        BRN_LAUNCH_OK("sum_slices_kernel");
+    } else if (N > 0) {
+        StageTimer st("linreg.fused", stream);
+        if (int e = launch_linear_fused(X, y, 2, N, F, 1, S, ws.W, ws.dW, 0.f, nullptr, stream, ws.R)) return e;
+    }
+    {
+        StageTimer st("linreg.finish", stream);
+        const int64_t tot = (int64_t)S * F;
+        brn_mf_var nv = nu ? *nu : brn_mf_var{};
+        linreg_finish_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(ws.dW, ws.R, F, N, nv, nu != nullptr, noise_scale, *r,
+                                                                              with_prior, loss);
+        BRN_LAUNCH_OK("linreg_finish_kernel");
+    }
+    StageTimer st3("linreg.reduce_finalize", stream);
+    return launch_mf_reduce_finalize(*w, eps, F, ws.dW, F, ws.stats, *r, with_prior, loss, stream);
 }

@@ -97,6 +97,8 @@ struct LinearFlashParams {
     double* loss; float loss_scale;
     int groups;
     int y_bulk;                   // y is 16-byte aligned: full blocks of it travel with the X block (bulk copy) into shared memory
+    const float* scal_y;          // Gaussian: max |y|  (device scalar)
+    double* R;                    // Gaussian: [S] += sum of squared residuals per vector (loss and loss_scale unused)
 };
 
 // tcgen05.mma kind::f16 with both shared-memory descriptors given as (low word, shared high word)
@@ -134,7 +136,9 @@ __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.
 // DTMEM: the d tile (A operand of the gradient MMA) lives in tensor memory (64 columns: hi pair words, lo pair words) instead of
 // shared memory -- the epilogue thread that owns TMEM lane s writes row s with tcgen05.st: no shared-memory round trip, no
 // generic -> async proxy fence, half the shared-memory operand reads of the gradient MMA.
-template <int KS1, int DTMEM>
+// LIK: 0 = Bernoulli (d = y - sigmoid(l), loss += loss_scale * sum ll), 1 = Gaussian residuals (d = r = y - l, R[s] += sum r^2;
+// the noise scale is applied afterwards, per vector, by the caller).
+template <int KS1, int DTMEM, int LIK = 0>
 __global__ void __launch_bounds__(LF_THREADS, 1)
 linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_constant__ CUtensorMap tmWl,
                     const __grid_constant__ CUtensorMap tmXh, const __grid_constant__ CUtensorMap tmXl, LinearFlashParams p) {
@@ -310,6 +314,9 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
             ++chain;
         };
         const int n_chains = (my_blocks + LF_D2_CHAIN - 1) / LF_D2_CHAIN;
+        // Gaussian: d = r * r_scale with r_scale = p2_scale(max|y| + F max|W| max|X|) >= 2^13 / max|r|: |d| < 2^14 fits fp16
+        float r_scale = 0.f;
+        if constexpr (LIK == 1) r_scale = p2_scale(*p.scal_y + (float)F * *p.scal_w * *p.scal_x);
         const uint64_t c2 = f2_pack(inv1 * 1.4426950408889634f, inv1 * 1.4426950408889634f);
         const uint64_t one2 = f2_pack(1.f, 1.f), ms2 = f2_pack(-LF_D_SCALE, -LF_D_SCALE), mone2 = f2_pack(-1.f, -1.f);
         int xs = grp % LF_XSTAGES;                     // X stage (and y slot) of this group's next block
@@ -340,75 +347,119 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
             if (lane == 0) umma::mbar_arrive(&d1_empty[b]);
             b += 2;
             if (b >= LF_D1BUF) { b -= LF_D1BUF; d1ph ^= 1; }
-            const float ys_lane = y_raw * LF_D_SCALE;
-            // Per element, with raw accumulator L (logit l = L * inv1), e = exp(-|l|), sig = sigmoid(l):
-            //   d * S = y S - S sig;   ll = y l - max(l, 0) - ln(1 + e)
-            // summed per block as inv1 * (sum(yS L) / S - sum(max(L, 0))) - ln 2 * log2(prod(1 + e))  -- ONE log per 16 elements
-            // (the product of 16 factors in (1, 2] cannot overflow), so 2 MUFU per element instead of 3.  Pairs of elements go
-            // through packed fp32x2 instructions.  Rows past the end of a ragged last block have X = 0 (L = 0), where
-            // d = y - 1/2 would be wrong: that block takes the predicated path.
             uint32_t dh_w[LF_EROWS / 2], dl_w[LF_EROWS / 2];
-            uint64_t acc_yl = f2_pack(0.f, 0.f), prod = one2;
-            float acc_mx = 0.f;
-            const uint64_t s2 = f2_pack(LF_D_SCALE, LF_D_SCALE);
-            auto body = [&](auto ragged, auto from_smem) {
+            float ll;                                  // Bernoulli: sum of the block's log-likelihoods; Gaussian: sum of r^2
+            if constexpr (LIK == 0) {
+                const float ys_lane = y_raw * LF_D_SCALE;
+                // Per element, with raw accumulator L (logit l = L * inv1), e = exp(-|l|), sig = sigmoid(l):
+                //   d * S = y S - S sig;   ll = y l - max(l, 0) - ln(1 + e)
+                // summed per block as inv1 * (sum(yS L) / S - sum(max(L, 0))) - ln 2 * log2(prod(1 + e))  -- ONE log per 16 elements
+                // (the product of 16 factors in (1, 2] cannot overflow), so 2 MUFU per element instead of 3.  Pairs of elements go
+                // through packed fp32x2 instructions.  Rows past the end of a ragged last block have X = 0 (L = 0), where
+                // d = y - 1/2 would be wrong: that block takes the predicated path.
+                uint64_t acc_yl = f2_pack(0.f, 0.f), prod = one2;
+                float acc_mx = 0.f;
+                const uint64_t s2 = f2_pack(LF_D_SCALE, LF_D_SCALE);
+                auto body = [&](auto ragged, auto from_smem) {
 #pragma unroll
-                for (int k = 0; k < LF_EROWS / 2; ++k) {
-                    uint64_t ys2;
-                    if (decltype(from_smem)::value) {
-                        const float2 yv = *reinterpret_cast<const float2*>(ysm + 2 * k);      // same address in every lane: broadcast
-                        ys2 = f2_mul(f2_pack(yv.x, yv.y), s2);
-                    } else {
-                        ys2 = f2_pack(__shfl_sync(0xffffffffu, ys_lane, 2 * k), __shfl_sync(0xffffffffu, ys_lane, 2 * k + 1));
+                    for (int k = 0; k < LF_EROWS / 2; ++k) {
+                        uint64_t ys2;
+                        if (decltype(from_smem)::value) {
+                            const float2 yv = *reinterpret_cast<const float2*>(ysm + 2 * k);      // same address in every lane: broadcast
+                            ys2 = f2_mul(f2_pack(yv.x, yv.y), s2);
+                        } else {
+                            ys2 = f2_pack(__shfl_sync(0xffffffffu, ys_lane, 2 * k), __shfl_sync(0xffffffffu, ys_lane, 2 * k + 1));
+                        }
+                        const uint64_t L2 = f2_pack(L[2 * k], L[2 * k + 1]);
+                        float a0, a1, e0, e1, i0, i1, r0f, r1f;
+                        f2_unpack(f2_mul(L2, c2), a0, a1);
+                        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e0) : "f"(-fabsf(a0)));
+                        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e1) : "f"(-fabsf(a1)));
+                        if (decltype(ragged)::value) {
+                            if (hp * LF_EROWS + 2 * k >= rows) e0 = 0.f;
+                            if (hp * LF_EROWS + 2 * k + 1 >= rows) e1 = 0.f;
+                        }
+                        const uint64_t e2 = f2_pack(e0, e1);
+                        const uint64_t ope2 = f2_add(e2, one2);
+                        float o0, o1;
+                        f2_unpack(ope2, o0, o1);
+                        asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(i0) : "f"(o0));
+                        asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(i1) : "f"(o1));
+                        f2_unpack(f2_mul(e2, f2_pack(i0, i1)), r0f, r1f);           // sigmoid(-|l|)
+                        const bool p0 = L[2 * k] >= 0.f, p1 = L[2 * k + 1] >= 0.f;
+                        const uint64_t sig2 = f2_pack(p0 ? i0 : r0f, p1 ? i1 : r1f);
+                        uint64_t ds2 = f2_fma(sig2, ms2, ys2);                      // S (y - sig)
+                        if (p0) acc_mx += L[2 * k];
+                        if (p1) acc_mx += L[2 * k + 1];
+                        acc_yl = f2_fma(ys2, L2, acc_yl);
+                        prod = f2_mul(prod, ope2);
+                        float d0, d1;
+                        f2_unpack(ds2, d0, d1);
+                        if (decltype(ragged)::value) {
+                            if (hp * LF_EROWS + 2 * k >= rows) d0 = 0.f;
+                            if (hp * LF_EROWS + 2 * k + 1 >= rows) d1 = 0.f;
+                            ds2 = f2_pack(d0, d1);
+                        }
+                        const __half2 h2 = __floats2half2_rn(d0, d1);
+                        const float2 hfv = __half22float2(h2);
+                        float l0, l1;
+                        f2_unpack(f2_fma(f2_pack(hfv.x, hfv.y), mone2, ds2), l0, l1);
+                        const __half2 l2 = __floats2half2_rn(l0, l1);
+                        dh_w[k] = *reinterpret_cast<const uint32_t*>(&h2);
+                        dl_w[k] = *reinterpret_cast<const uint32_t*>(&l2);
                     }
-                    const uint64_t L2 = f2_pack(L[2 * k], L[2 * k + 1]);
-                    float a0, a1, e0, e1, i0, i1, r0f, r1f;
-                    f2_unpack(f2_mul(L2, c2), a0, a1);
-                    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e0) : "f"(-fabsf(a0)));
-                    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e1) : "f"(-fabsf(a1)));
-                    if (decltype(ragged)::value) {
-                        if (hp * LF_EROWS + 2 * k >= rows) e0 = 0.f;
-                        if (hp * LF_EROWS + 2 * k + 1 >= rows) e1 = 0.f;
+                };
+                if (y_smem) body(std::false_type{}, std::true_type{});
+                else if (rows == LF_ROWS) body(std::false_type{}, std::false_type{});
+                else body(std::true_type{}, std::false_type{});
+                float ay0, ay1, pr0, pr1, lg0, lg1;
+                f2_unpack(acc_yl, ay0, ay1);
+                f2_unpack(prod, pr0, pr1);
+                asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg0) : "f"(pr0));
+                asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg1) : "f"(pr1));
+                ll = inv1 * ((ay0 + ay1) * (1.f / LF_D_SCALE) - acc_mx) - 0.6931471805599453f * (lg0 + lg1);
+            } else {
+                // r = y - L inv1 per element (no MUFU op); rows past the end of a ragged last block get r = 0
+                const uint64_t mi2 = f2_pack(-inv1, -inv1), rs2 = f2_pack(r_scale, r_scale);
+                uint64_t acc_rr = f2_pack(0.f, 0.f);
+                auto body = [&](auto ragged, auto from_smem) {
+#pragma unroll
+                    for (int k = 0; k < LF_EROWS / 2; ++k) {
+                        uint64_t y2;
+                        if (decltype(from_smem)::value) {
+                            const float2 yv = *reinterpret_cast<const float2*>(ysm + 2 * k);
+                            y2 = f2_pack(yv.x, yv.y);
+                        } else {
+                            y2 = f2_pack(__shfl_sync(0xffffffffu, y_raw, 2 * k), __shfl_sync(0xffffffffu, y_raw, 2 * k + 1));
+                        }
+                        uint64_t rr2 = f2_fma(f2_pack(L[2 * k], L[2 * k + 1]), mi2, y2);
+                        if (decltype(ragged)::value) {
+                            float q0, q1;
+                            f2_unpack(rr2, q0, q1);
+                            if (hp * LF_EROWS + 2 * k >= rows) q0 = 0.f;
+                            if (hp * LF_EROWS + 2 * k + 1 >= rows) q1 = 0.f;
+                            rr2 = f2_pack(q0, q1);
+                        }
+                        acc_rr = f2_fma(rr2, rr2, acc_rr);
+                        const uint64_t ds2 = f2_mul(rr2, rs2);
+                        float d0, d1;
+                        f2_unpack(ds2, d0, d1);
+                        const __half2 h2 = __floats2half2_rn(d0, d1);
+                        const float2 hfv = __half22float2(h2);
+                        float l0, l1;
+                        f2_unpack(f2_fma(f2_pack(hfv.x, hfv.y), f2_pack(-1.f, -1.f), ds2), l0, l1);
+                        const __half2 l2 = __floats2half2_rn(l0, l1);
+                        dh_w[k] = *reinterpret_cast<const uint32_t*>(&h2);
+                        dl_w[k] = *reinterpret_cast<const uint32_t*>(&l2);
                     }
-                    const uint64_t e2 = f2_pack(e0, e1);
-                    const uint64_t ope2 = f2_add(e2, one2);
-                    float o0, o1;
-                    f2_unpack(ope2, o0, o1);
-                    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(i0) : "f"(o0));
-                    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(i1) : "f"(o1));
-                    f2_unpack(f2_mul(e2, f2_pack(i0, i1)), r0f, r1f);           // sigmoid(-|l|)
-                    const bool p0 = L[2 * k] >= 0.f, p1 = L[2 * k + 1] >= 0.f;
-                    const uint64_t sig2 = f2_pack(p0 ? i0 : r0f, p1 ? i1 : r1f);
-                    uint64_t ds2 = f2_fma(sig2, ms2, ys2);                      // S (y - sig)
-                    if (p0) acc_mx += L[2 * k];
-                    if (p1) acc_mx += L[2 * k + 1];
-                    acc_yl = f2_fma(ys2, L2, acc_yl);
-                    prod = f2_mul(prod, ope2);
-                    float d0, d1;
-                    f2_unpack(ds2, d0, d1);
-                    if (decltype(ragged)::value) {
-                        if (hp * LF_EROWS + 2 * k >= rows) d0 = 0.f;
-                        if (hp * LF_EROWS + 2 * k + 1 >= rows) d1 = 0.f;
-                        ds2 = f2_pack(d0, d1);
-                    }
-                    const __half2 h2 = __floats2half2_rn(d0, d1);
-                    const float2 hfv = __half22float2(h2);
-                    float l0, l1;
-                    f2_unpack(f2_fma(f2_pack(hfv.x, hfv.y), mone2, ds2), l0, l1);
-                    const __half2 l2 = __floats2half2_rn(l0, l1);
-                    dh_w[k] = *reinterpret_cast<const uint32_t*>(&h2);
-                    dl_w[k] = *reinterpret_cast<const uint32_t*>(&l2);
-                }
-            };
-            if (y_smem) body(std::false_type{}, std::true_type{});
-            else if (rows == LF_ROWS) body(std::false_type{}, std::false_type{});
-            else body(std::true_type{}, std::false_type{});
-            float ay0, ay1, pr0, pr1, lg0, lg1;
-            f2_unpack(acc_yl, ay0, ay1);
-            f2_unpack(prod, pr0, pr1);
-            asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg0) : "f"(pr0));
-            asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg1) : "f"(pr1));
-            const float ll = inv1 * ((ay0 + ay1) * (1.f / LF_D_SCALE) - acc_mx) - 0.6931471805599453f * (lg0 + lg1);
+                };
+                if (y_smem) body(std::false_type{}, std::true_type{});
+                else if (rows == LF_ROWS) body(std::false_type{}, std::false_type{});
+                else body(std::true_type{}, std::false_type{});
+                float a0, a1;
+                f2_unpack(acc_rr, a0, a1);
+                ll = a0 + a1;
+            }
             // the d tile is free once the gradient MMA of the previous block (the other group's) has retired
             // (block i - 1: barrier of the other parity, its use (i - 1) / 2; the first block has nothing to wait for)
             if (i > 0) umma::mbar_wait_guarded(&d_empty[(i & 1) ^ 1], (uint32_t)(((i - 1) >> 1) & 1));
@@ -441,17 +492,22 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
         while ((int)chain < n_chains) drain();
         // this CTA's share of + d ll / d W for vector s_glob, features 32 part .. + 31
         if (s_ok) {
-            const float inv2 = 1.f / (LF_D_SCALE * p2_scale(*p.scal_x));
+            const float inv2 = 1.f / ((LIK == 1 ? r_scale : LF_D_SCALE) * p2_scale(*p.scal_x));
             float* o = p.part + (int64_t)g * p.part_stride + (int64_t)s_glob * F + part * LF_EFEAT;
 #pragma unroll
             for (int c = 0; c < LF_EFEAT; c += 4)
                 if (part * LF_EFEAT + c < F)
                     *reinterpret_cast<float4*>(o + c) = make_float4(r2[c] * inv2, r2[c + 1] * inv2, r2[c + 2] * inv2, r2[c + 3] * inv2);
         }
+        if constexpr (LIK == 1) {
+            // lane s owns vector s: the two epilogue groups and two row halves of this CTA and every row group add to R[s]
+            if (s_ok && ll_total != 0.0) atomicAdd(p.R + s_glob, ll_total);
+        } else {
         double tot = s_ok ? ll_total : 0.0;      // vectors past S are zero rows of the W tile: their terms are not part of the sum
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) tot += __shfl_xor_sync(0xffffffffu, tot, o);
         if (lane == 0 && tot != 0.0) atomicAdd(p.loss, tot * (double)p.loss_scale);
+        }
     }
     umma::tc_fence_before();
     __syncthreads();
@@ -560,8 +616,11 @@ static int launch_prepare_x(const float* X, int64_t N, int F, float* bound, __ha
 // dW [S][F] = + d ll / d W, loss += loss_scale * sum ll for S weight vectors W [S][F] over N rows (Bernoulli, C == 1).
 // px: a prepared X (the caller keeps it while X does not change: a training loop over fixed data then reads X once per
 // evaluation, as fp16 pairs, instead of three times), or NULL: X is split into the workspace on every call.
+// R != NULL selects the Gaussian epilogue: the per-slice partials of G_s = sum_b r_sb x_b, r_sb = y_b - w_s . x_b, go to b.part
+// and R[s] += sum_b r_sb^2 (loss is unused).
 static int launch_linear_flash(const float* X, const void* px, const float* y, int64_t N, int F, int S, const float* W, float* dW,
-                               float loss_scale, double* loss, const LinearFlashBuffers& b, cudaStream_t stream) {
+                               float loss_scale, double* loss, const LinearFlashBuffers& b, cudaStream_t stream,
+                               double* R = nullptr) {
     BRN_CUDA_OK(cudaMemsetAsync(b.scal, 0, 64 * sizeof(float), stream));
     lf_absmax_kernel<<<(unsigned)std::min<int64_t>(((int64_t)S * F / 4 + 255) / 256 + 1, 148), 256, 0, stream>>>(W, (int64_t)S * F, b.scal);
     BRN_LAUNCH_OK("lf_absmax_kernel");
@@ -575,6 +634,10 @@ static int launch_linear_flash(const float* X, const void* px, const float* y, i
     } else if (int e = launch_prepare_x(X, N, F, b.scal + 1, b.Xh, b.Xl, stream)) {
         return e;
     }
+    if (R) {
+        lf_absmax_kernel<<<(unsigned)std::min<int64_t>((N / 4 + 255) / 256 + 1, 148), 256, 0, stream>>>(y, N, b.scal + 2);
+        BRN_LAUNCH_OK("lf_absmax_kernel");
+    }
     CUtensorMap tWh, tWl, tXh, tXl;
     if (int e = make_tmap_2d_f16(&tWh, b.Wh, S, F, F, LF_MT, 64)) return e;
     if (int e = make_tmap_2d_f16(&tWl, b.Wl, S, F, F, LF_MT, 64)) return e;
@@ -583,6 +646,7 @@ static int launch_linear_flash(const float* X, const void* px, const float* y, i
     LinearFlashParams p;
     p.y = y; p.N = N; p.F = F; p.S = S; p.scal_w = b.scal; p.scal_x = scal_x; p.part = b.part; p.part_stride = (int64_t)S * F;
     p.loss = loss; p.loss_scale = loss_scale; p.groups = b.groups;
+    p.scal_y = b.scal + 2; p.R = R;
     p.y_bulk = (reinterpret_cast<uintptr_t>(y) & 15) == 0;
     if (const char* env = getenv("BRN_LINEAR_Y_BULK")) p.y_bulk = p.y_bulk && atoi(env) != 0;
     dim3 grid(b.tiles, b.groups);
@@ -593,7 +657,11 @@ static int launch_linear_flash(const float* X, const void* px, const float* y, i
         kern<<<grid, LF_THREADS, smem_bytes, stream>>>(tWh, tWl, tXh, tXl, p);
         return 0;
     };
-    if (F == 128) {
+    if (R) {      // the Gaussian epilogue exists with the d tile in tensor memory only
+        if (int e = F == 128 ? launch(linear_flash_kernel<8, 1, 1>, LinearFlashSmem<1>::TOTAL)
+                             : launch(linear_flash_kernel<0, 1, 1>, LinearFlashSmem<1>::TOTAL))
+            return e;
+    } else if (F == 128) {
         if (int e = dtmem ? launch(linear_flash_kernel<8, 1>, LinearFlashSmem<1>::TOTAL) : launch(linear_flash_kernel<8, 0>, LinearFlashSmem<0>::TOTAL)) return e;
     } else {
         if (int e = dtmem ? launch(linear_flash_kernel<0, 1>, LinearFlashSmem<1>::TOTAL) : launch(linear_flash_kernel<0, 0>, LinearFlashSmem<0>::TOTAL)) return e;

@@ -9,6 +9,7 @@ returns a 0-d tensor wired into autograd (so `loss.backward()` fills `.grad` of 
 
 Families
   LinearPlan  K2  observed Binomial(1)/Bernoulli/Categorical with logits = BF.matmul(W, x), W mean-field Normal
+  LinregPlan  K2g observed Normal(BF.matmul(W, x), sigma), W [1, F] mean-field Normal, sigma constant or a LogNormal latent
   BNNPlan     K3  observed Categorical with logits = BF.matmul(W2, BF.tanh(BF.matmul(W1, x) + b1)) + b2
 Unrecognised graphs raise `UnsupportedModelError` -- there is no eager / CPU fallback for the ELBO.
 """
@@ -93,12 +94,14 @@ def _var(e):
 class MeanFieldSpec:
     """One latent: q = Normal(root_loc, softplus(root_scale)) (learnable roots) and p = Normal prior of the
     same name, tied by root-name collision or declared."""
+    kind, kind_name = "normal", "Normal"
 
     def __init__(self, name, q_var, p_var, q_names):
         self.name = name
         lq = q_var.partial_links
-        if q_var.distribution.kind != "normal" or p_var.distribution.kind != "normal":
-            raise UnsupportedModelError("latent %r: only Normal q / Normal prior are lowered to the mean-field kernels" % name)
+        if q_var.distribution.kind != self.kind or p_var.distribution.kind != self.kind:
+            raise UnsupportedModelError("latent %r: only %s q / %s prior are lowered to the mean-field kernels"
+                                        % (name, self.kind_name, self.kind_name))
         self.loc_root = _as_root(lq["loc"].expr)
         self.scale_root = _softplus_root(lq["scale"].expr)
         if self.loc_root is None or self.scale_root is None:
@@ -151,6 +154,17 @@ class MeanFieldSpec:
         else:
             pl = ps = None
         return cu.MeanFieldVar(mu, rho, var_id=var_id, prior_loc=pl, prior_scale=ps, eps=eps, dmu=sinks[0], drho=sinks[1])
+
+
+class LogNormalSpec(MeanFieldSpec):
+    """A scalar latent with q = LogNormal(root_loc, softplus(root_scale)) and a LogNormal prior of the same name, tied or
+    declared: the noise scale of the linear-regression family (brn_mf_var read as a LogNormal, Philox var_id 1)."""
+    kind, kind_name = "lognormal", "LogNormal"
+
+    def __init__(self, name, q_var, p_var, q_names):
+        super().__init__(name, q_var, p_var, q_names)
+        if int(np.prod(self.shape)) != 1:
+            raise UnsupportedModelError("latent %r: the LogNormal noise scale must be a scalar (shape %s)" % (name, self.shape))
 
 
 class _FusedELBO(torch.autograd.Function):
@@ -270,6 +284,36 @@ class LinearPlan(Plan):
         return cu.linear_elbo_fwd_bwd(X, y, self.likelihood, mvars[0], self.C, r, loss=loss, prepared=self._prepared_x)
 
 
+class LinregPlan(Plan):
+    family = "linear regression (K2g)"
+
+    def __init__(self, joint, posterior, k, w_spec, x_var, nu_spec=None, scale=None):
+        """scale: (root, softplus) of a constant noise scale, or a number; None when nu_spec is given"""
+        super().__init__(joint, posterior)
+        self.k, self.x_var = k, x_var
+        self.latents = [w_spec] + ([nu_spec] if nu_spec is not None else [])
+        self._scale = scale
+        self._prepared_x = None
+
+    def noise_scale(self):
+        """the constant sigma as a 1-element device tensor, recomputed from its root at every evaluation (a constant root may be
+        re-assigned between evaluations; inside a captured graph this is one more captured kernel)"""
+        if isinstance(self._scale, float):
+            return torch.full((1,), self._scale, dtype=torch.float32, device=config.device)
+        root, sp = self._scale
+        v = root.value.detach().reshape(-1)[:1].to(device=config.device, dtype=torch.float32)
+        return (torch.nn.functional.softplus(v) if sp else v).contiguous()
+
+    def _launch(self, cu, mvars, r, empirical, loss=None):
+        X = _data_matrix(empirical[self.x_var], "x")
+        if self._prepared_x is None:
+            self._prepared_x = cu.PreparedX()
+        y = empirical[self.k].reshape(-1).to(torch.float32).contiguous()
+        nu = mvars[1] if len(mvars) > 1 else None
+        return cu.linreg_elbo_fwd_bwd(X, y, mvars[0], r, nu=nu, noise_scale=None if nu is not None else self.noise_scale(),
+                                      loss=loss, prepared=self._prepared_x)
+
+
 class BNNPlan(Plan):
     family = "bnn (K3)"
 
@@ -328,6 +372,8 @@ def _lower_dense(joint, posterior):
         raise UnsupportedModelError("fused families need exactly one observed likelihood node, found %d" % len(liks))
     k = liks[0]
     kind = k.distribution.kind
+    if kind == "normal":
+        return _lower_linreg(joint, posterior, k, latents, q_by_name, q_names)
     if "logits" not in k.partial_links:
         raise UnsupportedModelError("likelihood %r: only logits= parametrisations are lowered" % k.name)
     if kind == "binomial":
@@ -371,6 +417,52 @@ def _lower_dense(joint, posterior):
     raise UnsupportedModelError("model graph is not recognised by any fused kernel family "
                                 "(linear K2, bnn K3); likelihood link: %s" % k.partial_links["logits"].string)
 
+
+def _lower_linreg(joint, posterior, k, latents, q_by_name, q_names):
+    """K2g: observed Normal(loc = matmul(W, x), scale) with W the [1, F] mean-field Normal weights and x data; scale a
+    non-learnable constant (a root, behind softplus when auto-named, or a number) or a scalar LogNormal latent."""
+    loc, scale = k.partial_links["loc"].expr, k.partial_links["scale"].expr
+    if not _is_call(loc, "matmul", 2):
+        for a, b in _commutative_add(loc):
+            if _is_call(a, "matmul", 2):
+                raise UnsupportedModelError("linear regression %r: a bias added to BF.matmul(weights, x) is not lowered -- "
+                                            "append a column of ones to x instead" % k.name)
+        raise UnsupportedModelError("likelihood %r: a Normal likelihood is lowered for loc = BF.matmul(weights, x) only" % k.name)
+    W, x = _var(loc.args[0]), _var(loc.args[1])
+    if W not in latents or not _is_data(x):
+        raise UnsupportedModelError("linear regression %r: loc must be BF.matmul(weights, x) with weights a latent and x data" % k.name)
+    ws = MeanFieldSpec(W.name, q_by_name[W.name], W, q_names)
+    if len(ws.shape) != 2 or ws.shape[0] != 1:
+        raise UnsupportedModelError("linear regression %r: weights must have shape [1, F] (multi-output regression is not "
+                                    "lowered), got %s" % (k.name, ws.shape))
+    nu_spec, const = None, None
+    nu = _var(scale)
+    if nu is not None and nu in latents:
+        if nu.distribution.kind != "lognormal":
+            raise UnsupportedModelError("linear regression %r: a %s-distributed noise scale is not lowered (a LogNormal "
+                                        "latent or a constant is)" % (k.name, nu.distribution.kind))
+        nu_spec = LogNormalSpec(nu.name, q_by_name[nu.name], nu, q_names)
+    else:
+        root, sp = _softplus_root(scale), True
+        if root is None:
+            root, sp = _as_root(scale), False
+        if root is not None and not root.is_observed:
+            if getattr(root, "learnable", False):
+                raise UnsupportedModelError("linear regression %r: a learnable point-estimate noise scale (root %r) is not "
+                                            "lowered" % (k.name, root.name))
+            if root._value.numel() != 1:
+                raise UnsupportedModelError("linear regression %r: the noise scale must be a scalar" % k.name)
+            const = (root, sp)
+        elif _const_value(scale) is not None:
+            const = _const_value(scale)
+        else:
+            raise UnsupportedModelError("linear regression %r: the noise scale must be a constant or a scalar LogNormal latent "
+                                        "(deterministic or data-dependent scales are not lowered)" % k.name)
+    extra = [v.name for v in latents if v is not W and v is not nu]
+    if extra:
+        raise UnsupportedModelError("linear regression %r: latent variables other than the weights and the noise scale are not "
+                                    "lowered: %s" % (k.name, sorted(extra)))
+    return LinregPlan(joint, posterior, k, ws, x, nu_spec=nu_spec, scale=const)
 
 
 # ---------------------------------------------------------------------------------------------------

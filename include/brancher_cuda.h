@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define BRN_ABI_VERSION 2
+#define BRN_ABI_VERSION 3
 
 /* One mean-field Normal variational variable  q(w) = N(mu, softplus(rho))  together with the Normal
  * prior p(w) = N(prior_loc, prior_scale) of the same name.
@@ -151,6 +151,29 @@ int brn_linear_elbo_fwd_bwd_px(const float* X, const void* px, const void* y, in
                                const brn_mf_var* w, const brn_sample_range* r,
                                void* workspace, size_t workspace_bytes, int with_prior,
                                double* loss, void* stream);
+
+/* K2g -- Bayesian linear regression: y_b ~ Normal(sum_f w_sf X_bf, sigma_s) over N observed rows (summed, variables.py:513-514),
+ * w ~ q mean-field [1, F] (`w`, Philox var_id 0 by convention).  Per sample, with r_sb = y_b - w_s . x_b and R_s = sum_b r_sb^2:
+ *   ll_s = -R_s / (2 sigma_s^2) - N log sigma_s - N/2 log(2 pi) ;  loss += -(1/S_total) sum_{s local} ll_s
+ * plus the prior / entropy terms of both latents (with_prior != 0; 0 drops them, for row-sharded callers).  Same accumulation
+ * contract as K2.  Exactly one noise form is given:
+ *   noise_scale != NULL: sigma_s = *noise_scale, a DEVICE fp32 scalar read on every call (a replayed CUDA graph sees a
+ *                        re-assigned constant); nu must be NULL.
+ *   nu != NULL:          sigma_s = nu_s, a scalar LogNormal latent (numel 1, Philox var_id 1 by convention):
+ *                        q(nu) = LogNormal(mu, softplus(rho)), nu_s = exp(mu + softplus(rho) eps_s); the prior is
+ *                        LogNormal(prior_loc, prior_scale), or q's own roots when tied.  log p(nu) = log N(log nu; a, b) - log nu
+ *                        and H[q(nu)] = H[N(mu, softplus(rho))] + mu, as torch's LogNormal (TransformedDistribution) gives them.
+ * y fp32 [N]; X fp32 [N, F], F <= 128; px: the prepared X of brn_linear_prepare_x, or NULL (used only when the call takes the
+ * one-pass tensor-core kernel, as for brn_linear_elbo_fwd_bwd_px).  workspace: brn_linreg_workspace_bytes() bytes of scratch.
+ * Replaces the graph walk of estimate_log_model_evidence (variables.py:843-870) for
+ * NormalVariable(BF.matmul(weights, x), nu_or_constant, "y") -- examples/multivariate_regression.py with the regressors in a
+ * matrix: _get_sample, _apply_link's batched matmul (variables.py:436-449), Normal / LogNormal log_prob and entropy
+ * (distributions.py:111-124,170-181,493-507) and loss.backward() (inference.py:100). */
+size_t brn_linreg_workspace_bytes(int64_t N, int F, int s_local);
+int brn_linreg_elbo_fwd_bwd(const float* X, const void* px, const float* y, int64_t N, int F,
+                            const brn_mf_var* w, const brn_mf_var* nu, const float* noise_scale,
+                            const brn_sample_range* r, void* workspace, size_t workspace_bytes, int with_prior,
+                            double* loss, void* stream);
 
 /* K1 -- generic scalar-DAG ELBO: fused reparameterised sampling + log-probs + reduction over samples and data rows +
  * backward, for models whose variables are scalars (README.md:22-75 AR(1); examples/logNormal_normal.py;
