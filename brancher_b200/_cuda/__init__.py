@@ -12,7 +12,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libbrancher_cuda.so")
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 _lib = None
 
@@ -121,6 +121,10 @@ SYMBOLS = {
                                                ctypes.POINTER(MFVar), ctypes.POINTER(MFVar), ctypes.c_void_p,
                                                ctypes.POINTER(SampleRange), ctypes.c_void_p, ctypes.c_size_t, ctypes.c_int,
                                                ctypes.c_void_p, ctypes.c_void_p]),
+    "brn_linreg_elbo_fwd_bwd_lik": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int64,
+                                                   ctypes.c_int, ctypes.POINTER(MFVar), ctypes.POINTER(MFVar), ctypes.c_void_p,
+                                                   ctypes.POINTER(SampleRange), ctypes.c_void_p, ctypes.c_size_t, ctypes.c_int,
+                                                   ctypes.c_void_p, ctypes.c_void_p]),
     "brn_svgd_sharded_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int, ctypes.c_int]),
     "brn_svgd_sharded_offsets": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.c_int] + [ctypes.POINTER(ctypes.c_size_t)] * 4),
     "brn_svgd_sharded_phase": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p] + [ctypes.c_int] * 5 +
@@ -364,6 +368,7 @@ def bnn_predict(X, vars4, r, labels=True, probs=True, activation="tanh"):
 
 
 BERNOULLI, CATEGORICAL, GAUSSIAN = 0, 1, 2
+CAUCHY, LAPLACE = 3, 4          # regression likelihoods of linreg_elbo_fwd_bwd (with GAUSSIAN: include/brancher_cuda.h, BRN_LINREG_*)
 
 
 class PreparedX:
@@ -377,7 +382,7 @@ class PreparedX:
     def get(self, X, likelihood, C):
         """pointer-carrying uint8 tensor for `px`, or None when this call has no prepared form"""
         N, F = X.shape
-        nbytes = lib().brn_linear_prepared_x_bytes(N, F) if (likelihood in (BERNOULLI, GAUSSIAN) and C == 1) else 0
+        nbytes = lib().brn_linear_prepared_x_bytes(N, F) if (likelihood in (BERNOULLI, GAUSSIAN, CAUCHY, LAPLACE) and C == 1) else 0
         if nbytes == 0 or X.data_ptr() % 16:
             return None
         same = (self.src is not None and self.src.data_ptr() == X.data_ptr() and self.src.shape == X.shape
@@ -413,8 +418,9 @@ def linear_elbo_fwd_bwd(X, y, likelihood, w, C, r, with_prior=True, loss=None, p
     return loss
 
 
-def linreg_elbo_fwd_bwd(X, y, w, r, nu=None, noise_scale=None, with_prior=True, loss=None, prepared=None):
-    """K2g, Bayesian linear regression y ~ Normal(X w, sigma).  X [N,F] fp32; y [N] fp32; w MeanFieldVar [1,F] (var_id 0).
+def linreg_elbo_fwd_bwd(X, y, w, r, nu=None, noise_scale=None, with_prior=True, loss=None, prepared=None, likelihood=GAUSSIAN):
+    """K2g, Bayesian linear regression y ~ Normal(X w, sigma), or the robust Cauchy(X w, sigma) / Laplace(X w, sigma) with
+    likelihood=CAUCHY / LAPLACE.  X [N,F] fp32; y [N] fp32; w MeanFieldVar [1,F] (var_id 0).
     Exactly one noise form: nu, a MeanFieldVar of one element read as q = LogNormal(mu, softplus(rho)) with a LogNormal prior
     (var_id 1), or noise_scale, a 1-element fp32 CUDA tensor holding sigma (read on the device at every call).
     prepared: a PreparedX kept by the caller across evaluations of the same data matrix (optional)."""
@@ -422,6 +428,8 @@ def linreg_elbo_fwd_bwd(X, y, w, r, nu=None, noise_scale=None, with_prior=True, 
     N, F = X.shape
     if (nu is None) == (noise_scale is None):
         raise BrancherCudaError("linreg_elbo_fwd_bwd: give exactly one of nu and noise_scale")
+    if likelihood not in (GAUSSIAN, CAUCHY, LAPLACE):
+        raise BrancherCudaError("linreg_elbo_fwd_bwd: unknown likelihood %r (GAUSSIAN, CAUCHY or LAPLACE)" % (likelihood,))
     if w.numel != F:
         raise BrancherCudaError("linreg_elbo_fwd_bwd: weights have %d elements, expected F = %d" % (w.numel, F))
     if y.numel() != N:
@@ -435,11 +443,11 @@ def linreg_elbo_fwd_bwd(X, y, w, r, nu=None, noise_scale=None, with_prior=True, 
     ws = _workspace(dev, lib().brn_linreg_workspace_bytes(N, F, r.s_local))
     st = w.struct()
     nst = nu.struct() if nu is not None else None
-    px = prepared.get(X, GAUSSIAN, 1) if (prepared is not None and N > 0) else None
-    _check(lib().brn_linreg_elbo_fwd_bwd(_ptr(X, what="X"), px.data_ptr() if px is not None else None, _ptr(y, what="y"), N, F,
-                                         ctypes.byref(st), ctypes.byref(nst) if nst is not None else None,
-                                         _ptr(noise_scale, what="noise_scale"), ctypes.byref(r), ws.data_ptr(), ws.numel(),
-                                         int(with_prior), _ptr(loss, torch.float64), _stream(dev)), "brn_linreg_elbo_fwd_bwd")
+    px = prepared.get(X, likelihood, 1) if (prepared is not None and N > 0) else None
+    _check(lib().brn_linreg_elbo_fwd_bwd_lik(_ptr(X, what="X"), px.data_ptr() if px is not None else None, _ptr(y, what="y"),
+                                             likelihood, N, F, ctypes.byref(st), ctypes.byref(nst) if nst is not None else None,
+                                             _ptr(noise_scale, what="noise_scale"), ctypes.byref(r), ws.data_ptr(), ws.numel(),
+                                             int(with_prior), _ptr(loss, torch.float64), _stream(dev)), "brn_linreg_elbo_fwd_bwd")
     return loss
 
 

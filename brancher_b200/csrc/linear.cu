@@ -24,10 +24,14 @@ struct LinearArgs {
     int tiles_per_group; int64_t n_row_tiles;
     float inv_S; double* loss;
     double* ll_cols;                 // optional [S]: per-sample log-likelihood sums (K6), += ; loss may then be NULL
+    const float* sigma;              // LIK == 3: [S] noise scale per sample
+    double* ll_cols2;                // LIK == 3: [S] += sum z^2 / (1 + z^2)
 };
 
 // 0: Bernoulli/Binomial(1) with float y, 1: Categorical with int32 labels, 2: Gaussian residuals with float y (C == 1): d = r =
-// y - l and ll_cols[s] += sum r^2 (loss unused; the noise scale is applied per sample afterwards, linreg_finish_kernel)
+// y - l and ll_cols[s] += sum r^2 (loss unused; the noise scale is applied per sample afterwards, linreg_finish_kernel),
+// 3: Cauchy residuals (C == 1): z = r / sigma_s, d = z / (1 + z^2), ll_cols[s] += sum log1p(z^2), ll_cols2[s] += sum z^2/(1 + z^2),
+// 4: Laplace residuals (C == 1): d = sign(r), ll_cols[s] += sum |r|  (3, 4: loss unused, finished by linreg_finish_kernel)
 template <int LIK>
 __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
     extern __shared__ __align__(16) float sm[];
@@ -62,8 +66,17 @@ __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
     double llc[8];                   // LIK == 0 / 2 with ll_cols: this thread's 8 columns, summed over its rows and tiles
 #pragma unroll
     for (int j = 0; j < 8; ++j) llc[j] = 0.0;
-    __shared__ double llcol_s[LN_T];  // LIK == 1 with ll_cols: per sample of the tile
+    __shared__ double llcol_s[LN_T];  // LIK == 1 with ll_cols: per sample of the tile; LIK == 3: sum z^2 / (1 + z^2) per column
     if (a.ll_cols && t < LN_T) llcol_s[t] = 0.0;
+    float isg[8];                    // LIK == 3: 1 / sigma of this thread's 8 columns
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        isg[j] = 1.f;
+        if (LIK == 3) {
+            const int col = (j < 4 ? tx * 4 + j : 64 + tx * 4 + (j - 4));
+            if (col < ncols && j0 + col < J) isg[j] = 1.f / a.sigma[j0 + col];
+        }
+    }
 
     const int64_t tile_begin = (int64_t)blockIdx.y * a.tiles_per_group;
     const int64_t tile_end = min(a.n_row_tiles, tile_begin + a.tiles_per_group);
@@ -137,6 +150,32 @@ __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
                     bool ok = rv && col < ncols && (j0 + col) < J;
                     d[j] = ok ? yv - acc[i][j] : 0.f;
                     if (a.ll_cols) llc[j] += (double)(d[j] * d[j]);
+                }
+                *reinterpret_cast<float4*>(&Ls[row][tx * 4]) = make_float4(d[0], d[1], d[2], d[3]);
+                *reinterpret_cast<float4*>(&Ls[row][64 + tx * 4]) = make_float4(d[4], d[5], d[6], d[7]);
+            }
+            __syncthreads();
+        } else if (LIK == 3 || LIK == 4) {
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+                int row = (i < 4 ? ty * 4 + i : 64 + ty * 4 + (i - 4));
+                bool rv = r0 + row < a.N;
+                float yv = ys[row];
+                float d[8];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    int col = (j < 4 ? tx * 4 + j : 64 + tx * 4 + (j - 4));
+                    bool ok = rv && col < ncols && (j0 + col) < J;
+                    const float r = ok ? yv - acc[i][j] : 0.f;
+                    if (LIK == 3) {
+                        const float z = r * isg[j], z2 = z * z, iq = 1.f / (1.f + z2);
+                        d[j] = z * iq;
+                        llc[j] += (double)log1pf(z2);
+                        if (z2 != 0.f) atomicAdd(&llcol_s[col], (double)(z2 * iq));      // sixteen threads share a column
+                    } else {
+                        d[j] = r > 0.f ? 1.f : (r < 0.f ? -1.f : 0.f);      // sign(0) = 0, as torch's abs gradient
+                        llc[j] += (double)fabsf(r);
+                    }
                 }
                 *reinterpret_cast<float4*>(&Ls[row][tx * 4]) = make_float4(d[0], d[1], d[2], d[3]);
                 *reinterpret_cast<float4*>(&Ls[row][64 + tx * 4]) = make_float4(d[4], d[5], d[6], d[7]);
@@ -229,6 +268,10 @@ __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
             for (int j = 0; j < 8; ++j) {
                 const int col = (j < 4 ? tx * 4 + j : 64 + tx * 4 + (j - 4));
                 if (col < ncols && j0 + col < J && llc[j] != 0.0) atomicAdd(&a.ll_cols[j0 + col], llc[j]);
+            }
+            if (LIK == 3) {
+                __syncthreads();
+                if (t < ncols && j0 + t < J && llcol_s[t] != 0.0) atomicAdd(&a.ll_cols2[j0 + t], llcol_s[t]);
             }
         } else {
             __syncthreads();
@@ -371,10 +414,11 @@ static bool linear_use_tc(int likelihood, int64_t N, int F, int C, int S) {
 using namespace brn;
 
 static int launch_linear_fused(const float* X, const void* y, int likelihood, int64_t N, int F, int C, int S, const float* W,
-                               float* dW, float inv_S, double* loss, cudaStream_t stream, double* ll_cols = nullptr) {
+                               float* dW, float inv_S, double* loss, cudaStream_t stream, double* ll_cols = nullptr,
+                               const float* sigma = nullptr, double* ll_cols2 = nullptr) {
     LinearArgs a;
     a.X = X; a.y = y; a.N = N; a.F = F; a.C = C; a.S = S; a.W = W; a.dW = dW;
-    a.inv_S = inv_S; a.loss = loss; a.ll_cols = ll_cols;
+    a.inv_S = inv_S; a.loss = loss; a.ll_cols = ll_cols; a.sigma = sigma; a.ll_cols2 = ll_cols2;
     const int spc = LN_T / C;
     const int col_tiles = (S + spc - 1) / spc;
     a.n_row_tiles = (N + LN_T - 1) / LN_T;
@@ -394,6 +438,12 @@ static int launch_linear_fused(const float* X, const void* y, int likelihood, in
     } else if (likelihood == 2) {
         BRN_CUDA_OK(cudaFuncSetAttribute(linear_fused_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         linear_fused_kernel<2><<<grid, 256, smem, stream>>>(a);
+    } else if (likelihood == 3) {
+        BRN_CUDA_OK(cudaFuncSetAttribute(linear_fused_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        linear_fused_kernel<3><<<grid, 256, smem, stream>>>(a);
+    } else if (likelihood == 4) {
+        BRN_CUDA_OK(cudaFuncSetAttribute(linear_fused_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        linear_fused_kernel<4><<<grid, 256, smem, stream>>>(a);
     } else {
         BRN_CUDA_OK(cudaFuncSetAttribute(linear_fused_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         linear_fused_kernel<1><<<grid, 256, smem, stream>>>(a);
@@ -653,15 +703,19 @@ extern "C" int brn_linear_elbo_fwd_bwd_px(const float* X, const void* px, const 
 }
 
 // ---------------------------------------------------------------------------------------------
-// Bayesian linear regression: y_b ~ Normal(w_s . x_b, sigma_s) (see include/brancher_cuda.h, brn_linreg_elbo_fwd_bwd).
-// The kernels that read X never see sigma: they produce G_s = sum_b r_sb x_b and R_s = sum_b r_sb^2 per sample, and
-// linreg_finish_kernel applies the noise scale, so both noise modes share one pass over X and sigma_s costs nothing there.
+// Bayesian linear regression: y_b ~ Normal / Cauchy / Laplace(w_s . x_b, sigma_s) (see include/brancher_cuda.h,
+// brn_linreg_elbo_fwd_bwd_lik).  Normal and Laplace are separable in sigma: the kernels that read X never see it, they produce
+// G_s = sum_b r_sb x_b and R_s = sum_b r_sb^2 (Laplace: sum_b sign(r_sb) x_b and sum_b |r_sb|) per sample, and
+// linreg_finish_kernel applies the noise scale.  Cauchy is not (d ll / d r = 2 r / (sigma^2 + r^2)): its kernels read sigma_s
+// from the array linreg_sigma_kernel writes, which the finisher reads too, so the two stages cannot disagree on it.
 // ---------------------------------------------------------------------------------------------
 namespace brn {
 
 struct LinregWorkspace {
     float *eps, *W, *dW, *stats;
-    double* R;                 // [S] sums of squared residuals
+    double* R;                 // [S] sums of squared residuals (Cauchy: of log1p(z^2); Laplace: of |r|)
+    float* sigma;              // [S] noise scale per sample
+    double* T;                 // [S] Cauchy: sums of z^2 / (1 + z^2)
     LinearFlashBuffers flash;
     size_t bytes;
     LinregWorkspace(void* base, int S, int64_t N, int F, bool flash_path, int sms) {
@@ -671,6 +725,8 @@ struct LinregWorkspace {
         dW = take((size_t)S * F);
         stats = take(4 * (size_t)((F + 3) / 4 * 4));
         R = reinterpret_cast<double*>(take(2 * (size_t)S));
+        sigma = take((size_t)S);
+        T = reinterpret_cast<double*>(take(2 * (size_t)S));
         flash = LinearFlashBuffers();
         if (flash_path) {
             flash.carve(take, S, F, sms);
@@ -686,17 +742,33 @@ static bool linreg_use_flash(const float* X, int64_t N, int F, int S) {
     return linear_use_tc(0, N, F, 1, S) && linear_flash_ok(X, N, F, S);
 }
 
-// One thread per element (s, f) of the per-sample gradient rows: dW_s *= 1 / sigma_s^2 in place.  The thread of f == 0 also owns
-// sample s's scalar terms, all scaled by 1 / S_total (the partial contract of brn_mf_normal_prior_entropy, so sharded samples
-// sum to the unsharded result):
-//   ll_s = -R_s / (2 sigma_s^2) - N log sigma_s - N log sqrt(2 pi)
-// and, for the LogNormal latent (u_s = m + softplus(rho) e_s, sigma_s = exp(u_s)), d ll_s / d u_s = R_s / sigma_s^2 - N chained to
+// sigma [s] = the noise scale of sample s: the constant *noise_scale, or nu_s = exp(m + softplus(rho) e_s) of the LogNormal latent
+__global__ void __launch_bounds__(256)
+linreg_sigma_kernel(float* __restrict__ sigma, brn_mf_var nu, int has_nu, const float* __restrict__ noise_scale, brn_sample_range r) {
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= r.s_local) return;
+    if (has_nu) {
+        const float e = nu.eps ? nu.eps[s] : philox_normal1(r.seed, philox_offset(r), nu.var_id, (uint32_t)(r.s0 + s), 0);
+        sigma[s] = expf(__fmaf_rn(e, softplusf(nu.rho[0]), nu.mu[0]));
+    } else {
+        sigma[s] = *noise_scale;
+    }
+}
+
+// One thread per element (s, f) of the per-sample gradient rows: dW_s *= 1 / sigma_s^2 in place (Cauchy: 2 / sigma_s, Laplace:
+// 1 / sigma_s).  The thread of f == 0 also owns sample s's scalar terms, all scaled by 1 / S_total (the partial contract of
+// brn_mf_normal_prior_entropy, so sharded samples sum to the unsharded result), with u_s = log sigma_s:
+//   Normal   ll_s = -R_s / (2 sigma_s^2) - N u_s - N log sqrt(2 pi)   d ll_s / d u_s = R_s / sigma_s^2 - N
+//   Cauchy   ll_s = -N (log pi + u_s) - R_s                            d ll_s / d u_s = 2 T_s - N
+//   Laplace  ll_s = -N (log 2 + u_s) - R_s / sigma_s                   d ll_s / d u_s = R_s / sigma_s - N
+// and, for the LogNormal latent (u_s = m + softplus(rho) e_s, sigma_s = exp(u_s)), d ll_s / d u_s chained to
 // (m, rho), with log p(nu_s) = NORMAL_LP(log nu_s; a, b) - log nu_s and H[q(nu)] = H_Normal(softplus(rho)) + m composed as the
 // scalar-DAG family composes them (tied: a = m, b = softplus(rho), differentiated through both the sample and the prior, where
-// the terms cancel in closed form as in the mean-field finalisation).
+// the terms cancel in closed form as in the mean-field finalisation).  lik: BRN_LINREG_NORMAL / _CAUCHY / _LAPLACE.
 __global__ void __launch_bounds__(256)
-linreg_finish_kernel(float* __restrict__ dW, const double* __restrict__ R, int F, int64_t N, brn_mf_var nu, int has_nu,
-                     const float* __restrict__ noise_scale, brn_sample_range r, int with_prior, double* __restrict__ loss) {
+linreg_finish_kernel(float* __restrict__ dW, const double* __restrict__ R, const double* __restrict__ T,
+                     const float* __restrict__ sig, int lik, int F, int64_t N, brn_mf_var nu, int has_nu, brn_sample_range r,
+                     int with_prior, double* __restrict__ loss) {
     __shared__ double red[32];
     __shared__ float red_m[32], red_s[32];
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -705,21 +777,31 @@ linreg_finish_kernel(float* __restrict__ dW, const double* __restrict__ R, int F
     float gm = 0.f, gs = 0.f;            // d ELBO_s / d m, d ELBO_s / d softplus(rho) of the noise latent
     if (i < total) {
         const int s = (int)(i / F);
-        float sigma, e = 0.f, m = 0.f, sg = 1.f;
+        const float sigma = sig[s];
+        float e = 0.f, m = 0.f, sg = 1.f;
         if (has_nu) {
             e = nu.eps ? nu.eps[s] : philox_normal1(r.seed, philox_offset(r), nu.var_id, (uint32_t)(r.s0 + s), 0);
             m = nu.mu[0];
             sg = softplusf(nu.rho[0]);
-            sigma = expf(__fmaf_rn(e, sg, m));
-        } else {
-            sigma = *noise_scale;
         }
-        dW[i] *= 1.0f / (sigma * sigma);
+        dW[i] *= lik == BRN_LINREG_CAUCHY ? 2.0f / sigma : lik == BRN_LINREG_LAPLACE ? 1.0f / sigma : 1.0f / (sigma * sigma);
         if (i % F == 0) {
-            const double sd = sigma, inv_s2 = 1.0 / (sd * sd), Rs = R[s];
-            elbo = -0.5 * Rs * inv_s2 - (double)N * (log(sd) + (double)BRN_HALF_LOG_2PI);
+            const double sd = sigma, Rs = R[s];
+            double gu_ll;                      // d ll_s / d u_s
+            if (lik == BRN_LINREG_CAUCHY) {
+                elbo = -(double)N * (log(sd) + 1.1447298858494002) - Rs;                   // log pi
+                gu_ll = 2.0 * T[s] - (double)N;
+            } else if (lik == BRN_LINREG_LAPLACE) {
+                const double a = Rs / sd;
+                elbo = -(double)N * (log(sd) + 0.6931471805599453) - a;                   // log 2
+                gu_ll = a - (double)N;
+            } else {
+                const double inv_s2 = 1.0 / (sd * sd);
+                elbo = -0.5 * Rs * inv_s2 - (double)N * (log(sd) + (double)BRN_HALF_LOG_2PI);
+                gu_ll = Rs * inv_s2 - (double)N;
+            }
             if (has_nu) {
-                const float gu = (float)(Rs * inv_s2 - (double)N);
+                const float gu = (float)gu_ll;
                 gm = gu;
                 gs = gu * e;
                 if (with_prior) {
@@ -768,7 +850,18 @@ extern "C" size_t brn_linreg_workspace_bytes(int64_t N, int F, int s_local) {
 extern "C" int brn_linreg_elbo_fwd_bwd(const float* X, const void* px, const float* y, int64_t N, int F, const brn_mf_var* w,
                                        const brn_mf_var* nu, const float* noise_scale, const brn_sample_range* r,
                                        void* workspace, size_t workspace_bytes, int with_prior, double* loss, void* stream_) {
+    return brn_linreg_elbo_fwd_bwd_lik(X, px, y, BRN_LINREG_NORMAL, N, F, w, nu, noise_scale, r, workspace, workspace_bytes,
+                                       with_prior, loss, stream_);
+}
+
+extern "C" int brn_linreg_elbo_fwd_bwd_lik(const float* X, const void* px, const float* y, int likelihood, int64_t N, int F,
+                                           const brn_mf_var* w, const brn_mf_var* nu, const float* noise_scale,
+                                           const brn_sample_range* r, void* workspace, size_t workspace_bytes, int with_prior,
+                                           double* loss, void* stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
+    BRN_CHECK_ARG(likelihood == BRN_LINREG_NORMAL || likelihood == BRN_LINREG_CAUCHY || likelihood == BRN_LINREG_LAPLACE,
+                  "brn_linreg_elbo_fwd_bwd: unknown likelihood %d (Normal %d, Cauchy %d, Laplace %d)", likelihood, BRN_LINREG_NORMAL,
+                  BRN_LINREG_CAUCHY, BRN_LINREG_LAPLACE);
     BRN_CHECK_ARG(w && r && loss, "brn_linreg_elbo_fwd_bwd: NULL pointer");
     BRN_CHECK_ARG(N >= 0 && F > 0, "brn_linreg_elbo_fwd_bwd: bad shape N=%lld F=%d", (long long)N, F);
     BRN_CHECK_ARG(N == 0 || (X && y), "brn_linreg_elbo_fwd_bwd: NULL data pointer");
@@ -806,24 +899,31 @@ extern "C" int brn_linreg_elbo_fwd_bwd(const float* X, const void* px, const flo
         }
         if (int e = launch_sample_weights(w->mu, w->rho, eps, F, ws.W, F, F, S, stream)) return e;
         BRN_CUDA_OK(cudaMemsetAsync(ws.R, 0, sizeof(double) * (size_t)S, stream));
+        if (likelihood == BRN_LINREG_CAUCHY) BRN_CUDA_OK(cudaMemsetAsync(ws.T, 0, sizeof(double) * (size_t)S, stream));
         if (!use_flash) BRN_CUDA_OK(cudaMemsetAsync(ws.dW, 0, sizeof(float) * (size_t)S * F, stream));
+        linreg_sigma_kernel<<<(unsigned)((S + 255) / 256), 256, 0, stream>>>(ws.sigma, nu ? *nu : brn_mf_var{}, nu != nullptr, noise_scale,
+                                                                            *r);
+        BRN_LAUNCH_OK("linreg_sigma_kernel");
     }
+    // likelihood codes of the one-pass kernel's LIK (1 Gaussian, 2 Cauchy, 3 Laplace) and of linear_fused_kernel (2, 3, 4)
+    const int lik_flash = likelihood - BRN_LINREG_NORMAL + 1, lik_simt = likelihood - BRN_LINREG_NORMAL + 2;
     if (use_flash) {
         StageTimer st("linreg.fused", stream);
-        if (int e = launch_linear_flash(X, px, y, N, F, S, ws.W, ws.dW, 0.f, nullptr, ws.flash, stream, ws.R)) return e;
+        if (int e = launch_linear_flash(X, px, y, N, F, S, ws.W, ws.dW, 0.f, nullptr, ws.flash, stream, ws.R, lik_flash, ws.sigma, ws.T))
+            return e;
         const int64_t tot = (int64_t)S * F;
         sum_slices_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(ws.flash.part, ws.flash.groups, tot, tot, ws.dW);
         BRN_LAUNCH_OK("sum_slices_kernel");
     } else if (N > 0) {
         StageTimer st("linreg.fused", stream);
-        if (int e = launch_linear_fused(X, y, 2, N, F, 1, S, ws.W, ws.dW, 0.f, nullptr, stream, ws.R)) return e;
+        if (int e = launch_linear_fused(X, y, lik_simt, N, F, 1, S, ws.W, ws.dW, 0.f, nullptr, stream, ws.R, ws.sigma, ws.T)) return e;
     }
     {
         StageTimer st("linreg.finish", stream);
         const int64_t tot = (int64_t)S * F;
         brn_mf_var nv = nu ? *nu : brn_mf_var{};
-        linreg_finish_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(ws.dW, ws.R, F, N, nv, nu != nullptr, noise_scale, *r,
-                                                                              with_prior, loss);
+        linreg_finish_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(ws.dW, ws.R, ws.T, ws.sigma, likelihood, F, N, nv,
+                                                                              nu != nullptr, *r, with_prior, loss);
         BRN_LAUNCH_OK("linreg_finish_kernel");
     }
     StageTimer st3("linreg.reduce_finalize", stream);

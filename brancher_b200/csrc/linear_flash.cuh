@@ -99,6 +99,9 @@ struct LinearFlashParams {
     int y_bulk;                   // y is 16-byte aligned: full blocks of it travel with the X block (bulk copy) into shared memory
     const float* scal_y;          // Gaussian: max |y|  (device scalar)
     double* R;                    // Gaussian: [S] += sum of squared residuals per vector (loss and loss_scale unused)
+                                  // Cauchy: [S] += sum log1p(z^2);  Laplace: [S] += sum |r|
+    const float* sigma;           // Cauchy: [S] noise scale per vector
+    double* T;                    // Cauchy: [S] += sum z^2 / (1 + z^2)
 };
 
 // tcgen05.mma kind::f16 with both shared-memory descriptors given as (low word, shared high word)
@@ -137,7 +140,8 @@ __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.
 // shared memory -- the epilogue thread that owns TMEM lane s writes row s with tcgen05.st: no shared-memory round trip, no
 // generic -> async proxy fence, half the shared-memory operand reads of the gradient MMA.
 // LIK: 0 = Bernoulli (d = y - sigmoid(l), loss += loss_scale * sum ll), 1 = Gaussian residuals (d = r = y - l, R[s] += sum r^2;
-// the noise scale is applied afterwards, per vector, by the caller).
+// the noise scale is applied afterwards, per vector, by the caller), 2 = Cauchy (z = r / sigma_s, d = z / (1 + z^2),
+// R[s] += sum log1p(z^2), T[s] += sum z^2 / (1 + z^2)), 3 = Laplace (d = sign(r), R[s] += sum |r|; sigma applied afterwards).
 template <int KS1, int DTMEM, int LIK = 0>
 __global__ void __launch_bounds__(LF_THREADS, 1)
 linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_constant__ CUtensorMap tmWl,
@@ -317,6 +321,10 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
         // Gaussian: d = r * r_scale with r_scale = p2_scale(max|y| + F max|W| max|X|) >= 2^13 / max|r|: |d| < 2^14 fits fp16
         float r_scale = 0.f;
         if constexpr (LIK == 1) r_scale = p2_scale(*p.scal_y + (float)F * *p.scal_w * *p.scal_x);
+        // Cauchy: lane s owns vector s, so 1 / sigma_s is one register, loaded once
+        float inv_sig = 1.f;
+        if constexpr (LIK == 2) inv_sig = s_ok ? 1.f / p.sigma[s_glob] : 1.f;
+        double ll2_total = 0.0;     // Cauchy: sum of z^2 / (1 + z^2)
         const uint64_t c2 = f2_pack(inv1 * 1.4426950408889634f, inv1 * 1.4426950408889634f);
         const uint64_t one2 = f2_pack(1.f, 1.f), ms2 = f2_pack(-LF_D_SCALE, -LF_D_SCALE), mone2 = f2_pack(-1.f, -1.f);
         int xs = grp % LF_XSTAGES;                     // X stage (and y slot) of this group's next block
@@ -349,6 +357,7 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
             if (b >= LF_D1BUF) { b -= LF_D1BUF; d1ph ^= 1; }
             uint32_t dh_w[LF_EROWS / 2], dl_w[LF_EROWS / 2];
             float ll;                                  // Bernoulli: sum of the block's log-likelihoods; Gaussian: sum of r^2
+                                                       // Cauchy: sum of log1p(z^2); Laplace: sum of |r|
             if constexpr (LIK == 0) {
                 const float ys_lane = y_raw * LF_D_SCALE;
                 // Per element, with raw accumulator L (logit l = L * inv1), e = exp(-|l|), sig = sigmoid(l):
@@ -418,6 +427,101 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
                 asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg0) : "f"(pr0));
                 asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg1) : "f"(pr1));
                 ll = inv1 * ((ay0 + ay1) * (1.f / LF_D_SCALE) - acc_mx) - 0.6931471805599453f * (lg0 + lg1);
+            } else if constexpr (LIK == 2) {
+                // Cauchy, per element: r = y - L inv1, z = r / sigma_s, q = 1 + z^2 and ONE rcp: d = z / q lies in [-1/2, 1/2] and
+                // goes out at 2^14 (the fp16 pair cannot overflow), z^2 / q adds to T.  log1p(z^2) = ln 2 (e + log2 m) with
+                // q = 2^e m, m in [1, 2): the biased exponents add as integers and ONE lg2 per 16 elements takes the product of
+                // 16 mantissas (< 2^16) -- the product of the factors themselves, as the Bernoulli epilogue forms it, overflows
+                // here (q is unbounded).  Rows past the end of a ragged last block get r = 0: d = 0, q = 1, z^2 / q = 0.
+                // (scalar instructions where a constant is involved: they take it as an immediate, a packed one needs a register
+                // pair, and this epilogue is short of registers)
+                const uint64_t mi2 = f2_pack(-inv1, -inv1);
+                uint64_t prod = one2;
+                float acc_t = 0.f;
+                uint32_t esum = 0;
+                auto body = [&](auto ragged, auto from_smem) {
+#pragma unroll
+                    for (int k = 0; k < LF_EROWS / 2; ++k) {
+                        uint64_t y2;
+                        if (decltype(from_smem)::value) {
+                            const float2 yv = *reinterpret_cast<const float2*>(ysm + 2 * k);
+                            y2 = f2_pack(yv.x, yv.y);
+                        } else {
+                            y2 = f2_pack(__shfl_sync(0xffffffffu, y_raw, 2 * k), __shfl_sync(0xffffffffu, y_raw, 2 * k + 1));
+                        }
+                        uint64_t rr2 = f2_fma(f2_pack(L[2 * k], L[2 * k + 1]), mi2, y2);
+                        if (decltype(ragged)::value) {
+                            float q0, q1;
+                            f2_unpack(rr2, q0, q1);
+                            if (hp * LF_EROWS + 2 * k >= rows) q0 = 0.f;
+                            if (hp * LF_EROWS + 2 * k + 1 >= rows) q1 = 0.f;
+                            rr2 = f2_pack(q0, q1);
+                        }
+                        float r0f, r1f, i0, i1;
+                        f2_unpack(rr2, r0f, r1f);
+                        const float z0 = r0f * inv_sig, z1 = r1f * inv_sig;
+                        const float zz0 = z0 * z0, zz1 = z1 * z1;
+                        const float o0 = zz0 + 1.f, o1 = zz1 + 1.f;
+                        asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(i0) : "f"(o0));
+                        asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(i1) : "f"(o1));
+                        acc_t = __fmaf_rn(zz0, i0, acc_t);
+                        acc_t = __fmaf_rn(zz1, i1, acc_t);
+                        const uint32_t b0 = __float_as_uint(o0), b1 = __float_as_uint(o1);
+                        esum += (b0 >> 23) + (b1 >> 23);
+                        prod = f2_mul(prod, f2_pack(__uint_as_float((b0 & 0x007fffffu) | 0x3f800000u),
+                                                    __uint_as_float((b1 & 0x007fffffu) | 0x3f800000u)));
+                        const float d0 = z0 * i0 * (2.f * LF_D_SCALE), d1 = z1 * i1 * (2.f * LF_D_SCALE);
+                        const __half2 h2 = __floats2half2_rn(d0, d1);
+                        const float2 hfv = __half22float2(h2);
+                        const __half2 l2 = __floats2half2_rn(d0 - hfv.x, d1 - hfv.y);
+                        dh_w[k] = *reinterpret_cast<const uint32_t*>(&h2);
+                        dl_w[k] = *reinterpret_cast<const uint32_t*>(&l2);
+                    }
+                };
+                if (y_smem) body(std::false_type{}, std::true_type{});
+                else if (rows == LF_ROWS) body(std::false_type{}, std::false_type{});
+                else body(std::true_type{}, std::false_type{});
+                float pr0, pr1, lg0, lg1;
+                f2_unpack(prod, pr0, pr1);
+                asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg0) : "f"(pr0));
+                asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg1) : "f"(pr1));
+                // every one of the 32 factors carries the exponent bias 127, padding rows (q = 1) included
+                ll = 0.6931471805599453f * ((float)((int)esum - 127 * LF_EROWS) + (lg0 + lg1));
+                ll2_total += (double)acc_t;
+            } else if constexpr (LIK == 3) {
+                // Laplace, per element: r = y - L inv1, d = sign(r) (sign(0) = 0, as torch's abs gradient), exact in fp16 at 2^13
+                // with a zero lo word; |r| adds to A.  No MUFU op.  Rows past the end of a ragged last block get r = 0: d = 0.
+                const uint64_t mi2 = f2_pack(-inv1, -inv1);
+                float acc_a0 = 0.f, acc_a1 = 0.f;
+                auto body = [&](auto ragged, auto from_smem) {
+#pragma unroll
+                    for (int k = 0; k < LF_EROWS / 2; ++k) {
+                        uint64_t y2;
+                        if (decltype(from_smem)::value) {
+                            const float2 yv = *reinterpret_cast<const float2*>(ysm + 2 * k);
+                            y2 = f2_pack(yv.x, yv.y);
+                        } else {
+                            y2 = f2_pack(__shfl_sync(0xffffffffu, y_raw, 2 * k), __shfl_sync(0xffffffffu, y_raw, 2 * k + 1));
+                        }
+                        float q0, q1;
+                        f2_unpack(f2_fma(f2_pack(L[2 * k], L[2 * k + 1]), mi2, y2), q0, q1);
+                        if (decltype(ragged)::value) {
+                            if (hp * LF_EROWS + 2 * k >= rows) q0 = 0.f;
+                            if (hp * LF_EROWS + 2 * k + 1 >= rows) q1 = 0.f;
+                        }
+                        acc_a0 += fabsf(q0);
+                        acc_a1 += fabsf(q1);
+                        const float d0 = q0 > 0.f ? LF_D_SCALE : (q0 < 0.f ? -LF_D_SCALE : 0.f);
+                        const float d1 = q1 > 0.f ? LF_D_SCALE : (q1 < 0.f ? -LF_D_SCALE : 0.f);
+                        const __half2 h2 = __floats2half2_rn(d0, d1);
+                        dh_w[k] = *reinterpret_cast<const uint32_t*>(&h2);
+                        dl_w[k] = 0u;
+                    }
+                };
+                if (y_smem) body(std::false_type{}, std::true_type{});
+                else if (rows == LF_ROWS) body(std::false_type{}, std::false_type{});
+                else body(std::true_type{}, std::false_type{});
+                ll = acc_a0 + acc_a1;
             } else {
                 // r = y - L inv1 per element (no MUFU op); rows past the end of a ragged last block get r = 0
                 const uint64_t mi2 = f2_pack(-inv1, -inv1), rs2 = f2_pack(r_scale, r_scale);
@@ -492,16 +596,19 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
         while ((int)chain < n_chains) drain();
         // this CTA's share of + d ll / d W for vector s_glob, features 32 part .. + 31
         if (s_ok) {
-            const float inv2 = 1.f / ((LIK == 1 ? r_scale : LF_D_SCALE) * p2_scale(*p.scal_x));
+            constexpr float d_scale = LIK == 2 ? 2.f * LF_D_SCALE : LF_D_SCALE;      // Cauchy: |d| <= 1/2 goes out at 2^14
+            const float inv2 = 1.f / ((LIK == 1 ? r_scale : d_scale) * p2_scale(*p.scal_x));
             float* o = p.part + (int64_t)g * p.part_stride + (int64_t)s_glob * F + part * LF_EFEAT;
 #pragma unroll
             for (int c = 0; c < LF_EFEAT; c += 4)
                 if (part * LF_EFEAT + c < F)
                     *reinterpret_cast<float4*>(o + c) = make_float4(r2[c] * inv2, r2[c + 1] * inv2, r2[c + 2] * inv2, r2[c + 3] * inv2);
         }
-        if constexpr (LIK == 1) {
+        if constexpr (LIK != 0) {
             // lane s owns vector s: the two epilogue groups and two row halves of this CTA and every row group add to R[s]
             if (s_ok && ll_total != 0.0) atomicAdd(p.R + s_glob, ll_total);
+            if constexpr (LIK == 2)
+                if (s_ok && ll2_total != 0.0) atomicAdd(p.T + s_glob, ll2_total);
         } else {
         double tot = s_ok ? ll_total : 0.0;      // vectors past S are zero rows of the W tile: their terms are not part of the sum
 #pragma unroll
@@ -616,11 +723,13 @@ static int launch_prepare_x(const float* X, int64_t N, int F, float* bound, __ha
 // dW [S][F] = + d ll / d W, loss += loss_scale * sum ll for S weight vectors W [S][F] over N rows (Bernoulli, C == 1).
 // px: a prepared X (the caller keeps it while X does not change: a training loop over fixed data then reads X once per
 // evaluation, as fp16 pairs, instead of three times), or NULL: X is split into the workspace on every call.
-// R != NULL selects the Gaussian epilogue: the per-slice partials of G_s = sum_b r_sb x_b, r_sb = y_b - w_s . x_b, go to b.part
-// and R[s] += sum_b r_sb^2 (loss is unused).
+// R != NULL selects a regression epilogue, lik (the LIK codes of linear_flash_kernel): 1 = Gaussian, the per-slice partials of
+// G_s = sum_b r_sb x_b, r_sb = y_b - w_s . x_b, go to b.part and R[s] += sum_b r_sb^2 (loss is unused); 2 = Cauchy, with the
+// noise scales sigma [S]: G_s = sum_b z/(1 + z^2) x_b, z = r_sb / sigma_s, R[s] += sum_b log1p(z^2), T[s] += sum_b z^2/(1 + z^2);
+// 3 = Laplace: G_s = sum_b sign(r_sb) x_b, R[s] += sum_b |r_sb|.
 static int launch_linear_flash(const float* X, const void* px, const float* y, int64_t N, int F, int S, const float* W, float* dW,
                                float loss_scale, double* loss, const LinearFlashBuffers& b, cudaStream_t stream,
-                               double* R = nullptr) {
+                               double* R = nullptr, int lik = 1, const float* sigma = nullptr, double* T = nullptr) {
     BRN_CUDA_OK(cudaMemsetAsync(b.scal, 0, 64 * sizeof(float), stream));
     lf_absmax_kernel<<<(unsigned)std::min<int64_t>(((int64_t)S * F / 4 + 255) / 256 + 1, 148), 256, 0, stream>>>(W, (int64_t)S * F, b.scal);
     BRN_LAUNCH_OK("lf_absmax_kernel");
@@ -634,7 +743,7 @@ static int launch_linear_flash(const float* X, const void* px, const float* y, i
     } else if (int e = launch_prepare_x(X, N, F, b.scal + 1, b.Xh, b.Xl, stream)) {
         return e;
     }
-    if (R) {
+    if (R && lik == 1) {
         lf_absmax_kernel<<<(unsigned)std::min<int64_t>((N / 4 + 255) / 256 + 1, 148), 256, 0, stream>>>(y, N, b.scal + 2);
         BRN_LAUNCH_OK("lf_absmax_kernel");
     }
@@ -647,6 +756,7 @@ static int launch_linear_flash(const float* X, const void* px, const float* y, i
     p.y = y; p.N = N; p.F = F; p.S = S; p.scal_w = b.scal; p.scal_x = scal_x; p.part = b.part; p.part_stride = (int64_t)S * F;
     p.loss = loss; p.loss_scale = loss_scale; p.groups = b.groups;
     p.scal_y = b.scal + 2; p.R = R;
+    p.sigma = sigma; p.T = T;
     p.y_bulk = (reinterpret_cast<uintptr_t>(y) & 15) == 0;
     if (const char* env = getenv("BRN_LINEAR_Y_BULK")) p.y_bulk = p.y_bulk && atoi(env) != 0;
     dim3 grid(b.tiles, b.groups);
@@ -657,7 +767,15 @@ static int launch_linear_flash(const float* X, const void* px, const float* y, i
         kern<<<grid, LF_THREADS, smem_bytes, stream>>>(tWh, tWl, tXh, tXl, p);
         return 0;
     };
-    if (R) {      // the Gaussian epilogue exists with the d tile in tensor memory only
+    if (R && lik == 2) {      // the regression epilogues exist with the d tile in tensor memory only
+        if (int e = F == 128 ? launch(linear_flash_kernel<8, 1, 2>, LinearFlashSmem<1>::TOTAL)
+                             : launch(linear_flash_kernel<0, 1, 2>, LinearFlashSmem<1>::TOTAL))
+            return e;
+    } else if (R && lik == 3) {
+        if (int e = F == 128 ? launch(linear_flash_kernel<8, 1, 3>, LinearFlashSmem<1>::TOTAL)
+                             : launch(linear_flash_kernel<0, 1, 3>, LinearFlashSmem<1>::TOTAL))
+            return e;
+    } else if (R) {
         if (int e = F == 128 ? launch(linear_flash_kernel<8, 1, 1>, LinearFlashSmem<1>::TOTAL)
                              : launch(linear_flash_kernel<0, 1, 1>, LinearFlashSmem<1>::TOTAL))
             return e;

@@ -9,7 +9,8 @@ returns a 0-d tensor wired into autograd (so `loss.backward()` fills `.grad` of 
 
 Families
   LinearPlan  K2  observed Binomial(1)/Bernoulli/Categorical with logits = BF.matmul(W, x), W mean-field Normal
-  LinregPlan  K2g observed Normal(BF.matmul(W, x), sigma), W [1, F] mean-field Normal, sigma constant or a LogNormal latent
+  LinregPlan  K2g observed Normal / Cauchy / Laplace(BF.matmul(W, x), sigma), W [1, F] mean-field Normal, sigma constant or a
+              LogNormal latent
   BNNPlan     K3  observed Categorical with logits = BF.matmul(W2, BF.tanh(BF.matmul(W1, x) + b1)) + b2
 Unrecognised graphs raise `UnsupportedModelError` -- there is no eager / CPU fallback for the ELBO.
 """
@@ -287,9 +288,14 @@ class LinearPlan(Plan):
 class LinregPlan(Plan):
     family = "linear regression (K2g)"
 
-    def __init__(self, joint, posterior, k, w_spec, x_var, nu_spec=None, scale=None):
-        """scale: (root, softplus) of a constant noise scale, or a number; None when nu_spec is given"""
+    def __init__(self, joint, posterior, k, w_spec, x_var, nu_spec=None, scale=None, likelihood=None):
+        """scale: (root, softplus) of a constant noise scale, or a number; None when nu_spec is given.
+        likelihood: cu.GAUSSIAN (None), cu.CAUCHY or cu.LAPLACE"""
         super().__init__(joint, posterior)
+        from brancher_b200 import _cuda as cu
+        self.likelihood = cu.GAUSSIAN if likelihood is None else likelihood
+        if self.likelihood != cu.GAUSSIAN:
+            self.family = "linear regression (K2g, %s likelihood)" % {cu.CAUCHY: "Cauchy", cu.LAPLACE: "Laplace"}[self.likelihood]
         self.k, self.x_var = k, x_var
         self.latents = [w_spec] + ([nu_spec] if nu_spec is not None else [])
         self._scale = scale
@@ -311,7 +317,7 @@ class LinregPlan(Plan):
         y = empirical[self.k].reshape(-1).to(torch.float32).contiguous()
         nu = mvars[1] if len(mvars) > 1 else None
         return cu.linreg_elbo_fwd_bwd(X, y, mvars[0], r, nu=nu, noise_scale=None if nu is not None else self.noise_scale(),
-                                      loss=loss, prepared=self._prepared_x)
+                                      loss=loss, prepared=self._prepared_x, likelihood=self.likelihood)
 
 
 class BNNPlan(Plan):
@@ -372,7 +378,7 @@ def _lower_dense(joint, posterior):
         raise UnsupportedModelError("fused families need exactly one observed likelihood node, found %d" % len(liks))
     k = liks[0]
     kind = k.distribution.kind
-    if kind == "normal":
+    if kind in ("normal", "cauchy", "laplace"):
         return _lower_linreg(joint, posterior, k, latents, q_by_name, q_names)
     if "logits" not in k.partial_links:
         raise UnsupportedModelError("likelihood %r: only logits= parametrisations are lowered" % k.name)
@@ -419,28 +425,34 @@ def _lower_dense(joint, posterior):
 
 
 def _lower_linreg(joint, posterior, k, latents, q_by_name, q_names):
-    """K2g: observed Normal(loc = matmul(W, x), scale) with W the [1, F] mean-field Normal weights and x data; scale a
-    non-learnable constant (a root, behind softplus when auto-named, or a number) or a scalar LogNormal latent."""
+    """K2g: observed Normal / Cauchy / Laplace(loc = matmul(W, x), scale) with W the [1, F] mean-field Normal weights and x
+    data; scale a non-learnable constant (a root, behind softplus when auto-named, or a number) or a scalar LogNormal latent."""
+    from brancher_b200 import _cuda as cu
+    kind = k.distribution.kind
+    likelihood = {"normal": cu.GAUSSIAN, "cauchy": cu.CAUCHY, "laplace": cu.LAPLACE}[kind]
+    lik_name = {"normal": "Normal", "cauchy": "Cauchy", "laplace": "Laplace"}[kind]
+    what = "linear regression" if kind == "normal" else "%s linear regression" % lik_name
     loc, scale = k.partial_links["loc"].expr, k.partial_links["scale"].expr
     if not _is_call(loc, "matmul", 2):
         for a, b in _commutative_add(loc):
             if _is_call(a, "matmul", 2):
-                raise UnsupportedModelError("linear regression %r: a bias added to BF.matmul(weights, x) is not lowered -- "
-                                            "append a column of ones to x instead" % k.name)
-        raise UnsupportedModelError("likelihood %r: a Normal likelihood is lowered for loc = BF.matmul(weights, x) only" % k.name)
+                raise UnsupportedModelError("%s %r: a bias added to BF.matmul(weights, x) is not lowered -- "
+                                            "append a column of ones to x instead" % (what, k.name))
+        raise UnsupportedModelError("likelihood %r: a %s likelihood is lowered for loc = BF.matmul(weights, x) only"
+                                    % (k.name, lik_name))
     W, x = _var(loc.args[0]), _var(loc.args[1])
     if W not in latents or not _is_data(x):
-        raise UnsupportedModelError("linear regression %r: loc must be BF.matmul(weights, x) with weights a latent and x data" % k.name)
+        raise UnsupportedModelError("%s %r: loc must be BF.matmul(weights, x) with weights a latent and x data" % (what, k.name))
     ws = MeanFieldSpec(W.name, q_by_name[W.name], W, q_names)
     if len(ws.shape) != 2 or ws.shape[0] != 1:
-        raise UnsupportedModelError("linear regression %r: weights must have shape [1, F] (multi-output regression is not "
-                                    "lowered), got %s" % (k.name, ws.shape))
+        raise UnsupportedModelError("%s %r: weights must have shape [1, F] (multi-output regression is not "
+                                    "lowered), got %s" % (what, k.name, ws.shape))
     nu_spec, const = None, None
     nu = _var(scale)
     if nu is not None and nu in latents:
         if nu.distribution.kind != "lognormal":
-            raise UnsupportedModelError("linear regression %r: a %s-distributed noise scale is not lowered (a LogNormal "
-                                        "latent or a constant is)" % (k.name, nu.distribution.kind))
+            raise UnsupportedModelError("%s %r: a %s-distributed noise scale is not lowered (a LogNormal "
+                                        "latent or a constant is)" % (what, k.name, nu.distribution.kind))
         nu_spec = LogNormalSpec(nu.name, q_by_name[nu.name], nu, q_names)
     else:
         root, sp = _softplus_root(scale), True
@@ -448,21 +460,21 @@ def _lower_linreg(joint, posterior, k, latents, q_by_name, q_names):
             root, sp = _as_root(scale), False
         if root is not None and not root.is_observed:
             if getattr(root, "learnable", False):
-                raise UnsupportedModelError("linear regression %r: a learnable point-estimate noise scale (root %r) is not "
-                                            "lowered" % (k.name, root.name))
+                raise UnsupportedModelError("%s %r: a learnable point-estimate noise scale (root %r) is not "
+                                            "lowered" % (what, k.name, root.name))
             if root._value.numel() != 1:
-                raise UnsupportedModelError("linear regression %r: the noise scale must be a scalar" % k.name)
+                raise UnsupportedModelError("%s %r: the noise scale must be a scalar" % (what, k.name))
             const = (root, sp)
         elif _const_value(scale) is not None:
             const = _const_value(scale)
         else:
-            raise UnsupportedModelError("linear regression %r: the noise scale must be a constant or a scalar LogNormal latent "
-                                        "(deterministic or data-dependent scales are not lowered)" % k.name)
+            raise UnsupportedModelError("%s %r: the noise scale must be a constant or a scalar LogNormal latent "
+                                        "(deterministic or data-dependent scales are not lowered)" % (what, k.name))
     extra = [v.name for v in latents if v is not W and v is not nu]
     if extra:
-        raise UnsupportedModelError("linear regression %r: latent variables other than the weights and the noise scale are not "
-                                    "lowered: %s" % (k.name, sorted(extra)))
-    return LinregPlan(joint, posterior, k, ws, x, nu_spec=nu_spec, scale=const)
+        raise UnsupportedModelError("%s %r: latent variables other than the weights and the noise scale are not "
+                                    "lowered: %s" % (what, k.name, sorted(extra)))
+    return LinregPlan(joint, posterior, k, ws, x, nu_spec=nu_spec, scale=const, likelihood=likelihood)
 
 
 # ---------------------------------------------------------------------------------------------------

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define BRN_ABI_VERSION 3
+#define BRN_ABI_VERSION 4
 
 /* One mean-field Normal variational variable  q(w) = N(mu, softplus(rho))  together with the Normal
  * prior p(w) = N(prior_loc, prior_scale) of the same name.
@@ -174,6 +174,23 @@ int brn_linreg_elbo_fwd_bwd(const float* X, const void* px, const float* y, int6
                             const brn_mf_var* w, const brn_mf_var* nu, const float* noise_scale,
                             const brn_sample_range* r, void* workspace, size_t workspace_bytes, int with_prior,
                             double* loss, void* stream);
+
+/* K2g with a choice of likelihood: robust (heavy-tailed) regression over the same dense design matrix.  The codes continue the
+ * likelihood codes of brn_linear_elbo_fwd_bwd (0 Bernoulli, 1 Categorical).  With r_sb = y_b - w_s . x_b, z_sb = r_sb / sigma_s
+ * and u_s = log sigma_s, per sample (torch's log_prob of each distribution, summed over the N rows):
+ *   BRN_LINREG_NORMAL   y_b ~ Normal(w_s . x_b, sigma_s):   ll_s = -sum_b r^2 / (2 sigma_s^2) - N u_s - N/2 log(2 pi)
+ *                       exactly brn_linreg_elbo_fwd_bwd
+ *   BRN_LINREG_CAUCHY   y_b ~ Cauchy(w_s . x_b, sigma_s):   ll_s = -N (log pi + u_s) - sum_b log1p(z^2)
+ *   BRN_LINREG_LAPLACE  y_b ~ Laplace(w_s . x_b, sigma_s):  ll_s = -N (log 2 + u_s) - sum_b |r| / sigma_s
+ *                       (the gradient of |r| at r = 0 is 0, as torch's abs gives it)
+ * Every other argument, the two noise forms, the prior / entropy terms, the prepared X and the workspace are as for
+ * brn_linreg_elbo_fwd_bwd.  Replaces the graph walk for CauchyVariable / LaplaceVariable(BF.matmul(weights, x), nu_or_constant,
+ * "y") (standard_variables.py:156-183, torch.distributions Cauchy / Laplace log_prob). */
+enum brn_linreg_likelihood { BRN_LINREG_NORMAL = 2, BRN_LINREG_CAUCHY = 3, BRN_LINREG_LAPLACE = 4 };
+int brn_linreg_elbo_fwd_bwd_lik(const float* X, const void* px, const float* y, int likelihood, int64_t N, int F,
+                                const brn_mf_var* w, const brn_mf_var* nu, const float* noise_scale,
+                                const brn_sample_range* r, void* workspace, size_t workspace_bytes, int with_prior,
+                                double* loss, void* stream);
 
 /* K1 -- generic scalar-DAG ELBO: fused reparameterised sampling + log-probs + reduction over samples and data rows +
  * backward, for models whose variables are scalars (README.md:22-75 AR(1); examples/logNormal_normal.py;

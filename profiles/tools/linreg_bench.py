@@ -1,12 +1,14 @@
-"""Bayesian linear regression (K2g, brn_linreg_elbo_fwd_bwd) against the Bernoulli K2 evaluation on the same data matrix.
+"""Bayesian linear regression (K2g, brn_linreg_elbo_fwd_bwd_lik: Normal, Cauchy and Laplace likelihoods) against the Bernoulli K2
+evaluation on the same data matrix.
 
     python profiles/tools/linreg_bench.py [--N 1000000 --F 128 --S 1024 --steps 60 --warmup 10]
 
 N = 10^6 rows, F = 128 features, S = 1024 samples, one prepared X shared by every evaluation.  Method of bench.py (DESIGN.md
 section 6): each evaluation (loss and gradient buffers zeroed, then one fused call) is captured once in a CUDA graph and
-replayed; a 256 MiB buffer is overwritten between timed replays to flush the L2; CUDA events time each replay.  The three
-evaluations -- Bernoulli, Gaussian with a fixed noise scale, Gaussian with a LogNormal noise latent -- alternate replay by
-replay in one process, so clock and neighbour effects fall on all three alike.  Prints one JSON line: GPU name and power limit
+replayed; a 256 MiB buffer is overwritten between timed replays to flush the L2; CUDA events time each replay.  The seven
+evaluations -- Bernoulli, then Gaussian, Cauchy and Laplace each with a fixed noise scale and with a LogNormal noise latent --
+alternate replay by replay in one process, so clock and neighbour effects fall on all of them alike.  The Cauchy and Laplace
+targets are y = X w* + 0.3 standard-Cauchy noise.  Prints one JSON line: GPU name and power limit
 (read-only nvidia-smi query), ms per evaluation, the ratio to Bernoulli and the fraction of the 3xFP16 roofline (4 S N F flop
 at a third of the bf16 dense rate).  Needs a GPU: there is no CPU path.
 """
@@ -57,6 +59,7 @@ def main():
     wstar = torch.randn(F, generator=g) / F ** 0.5
     y_gauss = (X @ wstar + 0.3 * torch.randn(N, generator=g)).to(dev)
     y_bern = (torch.rand(N, generator=g) < torch.sigmoid(X @ wstar)).float().to(dev)
+    y_heavy = (X @ wstar + 0.3 * torch.tan(np.pi * (torch.rand(N, generator=g, dtype=torch.float64) - 0.5)).float()).to(dev)
     X = X.to(dev).contiguous()
     px = cu.PreparedX()
     mu = torch.zeros(1, F, device=dev)
@@ -75,6 +78,11 @@ def main():
         "gaussian_fixed": lambda: cu.linreg_elbo_fwd_bwd(X, y_gauss, w, r, noise_scale=scale, loss=loss, prepared=px),
         "gaussian_lognormal": lambda: cu.linreg_elbo_fwd_bwd(X, y_gauss, w, r, nu=nu, loss=loss, prepared=px),
     }
+    for lik, name in ((cu.CAUCHY, "cauchy"), (cu.LAPLACE, "laplace")):
+        evals[name + "_fixed"] = (lambda lik=lik: cu.linreg_elbo_fwd_bwd(X, y_heavy, w, r, noise_scale=scale, loss=loss, prepared=px,
+                                                                          likelihood=lik))
+        evals[name + "_lognormal"] = (lambda lik=lik: cu.linreg_elbo_fwd_bwd(X, y_heavy, w, r, nu=nu, loss=loss, prepared=px,
+                                                                              likelihood=lik))
     variants = {}
     for name, fn in evals.items():          # every workspace is grown (and X prepared) before the first capture
         zero(); fn()
@@ -101,12 +109,22 @@ def main():
     torch.cuda.synchronize()
     ms = {n: float(np.mean([s.elapsed_time(e) for s, e in evs[n]])) for n in graphs}
     spread = {n: [float(np.percentile([s.elapsed_time(e) for s, e in evs[n]], q)) for q in (10, 50, 90)] for n in graphs}
+    # per-stage split (StageTimer events), in a separate eager pass after the timed replays: the events are not in the graphs
+    stages = {}
+    for name, fn in evals.items():
+        cu.profile_reset(); cu.profile_enable(True)
+        for _ in range(10):
+            flush.fill_(0.0); zero(); fn()
+        st = cu.profile_collect()
+        cu.profile_enable(False)
+        stages[name] = {k: v[0] / v[1] for k, v in st.items() if v[1] > 0}
     bf16, peak_src = bf16_burst_tflops()
     roof_ms = 4.0 * S * N * F / (bf16 / 3 * 1e12) * 1e3
     out = dict(gpu_info(), N=N, F=F, S=S, steps=a.steps, warmup=a.warmup, method="CUDA graph replay, 256 MiB L2 flush between "
-               "replays, CUDA events, the three evaluations alternating", variants=variants,
+               "replays, CUDA events, the evaluations alternating", variants=variants,
                ms_per_eval=ms, ms_p10_p50_p90=spread, ratio_to_bernoulli={n: ms[n] / ms["bernoulli"] for n in ms},
                frac_3xfp16_roofline={n: roof_ms / ms[n] for n in ms}, roofline_ms=roof_ms,
+               stage_ms_eager=stages,
                roofline="4 S N F flop at bf16 burst / 3 = %.0f TFLOP/s, peak %s" % (bf16 / 3, peak_src))
     line = json.dumps(out)
     print(line)
