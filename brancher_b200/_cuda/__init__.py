@@ -12,7 +12,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libbrancher_cuda.so")
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 _lib = None
 
@@ -125,6 +125,14 @@ SYMBOLS = {
                                                    ctypes.c_int, ctypes.POINTER(MFVar), ctypes.POINTER(MFVar), ctypes.c_void_p,
                                                    ctypes.POINTER(SampleRange), ctypes.c_void_p, ctypes.c_size_t, ctypes.c_int,
                                                    ctypes.c_void_p, ctypes.c_void_p]),
+    "brn_linreg_vectors_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int64, ctypes.c_int, ctypes.c_int]),
+    "brn_linreg_particles_loss_grad": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int64,
+                                                      ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
+                                                      ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                                      ctypes.c_size_t, ctypes.c_void_p]),
+    "brn_linreg_vectors_loglik_grad": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int64,
+                                                      ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
+                                                      ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]),
     "brn_svgd_sharded_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int, ctypes.c_int]),
     "brn_svgd_sharded_offsets": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.c_int] + [ctypes.POINTER(ctypes.c_size_t)] * 4),
     "brn_svgd_sharded_phase": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p] + [ctypes.c_int] * 5 +
@@ -547,6 +555,58 @@ def linear_particles_loss_grad(X, y, likelihood, theta, C, prior_loc=None, prior
     return loss, G
 
 
+def _regression_args(fn, X, y, likelihood, V, noise_scale):
+    N, F = X.shape
+    if likelihood not in (GAUSSIAN, CAUCHY, LAPLACE):
+        raise BrancherCudaError("%s: unknown likelihood %r (GAUSSIAN, CAUCHY or LAPLACE)" % (fn, likelihood))
+    if V.shape[1] != F:
+        raise BrancherCudaError("%s: weight vectors have %d elements, expected F = %d" % (fn, V.shape[1], F))
+    if y.numel() != N:
+        raise BrancherCudaError("%s: y has %d entries for %d rows" % (fn, y.numel(), N))
+    if noise_scale is None or noise_scale.numel() != 1:
+        raise BrancherCudaError("%s: noise_scale must be a 1-element fp32 CUDA tensor" % fn)
+
+
+def linreg_particles_loss_grad(X, y, likelihood, theta, noise_scale, prior_loc=None, prior_scale=None, loss=None, prepared=None):
+    """K4a for regression particles: y ~ Normal / Cauchy / Laplace(X theta_k, sigma) (likelihood GAUSSIAN / CAUCHY / LAPLACE), theta
+    [n, F], noise_scale a 1-element fp32 CUDA tensor holding sigma -> (loss fp64 [1] accumulator, G [n, F] = d loss / d theta) with
+    loss += sum_k [-ll_k - log N(theta_k; prior)].  prepared: a PreparedX kept by the caller for a fixed X (optional)."""
+    dev = X.device
+    N, F = X.shape
+    n = theta.shape[0]
+    theta = theta.reshape(n, -1) if n else theta.reshape(0, F)
+    _regression_args("linreg_particles_loss_grad", X, y, likelihood, theta, noise_scale)
+    loss = torch.zeros(1, dtype=torch.float64, device=dev) if loss is None else loss
+    G = torch.empty_like(theta)
+    ws = _workspace(dev, lib().brn_linreg_vectors_workspace_bytes(N, F, n))
+    px = prepared.get(X, likelihood, 1) if (prepared is not None and N > 0) else None
+    _check(lib().brn_linreg_particles_loss_grad(_ptr(X, what="X"), px.data_ptr() if px is not None else None, _ptr(y, what="y"),
+                                                likelihood, N, F, _ptr(theta, what="theta"), n, _ptr(prior_loc, what="prior_loc"),
+                                                _ptr(prior_scale, what="prior_scale"), _ptr(noise_scale, what="noise_scale"), _ptr(G),
+                                                _ptr(loss, torch.float64), ws.data_ptr(), ws.numel(), _stream(dev)),
+           "brn_linreg_particles_loss_grad")
+    return loss, G
+
+
+def linreg_vectors_loglik_grad(X, y, likelihood, V, noise_scale, want_grad=True, prepared=None):
+    """K6b for regression: V [n, F] weight vectors -> (ll fp64 [n], G [n, F] = -d ll / d V or None); arguments as for
+    linreg_particles_loss_grad."""
+    dev = X.device
+    N, F = X.shape
+    n = V.shape[0]
+    V = V.reshape(n, -1) if n else V.reshape(0, F)
+    _regression_args("linreg_vectors_loglik_grad", X, y, likelihood, V, noise_scale)
+    ll = torch.empty(n, dtype=torch.float64, device=dev)
+    G = torch.empty_like(V) if want_grad else None
+    ws = _workspace(dev, lib().brn_linreg_vectors_workspace_bytes(N, F, n))
+    px = prepared.get(X, likelihood, 1) if (prepared is not None and N > 0) else None
+    _check(lib().brn_linreg_vectors_loglik_grad(_ptr(X, what="X"), px.data_ptr() if px is not None else None, _ptr(y, what="y"),
+                                                likelihood, N, F, _ptr(V, what="V"), n, _ptr(noise_scale, what="noise_scale"), _ptr(G),
+                                                _ptr(ll, torch.float64), ws.data_ptr(), ws.numel(), _stream(dev)),
+           "brn_linreg_vectors_loglik_grad")
+    return ll, G
+
+
 def svgd_direction(theta, grad, row0=0, rows=None, bandwidth=None):
     """K4b.  theta, grad [n, d] (all particles) -> (out [rows, d], bandwidth device float [1]).  bandwidth=None applies
     the reference's median heuristic (inference.py:317-324); pass a device tensor to reuse a fixed bandwidth."""
@@ -639,17 +699,23 @@ def wvgd_sample_assign(loc, rho, theta, S, F_last, r, draw, eps=None, first_colu
 
 
 def wvgd_loss_grad(X, y, likelihood, C, loc, rho, theta, S, r, eps0=None, eps1=None, prior=None, biased=False,
-                   first_column_only=True, loss=None):
+                   first_column_only=True, loss=None, noise_scale=None, prepared=None):
     """K6: one WassersteinVariationalGradientDescent.compute_loss + backward (inference.py:203-229) for P (sampler, particle)
-    pairs.  loc, theta [P, C*F]; rho [P] or [P, C*F]; prior = (loc [C*F], scale [C*F]) or None (tied).
+    pairs.  loc, theta [P, C*F]; rho [P] or [P, C*F]; prior = (loc [C*F], scale [C*F]) or None (tied).  For the regression
+    likelihoods GAUSSIAN / CAUCHY / LAPLACE (C = 1) noise_scale is the 1-element device tensor holding sigma and prepared an
+    optional PreparedX, as for linreg_vectors_loglik_grad.
     Returns (loss fp64 [1], dloc [P,d], drho [P,d] per element, dtheta [P,d], counts int32 [P,2])."""
     P, d = loc.shape
     dev = loc.device
     F_last = d // C
     Z0, e0, o0 = wvgd_sample_assign(loc, rho, theta, S, F_last, r, 0, eps0, first_column_only)
     Z1, e1, o1 = wvgd_sample_assign(loc, rho, theta, S, F_last, r, 1, eps1, first_column_only)
-    ll0, G0 = linear_vectors_loglik_grad(X, y, likelihood, Z0.reshape(P * S, d), C, True)
-    ll1, _ = linear_vectors_loglik_grad(X, y, likelihood, Z1.reshape(P * S, d), C, False)
+    if likelihood in (GAUSSIAN, CAUCHY, LAPLACE):
+        ll0, G0 = linreg_vectors_loglik_grad(X, y, likelihood, Z0.reshape(P * S, d), noise_scale, True, prepared)
+        ll1, _ = linreg_vectors_loglik_grad(X, y, likelihood, Z1.reshape(P * S, d), noise_scale, False, prepared)
+    else:
+        ll0, G0 = linear_vectors_loglik_grad(X, y, likelihood, Z0.reshape(P * S, d), C, True)
+        ll1, _ = linear_vectors_loglik_grad(X, y, likelihood, Z1.reshape(P * S, d), C, False)
     loss = torch.zeros(1, dtype=torch.float64, device=dev) if loss is None else loss
     dloc, drho, dtheta = torch.empty_like(loc), torch.empty_like(loc), torch.empty_like(loc)
     counts = torch.empty((P, 2), dtype=torch.int32, device=dev)

@@ -755,6 +755,30 @@ linreg_sigma_kernel(float* __restrict__ sigma, brn_mf_var nu, int has_nu, const 
     }
 }
 
+// The per-vector finishing formulas shared by the mean-field finisher and the particle / vector finisher, so the two families
+// cannot disagree.  linreg_grad_scale: the factor that turns the X pass's G_s into d ll_s / d w_s.  linreg_loglik: ll_s from the
+// X pass's sums (R_s, and T_s for Cauchy) and, in *gu, d ll_s / d u_s with u_s = log sigma_s (formulas below).
+__device__ __forceinline__ float linreg_grad_scale(int lik, float sigma) {
+    return lik == BRN_LINREG_CAUCHY ? 2.0f / sigma : lik == BRN_LINREG_LAPLACE ? 1.0f / sigma : 1.0f / (sigma * sigma);
+}
+__device__ __forceinline__ double linreg_loglik(int lik, double sd, double Rs, const double* __restrict__ T, int s, int64_t N,
+                                                double* gu) {
+    double ll;
+    if (lik == BRN_LINREG_CAUCHY) {
+        ll = -(double)N * (log(sd) + 1.1447298858494002) - Rs;                     // log pi
+        *gu = 2.0 * T[s] - (double)N;
+    } else if (lik == BRN_LINREG_LAPLACE) {
+        const double a = Rs / sd;
+        ll = -(double)N * (log(sd) + 0.6931471805599453) - a;                      // log 2
+        *gu = a - (double)N;
+    } else {
+        const double inv_s2 = 1.0 / (sd * sd);
+        ll = -0.5 * Rs * inv_s2 - (double)N * (log(sd) + (double)BRN_HALF_LOG_2PI);
+        *gu = Rs * inv_s2 - (double)N;
+    }
+    return ll;
+}
+
 // One thread per element (s, f) of the per-sample gradient rows: dW_s *= 1 / sigma_s^2 in place (Cauchy: 2 / sigma_s, Laplace:
 // 1 / sigma_s).  The thread of f == 0 also owns sample s's scalar terms, all scaled by 1 / S_total (the partial contract of
 // brn_mf_normal_prior_entropy, so sharded samples sum to the unsharded result), with u_s = log sigma_s:
@@ -784,22 +808,10 @@ linreg_finish_kernel(float* __restrict__ dW, const double* __restrict__ R, const
             m = nu.mu[0];
             sg = softplusf(nu.rho[0]);
         }
-        dW[i] *= lik == BRN_LINREG_CAUCHY ? 2.0f / sigma : lik == BRN_LINREG_LAPLACE ? 1.0f / sigma : 1.0f / (sigma * sigma);
+        dW[i] *= linreg_grad_scale(lik, sigma);
         if (i % F == 0) {
-            const double sd = sigma, Rs = R[s];
             double gu_ll;                      // d ll_s / d u_s
-            if (lik == BRN_LINREG_CAUCHY) {
-                elbo = -(double)N * (log(sd) + 1.1447298858494002) - Rs;                   // log pi
-                gu_ll = 2.0 * T[s] - (double)N;
-            } else if (lik == BRN_LINREG_LAPLACE) {
-                const double a = Rs / sd;
-                elbo = -(double)N * (log(sd) + 0.6931471805599453) - a;                   // log 2
-                gu_ll = a - (double)N;
-            } else {
-                const double inv_s2 = 1.0 / (sd * sd);
-                elbo = -0.5 * Rs * inv_s2 - (double)N * (log(sd) + (double)BRN_HALF_LOG_2PI);
-                gu_ll = Rs * inv_s2 - (double)N;
-            }
+            elbo = linreg_loglik(lik, sigma, R[s], T, s, N, &gu_ll);
             if (has_nu) {
                 const float gu = (float)gu_ll;
                 gm = gu;
@@ -833,6 +845,53 @@ linreg_finish_kernel(float* __restrict__ dW, const double* __restrict__ R, const
             atomicAdd(nu.dmu, -tm * inv_S);
             atomicAdd(nu.drho, -ts * inv_S * sigmoidf(nu.rho[0]));
         }
+    }
+}
+
+// The finisher of n weight vectors (particles, or WVGD's draws) at a fixed noise scale: one thread per element (k, f) of G,
+// G_k *= the likelihood's scale (G may be NULL); the thread of f == 0 computes ll_k in fp64 and writes ll[k] (ll != NULL) or adds
+// -ll_k to *loss.  No 1/S factor: particle losses are sums over the particles.
+struct LinregVectorsWorkspace {
+    double *R, *T;
+    float* sigma;
+    LinearFlashBuffers flash;
+    size_t bytes;
+    LinregVectorsWorkspace(void* base, int n, int64_t N, int F, bool flash_path, int sms) {
+        WorkspaceCarver take(base);
+        R = reinterpret_cast<double*>(take(2 * (size_t)n));
+        T = reinterpret_cast<double*>(take(2 * (size_t)n));
+        sigma = take((size_t)n);
+        flash = LinearFlashBuffers();
+        if (flash_path) {
+            flash.carve(take, n, F, sms);
+            flash.Xh = reinterpret_cast<__half*>(take(((size_t)N * F + 1) / 2));
+            flash.Xl = reinterpret_cast<__half*>(take(((size_t)N * F + 1) / 2));
+        }
+        bytes = take.off;
+    }
+};
+
+__global__ void __launch_bounds__(256)
+linreg_vectors_finish_kernel(float* __restrict__ G, const double* __restrict__ R, const double* __restrict__ T,
+                             const float* __restrict__ sig, int lik, int F, int64_t N, int n, double* __restrict__ ll,
+                             double* __restrict__ loss) {
+    __shared__ double red[32];
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    double nll = 0.0;
+    if (i < (int64_t)n * F) {
+        const int k = (int)(i / F);
+        const float sigma = sig[k];
+        if (G) G[i] *= linreg_grad_scale(lik, sigma);
+        if (i % F == 0) {
+            double gu;
+            const double l = linreg_loglik(lik, sigma, R[k], T, k, N, &gu);
+            if (ll) ll[k] = l;
+            else nll = -l;
+        }
+    }
+    if (loss) {
+        const double tot = block_sum<double>(nll, red);
+        if (threadIdx.x == 0 && tot != 0.0) atomicAdd(loss, tot);
     }
 }
 
@@ -928,4 +987,107 @@ extern "C" int brn_linreg_elbo_fwd_bwd_lik(const float* X, const void* px, const
     }
     StageTimer st3("linreg.reduce_finalize", stream);
     return launch_mf_reduce_finalize(*w, eps, F, ws.dW, F, ws.stats, *r, with_prior, loss, stream);
+}
+
+// ---------------------------------------------------------------------------------------------
+// K4a / K6b for regression particles and vectors (brn_linreg_particles_loss_grad, brn_linreg_vectors_loglik_grad): the K2g X pass
+// with the n particles as the weight vectors at a fixed noise scale, then linreg_vectors_finish_kernel instead of the mean-field
+// finisher.  G (when given) leaves holding + d ll / d theta; the callers negate it and add the prior (particles_prior_kernel).
+// ---------------------------------------------------------------------------------------------
+static int linreg_vectors_check(const char* fn, const float* X, const void* px, const float* y, int likelihood, int64_t N, int F,
+                                const float* V, int n, const float* noise_scale) {
+    BRN_CHECK_ARG(likelihood == BRN_LINREG_NORMAL || likelihood == BRN_LINREG_CAUCHY || likelihood == BRN_LINREG_LAPLACE,
+                  "%s: unknown likelihood %d (Normal %d, Cauchy %d, Laplace %d)", fn, likelihood, BRN_LINREG_NORMAL, BRN_LINREG_CAUCHY,
+                  BRN_LINREG_LAPLACE);
+    BRN_CHECK_ARG((V || n == 0) && noise_scale, "%s: NULL pointer (weight vectors or noise_scale)", fn);
+    BRN_CHECK_ARG(N >= 0 && F > 0 && n >= 0, "%s: bad shape N=%lld F=%d n=%d", fn, (long long)N, F, n);
+    BRN_CHECK_ARG(N == 0 || (X && y), "%s: NULL data pointer", fn);
+    BRN_CHECK_ARG(F <= LN_T, "%s: F=%d exceeds the supported maximum %d", fn, F, LN_T);
+    BRN_CHECK_ARG(!px || (linear_prepared_x_bytes(N, F) > 0 && (reinterpret_cast<uintptr_t>(px) & 255) == 0),
+                  "%s: a prepared X does not exist for N=%lld F=%d, or px is not 256-byte aligned", fn, (long long)N, F);
+    return 0;
+}
+
+static int linreg_vectors_run(const float* X, const void* px, const float* y, int likelihood, int64_t N, int F, const float* V, int n,
+                              const float* noise_scale, float* G, double* ll, double* loss, void* workspace, size_t workspace_bytes,
+                              const char* stage, cudaStream_t stream) {
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const bool use_flash = N > 0 && linreg_use_flash(X, N, F, n);
+    LinregVectorsWorkspace ws(workspace, n, N, F, use_flash, sms);
+    BRN_CHECK_ARG(workspace && workspace_bytes >= ws.bytes, "workspace too small: %zu < %zu", workspace_bytes, ws.bytes);
+    set_variant(use_flash ? "tcgen05-flash" : "simt");
+    const int64_t tot = (int64_t)n * F;
+    StageTimer st(stage, stream);
+    BRN_CUDA_OK(cudaMemsetAsync(ws.R, 0, sizeof(double) * (size_t)n, stream));
+    if (likelihood == BRN_LINREG_CAUCHY) BRN_CUDA_OK(cudaMemsetAsync(ws.T, 0, sizeof(double) * (size_t)n, stream));
+    brn_sample_range r{};
+    r.s_local = n;
+    r.s_total = n;
+    linreg_sigma_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(ws.sigma, brn_mf_var{}, 0, noise_scale, r);
+    BRN_LAUNCH_OK("linreg_sigma_kernel");
+    const int lik_flash = likelihood - BRN_LINREG_NORMAL + 1, lik_simt = likelihood - BRN_LINREG_NORMAL + 2;
+    if (use_flash) {
+        if (int e = launch_linear_flash(X, px, y, N, F, n, V, G, 0.f, nullptr, ws.flash, stream, ws.R, lik_flash, ws.sigma, ws.T))
+            return e;
+        if (G) {
+            sum_slices_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(ws.flash.part, ws.flash.groups, tot, tot, G);
+            BRN_LAUNCH_OK("sum_slices_kernel");
+        }
+    } else {
+        if (G) BRN_CUDA_OK(cudaMemsetAsync(G, 0, sizeof(float) * (size_t)tot, stream));
+        if (N > 0)
+            if (int e = launch_linear_fused(X, y, lik_simt, N, F, 1, n, V, G, 0.f, nullptr, stream, ws.R, ws.sigma, ws.T)) return e;
+    }
+    linreg_vectors_finish_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(G, ws.R, ws.T, ws.sigma, likelihood, F, N, n, ll,
+                                                                                  loss);
+    BRN_LAUNCH_OK("linreg_vectors_finish_kernel");
+    return 0;
+}
+
+extern "C" size_t brn_linreg_vectors_workspace_bytes(int64_t N, int F, int n) {
+    if (N < 0 || F <= 0 || n < 0) return 0;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    // sized for the one-pass kernel whenever a call of this shape may take it (X's alignment is not known here)
+    return LinregVectorsWorkspace(nullptr, n, N, F, N > 0 && linreg_use_flash(nullptr, N, F, n), sms).bytes;
+}
+
+extern "C" int brn_linreg_particles_loss_grad(const float* X, const void* px, const float* y, int likelihood, int64_t N, int F,
+                                              const float* theta, int n, const float* prior_loc, const float* prior_scale,
+                                              const float* noise_scale, float* G, double* loss, void* workspace,
+                                              size_t workspace_bytes, void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    if (int e = linreg_vectors_check("brn_linreg_particles_loss_grad", X, px, y, likelihood, N, F, theta, n, noise_scale)) return e;
+    BRN_CHECK_ARG((G || n == 0) && loss, "brn_linreg_particles_loss_grad: NULL pointer (G or loss)");
+    BRN_CHECK_ARG((prior_loc == nullptr) == (prior_scale == nullptr), "prior_loc and prior_scale must both be given or both NULL");
+    if (n == 0) return 0;
+    if (int e = linreg_vectors_run(X, px, y, likelihood, N, F, theta, n, noise_scale, G, nullptr, loss, workspace, workspace_bytes,
+                                   "linreg_particles.loglik_grad", stream))
+        return e;
+    const int64_t total = (int64_t)n * F;
+    StageTimer st("linreg_particles.prior", stream);
+    particles_prior_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(theta, prior_loc, prior_scale, F, total, G, loss);
+    BRN_LAUNCH_OK("particles_prior_kernel");
+    return 0;
+}
+
+extern "C" int brn_linreg_vectors_loglik_grad(const float* X, const void* px, const float* y, int likelihood, int64_t N, int F,
+                                              const float* V, int n, const float* noise_scale, float* G, double* ll, void* workspace,
+                                              size_t workspace_bytes, void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    if (int e = linreg_vectors_check("brn_linreg_vectors_loglik_grad", X, px, y, likelihood, N, F, V, n, noise_scale)) return e;
+    BRN_CHECK_ARG(ll || n == 0, "brn_linreg_vectors_loglik_grad: NULL pointer (ll)");
+    if (n == 0) return 0;
+    if (int e = linreg_vectors_run(X, px, y, likelihood, N, F, V, n, noise_scale, G, ll, nullptr, workspace, workspace_bytes,
+                                   "linreg_vectors.loglik_grad", stream))
+        return e;
+    if (G) {       // + d ll / d V -> the ABI's loss gradient - d ll / d V
+        const int64_t total = (int64_t)n * F;
+        particles_prior_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(V, nullptr, nullptr, F, total, G, nullptr);
+        BRN_LAUNCH_OK("particles_prior_kernel");
+    }
+    return 0;
 }

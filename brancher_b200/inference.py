@@ -274,8 +274,9 @@ class SteinVariationalGradientDescent(InferenceMethod):
 
 class MAP(InferenceMethod):
     """Maximum a posteriori (inference.py:251-274): the posterior model holds one learnable RootVariable per latent,
-    loss = -log p(data, theta).  The point estimate is a one-particle ensemble of the linear family (K4a: one fused launch
-    for the joint log-probability and its gradient), any scalar model goes through the scalar-DAG family (K1)."""
+    loss = -log p(data, theta).  The point estimate is a one-particle ensemble of the linear family or of the dense regression
+    family at a constant noise scale (K4a: one fused launch for the joint log-probability and its gradient), any scalar model goes
+    through the scalar-DAG family (K1)."""
 
     def __init__(self):
         self.learnable_model = False

@@ -12,6 +12,8 @@ Families
   LinregPlan  K2g observed Normal / Cauchy / Laplace(BF.matmul(W, x), sigma), W [1, F] mean-field Normal, sigma constant or a
               LogNormal latent
   BNNPlan     K3  observed Categorical with logits = BF.matmul(W2, BF.tanh(BF.matmul(W1, x) + b1)) + b2
+  ParticlePlan / WvgdPlan  K4 / K6  particle ensembles (SVGD, MAP, WVGD) of the K2 graph, or of the K2g graph at a constant
+              noise scale
 Unrecognised graphs raise `UnsupportedModelError` -- there is no eager / CPU fallback for the ELBO.
 """
 import contextlib
@@ -99,6 +101,8 @@ class MeanFieldSpec:
 
     def __init__(self, name, q_var, p_var, q_names):
         self.name = name
+        if not isinstance(q_var, RandomVariable):          # MAP's point estimate reaches here when its particle lowering fails
+            raise UnsupportedModelError("latent %r: q is a point estimate (a root), not a %s variable" % (name, self.kind_name))
         lq = q_var.partial_links
         if q_var.distribution.kind != self.kind or p_var.distribution.kind != self.kind:
             raise UnsupportedModelError("latent %r: only %s q / %s prior are lowered to the mean-field kernels"
@@ -302,13 +306,7 @@ class LinregPlan(Plan):
         self._prepared_x = None
 
     def noise_scale(self):
-        """the constant sigma as a 1-element device tensor, recomputed from its root at every evaluation (a constant root may be
-        re-assigned between evaluations; inside a captured graph this is one more captured kernel)"""
-        if isinstance(self._scale, float):
-            return torch.full((1,), self._scale, dtype=torch.float32, device=config.device)
-        root, sp = self._scale
-        v = root.value.detach().reshape(-1)[:1].to(device=config.device, dtype=torch.float32)
-        return (torch.nn.functional.softplus(v) if sp else v).contiguous()
+        return _noise_scale_tensor(self._scale)
 
     def _launch(self, cu, mvars, r, empirical, loss=None):
         X = _data_matrix(empirical[self.x_var], "x")
@@ -424,6 +422,35 @@ def _lower_dense(joint, posterior):
                                 "(linear K2, bnn K3); likelihood link: %s" % k.partial_links["logits"].string)
 
 
+REGRESSION_KINDS = {"normal": "Normal", "cauchy": "Cauchy", "laplace": "Laplace"}
+
+
+def _constant_scale(scale, what, k):
+    """The constant noise scale of likelihood node k: (root, softplus?) for a non-learnable scalar root (an auto-named root sits
+    behind a softplus), a float for a number, None for anything else.  Shared by the mean-field and the particle regressions."""
+    root, sp = _softplus_root(scale), True
+    if root is None:
+        root, sp = _as_root(scale), False
+    if root is not None and not root.is_observed:
+        if getattr(root, "learnable", False):
+            raise UnsupportedModelError("%s %r: a learnable point-estimate noise scale (root %r) is not "
+                                        "lowered" % (what, k.name, root.name))
+        if root._value.numel() != 1:
+            raise UnsupportedModelError("%s %r: the noise scale must be a scalar" % (what, k.name))
+        return (root, sp)
+    return _const_value(scale)
+
+
+def _noise_scale_tensor(scale):
+    """a constant scale of _constant_scale as a 1-element device tensor, recomputed from its root at every evaluation (a constant
+    root may be re-assigned between evaluations; inside a captured graph this is one more captured kernel)"""
+    if isinstance(scale, float):
+        return torch.full((1,), scale, dtype=torch.float32, device=config.device)
+    root, sp = scale
+    v = root.value.detach().reshape(-1)[:1].to(device=config.device, dtype=torch.float32)
+    return (torch.nn.functional.softplus(v) if sp else v).contiguous()
+
+
 def _lower_linreg(joint, posterior, k, latents, q_by_name, q_names):
     """K2g: observed Normal / Cauchy / Laplace(loc = matmul(W, x), scale) with W the [1, F] mean-field Normal weights and x
     data; scale a non-learnable constant (a root, behind softplus when auto-named, or a number) or a scalar LogNormal latent."""
@@ -455,19 +482,8 @@ def _lower_linreg(joint, posterior, k, latents, q_by_name, q_names):
                                         "latent or a constant is)" % (what, k.name, nu.distribution.kind))
         nu_spec = LogNormalSpec(nu.name, q_by_name[nu.name], nu, q_names)
     else:
-        root, sp = _softplus_root(scale), True
-        if root is None:
-            root, sp = _as_root(scale), False
-        if root is not None and not root.is_observed:
-            if getattr(root, "learnable", False):
-                raise UnsupportedModelError("%s %r: a learnable point-estimate noise scale (root %r) is not "
-                                            "lowered" % (what, k.name, root.name))
-            if root._value.numel() != 1:
-                raise UnsupportedModelError("%s %r: the noise scale must be a scalar" % (what, k.name))
-            const = (root, sp)
-        elif _const_value(scale) is not None:
-            const = _const_value(scale)
-        else:
+        const = _constant_scale(scale, what, k)
+        if const is None:
             raise UnsupportedModelError("%s %r: the noise scale must be a constant or a scalar LogNormal latent "
                                         "(deterministic or data-dependent scales are not lowered)" % (what, k.name))
     extra = [v.name for v in latents if v is not W and v is not nu]
@@ -1123,11 +1139,19 @@ class _ParticleLoss(torch.autograd.Function):
 class ParticlePlan:
     """SVGD over (multi-class) logistic-regression particles: the joint model is the linear family (K2's graph), every
     particle is a ProbabilisticModel holding ONE learnable RootVariable named like the weights latent
-    (development_playgrounds/SVGD_logistic_regression.py:34-48)."""
+    (development_playgrounds/SVGD_logistic_regression.py:34-48).  The same holds for regression particles: the joint model is
+    Normal / Cauchy / Laplace(BF.matmul(weights, x), constant scale) (likelihood cu.GAUSSIAN / CAUCHY / LAPLACE, C = 1)."""
     family = "particles (K4)"
 
-    def __init__(self, joint, particles, k, W, x_var, likelihood, C):
+    def __init__(self, joint, particles, k, W, x_var, likelihood, C, scale=None):
+        """scale: the constant noise scale of a regression likelihood (_constant_scale), None for the logistic ones"""
+        from brancher_b200 import _cuda as cu
         self.joint, self.particles, self.k, self.x_var, self.likelihood, self.C = joint, particles, k, x_var, likelihood, C
+        self.regression = likelihood in (cu.GAUSSIAN, cu.CAUCHY, cu.LAPLACE)
+        if self.regression:
+            self.family = "particles (K4, %s likelihood)" % {cu.GAUSSIAN: "Normal", cu.CAUCHY: "Cauchy", cu.LAPLACE: "Laplace"}[likelihood]
+        self._scale = scale
+        self.prepared_x = None       # fp16-pair form of a fixed observed matrix (regression), rebuilt when the matrix changes
         self.W = W
         lp = W.partial_links
         loc, sc_sp = _as_root(lp["loc"].expr), _softplus_root(lp["scale"].expr)
@@ -1151,6 +1175,18 @@ class ParticlePlan:
     def stacked(self):
         return torch.stack([p.detach().reshape(-1) for p in self.parameters()]).contiguous()
 
+    def noise_scale(self):
+        return _noise_scale_tensor(self._scale)
+
+    def observations(self, cu, empirical):
+        """(X [N, F], y [N]) of one evaluation, y in the dtype the likelihood's kernels read"""
+        X = _data_matrix(empirical[self.x_var], "x")
+        yv = empirical[self.k].reshape(-1)
+        y = yv.to(torch.int32).contiguous() if self.likelihood == cu.CATEGORICAL else yv.to(torch.float32).contiguous()
+        if self.regression and self.prepared_x is None:
+            self.prepared_x = cu.PreparedX()
+        return X, y
+
     def loss(self, empirical):
         if config.device.type != "cuda":
             raise RuntimeError("brancher_b200 evaluates particle losses only on CUDA devices (no CPU fallback)")
@@ -1158,18 +1194,60 @@ class ParticlePlan:
         cu.lib()
 
         def runner():
-            X = _data_matrix(empirical[self.x_var], "x")
-            yv = empirical[self.k].reshape(-1)
-            y = yv.to(torch.float32).contiguous() if self.likelihood == cu.BERNOULLI else yv.to(torch.int32).contiguous()
+            X, y = self.observations(cu, empirical)
+            if self.regression:
+                return cu.linreg_particles_loss_grad(X, y, self.likelihood, self.stacked(), self.noise_scale(), self.prior_loc,
+                                                     self.prior_scale, prepared=self.prepared_x)
             return cu.linear_particles_loss_grad(X, y, self.likelihood, self.stacked(), self.C, self.prior_loc, self.prior_scale)
 
         return _ParticleLoss.apply(runner, *self.parameters())
+
+
+def _lower_regression_particles(joint, particles, k, latents):
+    """Particles of Normal / Cauchy / Laplace(loc = BF.matmul(W, x), scale): W the one latent, [1, F] with a Normal prior, x data,
+    the scale a constant (a particle holds one root: there is no noise latent to carry)."""
+    from brancher_b200 import _cuda as cu
+    lik_name = REGRESSION_KINDS[k.distribution.kind]
+    what = "particle family: %s likelihood" % lik_name
+    loc, scale = k.partial_links["loc"].expr, k.partial_links["scale"].expr
+    if not _is_call(loc, "matmul", 2):
+        if any(_is_call(a, "matmul", 2) for a, _ in _commutative_add(loc)):
+            raise UnsupportedModelError("%s %r: a bias added to BF.matmul(weights, x) is not lowered -- append a column of ones "
+                                        "to x instead" % (what, k.name))
+        raise UnsupportedModelError("%s %r: loc must be BF.matmul(weights, x)" % (what, k.name))
+    W, x = _var(loc.args[0]), _var(loc.args[1])
+    if W not in latents or not _is_data(x):
+        raise UnsupportedModelError("%s %r: loc must be BF.matmul(weights, x) with weights a latent and x data" % (what, k.name))
+    nu = _var(scale)
+    if nu is not None and nu in latents:
+        raise UnsupportedModelError("%s %r: a %s-distributed noise latent is not lowered -- a particle holds one root, the "
+                                    "weights; give the noise scale as a constant" % (what, k.name, nu.distribution.kind))
+    const = _constant_scale(scale, what, k)
+    if const is None:
+        raise UnsupportedModelError("%s %r: the noise scale must be a constant (deterministic or data-dependent scales are not "
+                                    "lowered)" % (what, k.name))
+    extra = sorted(v.name for v in latents if v is not W)
+    if extra:
+        raise UnsupportedModelError("%s %r: latent variables other than the weights are not lowered: %s" % (what, k.name, extra))
+    if W.distribution.kind != "normal":
+        raise UnsupportedModelError("%s %r: only a Normal prior on the weights is lowered (got %s)" % (what, k.name,
+                                                                                                      W.distribution.kind))
+    shape = tuple(W.partial_links["loc"].expr.var._value.shape[2:]) if _as_root(W.partial_links["loc"].expr) else ()
+    if len(shape) != 2 or shape[0] != 1:
+        raise UnsupportedModelError("%s %r: weights must have shape [1, F] (multi-output regression is not lowered), got %s"
+                                    % (what, k.name, shape))
+    if shape[1] > 128:
+        raise UnsupportedModelError("%s %r: at most 128 features are lowered, got F = %d" % (what, k.name, shape[1]))
+    likelihood = {"normal": cu.GAUSSIAN, "cauchy": cu.CAUCHY, "laplace": cu.LAPLACE}[k.distribution.kind]
+    return ParticlePlan(joint, particles, k, W, x, likelihood, 1, scale=const)
 
 
 def lower_particles(joint, particles):
     from brancher_b200 import _cuda as cu
     latents = _latent_random_variables(joint)
     liks = _observed_likelihood_nodes(joint)
+    if len(liks) == 1 and liks[0].distribution.kind in REGRESSION_KINDS:
+        return _lower_regression_particles(joint, particles, liks[0], latents)
     if len(liks) != 1 or len(latents) != 1:
         raise UnsupportedModelError("particle family needs one observed likelihood node and one latent weight matrix")
     k, W = liks[0], latents[0]
@@ -1208,7 +1286,7 @@ class _WvgdLoss(torch.autograd.Function):
 
 
 class WvgdPlan:
-    """WVGD over (multi-class) logistic-regression ensembles (development_playgrounds/WVGD_logistic_regression.py:33-58): the
+    """WVGD over (multi-class) logistic-regression or regression ensembles (development_playgrounds/WVGD_logistic_regression.py:33-58): the
     joint model is the linear family, particle k holds one learnable root named like the weights latent, sampler k one
     learnable Normal of the same name whose loc/scale are roots (scale a scalar or a full tensor)."""
     family = "wvgd (K6)"
@@ -1257,9 +1335,7 @@ class WvgdPlan:
         r = cu.sample_range(number_samples, seed=config.seed, offset=config.next_offset())
 
         def runner():
-            X = _data_matrix(empirical[pp.x_var], "x")
-            yv = empirical[pp.k].reshape(-1)
-            y = yv.to(torch.float32).contiguous() if pp.likelihood == cu.BERNOULLI else yv.to(torch.int32).contiguous()
+            X, y = pp.observations(cu, empirical)
             theta = pp.stacked()
             loc = torch.stack([p.value.detach().reshape(-1) for p in self.loc_roots]).contiguous()
             scalar = self.scale_roots[0]._value.numel() == 1
@@ -1271,7 +1347,9 @@ class WvgdPlan:
                 eps0, eps1 = cv(_INJECTED["elbo"]), cv(_INJECTED["particle"])
             prior = None if self.tied else (pp.prior_loc, pp.prior_scale)
             loss, dloc, drho, dth, counts = cu.wvgd_loss_grad(X, y, pp.likelihood, pp.C, loc, rho, theta, number_samples, r, eps0, eps1,
-                                                              prior=prior, biased=biased, first_column_only=first_column_only)
+                                                              prior=prior, biased=biased, first_column_only=first_column_only,
+                                                              noise_scale=pp.noise_scale() if pp.regression else None,
+                                                              prepared=pp.prepared_x)
             self.accepted = counts
             drho = drho.sum(1, keepdim=True) if scalar else drho
             grads = [dth[i].reshape(params[i].shape) for i in range(n)]
@@ -1294,9 +1372,8 @@ def _wvgd_ensemble_weights(self, empirical, number_post_samples, first_column_on
     pp = self.pplan
     n = len(pp.roots)
     dev = config.device
-    X = _data_matrix(empirical[pp.x_var], "x")
-    yv = empirical[pp.k].reshape(-1)
-    y = yv.to(torch.float32).contiguous() if pp.likelihood == cu.BERNOULLI else yv.to(torch.int32).contiguous()
+    X, y = pp.observations(cu, empirical)
+    sigma = pp.noise_scale() if pp.regression else None
     theta = pp.stacked()
     loc = torch.stack([p.value.detach().reshape(-1) for p in self.loc_roots]).contiguous()
     scalar = self.scale_roots[0]._value.numel() == 1
@@ -1320,7 +1397,10 @@ def _wvgd_ensemble_weights(self, empirical, number_post_samples, first_column_on
         eps = None if injected is None else injected[:, done:done + S].contiguous()
         r = cu.sample_range(S, seed=config.seed, offset=config.next_offset())
         Z, e, owner = cu.wvgd_sample_assign(loc, rho, theta, S, F_last, r, 0, eps, first_column_only)
-        ll, _ = cu.linear_vectors_loglik_grad(X, y, pp.likelihood, Z.reshape(n * S, d), pp.C, False)
+        if pp.regression:
+            ll, _ = cu.linreg_vectors_loglik_grad(X, y, pp.likelihood, Z.reshape(n * S, d), sigma, False, pp.prepared_x)
+        else:
+            ll, _ = cu.linear_vectors_loglik_grad(X, y, pp.likelihood, Z.reshape(n * S, d), pp.C, False)
         logw = ll.reshape(n, S)
         if not self.tied:          # tied: the prior's roots take sampler k's values, log p(z) == log q_k(z) and the pair cancels
             c = 0.5 * float(np.log(2 * np.pi))

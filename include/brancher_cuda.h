@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define BRN_ABI_VERSION 4
+#define BRN_ABI_VERSION 5
 
 /* One mean-field Normal variational variable  q(w) = N(mu, softplus(rho))  together with the Normal
  * prior p(w) = N(prior_loc, prior_scale) of the same name.
@@ -192,6 +192,29 @@ int brn_linreg_elbo_fwd_bwd_lik(const float* X, const void* px, const float* y, 
                                 const brn_sample_range* r, void* workspace, size_t workspace_bytes, int with_prior,
                                 double* loss, void* stream);
 
+/* K4a / K6b for regression: n weight vectors theta_k (or V_k) [n, F] at a FIXED noise scale, with ll_k the log-likelihood of
+ * BRN_LINREG_NORMAL / _CAUCHY / _LAPLACE above (torch's log_prob summed over the N rows) at w_s = theta_k, sigma_s = *noise_scale.
+ * The X pass is K2g's (the one-pass tensor-core kernel where the K2g evaluation of the same shape takes it, else the SIMT kernel)
+ * with the vectors in place of the MC samples; a per-vector finisher replaces the mean-field one.  noise_scale: a DEVICE fp32
+ * scalar, as for brn_linreg_elbo_fwd_bwd_lik; px: the prepared X of brn_linear_prepare_x, or NULL.  F <= 128; n == 0 and N == 0
+ * are valid (N == 0: ll = 0).  workspace: brn_linreg_vectors_workspace_bytes() bytes of scratch.
+ *   brn_linreg_particles_loss_grad:  loss += sum_k [ -ll_k - sum log N(theta_k; prior_loc, prior_scale) ]  (prior optional; a SUM
+ *                                    over the particles, as brn_linear_particles_loss_grad), G = d loss / d theta (overwritten).
+ *                                    Replaces SteinVariationalGradientDescent.compute_loss + loss.backward() (inference.py:292-299,
+ *                                    100) and MAP's -log p(data, theta) + backward (inference.py:251-274) for
+ *                                    Normal / Cauchy / LaplaceVariable(BF.matmul(weights, x), scale, "y").
+ *   brn_linreg_vectors_loglik_grad:  ll[k] = ll_k (overwritten, fp64), G = -d ll_k / d V_k (overwritten) or G == NULL.
+ *                                    Replaces the per-draw log-likelihoods of WassersteinVariationalGradientDescent.compute_loss
+ *                                    (inference.py:203-229) for the same models; the rest of K6 is unchanged. */
+size_t brn_linreg_vectors_workspace_bytes(int64_t N, int F, int n);
+int brn_linreg_particles_loss_grad(const float* X, const void* px, const float* y, int likelihood, int64_t N, int F,
+                                   const float* theta, int n, const float* prior_loc, const float* prior_scale,
+                                   const float* noise_scale, float* G, double* loss,
+                                   void* workspace, size_t workspace_bytes, void* stream);
+int brn_linreg_vectors_loglik_grad(const float* X, const void* px, const float* y, int likelihood, int64_t N, int F,
+                                   const float* V, int n, const float* noise_scale, float* G, double* ll,
+                                   void* workspace, size_t workspace_bytes, void* stream);
+
 /* K1 -- generic scalar-DAG ELBO: fused reparameterised sampling + log-probs + reduction over samples and data rows +
  * backward, for models whose variables are scalars (README.md:22-75 AR(1); examples/logNormal_normal.py;
  * examples/multivariate_regression.py).  The host flattens (joint, posterior) into a straight-line SSA program;
@@ -336,7 +359,8 @@ int brn_vae_elbo_fwd_bwd(const float* X, int B, int64_t row0, int64_t B_total, c
  *     the reference's numpy cost (utilities.py:125-126: only index 0 of the last axis, F_last elements apart, enters
  *     the squared distance); 0 = full squared distance.
  * (b) brn_linear_vectors_loglik_grad: ll[i] = sum_rows log-lik(data | weights = V[i]) and G[i] = -d ll[i] / d V[i] for
- *     n = P*S weight vectors in one fused pass over X (same kernel as K4a; G may be NULL).
+ *     n = P*S weight vectors in one fused pass over X (same kernel as K4a; G may be NULL).  Regression models (Normal / Cauchy /
+ *     Laplace likelihood at a fixed noise scale) use brn_linreg_vectors_loglik_grad here instead.
  * (c) brn_wvgd_reduce: per sampler k, over its accepted samples A_k (draw 0) and A'_k (draw 1):
  *       loss += -mean_{A_k}[ll + log prior(z)]  +  sum_{A'_k} w_s ||theta_k - z'_s||^2
  *       w = softmax_{A'_k}(ll' + log prior(z') - log q_k(z'))   (1/S if biased)         (variables.py:821-841)
