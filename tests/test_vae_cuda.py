@@ -21,11 +21,11 @@ def dev(a):
     return torch.as_tensor(np.asarray(a), dtype=torch.float32).to(DEV).contiguous()
 
 
-def make_net(cu, enc, dec):
+def make_net(cu, enc, dec, sd_offset=0.1):
     pair = lambda W, b: (dev(W), dev(b))
     return cu.VaeNet([pair(W, b) for W, b in zip(enc["W"], enc["b"])], pair(enc["W_mean"], enc["b_mean"]),
                      pair(enc["W_sd"], enc["b_sd"]), [pair(W, b) for W, b in zip(dec["W"], dec["b"])],
-                     pair(dec["W_out"], dec["b_out"]))
+                     pair(dec["W_out"], dec["b_out"]), sd_offset=sd_offset)
 
 
 def grads_of(net):
