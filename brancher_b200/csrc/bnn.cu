@@ -488,8 +488,6 @@ extern "C" int brn_bnn_elbo_fwd_bwd_act(const float* X, const int32_t* y, int B,
     // variant: tcgen05 (TMA + 3xFP16 tensor-core GEMMs) when the padded hidden width matches the instantiated
     // tile, else the fp32 SIMT GEMMs.  BRN_BNN_VARIANT=simt|tcgen05 forces one (tests compare both).
     const char* env_variant = getenv("BRN_BNN_VARIANT");
-    const char* env_drain = getenv("BRN_UMMA_DRAIN");
-    const char* env_mid = getenv("BRN_BNN_MID");
     bool use_tc = (H > BNN_UMMA_HP - 16 && H <= BNN_UMMA_HP);
     if (env_variant) {
         if (!strcmp(env_variant, "simt")) use_tc = false;
@@ -499,18 +497,7 @@ extern "C" int brn_bnn_elbo_fwd_bwd_act(const float* X, const int32_t* y, int B,
         }
     }
     set_variant(use_tc ? "tcgen05" : "simt");
-    if (use_tc) {
-        // TMEM accumulation chain = 2 x 32 words = 128 fp16 elements of K between register drains (umma_gemm.cuh): the error
-        // of the evaluation grows with the chain (max gradient error / scale at the C3 shape: 0.9e-6 / 1.1e-6 / 1.3e-6 /
-        // 2.3e-6 for 1 / 2 / 4 / 8, profiles/tools/bnn_err_probe.py) -- 128 elements is the chain length round 1 settled on.
-        // The backward GEMM's accumulator is the per-sample weight gradient, summed over 256 samples afterwards: its chain
-        // may be twice as long (measured: no change of the parity margins, 8 us per evaluation).
-        const int drain = env_drain ? atoi(env_drain) : 2, drain_bwd = env_drain ? atoi(env_drain) : 4;
-        // BRN_BNN_MID=5 selects the fully fused pipeline (mid stage in the forward GEMM's epilogue, sample-axis reduction
-        // in the backward GEMM's); measured slower than the staged one on B200 (profiles/r2*), kept for A/B and tests
-        const bool fused = env_mid && atoi(env_mid) == 5;
-        return bnn_tc_eval(X, y, L, vars, r, ws.tc, ws.eps, ws.W, ws.dW, ws.pre, ws.stats, with_prior, loss, drain, drain_bwd, fused, stream);
-    }
+    if (use_tc) return bnn_tc_eval(X, y, L, vars, r, ws.tc, ws.eps, ws.W, ws.dW, ws.pre, ws.stats, with_prior, loss, stream);
 
     // ---- SIMT variant
     // 1. noise + weights: noise in ws.eps [S][ldw], sampled weights in ws.W, the four variables back to back inside a row
@@ -588,7 +575,7 @@ extern "C" int brn_bnn_predict(const float* X, int B, int P, int H, int C, int a
     }
     set_variant(use_tc ? "tcgen05" : "simt");
     if (use_tc) {
-        if (int e = bnn_tc_eval(X, nullptr, L, vars, r, ws.tc, ws.eps, ws.W, ws.dW, ws.pre, ws.stats, 0, nullptr, 2, 4, false, stream, true))
+        if (int e = bnn_tc_eval(X, nullptr, L, vars, r, ws.tc, ws.eps, ws.W, ws.dW, ws.pre, ws.stats, 0, nullptr, stream, true))
             return e;
     } else {
         if (int e = launch_sample_multi(vars, offs, 4, ws.eps, ws.W, L.ldw, *r, stream)) return e;

@@ -464,555 +464,10 @@ static int launch_mid4(const float* pre, const float* W, float* dW, const int32_
     return 0;
 }
 
-
-// K3, fused forward: layer-1 GEMM on tcgen05 with the whole "mid" stage in its epilogue.
-//
-//   pre_s[b, h] = sum_p X[b, p] W1_s[h, p]          tcgen05 3xTF32, accumulators in TMEM (M = 128 batch rows,
-//                                                   N = 2 samples x 104 hidden units, K = P)
-//   epilogue (never leaves the SM):  h = tanh(pre + b1_s), a = W2_s h + b2_s, log-softmax, ll, da,
-//                                    dW2_s / db2_s / db1_s, dpre = (W2_s^T da)(1 - h^2)
-//   out: dpre^T (TF32-split, K-major B operand of the weight-gradient GEMM), the small per-sample gradients, the loss.
-//
-// The pre-activations (105 MB at the C3 shape) used to cross HBM twice between the GEMM and a separate mid kernel
-// (137 us, latency-bound).  Here the accumulator is read from TMEM with the 16x256b shape, which delivers each warp's
-// 32 rows as two m16 tiles in exactly the mma.sync accumulator-fragment layout (thread (g, t): rows g / g+8, columns
-// 2t / 2t+1 of every 8-column group).  The three small layer-2 contractions then run on the warp-level tensor cores
-// (mma.sync m16n8k8 tf32, 3xTF32 split) chained fragment-to-fragment:
-//   A  a[b, c]   = sum_h h[b, h] W2[c, h]     the C fragment of pre IS the A fragment after permuting the contraction
-//                                             index (k columns (t, t+4) <-> hidden (2t, 2t+1)); B fragments from smem
-//   B  dh[b, h]  = sum_c da[b, c] W2[c, h]    same trick on the class index
-//   C  dW2[c, h] = sum_b da[b, c] h[b, h]     contraction over rows: both operands transposed inside the warp with
-//                                             shuffles (2 per element), K = the warp's 32 rows, RED into dW2_s
-// Everything is per warp except the per-sample weights (W2_s, b1_s, b2_s), which the four warps of a sample stage in
-// shared memory once per unit (two 128-thread named barriers per unit).
-// ---- TMEM -> registers, 16 lanes x (8 columns x NUM): regs [4n .. 4n+3] = C fragment of column group n
-#define BRN_R4(a, i) "=r"(a[i]), "=r"(a[i + 1]), "=r"(a[i + 2]), "=r"(a[i + 3])
-__device__ __forceinline__ void tmem_ld_16x256b_x8(uint32_t taddr, float* v) {
-    uint32_t* r = reinterpret_cast<uint32_t*>(v);
-    asm volatile(
-        "tcgen05.ld.sync.aligned.16x256b.x8.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : BRN_R4(r, 0), BRN_R4(r, 4), BRN_R4(r, 8), BRN_R4(r, 12), BRN_R4(r, 16), BRN_R4(r, 20), BRN_R4(r, 24), BRN_R4(r, 28)
-        : "r"(taddr)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_ld_16x256b_x4(uint32_t taddr, float* v) {
-    uint32_t* r = reinterpret_cast<uint32_t*>(v);
-    asm volatile(
-        "tcgen05.ld.sync.aligned.16x256b.x4.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : BRN_R4(r, 0), BRN_R4(r, 4), BRN_R4(r, 8), BRN_R4(r, 12)
-        : "r"(taddr)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_ld_16x256b_x1(uint32_t taddr, float* v) {
-    uint32_t* r = reinterpret_cast<uint32_t*>(v);
-    asm volatile("tcgen05.ld.sync.aligned.16x256b.x1.b32 {%0, %1, %2, %3}, [%4];" : BRN_R4(r, 0) : "r"(taddr) : "memory");
-}
-#undef BRN_R4
-
-__device__ __forceinline__ void named_bar_sync(int id, int threads) {
-    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory");
-}
-__device__ __forceinline__ void red_add_v2(float* p, float a, float b) {
-    asm volatile("red.global.add.v2.f32 [%0], {%1, %2};" ::"l"(p), "f"(a), "f"(b) : "memory");
-}
-__device__ __forceinline__ void red_add_v4(float* p, float a, float b, float c, float d) {
-    asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
-}
-
-constexpr int FM_W2_PITCH = 104;      // == 8 (mod 32): the 64-bit B-fragment loads of phase A are conflict-free
-constexpr int FM_W2_ROWS = 16;
-
-template <int HP, int BK>
-struct FwdMidSmem {
-    using Ring = UmmaSmem<2 * HP, BK>;
-    static constexpr int W2_FLOATS = FM_W2_ROWS * FM_W2_PITCH;
-    static constexpr int SAMPLE_FLOATS = W2_FLOATS + HP + 16;          // W2 [16][104], b1 [HP], b2 [16]
-    static constexpr int EXTRA_BYTES = 2 * SAMPLE_FLOATS * 4;
-    static constexpr int TOTAL = Ring::STAGES * Ring::STAGE_BYTES + 1024 + EXTRA_BYTES;
-    static_assert(HP <= FM_W2_PITCH, "hidden width exceeds the staged W2 pitch");
-    static_assert(TOTAL <= 227 * 1024, "shared memory budget exceeded");
-};
-
-struct FwdMidParams {
-    const float* W;        // sampled small variables [S][ldw] (b1, W2, b2 at L.ob1 / L.oW2 / L.ob2)
-    float* dW;             // per-sample gradient slots [S][ldw] (b1 / W2 / b2 slots pre-zeroed, accumulated with RED)
-    const int32_t* y;
-    BnnLayout L;
-    int S;
-    float inv_S;
-    double* loss;
-    __half* dpT_hi; __half* dpT_lo; int64_t ldB;    // [(S + pad) * HP][ldB], scaled by dpre_scale
-    const float* scal;                              // operand bounds (see the top of this file)
-};
-
-// 12 warps = 3 warpgroups: WG0 = {TMA producer, MMA issuer, 2 idle warps} gives registers back (setmaxnreg.dec 40), the 8
-// epilogue warps of WG1 / WG2 take them (setmaxnreg.inc 232): each SM sub-partition hosts one warp of every warpgroup,
-// 32 x (40 + 2 x 232) = 16128 <= 16384 registers.  (With 10 warps a sub-partition hosts three and the cap is 168.)
-constexpr int FM_THREADS = 384, FM_EPI_WARP0 = 4;
-__device__ __forceinline__ void setmaxnreg_dec40() { asm volatile("setmaxnreg.dec.sync.aligned.u32 40;"); }
-__device__ __forceinline__ void setmaxnreg_inc232() { asm volatile("setmaxnreg.inc.sync.aligned.u32 232;"); }
-
-template <int HP, int BK>
-__global__ void __launch_bounds__(FM_THREADS, 1)
-bnn_fwd_mid_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUtensorMap tmAl,
-                   const __grid_constant__ CUtensorMap tmBh, const __grid_constant__ CUtensorMap tmBl,
-                   int m_tiles, int n_tiles, int k_chunks, int drain_chunks, FwdMidParams p) {
-    constexpr int BN = 2 * HP, EW = 8, KS = HP / 8;
-    using SM = UmmaSmem<BN, BK>;
-    using FS = FwdMidSmem<HP, BK>;
-    constexpr int UG_STAGES = SM::STAGES, SW = BK * 4;
-    static_assert(HP % 8 == 0 && KS == 13, "the TMEM drain below is written for HP = 104 (x8 + x4 + x1 column groups)");
-    constexpr uint32_t TMEM_COLS = 512;
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    float* extra = reinterpret_cast<float*>(smem + UG_STAGES * SM::STAGE_BYTES);
-    __shared__ __align__(8) uint64_t full_bar[UG_STAGES], empty_bar[UG_STAGES], acc_full[2], acc_empty[2];
-    __shared__ uint32_t tmem_base_slot;
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-    if (warp == 0 && lane == 0) {
-        umma::tma_prefetch_desc(&tmAh); umma::tma_prefetch_desc(&tmAl);
-        umma::tma_prefetch_desc(&tmBh); umma::tma_prefetch_desc(&tmBl);
-        for (int s = 0; s < UG_STAGES; ++s) { umma::mbar_init(&full_bar[s], 1); umma::mbar_init(&empty_bar[s], 1); }
-        for (int b = 0; b < 2; ++b) { umma::mbar_init(&acc_full[b], 1); umma::mbar_init(&acc_empty[b], EW); }
-        umma::fence_barrier_init();
-    }
-    if (warp == 1) umma::tmem_alloc(&tmem_base_slot, TMEM_COLS);
-    // zero the staged-weight region once: pad classes / pad hidden units stay zero for the whole kernel
-    for (int i = threadIdx.x; i < 2 * FS::SAMPLE_FLOATS; i += blockDim.x) extra[i] = 0.f;
-    umma::tc_fence_before();
-    __syncthreads();
-    umma::tc_fence_after();
-    const uint32_t tmem_base = tmem_base_slot;
-
-    if (warp < FM_EPI_WARP0) {
-    setmaxnreg_dec40();
-    if (warp == 0) {
-        // ===================== TMA producer =====================
-        if (umma::elect_one()) {
-            int stage = 0; uint32_t phase = 0;
-            for (UnitIter it(m_tiles, n_tiles, k_chunks, 0, 0, m_tiles * n_tiles); it.valid(); it.next()) {
-                const int m0 = it.mt() * UG_BM, n0 = it.nt() * BN;
-                for (int kc = 0; kc < k_chunks; ++kc) {
-                    umma::mbar_wait(&empty_bar[stage], phase ^ 1);
-                    uint8_t* st = smem + stage * SM::STAGE_BYTES;
-                    umma::mbar_arrive_expect_tx(&full_bar[stage], SM::STAGE_BYTES);
-                    const int k0 = kc * BK * 2;          // fp16 elements
-                    umma::tma_load_2d(st, &tmAh, &full_bar[stage], k0, m0);
-                    umma::tma_load_2d(st + SM::A_BYTES, &tmAl, &full_bar[stage], k0, m0);
-                    umma::tma_load_2d(st + 2 * SM::A_BYTES, &tmBh, &full_bar[stage], k0, n0);
-                    umma::tma_load_2d(st + 2 * SM::A_BYTES + SM::B_BYTES, &tmBl, &full_bar[stage], k0, n0);
-                    if (++stage == UG_STAGES) { stage = 0; phase ^= 1; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ===================== MMA issuer =====================
-        if (umma::elect_one()) {      // not `lane == 0`: ptxas then issues each UTCHMMA once instead of inside an ELECT loop
-            constexpr uint32_t idesc = umma::idesc_f16(UG_BM, BN);
-            int stage = 0; uint32_t phase = 0, blk = 0;
-            for (UnitIter it(m_tiles, n_tiles, k_chunks, 0, 0, m_tiles * n_tiles); it.valid(); it.next()) {
-                for (int kc0 = 0; kc0 < k_chunks; kc0 += drain_chunks, ++blk) {
-                    const uint32_t buf = blk & 1, use = (blk >> 1) & 1;
-                    umma::mbar_wait(&acc_empty[buf], use ^ 1);
-                    umma::tc_fence_after();
-                    const uint32_t d_tmem = tmem_base + buf * UG_BUF_COLS;
-                    const int kc1 = min(kc0 + drain_chunks, k_chunks);
-                    for (int kc = kc0; kc < kc1; ++kc) {
-                        umma::mbar_wait(&full_bar[stage], phase);
-                        umma::tc_fence_after();
-                        const uint32_t st = umma::smem_u32(smem + stage * SM::STAGE_BYTES);
-                        const uint32_t ah = st, al = st + SM::A_BYTES, bh = st + 2 * SM::A_BYTES, bl = bh + SM::B_BYTES;
-#pragma unroll
-                        for (int ks = 0; ks < BK / 8; ++ks) {
-                            const uint32_t ko = ks * 32;
-                            const uint64_t dah = umma::smem_desc_k<SW>(ah + ko), dal = umma::smem_desc_k<SW>(al + ko);
-                            const uint64_t dbh = umma::smem_desc_k<SW>(bh + ko), dbl = umma::smem_desc_k<SW>(bl + ko);
-                            umma::mma_f16_ss(d_tmem, dal, dbh, idesc, kc != kc0 || ks != 0);
-                            umma::mma_f16_ss(d_tmem, dah, dbl, idesc, true);
-                            umma::mma_f16_ss(d_tmem, dah, dbh, idesc, true);
-                        }
-                        umma::mma_commit(&empty_bar[stage]);
-                        if (++stage == UG_STAGES) { stage = 0; phase ^= 1; }
-                    }
-                    umma::mma_commit(&acc_full[buf]);
-                }
-            }
-        }
-    }
-    } else {
-        // ===================== epilogue warps: drain + mid =====================
-        setmaxnreg_inc232();
-        const int ew = warp - FM_EPI_WARP0;
-        const int q = warp & 3;                   // TMEM lane quarter this warp may access (warp id % 4)
-        const int hf = ew >> 2;                   // sample of the pair (column half of the tile)
-        const int g = lane >> 2, t = lane & 3;
-        const int gt = (ew & 3) * 32 + lane;      // thread index inside the sample's 4-warp group
-        const int H = p.L.H, C = p.L.C, B = p.L.B, act = p.L.act;
-        float* W2s = extra + hf * FS::SAMPLE_FLOATS;
-        float* b1s = W2s + FS::W2_FLOATS;
-        float* b2s = b1s + HP;
-        const bool two_q = C > 8;                 // classes 8..15 present
-        const float inv_pre = 1.f / (x_scale(p.scal) * w1_scale(p.scal)), sD = dpre_scale(p.scal);
-        uint32_t blk = 0;
-        for (UnitIter it(m_tiles, n_tiles, k_chunks, 0, 0, m_tiles * n_tiles); it.valid(); it.next()) {
-            const int s = it.nt() * 2 + hf;
-            const bool s_ok = s < p.S;
-            const int b0 = it.mt() * UG_BM;
-            // ---- stage this sample's layer-2 weights (overlaps the MMAs of the unit)
-            named_bar_sync(1 + hf, 128);                                 // previous unit's readers are done
-            if (s_ok) {
-                const float* Ws = p.W + (int64_t)s * p.L.ldw;
-                for (int c = 0; c < C; ++c)
-                    for (int h = gt; h < H; h += 128) W2s[c * FM_W2_PITCH + h] = Ws[p.L.oW2 + (int64_t)c * H + h];
-                for (int h = gt; h < H; h += 128) b1s[h] = Ws[p.L.ob1 + h];
-                if (gt < C) b2s[gt] = Ws[p.L.ob2 + gt];
-            }
-            named_bar_sync(1 + hf, 128);
-
-            // ---- drain the accumulator blocks into registers (round-to-nearest adds, see umma_gemm.cuh)
-            float acc[2][KS][4];
-#pragma unroll
-            for (int m = 0; m < 2; ++m)
-#pragma unroll
-                for (int k = 0; k < KS; ++k)
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) acc[m][k][i] = 0.f;
-            for (int kc0 = 0; kc0 < k_chunks; kc0 += drain_chunks, ++blk) {
-                const uint32_t buf = blk & 1, use = (blk >> 1) & 1;
-                umma::mbar_wait(&acc_full[buf], use);
-                umma::tc_fence_after();
-#pragma unroll
-                for (int m = 0; m < 2; ++m) {
-                    const uint32_t t0 = tmem_base + ((uint32_t)(q * 32 + m * 16) << 16) + buf * UG_BUF_COLS + hf * HP;
-                    float v[4 * KS];
-                    tmem_ld_16x256b_x8(t0, v);
-                    tmem_ld_16x256b_x4(t0 + 64, v + 32);
-                    tmem_ld_16x256b_x1(t0 + 96, v + 48);
-                    umma::tmem_ld_wait();
-#pragma unroll
-                    for (int k = 0; k < KS; ++k)
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) acc[m][k][i] += v[4 * k + i];
-                }
-                umma::tc_fence_before();
-                __syncwarp();
-                if (lane == 0) umma::mbar_arrive(&acc_empty[buf]);
-            }
-            if (!s_ok) continue;                 // odd sample count: the pair's second half is padding (warp-uniform)
-
-            // rows of this thread: r[m][0] = 32q + 16m + g, r[m][1] = +8   (inside the 128-row tile)
-            const int rbase = q * 32 + g;
-            bool ok[2][2];
-#pragma unroll
-            for (int m = 0; m < 2; ++m) {
-                ok[m][0] = b0 + rbase + 16 * m < B;
-                ok[m][1] = b0 + rbase + 16 * m + 8 < B;
-            }
-
-            // ---- phase A: h = tanh(pre + b1) (kept in acc), a = h W2^T
-            float ahh[2][2][4], acr[2][2][4];
-#pragma unroll
-            for (int m = 0; m < 2; ++m)
-#pragma unroll
-                for (int qq = 0; qq < 2; ++qq)
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) ahh[m][qq][i] = acr[m][qq][i] = 0.f;
-#pragma unroll
-            for (int k = 0; k < KS; ++k) {
-                const int h0 = 8 * k + 2 * t;
-                const float2 bb = *reinterpret_cast<const float2*>(b1s + h0);
-                const bool v0 = h0 < H, v1 = h0 + 1 < H;       // pad hidden units: the accumulator columns are garbage
-                float bh[2][2], bl[2][2];
-#pragma unroll
-                for (int qq = 0; qq < 2; ++qq) {
-                    const float2 w = *reinterpret_cast<const float2*>(W2s + (8 * qq + g) * FM_W2_PITCH + h0);
-                    split_tf32_trunc_lo(w.x, bh[qq][0], bl[qq][0]);
-                    split_tf32_trunc_lo(w.y, bh[qq][1], bl[qq][1]);
-                }
-#pragma unroll
-                for (int m = 0; m < 2; ++m) {
-                    float* a = acc[m][k];
-                    a[0] = v0 ? act_fast(act, __fmaf_rn(a[0], inv_pre, bb.x)) : 0.f;      // (row g,   h0)
-                    a[1] = v1 ? act_fast(act, __fmaf_rn(a[1], inv_pre, bb.y)) : 0.f;      // (row g,   h0 + 1)
-                    a[2] = v0 ? act_fast(act, __fmaf_rn(a[2], inv_pre, bb.x)) : 0.f;      // (row g+8, h0)
-                    a[3] = v1 ? act_fast(act, __fmaf_rn(a[3], inv_pre, bb.y)) : 0.f;      // (row g+8, h0 + 1)
-                    // A fragment (k columns t, t+4 <-> hidden h0, h0+1): (g, h0), (g+8, h0), (g, h0+1), (g+8, h0+1)
-                    float hi[4], lo[4];
-                    split_tf32_trunc_lo(a[0], hi[0], lo[0]);
-                    split_tf32_trunc_lo(a[2], hi[1], lo[1]);
-                    split_tf32_trunc_lo(a[1], hi[2], lo[2]);
-                    split_tf32_trunc_lo(a[3], hi[3], lo[3]);
-                    mma_tf32(ahh[m][0], hi, bh[0][0], bh[0][1]);
-                    mma_tf32(acr[m][0], lo, bh[0][0], bh[0][1]);
-                    mma_tf32(acr[m][0], hi, bl[0][0], bl[0][1]);
-                    if (two_q) {
-                        mma_tf32(ahh[m][1], hi, bh[1][0], bh[1][1]);
-                        mma_tf32(acr[m][1], lo, bh[1][0], bh[1][1]);
-                        mma_tf32(acr[m][1], hi, bl[1][0], bl[1][1]);
-                    }
-                }
-            }
-
-            // ---- log-softmax: rows (g, g+8) of each m-tile, classes {2t, 2t+1, 8+2t, 9+2t}
-            float dahi[2][2][4], dalo[2][2][4];          // phase-B A fragments: (r0, 2t), (r1, 2t), (r0, 2t+1), (r1, 2t+1)
-            float ll = 0.f;
-#pragma unroll
-            for (int m = 0; m < 2; ++m) {
-                const int lab0 = ok[m][0] ? p.y[b0 + rbase + 16 * m] : -1, lab1 = ok[m][1] ? p.y[b0 + rbase + 16 * m + 8] : -1;
-                float a[2][4];
-                float m0 = -INFINITY, m1 = -INFINITY;
-#pragma unroll
-                for (int qq = 0; qq < 2; ++qq)
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const int c = 8 * qq + 2 * t + (i & 1);
-                        a[qq][i] = c < C ? ahh[m][qq][i] + acr[m][qq][i] + b2s[c] : -INFINITY;
-                        if (i < 2) m0 = fmaxf(m0, a[qq][i]);
-                        else m1 = fmaxf(m1, a[qq][i]);
-                    }
-                m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 1)); m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 2));
-                m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 1)); m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 2));
-                float ex[2][4];
-                float se0 = 0.f, se1 = 0.f;
-#pragma unroll
-                for (int qq = 0; qq < 2; ++qq)
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        ex[qq][i] = expf(a[qq][i] - (i < 2 ? m0 : m1));          // exp(-inf) = 0 for the pad classes
-                        if (i < 2) se0 += ex[qq][i];
-                        else se1 += ex[qq][i];
-                    }
-                se0 += __shfl_xor_sync(0xffffffffu, se0, 1); se0 += __shfl_xor_sync(0xffffffffu, se0, 2);
-                se1 += __shfl_xor_sync(0xffffffffu, se1, 1); se1 += __shfl_xor_sync(0xffffffffu, se1, 2);
-                const float lse0 = m0 + logf(se0), lse1 = m1 + logf(se1);
-                const float inv0 = 1.f / se0, inv1 = 1.f / se1;
-#pragma unroll
-                for (int qq = 0; qq < 2; ++qq) {
-                    float da[4];
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const int c = 8 * qq + 2 * t + (i & 1);
-                        const bool okc = (i < 2 ? ok[m][0] : ok[m][1]) && c < C;
-                        const int lab = i < 2 ? lab0 : lab1;
-                        const float lse = i < 2 ? lse0 : lse1;
-                        const float sm_ = ex[qq][i] * (i < 2 ? inv0 : inv1);
-                        da[i] = okc ? (c == lab ? 1.f : 0.f) - sm_ : 0.f;            // d ll / d a_c
-                        if (okc && c == lab) ll += a[qq][i] - lse;
-                    }
-                    split_tf32_trunc_lo(da[0], dahi[m][qq][0], dalo[m][qq][0]);
-                    split_tf32_trunc_lo(da[2], dahi[m][qq][1], dalo[m][qq][1]);
-                    split_tf32_trunc_lo(da[1], dahi[m][qq][2], dalo[m][qq][2]);
-                    split_tf32_trunc_lo(da[3], dahi[m][qq][3], dalo[m][qq][3]);
-                }
-            }
-
-            float* dWs = p.dW + (int64_t)s * p.L.ldw;
-            // ---- db2[c] = sum_rows da[row, c]: this thread holds classes 8qq + 2t (+1) of 4 rows
-            {
-#pragma unroll
-                for (int qq = 0; qq < 2; ++qq) {
-                    // fragment order: [0] = (r0, 2t), [1] = (r1, 2t), [2] = (r0, 2t+1), [3] = (r1, 2t+1); hi + lo == da exactly
-                    float c0 = 0.f, c1 = 0.f;
-#pragma unroll
-                    for (int m = 0; m < 2; ++m) {
-                        c0 += (dahi[m][qq][0] + dalo[m][qq][0]) + (dahi[m][qq][1] + dalo[m][qq][1]);
-                        c1 += (dahi[m][qq][2] + dalo[m][qq][2]) + (dahi[m][qq][3] + dalo[m][qq][3]);
-                    }
-#pragma unroll
-                    for (int o = 4; o < 32; o <<= 1) {
-                        c0 += __shfl_xor_sync(0xffffffffu, c0, o);
-                        c1 += __shfl_xor_sync(0xffffffffu, c1, o);
-                    }
-                    const int c = 8 * qq + 2 * t;
-                    if (g == 0 && c < C) atomicAdd(&dWs[p.L.ob2 + c], c0);
-                    if (g == 0 && c + 1 < C) atomicAdd(&dWs[p.L.ob2 + c + 1], c1);
-                }
-            }
-
-            // ---- phase B: dh = da W2, dpre = dh (1 - h^2) -> TF32 split, transposed store; db1 column sums
-            {
-                __half* ohi = p.dpT_hi + ((int64_t)s * HP + 2 * t) * p.ldB + b0 + rbase;
-                const int64_t lo_off = p.dpT_lo - p.dpT_hi;
-                const int64_t ldB = p.ldB;
-#pragma unroll
-                for (int j = 0; j < KS; ++j) {
-                    float bh[2][2], bl[2][2];
-#pragma unroll
-                    for (int qq = 0; qq < 2; ++qq) {
-                        const float w0 = W2s[(8 * qq + 2 * t) * FM_W2_PITCH + 8 * j + g];
-                        const float w1 = W2s[(8 * qq + 2 * t + 1) * FM_W2_PITCH + 8 * j + g];
-                        split_tf32_trunc_lo(w0, bh[qq][0], bl[qq][0]);
-                        split_tf32_trunc_lo(w1, bh[qq][1], bl[qq][1]);
-                    }
-                    float cs0 = 0.f, cs1 = 0.f;
-#pragma unroll
-                    for (int m = 0; m < 2; ++m) {
-                        float dh[4] = {0.f, 0.f, 0.f, 0.f};
-                        mma_tf32(dh, dalo[m][0], bh[0][0], bh[0][1]);
-                        mma_tf32(dh, dahi[m][0], bl[0][0], bl[0][1]);
-                        if (two_q) {
-                            mma_tf32(dh, dalo[m][1], bh[1][0], bh[1][1]);
-                            mma_tf32(dh, dahi[m][1], bl[1][0], bl[1][1]);
-                            mma_tf32(dh, dahi[m][1], bh[1][0], bh[1][1]);
-                        }
-                        mma_tf32(dh, dahi[m][0], bh[0][0], bh[0][1]);
-                        // C fragment: (r0, h0), (r0, h0+1), (r1, h0), (r1, h0+1), h0 = 8j + 2t -- same order as acc[m][j]
-                        const float* hv = acc[m][j];
-                        float dp[4];
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) dp[i] = dh[i] * act_grad_from_h(act, hv[i]);
-                        __half hi[4], lo[4];
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) split_f16(dp[i] * sD, hi[i], lo[i]);
-                        // pad hidden units: zero W2 columns -> dp == 0, and the pad rows of dpT exist: no guard needed
-                        __half* o0 = ohi + (int64_t)(8 * j) * ldB + 16 * m;
-                        if (ok[m][0]) {
-                            o0[0] = hi[0]; o0[lo_off] = lo[0];
-                            o0[ldB] = hi[1]; o0[ldB + lo_off] = lo[1];
-                        }
-                        if (ok[m][1]) {
-                            o0[8] = hi[2]; o0[8 + lo_off] = lo[2];
-                            o0[ldB + 8] = hi[3]; o0[ldB + 8 + lo_off] = lo[3];
-                        }
-                        cs0 += dp[0] + dp[2];
-                        cs1 += dp[1] + dp[3];
-                    }
-#pragma unroll
-                    for (int o = 4; o < 32; o <<= 1) {
-                        cs0 += __shfl_xor_sync(0xffffffffu, cs0, o);
-                        cs1 += __shfl_xor_sync(0xffffffffu, cs1, o);
-                    }
-                    const int h0 = 8 * j + 2 * t;
-                    if (g == 0 && h0 < H) atomicAdd(&dWs[p.L.ob1 + h0], cs0);
-                    if (g == 0 && h0 + 1 < H) atomicAdd(&dWs[p.L.ob1 + h0 + 1], cs1);
-                }
-            }
-
-            // ---- phase C: dW2[c, h] += sum over this warp's 32 rows of da[row, c] h[row, h]
-            // k-step (m, hh) = rows {16m + 8hh + 0..7}.  A[class][k = row]: a0 = da[row t][g], a1 = da[row t][g + 8],
-            // a2 = da[row t+4][g], a3 = da[row t+4][g + 8]; B[k = row][n = hidden]: b0 = h[row t][8n + g], b1 = h[row t+4][8n + g].
-            // Source of (row r', column 2t' + par) is lane 4 r' + t' -- two shuffles (par = 0 / 1) and a select per element.
-            {
-                const int srcA = 4 * t + (g >> 1), srcB = 4 * (t + 4) + (g >> 1);
-                const bool odd = g & 1;
-                float Ahi[4][4], Alo[4][4];
-#pragma unroll
-                for (int m = 0; m < 2; ++m)
-#pragma unroll
-                    for (int hh = 0; hh < 2; ++hh) {
-                        const int ks = 2 * m + hh;
-#pragma unroll
-                        for (int qq = 0; qq < 2; ++qq) {
-                            // da of row half hh: even class -> fragment slot hh, odd class -> slot 2 + hh
-                            const float de = dahi[m][qq][hh] + dalo[m][qq][hh], dod = dahi[m][qq][2 + hh] + dalo[m][qq][2 + hh];
-                            const float ea = __shfl_sync(0xffffffffu, de, srcA), oa = __shfl_sync(0xffffffffu, dod, srcA);
-                            const float eb = __shfl_sync(0xffffffffu, de, srcB), ob = __shfl_sync(0xffffffffu, dod, srcB);
-                            split_tf32_trunc_lo(odd ? oa : ea, Ahi[ks][qq], Alo[ks][qq]);             // a0 / a1
-                            split_tf32_trunc_lo(odd ? ob : eb, Ahi[ks][2 + qq], Alo[ks][2 + qq]);     // a2 / a3
-                        }
-                    }
-                float* dW2 = dWs + p.L.oW2;
-                const bool vec2 = ((H & 1) == 0) && ((p.L.oW2 & 1) == 0) && ((p.L.ldw & 1) == 0);
-#pragma unroll
-                for (int n = 0; n < KS; ++n) {
-                    float cacc[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-                    for (int m = 0; m < 2; ++m)
-#pragma unroll
-                        for (int hh = 0; hh < 2; ++hh) {
-                            const int ks = 2 * m + hh;
-                            const float he = acc[m][n][2 * hh], ho = acc[m][n][2 * hh + 1];
-                            const float ea = __shfl_sync(0xffffffffu, he, srcA), oa = __shfl_sync(0xffffffffu, ho, srcA);
-                            const float eb = __shfl_sync(0xffffffffu, he, srcB), ob = __shfl_sync(0xffffffffu, ho, srcB);
-                            float bh0, bl0, bh1, bl1;
-                            split_tf32_trunc_lo(odd ? oa : ea, bh0, bl0);
-                            split_tf32_trunc_lo(odd ? ob : eb, bh1, bl1);
-                            mma_tf32(cacc, Alo[ks], bh0, bh1);
-                            mma_tf32(cacc, Ahi[ks], bl0, bl1);
-                            mma_tf32(cacc, Ahi[ks], bh0, bh1);
-                        }
-                    // C fragment: (class g, 8n + 2t), (g, 8n + 2t + 1), (g + 8, 8n + 2t), (g + 8, 8n + 2t + 1)
-                    const int h0 = 8 * n + 2 * t;
-                    if (vec2) {
-                        if (h0 < H) {           // H even: h0 + 1 < H as well
-                            if (g < C) red_add_v2(dW2 + (int64_t)g * H + h0, cacc[0], cacc[1]);
-                            if (g + 8 < C) red_add_v2(dW2 + (int64_t)(g + 8) * H + h0, cacc[2], cacc[3]);
-                        }
-                    } else {
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            const int c = g + (i >= 2 ? 8 : 0), h = h0 + (i & 1);
-                            if (c < C && h < H) atomicAdd(&dW2[(int64_t)c * H + h], cacc[i]);
-                        }
-                    }
-                }
-            }
-            double tot = (double)ll;
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) tot += __shfl_xor_sync(0xffffffffu, tot, o);
-            if (lane == 0) atomicAdd(p.loss, -tot * (double)p.inv_S);
-        }
-    }
-    umma::tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        umma::tc_fence_after();
-        umma::tmem_dealloc(tmem_base, TMEM_COLS);
-    }
-}
-
-// ---------------------------------------------------------------------------------------------------
-// backward GEMM epilogue: the per-sample weight gradient dW1_s never reaches HBM.  An epilogue thread owns one input
-// feature p (tile row) and the HP hidden units of ONE sample; it folds its accumulator row into the sample-axis sums
-//     gwT[p][h] += dW1_s[h, p]            gweT[p][h] += dW1_s[h, p] * eps_s[h, p]
-// with 16-byte vector REDs (the [p][h] layout makes a thread's hidden units contiguous).  eps_s[h][p] is read coalesced
-// across the warp (32 consecutive p).  Linear in the accumulator, so K-split partial sums need no special case.
-// ---------------------------------------------------------------------------------------------------
-struct EpiSampleReduce {
-    struct Params {
-        float* gwT; float* gweT;       // [P][HP], zeroed by the caller
-        const float* eps; int64_t lde; // eps[s * lde + h * P + p]
-        int P, H, HP, S;
-        const float* scal;             // operand bounds: the accumulator is (x_scale * dpre_scale) times the gradient
-    };
-    template <int CPT>
-    static __device__ __forceinline__ void finish(const Params& p, float (&r)[CPT], int row, int blk, bool, int) {
-        if (row >= p.P || blk >= p.S) return;
-        const float* e = p.eps + (int64_t)blk * p.lde + row;
-        float* ow = p.gwT + (int64_t)row * p.HP;
-        float* oe = p.gweT + (int64_t)row * p.HP;
-        const float inv = 1.f / (x_scale(p.scal) * dpre_scale(p.scal));
-#pragma unroll
-        for (int i0 = 0; i0 < CPT; i0 += 8) {        // 8 independent loads in flight per batch
-            float ev[8];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) ev[j] = (i0 + j < p.H) ? __ldg(e + (int64_t)(i0 + j) * p.P) : 0.f;
-#pragma unroll
-            for (int j = 0; j < 8; j += 4) {
-                const int i = i0 + j;
-                if (i >= p.H) break;
-                float a[4];
-#pragma unroll
-                for (int u = 0; u < 4; ++u) a[u] = (i + u < p.H) ? r[i + u] * inv : 0.f;      // pad columns hold garbage
-                red_add_v4(ow + i, a[0], a[1], a[2], a[3]);
-                red_add_v4(oe + i, a[0] * ev[j], a[1] * ev[j + 1], a[2] * ev[j + 2], a[3] * ev[j + 3]);
-            }
-        }
-    }
-};
-
-
 // ---------------------------------------------------------------------------------------------------
 // layer-1 sampler: noise + W1_s = mu + softplus(rho) eps_s + fp16 (hi, lo) split, scaled by w1_scale, in the padded K-major
 // layout Wh/Wl [(s * Hp + h)][ldP] the GEMMs read through TMA.  Sample-group version (P % 4 == 0): one thread = 4
-// consecutive weights, walking SG consecutive samples; sigma is evaluated once per thread, and the sample-axis noise
-// statistics the closed-form prior / entropy terms need,  e1 = sum_s eps,  e2 = sum_s eps^2,  are accumulated in registers
-// and added to e1/e2 [H*P] with one 16-byte RED each -- the statistics stage never re-reads the noise.
+// consecutive weights, walking SG consecutive samples; sigma is evaluated once per thread.
 // Pad rows h in [H, Hp) are never written: they only feed accumulator columns the epilogues mask.
 // ---------------------------------------------------------------------------------------------------
 template <int SG>
@@ -1020,7 +475,7 @@ __global__ void __launch_bounds__(256)
 sample_w1_group_kernel(const float* __restrict__ mu, const float* __restrict__ rho, const float* __restrict__ eps_in,
                        int64_t lde_in, float* __restrict__ eps_out, int64_t lde_out, __half* __restrict__ hi,
                        __half* __restrict__ lo, int H, int P, int Hp, int64_t ldP, brn_sample_range r, uint32_t var_id,
-                       float* __restrict__ e1, float* __restrict__ e2, const float* __restrict__ scal) {
+                       const float* __restrict__ scal) {
     const int64_t qq = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (qq * 4 >= (int64_t)H * P) return;
     const int h = (int)((qq * 4) / P), p = (int)((qq * 4) - (int64_t)h * P);
@@ -1029,7 +484,6 @@ sample_w1_group_kernel(const float* __restrict__ mu, const float* __restrict__ r
     const float4 m = *reinterpret_cast<const float4*>(mu + i);
     const float4 rh = *reinterpret_cast<const float4*>(rho + i);
     const float4 sg = make_float4(softplusf(rh.x), softplusf(rh.y), softplusf(rh.z), softplusf(rh.w));
-    float4 a1 = make_float4(0.f, 0.f, 0.f, 0.f), a2 = a1;
     const int s_begin = blockIdx.y * SG, s_end = min(r.s_local, s_begin + SG);
     const int64_t o0 = (int64_t)h * ldP + p;
 #pragma unroll 2
@@ -1055,12 +509,7 @@ sample_w1_group_kernel(const float* __restrict__ mu, const float* __restrict__ r
         pl.y = (uint32_t)__half_as_ushort(vl[2]) | ((uint32_t)__half_as_ushort(vl[3]) << 16);
         *reinterpret_cast<uint2*>(hi + o) = ph;
         *reinterpret_cast<uint2*>(lo + o) = pl;
-        a1.x += e.x; a1.y += e.y; a1.z += e.z; a1.w += e.w;
-        a2.x = __fmaf_rn(e.x, e.x, a2.x); a2.y = __fmaf_rn(e.y, e.y, a2.y);
-        a2.z = __fmaf_rn(e.z, e.z, a2.z); a2.w = __fmaf_rn(e.w, e.w, a2.w);
     }
-    red_add_v4(e1 + i, a1.x, a1.y, a1.z, a1.w);
-    red_add_v4(e2 + i, a2.x, a2.y, a2.z, a2.w);
 }
 
 // any shape / alignment: one thread per (p, h, s), noise already materialised in eps [S][lde]
@@ -1077,63 +526,6 @@ __global__ void sample_w1_generic_kernel(const float* __restrict__ mu, const flo
     lo[o] = vl;
 }
 
-// e1 = sum_s eps, e2 = sum_s eps^2 from stored noise (shapes the vectorised sampler does not cover)
-__global__ void __launch_bounds__(256)
-eps_stats_kernel(const float* __restrict__ eps, int64_t lde, int64_t numel, int S, float* __restrict__ e1, float* __restrict__ e2) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= numel) return;
-    float a1 = 0.f, a2 = 0.f;
-    for (int s = 0; s < S; ++s) {
-        const float e = eps[(int64_t)s * lde + i];
-        a1 += e;
-        a2 = __fmaf_rn(e, e, a2);
-    }
-    e1[i] += a1;
-    e2[i] += a2;
-}
-
-// layer-1 finalisation: sample-axis sums gw / gwe (HP > 0: stored transposed [P][HP] by the backward GEMM's epilogue; HP == 0:
-// natural [H*P] order) + e1 / e2 [H*P] (sampler) -> closed-form prior / entropy terms, chain rule to (mu, rho), loss.
-__global__ void __launch_bounds__(256)
-bnn_w1_finalize_kernel(brn_mf_var v, const float* __restrict__ gwT, const float* __restrict__ gweT, int HP, int P,
-                       const float* __restrict__ e1, const float* __restrict__ e2, brn_sample_range r, int with_prior,
-                       double* __restrict__ loss) {
-    __shared__ double red[32];
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    double elbo = 0.0;
-    if (i < v.numel) {
-        const int h = (int)(i / P), p = (int)(i - (int64_t)h * P);
-        const int64_t o = HP > 0 ? (int64_t)p * HP + h : i;
-        elbo = mf_finalize_element(v, i, gwT[o], gweT[o], e1[i], e2[i], r, with_prior);
-    }
-    const double tot = block_sum<double>(elbo, red);
-    if (threadIdx.x == 0 && with_prior) atomicAdd(loss, -tot);
-}
-
-template <int HP, int BK>
-static int launch_fwd_mid(const __half* Ah, const __half* Al, int M, int64_t lda, const __half* Bh, const __half* Bl, int N,
-                          int64_t ldb, int K, int drain_chunks, const FwdMidParams& fp, cudaStream_t stream) {
-    constexpr int BN = 2 * HP;
-    CUtensorMap tAh, tAl, tBh, tBl;
-    if (int e = make_tmap_2d_f16(&tAh, Ah, M, K, lda, UG_BM, BK * 2)) return e;
-    if (int e = make_tmap_2d_f16(&tAl, Al, M, K, lda, UG_BM, BK * 2)) return e;
-    if (int e = make_tmap_2d_f16(&tBh, Bh, N, K, ldb, BN, BK * 2)) return e;
-    if (int e = make_tmap_2d_f16(&tBl, Bl, N, K, ldb, BN, BK * 2)) return e;
-    const int m_tiles = (M + UG_BM - 1) / UG_BM, n_tiles = (N + BN - 1) / BN, k_chunks = (K + 2 * BK - 1) / (2 * BK);
-    drain_chunks = drain_chunks * 32 / BK;
-    if (drain_chunks < 1) drain_chunks = 2 * 32 / BK;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int U = m_tiles * n_tiles, grid = U < sms ? U : sms;
-    auto kern = bnn_fwd_mid_kernel<HP, BK>;
-    const int smem = FwdMidSmem<HP, BK>::TOTAL;
-    BRN_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    kern<<<grid, FM_THREADS, smem, stream>>>(tAh, tAl, tBh, tBl, m_tiles, n_tiles, k_chunks, drain_chunks, fp);
-    BRN_LAUNCH_OK("bnn_fwd_mid_kernel");
-    return 0;
-}
-
 constexpr int BNN_UMMA_HP = 104;     // padded hidden width of the instantiated tcgen05 variant (multiple of 8)
 constexpr int BNN_UMMA_BK = 16;      // K chunk: 16 words = 64 bytes = 32 fp16 (64-byte swizzle), 5-stage TMA ring
 constexpr int BNN_UMMA_NSAMP = 2;    // samples per MMA N tile (N = 208)
@@ -1141,8 +533,7 @@ constexpr int BNN_UMMA_NSAMP = 2;    // samples per MMA N tile (N = 208)
 // workspace of the tcgen05 variant (appended to the SIMT variant's blocks by BnnWorkspace in bnn.cu)
 struct BnnTcWorkspace {
     __half *Xh, *Xl, *Xth, *Xtl, *Wh, *Wl, *dph, *dpl;   // fp16 (hi, lo) operands
-    float *scal, *gwT, *gweT, *e1, *e2;                  // one block, zeroed per call: bounds + sample-axis sums of layer 1
-    size_t zero_floats;
+    float* scal;                                         // operand bounds (SC_*), zeroed per call
     int64_t ldP, ldB;
     template <class Take>
     void carve(Take&& take, const BnnLayout& L, int S) {
@@ -1154,46 +545,42 @@ struct BnnTcWorkspace {
         const size_t rowsW = (size_t)(S + BNN_UMMA_NSAMP) * BNN_UMMA_HP;
         Wh = half_block(rowsW * ldP); Wl = half_block(rowsW * ldP);
         dph = half_block(rowsW * ldB); dpl = half_block(rowsW * ldB);
-        const size_t gT = ((size_t)L.P * BNN_UMMA_HP + 63) / 64 * 64, ne = ((size_t)L.H * L.P + 63) / 64 * 64;
-        zero_floats = 64 + 2 * gT + 2 * ne;
-        scal = take(zero_floats);                        // contiguous: [scal | gwT | gweT | e1 | e2]
-        gwT = scal ? scal + 64 : nullptr;
-        gweT = scal ? gwT + gT : nullptr;
-        e1 = scal ? gweT + gT : nullptr;
-        e2 = scal ? e1 + ne : nullptr;
+        scal = take(SC_SLOTS);
     }
 };
 
-// The tcgen05 variant of brn_bnn_elbo_fwd_bwd.  fused != 0 (default): sampler (+ noise statistics) -> forward GEMM with the
-// mid stage in its epilogue -> backward GEMM with the sample-axis reduction in its epilogue -> finalisation; pre_s and dW1_s
-// never reach HBM.  fused == 0: the staged pipeline (forward GEMM -> mid kernel -> backward GEMM -> statistics), kept for A/B
-// measurements and tests (BRN_BNN_MID=4).
+// The tcgen05 variant of brn_bnn_elbo_fwd_bwd: sampler -> forward GEMM -> mid kernel -> backward GEMM -> statistics.
+// forward_only (brn_bnn_predict) stops after the forward GEMM.
 static int bnn_tc_eval(const float* X, const int32_t* y, const BnnLayout& L, const brn_mf_var vars[4], const brn_sample_range* r,
                        const BnnTcWorkspace& ws, float* ws_eps, float* ws_W, float* ws_dW, float* ws_pre, float* ws_stats,
-                       int with_prior, double* loss, int drain, int drain_bwd, bool fused, cudaStream_t stream, bool forward_only = false) {
+                       int with_prior, double* loss, cudaStream_t stream, bool forward_only = false) {
     constexpr int HP = BNN_UMMA_HP, NS = BNN_UMMA_NSAMP, BN = HP * NS;
+    // TMEM accumulation chain = 2 x 32 words = 128 fp16 elements of K between register drains (umma_gemm.cuh): the error
+    // of the evaluation grows with the chain (max gradient error / scale at the C3 shape: 0.9e-6 / 1.1e-6 / 1.3e-6 /
+    // 2.3e-6 for 1 / 2 / 4 / 8, profiles/tools/bnn_err_probe.py) -- 128 elements is the chain length round 1 settled on.
+    // The backward GEMM's accumulator is the per-sample weight gradient, summed over 256 samples afterwards: its chain
+    // may be twice as long (measured: no change of the parity margins, 8 us per evaluation).
+    constexpr int drain = 2, drain_bwd = 4;
     const int B = L.B, P = L.P, H = L.H, S = r->s_local;
     const int64_t numels[4] = {(int64_t)H * P, H, (int64_t)L.C * H, L.C};
     const int64_t offs[4] = {L.oW1, L.ob1, L.oW2, L.ob2};
     const float inv_S = 1.0f / (float)r->s_total;
-    bool fast_sampler = false;
     {
         StageTimer st("bnn.sample_weights", stream);
-        BRN_CUDA_OK(cudaMemsetAsync(ws.scal, 0, sizeof(float) * ws.zero_floats, stream));
+        BRN_CUDA_OK(cudaMemsetAsync(ws.scal, 0, sizeof(float) * SC_SLOTS, stream));
         // operand bounds (device scalars): injected noise is not bounded a priori
         if (vars[0].eps) if (int e = launch_absmax(vars[0].eps, (int64_t)S * numels[0], ws.scal + SC_EPS, stream)) return e;
         if (vars[2].eps) if (int e = launch_absmax(vars[2].eps, (int64_t)S * numels[2], ws.scal + SC_EPS, stream)) return e;
         bnn_bounds_kernel<<<(unsigned)std::min<int64_t>((numels[0] + numels[2] + 255) / 256, 296), 256, 0, stream>>>(
             vars[0].mu, vars[0].rho, numels[0], vars[2].mu, vars[2].rho, numels[2], ws.scal);
         BRN_LAUNCH_OK("bnn_bounds_kernel");
-        fast_sampler = (P % 4 == 0) && ((uintptr_t)vars[0].mu % 16 == 0) && ((uintptr_t)vars[0].rho % 16 == 0) &&
-                       (!vars[0].eps || ((uintptr_t)vars[0].eps % 16 == 0));
-        const bool fast = fast_sampler;
+        const bool fast = (P % 4 == 0) && ((uintptr_t)vars[0].mu % 16 == 0) && ((uintptr_t)vars[0].rho % 16 == 0) &&
+                          (!vars[0].eps || ((uintptr_t)vars[0].eps % 16 == 0));
         if (fast) {
             constexpr int SG = 8;
             dim3 grid((unsigned)(((int64_t)H * P / 4 + 255) / 256), (unsigned)((S + SG - 1) / SG));
             sample_w1_group_kernel<SG><<<grid, 256, 0, stream>>>(vars[0].mu, vars[0].rho, vars[0].eps, numels[0], ws_eps + offs[0], L.ldw,
-                                                                 ws.Wh, ws.Wl, H, P, HP, ws.ldP, *r, vars[0].var_id, ws.e1, ws.e2, ws.scal);
+                                                                 ws.Wh, ws.Wl, H, P, HP, ws.ldP, *r, vars[0].var_id, ws.scal);
             BRN_LAUNCH_OK("sample_w1_group_kernel");
         } else {
             if (vars[0].eps)
@@ -1204,8 +591,6 @@ static int bnn_tc_eval(const float* X, const int32_t* y, const BnnLayout& L, con
             sample_w1_generic_kernel<<<grid, 256, 0, stream>>>(vars[0].mu, vars[0].rho, ws_eps + offs[0], L.ldw, ws.Wh, ws.Wl, H, P, HP,
                                                                ws.ldP, ws.scal);
             BRN_LAUNCH_OK("sample_w1_generic_kernel");
-            eps_stats_kernel<<<(unsigned)((numels[0] + 255) / 256), 256, 0, stream>>>(ws_eps + offs[0], L.ldw, numels[0], S, ws.e1, ws.e2);
-            BRN_LAUNCH_OK("eps_stats_kernel");
         }
         if (S % NS) {   // the odd tail tile reads one more sample block: keep it finite
             BRN_CUDA_OK(cudaMemsetAsync(ws.Wh + (size_t)S * HP * ws.ldP, 0, sizeof(__half) * HP * ws.ldP, stream));
@@ -1222,31 +607,6 @@ static int bnn_tc_eval(const float* X, const int32_t* y, const BnnLayout& L, con
         split_f16_kernel<<<grid, block, 0, stream>>>(X, P, B, P, ws.Xh, ws.Xl, ws.ldP, ws.Xth, ws.Xtl, ws.ldB, ws.scal);
         BRN_LAUNCH_OK("split_f16_kernel");
     }
-    if (fused && !forward_only) {
-        {
-            StageTimer st("bnn.gemm_fwd", stream);      // forward GEMM + mid in its epilogue
-            FwdMidParams fp{ws_W, ws_dW, y, L, S, inv_S, loss, ws.dph, ws.dpl, ws.ldB, ws.scal};
-            if (int e = launch_fwd_mid<HP, BNN_UMMA_BK>(ws.Xh, ws.Xl, B, ws.ldP, ws.Wh, ws.Wl, S * HP, ws.ldP, P, drain, fp, stream))
-                return e;
-        }
-        {
-            StageTimer st("bnn.gemm_bwd", stream);      // dW1_s = dpre_s^T . X, folded over samples in the epilogue
-            EpiSampleReduce::Params ep{ws.gwT, ws.gweT, ws_eps + offs[0], L.ldw, P, H, HP, S, ws.scal};
-            if (int e = launch_umma_nt_kind<BN, BNN_UMMA_BK, EpiSampleReduce, 8, 0, 4, 1>(ws.Xth, ws.Xtl, P, ws.ldB, ws.dph, ws.dpl, S * HP,
-                                                                                          ws.ldB, B, 0, drain_bwd, ep, stream, true))
-                return e;
-        }
-        StageTimer st5("bnn.reduce_finalize", stream);
-        const int64_t offs_small[3] = {0, offs[2] - offs[1], offs[3] - offs[1]};
-        if (int e = launch_mf_reduce_finalize_multi(vars + 1, offs_small, 3, L.numel - offs[1], ws_eps + offs[1], L.ldw, ws_dW + offs[1],
-                                                    L.ldw, ws_stats, *r, with_prior, loss, stream, 0))
-            return e;
-        bnn_w1_finalize_kernel<<<(unsigned)((numels[0] + 255) / 256), 256, 0, stream>>>(vars[0], ws.gwT, ws.gweT, HP, P, ws.e1, ws.e2, *r,
-                                                                                       with_prior, loss);
-        BRN_LAUNCH_OK("bnn_w1_finalize_kernel");
-        return 0;
-    }
-    // ---- staged pipeline
     {
         StageTimer st("bnn.gemm_fwd", stream);
         EpiStore::Params ep;      // pre^T: [S][H][B], coalesced across the warp's rows b

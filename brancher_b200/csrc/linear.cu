@@ -302,8 +302,7 @@ constexpr int LT_BK2 = 32;        // gradient GEMM: 128-byte operand rows (both 
 // rows per chunk of the tcgen05 path: whole 128-row tiles such that (m-tiles x n-tiles) fills ~2 rounds of the grid
 static int linear_tc_chunk_rows(int S, int sms) {
     const int n_tiles = (S + LT_BN1 - 1) / LT_BN1;
-    int rounds = 12;     // measured at C2 on B200 (profiles/r1k_*, r1l_*): 2: 7.06 ms, 4: 5.90, 8: 5.43, 12: 5.14, 16: 5.19, 24: 5.14
-    if (const char* env = getenv("BRN_LINEAR_ROUNDS")) rounds = atoi(env) > 0 ? atoi(env) : rounds;
+    const int rounds = 12;     // measured at C2 on B200 (profiles/r1k_*, r1l_*): 2: 7.06 ms, 4: 5.90, 8: 5.43, 12: 5.14, 16: 5.19, 24: 5.14
     int mt = rounds * sms / n_tiles;
     if (mt < 1) mt = 1;
     if (mt > 512) mt = 512;
@@ -317,7 +316,7 @@ namespace brn {
 // TF32-split operands and scratch of the tcgen05 variant (Bernoulli, C == 1); S = weight vectors (MC samples or particles)
 struct LinearTcBuffers {
     LinearFlashBuffers flash;
-    float *Wh, *Wl, *Xh, *Xl, *Xth, *Xtl, *dTh, *dTl, *dWpart;
+    float *Wh, *Wl, *Xh, *Xl, *Xth, *Xtl, *dT, *dWpart;
     int64_t ldF, ldN, ldNB, n_chunks;
     int nb, slices;
     template <class Take>
@@ -336,7 +335,7 @@ struct LinearTcBuffers {
         // per TMA request -- measured: the gradient GEMM spent 71 % of its time waiting for those loads)
         n_chunks = nb > 0 ? (N + nb - 1) / nb : 0;
         Xth = take((size_t)n_chunks * F * ldNB); Xtl = take((size_t)n_chunks * F * ldNB);
-        dTh = take((size_t)S * ldNB); dTl = take((size_t)S * ldNB);
+        dT = take((size_t)S * ldNB);
         dWpart = take((size_t)slices * S * F);
         flash.carve(take, S, F, sms);
         flash.Xh = reinterpret_cast<__half*>(Xh);        // the one-pass kernel's fp16 pair of X lives in the staged pair's buffers
@@ -469,37 +468,24 @@ static int launch_linear_tc(const float* X, const float* y, int64_t N, int F, in
         BRN_LAUNCH_OK("sum_slices_kernel");
         return 0;
     }
-    int drain = 2;
-    if (const char* env = getenv("BRN_UMMA_DRAIN")) drain = atoi(env);
+    constexpr int drain = 2;
     // Operands that cross HBM once are kept as ONE fp32 matrix and split into TF32 (hi, lo) inside the GEMMs by converter warps
-    // (SPLIT mask, umma_gemm.cuh): d^T between the two GEMMs, X itself (read in place: no row-major copy at all) and the
-    // per-chunk X^T.  BRN_LINEAR_SPLIT_A=0 restores the pre-split operand pairs everywhere (A/B measurements, tests).
-    // BRN_LINEAR_SPLIT_A is a bit mask: 1 = d^T plain, 2 = X^T plain, 4 = X read in place (0 = every operand pre-split)
-    // measured at C2 on B200 (profiles/r1t_*): 0: 5.44 ms, 1: 4.75, 3: 5.07, 5: 4.57, 7: 4.69 -- converting the B tile too slows
-    // the gradient GEMM more than the smaller split pass saves
-    int sm = 5;
-    if (const char* env = getenv("BRN_LINEAR_SPLIT_A")) sm = atoi(env) & 7;
-    if (reinterpret_cast<uintptr_t>(X) % 16 != 0) sm &= ~4;      // TMA needs a 16-byte aligned base
-    const bool d_plain = sm & 1, xt_plain = sm & 2, x_in_place = sm & 4;
+    // (SPLIT mask, umma_gemm.cuh): d^T between the two GEMMs, and X itself (read in place: no row-major copy at all) when
+    // TMA can read it (16-byte aligned base); the per-chunk X^T stays pre-split.  Measured at C2 on B200 (profiles/r1t_*,
+    // mask of plain operands 1 = d^T, 2 = X^T, 4 = X): 0: 5.44 ms, 1: 4.75, 3: 5.07, 5: 4.57, 7: 4.69 -- converting the B
+    // tile too slows the gradient GEMM more than the smaller split pass saves
+    const bool x_in_place = reinterpret_cast<uintptr_t>(X) % 16 == 0;
     {
         StageTimer sp(stage_split, stream);
         if (int e = launch_split_tf32(W, F, S, F, b.Wh, b.Wl, b.ldF, nullptr, nullptr, 0, stream)) return e;
         for (int64_t c = 0; c < b.n_chunks; ++c) {
             const int64_t r0 = c * b.nb;
             const int nb = (int)((N - r0 < b.nb) ? (N - r0) : b.nb);
-            float* xth = b.Xth + c * F * b.ldNB;
-            float* xtl = b.Xtl + c * F * b.ldNB;
-            if (x_in_place && xt_plain) {
-                if (int e = launch_transpose_f32(X + r0 * F, F, nb, F, xth, b.ldNB, stream)) return e;
-            } else {
-                // (hi, lo) of X row-major and / or transposed; an unused output pair is skipped by the kernel
-                if (int e = launch_split_tf32(X + r0 * F, F, nb, F, x_in_place ? nullptr : b.Xh + r0 * b.ldF,
-                                              x_in_place ? nullptr : b.Xl + r0 * b.ldF, b.ldF, xt_plain ? nullptr : xth,
-                                              xt_plain ? nullptr : xtl, b.ldNB, stream))
-                    return e;
-                if (xt_plain)
-                    if (int e = launch_transpose_f32(X + r0 * F, F, nb, F, xth, b.ldNB, stream)) return e;
-            }
+            // (hi, lo) of X transposed and, unless X is read in place, row-major; an unused output pair is skipped by the kernel
+            if (int e = launch_split_tf32(X + r0 * F, F, nb, F, x_in_place ? nullptr : b.Xh + r0 * b.ldF,
+                                          x_in_place ? nullptr : b.Xl + r0 * b.ldF, b.ldF, b.Xth + c * F * b.ldNB,
+                                          b.Xtl + c * F * b.ldNB, b.ldNB, stream))
+                return e;
         }
         BRN_CUDA_OK(cudaMemsetAsync(b.dWpart, 0, sizeof(float) * (size_t)b.slices * S * F, stream));
     }
@@ -507,7 +493,7 @@ static int launch_linear_tc(const float* X, const float* y, int64_t N, int F, in
     for (int64_t r0 = 0; r0 < N; r0 += b.nb) {
         const int nb = (int)((N - r0 < b.nb) ? (N - r0) : b.nb);
         EpiBernoulli::Params e1;
-        e1.y = y + r0; e1.dT_hi = b.dTh; e1.dT_lo = d_plain ? nullptr : b.dTl; e1.rows = nb; e1.cols = S;
+        e1.y = y + r0; e1.dT = b.dT; e1.rows = nb; e1.cols = S;
         e1.ld = b.ldNB; e1.loss = loss; e1.neg_inv_S = loss_scale;
         if (x_in_place) {
             if (int e = launch_umma_nt<LT_BN1, LT_BK, EpiBernoulli, LT_EW1, 1, 2>(X + r0 * F, nullptr, nb, F, b.Wh, b.Wl, S, b.ldF, F, 0,
@@ -520,20 +506,9 @@ static int launch_linear_tc(const float* X, const float* y, int64_t N, int F, in
         EpiAccum::Params e2;
         e2.out = b.dWpart; e2.rows = S; e2.cols = F; e2.ld = F; e2.slice_stride = (int64_t)S * F;
         const int64_t xt = (r0 / b.nb) * F * b.ldNB;
-        int e = 0;
-        if (d_plain && xt_plain)
-            e = launch_umma_nt<LT_BN2, LT_BK2, EpiAccum, UG_EPI_WARPS, 3>(b.dTh, nullptr, S, b.ldNB, b.Xth + xt, nullptr, F, b.ldNB, nb, 0,
-                                                                         drain, e2, stream, b.slices > 1);
-        else if (d_plain)
-            e = launch_umma_nt<LT_BN2, LT_BK2, EpiAccum, UG_EPI_WARPS, 1>(b.dTh, nullptr, S, b.ldNB, b.Xth + xt, b.Xtl + xt, F, b.ldNB, nb,
-                                                                         0, drain, e2, stream, b.slices > 1);
-        else if (xt_plain)
-            e = launch_umma_nt<LT_BN2, LT_BK2, EpiAccum, UG_EPI_WARPS, 2>(b.dTh, b.dTl, S, b.ldNB, b.Xth + xt, nullptr, F, b.ldNB, nb, 0,
-                                                                         drain, e2, stream, b.slices > 1);
-        else
-            e = launch_umma_nt<LT_BN2, LT_BK2, EpiAccum>(b.dTh, b.dTl, S, b.ldNB, b.Xth + xt, b.Xtl + xt, F, b.ldNB, nb, 0, drain, e2,
-                                                        stream, b.slices > 1);
-        if (e) return e;
+        if (int e = launch_umma_nt<LT_BN2, LT_BK2, EpiAccum, UG_EPI_WARPS, 1>(b.dT, nullptr, S, b.ldNB, b.Xth + xt, b.Xtl + xt, F, b.ldNB,
+                                                                               nb, 0, drain, e2, stream, b.slices > 1))
+            return e;
     }
     const int64_t tot = (int64_t)S * F;
     sum_slices_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(b.dWpart, b.slices, tot, tot, dW);

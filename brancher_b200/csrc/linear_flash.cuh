@@ -5,7 +5,7 @@
 //     MMA1   L[s, r]   = sum_f W[s, f] X[r, f]              M = 128 vectors, N = 64 rows,  K = F   (D1 in TMEM, 64 columns)
 //     epilogue         d = y_r - sigmoid(L), ll += y L - softplus(L); d -> fp16 (hi, lo) pair, written with tcgen05.st to
 //                      TENSOR memory as the A operand of MMA2 (the thread that owns TMEM lane s writes row s: no
-//                      transposition; DTMEM = 0 keeps the round-trip through a K-major shared-memory tile)
+//                      transposition)
 //     MMA2   dW[s, f] += sum_r d[s, r] X[r, f]             M = 128 vectors, N = F,        K = 64 rows (D2 in TMEM, F columns)
 //   The SAME shared-memory image of the X block serves MMA1 as a K-major B operand (K = f, contiguous) and MMA2 as an
 //   MN-major B operand (N = f contiguous, K = rows): no transposed copy of X exists anywhere.
@@ -31,7 +31,7 @@ namespace brn {
 constexpr int LF_ROWS = 64;            // rows of X per block (N of MMA1, K of MMA2)
 constexpr int LF_MT = 128;             // weight vectors per CTA tile (M of both MMAs)
 constexpr int LF_FMAX = 128;           // features (K of MMA1, N of MMA2): multiple of 16, at most 128
-constexpr int LF_XSTAGES_SMEM_D = 4;   // X blocks (fp16 pair images, 32 KB each) in flight; 5 when the d tile lives in TMEM
+constexpr int LF_XSTAGES = 5;          // X blocks (fp16 pair images, 32 KB each) in flight
 constexpr int LF_D1BUF = 3;            // logits accumulators in TMEM: the logits MMA runs two blocks ahead of the gradient MMA
 constexpr int LF_THREADS = 640;        // 20 warps: TMA, 2 MMA issuers, 1 idle | 16 epilogue
 constexpr int LF_EPI_WARP0 = 4, LF_EPI_WARPS = 16;
@@ -40,18 +40,14 @@ constexpr int LF_EFEAT = 32;           // gradient features per epilogue warp (a
 constexpr int LF_D2_CHAIN = 2;         // blocks per D2 accumulation chain
 constexpr float LF_D_SCALE = 8192.f;   // 2^13: |d| < 1
 
-template <int DTMEM>
 struct LinearFlashSmem {
-    static constexpr int XSTAGES = DTMEM ? LF_XSTAGES_SMEM_D + 1 : LF_XSTAGES_SMEM_D;
     static constexpr int W_BYTES = 2 * LF_MT * LF_FMAX * 2;                 // (hi, lo) [128][128] fp16 = 64 KB
     static constexpr int X16_BYTES = 2 * LF_ROWS * LF_FMAX * 2;             // (hi, lo) [64][128] fp16 = 32 KB
-    static constexpr int D_BYTES = DTMEM ? 0 : 2 * LF_MT * LF_ROWS * 2;     // (hi, lo) [128][64] fp16 = 32 KB (shared-memory d tile)
     static constexpr int off_w = 0;
     static constexpr int off_x16 = off_w + W_BYTES;
-    static constexpr int off_d = off_x16 + XSTAGES * X16_BYTES;
-    static constexpr int off_y = off_d + D_BYTES;                           // y of the block in each X stage: 64 floats
+    static constexpr int off_y = off_x16 + LF_XSTAGES * X16_BYTES;          // y of the block in each X stage: 64 floats
     static constexpr int Y_BYTES = LF_ROWS * 4;
-    static constexpr int TOTAL = off_y + XSTAGES * Y_BYTES + 1024;          // + alignment slack
+    static constexpr int TOTAL = off_y + LF_XSTAGES * Y_BYTES + 1024;       // + alignment slack
     static_assert(TOTAL <= 227 * 1024, "shared memory budget exceeded");
 };
 
@@ -136,18 +132,17 @@ __device__ __forceinline__ void tmem_st_32x16(uint32_t taddr, const uint32_t (&v
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 // KS1 = F / 16 at compile time (the logits MMA loop is then fully unrolled), 0 = any F.
-// DTMEM: the d tile (A operand of the gradient MMA) lives in tensor memory (64 columns: hi pair words, lo pair words) instead of
-// shared memory -- the epilogue thread that owns TMEM lane s writes row s with tcgen05.st: no shared-memory round trip, no
-// generic -> async proxy fence, half the shared-memory operand reads of the gradient MMA.
+// The d tile (A operand of the gradient MMA) lives in tensor memory (64 columns: hi pair words, lo pair words): the epilogue
+// thread that owns TMEM lane s writes row s with tcgen05.st -- no shared-memory round trip, no generic -> async proxy fence,
+// half the shared-memory operand reads of the gradient MMA.
 // LIK: 0 = Bernoulli (d = y - sigmoid(l), loss += loss_scale * sum ll), 1 = Gaussian residuals (d = r = y - l, R[s] += sum r^2;
 // the noise scale is applied afterwards, per vector, by the caller), 2 = Cauchy (z = r / sigma_s, d = z / (1 + z^2),
 // R[s] += sum log1p(z^2), T[s] += sum z^2 / (1 + z^2)), 3 = Laplace (d = sign(r), R[s] += sum |r|; sigma applied afterwards).
-template <int KS1, int DTMEM, int LIK = 0>
+template <int KS1, int LIK = 0>
 __global__ void __launch_bounds__(LF_THREADS, 1)
 linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_constant__ CUtensorMap tmWl,
                     const __grid_constant__ CUtensorMap tmXh, const __grid_constant__ CUtensorMap tmXl, LinearFlashParams p) {
-    using SM = LinearFlashSmem<DTMEM>;
-    constexpr int LF_XSTAGES = SM::XSTAGES;
+    using SM = LinearFlashSmem;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     __shared__ __align__(8) uint64_t w_full, x_full[LF_XSTAGES], x_empty[LF_XSTAGES], d1_full[LF_D1BUF], d1_empty[LF_D1BUF],
@@ -178,7 +173,7 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
     umma::tc_fence_after();
     const uint32_t tmem_base = tmem_base_slot;
     const uint32_t t_d1 = tmem_base, t_d2 = tmem_base + 256;        // D1: 3 x 64 columns at 0 / 64 / 128; D2: 2 x 128 at 256 / 384
-    const uint32_t t_dt = tmem_base + 192;                          // d tile (DTMEM): hi words at 192..223, lo words at 224..255
+    const uint32_t t_dt = tmem_base + 192;                          // d tile: hi words at 192..223, lo words at 224..255
 
     // register budget: the CTA owns 96 registers x 640 threads (launch bounds); setmaxnreg only moves registers INSIDE that
     // allocation (asking for more blocks forever), so per warpgroup 32 + 4 x 112 = 480 = 5 x 96
@@ -246,7 +241,6 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
         if (umma::elect_one()) {
             constexpr uint32_t HI = 0x40004040u;
             const uint32_t idesc2 = idesc_f16_major(LF_MT, F, true);
-            const uint32_t d_h = (umma::smem_u32(smem + SM::off_d) >> 4) | (1u << 16), d_l = d_h + (SM::D_BYTES / 2 >> 4);
             const uint32_t x0 = (umma::smem_u32(smem + SM::off_x16) >> 4) | ((LF_ROWS * 128 >> 4) << 16);   // MN-major view: LBO = one box
             int xs = 0;
             uint32_t chain = 0;                        // index of the current D2 accumulation chain
@@ -260,16 +254,10 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
                 const uint32_t d_t = t_d2 + buf * 128;
 #pragma unroll
                 for (int ks = 0; ks < LF_ROWS / 16; ++ks) {
-                    // A = d tile, K-major (32 bytes per k-step); B: 16 K-indices (rows of X) = 2 KB per k-step
-                    if (DTMEM) {      // 16 K elements = 8 columns per k-step
-                        mma_f16_ts_lohi(d_t, t_dt + 32 + ks * 8, xm + ks * 128, HI, idesc2, !first || ks != 0);
-                        mma_f16_ts_lohi(d_t, t_dt + ks * 8, xm + (SM::X16_BYTES / 2 >> 4) + ks * 128, HI, idesc2, true);
-                        mma_f16_ts_lohi(d_t, t_dt + ks * 8, xm + ks * 128, HI, idesc2, true);
-                    } else {
-                        mma_f16_lohi(d_t, d_l + ks * 2, xm + ks * 128, HI, idesc2, !first || ks != 0);
-                        mma_f16_lohi(d_t, d_h + ks * 2, xm + (SM::X16_BYTES / 2 >> 4) + ks * 128, HI, idesc2, true);
-                        mma_f16_lohi(d_t, d_h + ks * 2, xm + ks * 128, HI, idesc2, true);
-                    }
+                    // A = d tile in TMEM: 16 K elements = 8 columns per k-step; B: 16 K-indices (rows of X) = 2 KB per k-step
+                    mma_f16_ts_lohi(d_t, t_dt + 32 + ks * 8, xm + ks * 128, HI, idesc2, !first || ks != 0);
+                    mma_f16_ts_lohi(d_t, t_dt + ks * 8, xm + (SM::X16_BYTES / 2 >> 4) + ks * 128, HI, idesc2, true);
+                    mma_f16_ts_lohi(d_t, t_dt + ks * 8, xm + ks * 128, HI, idesc2, true);
                 }
                 umma::mma_commit(&x_empty[xs]);        // X block and d tile are free once these MMAs retire (the logits MMA of
                 umma::mma_commit(&d_empty[i & 1]);     // this block retired long ago: d was computed from its result)
@@ -295,8 +283,6 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
         const bool s_ok = s_glob < p.S;
         const float inv1 = 1.f / (p2_scale(*p.scal_w) * p2_scale(*p.scal_x));      // logit = D1 * inv1
         const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
-        uint8_t* dh = smem + SM::off_d;
-        uint8_t* dl = dh + SM::D_BYTES / 2;
         float r2[LF_EFEAT];
 #pragma unroll
         for (int c = 0; c < LF_EFEAT; ++c) r2[c] = 0.f;
@@ -567,25 +553,12 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
             // the d tile is free once the gradient MMA of the previous block (the other group's) has retired
             // (block i - 1: barrier of the other parity, its use (i - 1) / 2; the first block has nothing to wait for)
             if (i > 0) umma::mbar_wait_guarded(&d_empty[(i & 1) ^ 1], (uint32_t)(((i - 1) >> 1) & 1));
-            if (DTMEM) {
-                // this thread owns TMEM lane s_local = row s of the A operand; column = pair of block rows (2k, 2k + 1)
-                umma::tc_fence_after();
-                tmem_st_32x16(t_dt + lane_addr + hp * (LF_EROWS / 2), dh_w);
-                tmem_st_32x16(t_dt + 32 + lane_addr + hp * (LF_EROWS / 2), dl_w);
-                tmem_st_wait();
-                umma::tc_fence_before();
-            } else {
-            // K-major A tile [128 vectors][64 rows] fp16, 128-byte rows, SWIZZLE_128B: this thread owns row s_local and writes
-            // the 4 chunks (8 rows of X each) of its rows
-#pragma unroll
-            for (int cc = 0; cc < LF_EROWS / 8; ++cc) {
-                const int c = hp * (LF_EROWS / 8) + cc;
-                const int off = s_local * 128 + ((c ^ (s_local & 7)) << 4);
-                *reinterpret_cast<uint4*>(dh + off) = make_uint4(dh_w[4 * cc], dh_w[4 * cc + 1], dh_w[4 * cc + 2], dh_w[4 * cc + 3]);
-                *reinterpret_cast<uint4*>(dl + off) = make_uint4(dl_w[4 * cc], dl_w[4 * cc + 1], dl_w[4 * cc + 2], dl_w[4 * cc + 3]);
-            }
-            umma::fence_proxy_async();
-            }
+            // this thread owns TMEM lane s_local = row s of the A operand; column = pair of block rows (2k, 2k + 1)
+            umma::tc_fence_after();
+            tmem_st_32x16(t_dt + lane_addr + hp * (LF_EROWS / 2), dh_w);
+            tmem_st_32x16(t_dt + 32 + lane_addr + hp * (LF_EROWS / 2), dl_w);
+            tmem_st_wait();
+            umma::tc_fence_before();
             ll_total += (double)ll;
             __syncwarp();
             if (lane == 0) umma::mbar_arrive(&d_full[grp]);
@@ -758,32 +731,18 @@ static int launch_linear_flash(const float* X, const void* px, const float* y, i
     p.scal_y = b.scal + 2; p.R = R;
     p.sigma = sigma; p.T = T;
     p.y_bulk = (reinterpret_cast<uintptr_t>(y) & 15) == 0;
-    if (const char* env = getenv("BRN_LINEAR_Y_BULK")) p.y_bulk = p.y_bulk && atoi(env) != 0;
     dim3 grid(b.tiles, b.groups);
-    int dtmem = 1;
-    if (const char* env = getenv("BRN_LINEAR_DTMEM")) dtmem = atoi(env) != 0;
-    auto launch = [&](auto kern, int smem_bytes) -> int {
-        BRN_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
-        kern<<<grid, LF_THREADS, smem_bytes, stream>>>(tWh, tWl, tXh, tXl, p);
+    auto launch = [&](auto kern) -> int {
+        BRN_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, LinearFlashSmem::TOTAL));
+        kern<<<grid, LF_THREADS, LinearFlashSmem::TOTAL, stream>>>(tWh, tWl, tXh, tXl, p);
         return 0;
     };
-    if (R && lik == 2) {      // the regression epilogues exist with the d tile in tensor memory only
-        if (int e = F == 128 ? launch(linear_flash_kernel<8, 1, 2>, LinearFlashSmem<1>::TOTAL)
-                             : launch(linear_flash_kernel<0, 1, 2>, LinearFlashSmem<1>::TOTAL))
-            return e;
-    } else if (R && lik == 3) {
-        if (int e = F == 128 ? launch(linear_flash_kernel<8, 1, 3>, LinearFlashSmem<1>::TOTAL)
-                             : launch(linear_flash_kernel<0, 1, 3>, LinearFlashSmem<1>::TOTAL))
-            return e;
-    } else if (R) {
-        if (int e = F == 128 ? launch(linear_flash_kernel<8, 1, 1>, LinearFlashSmem<1>::TOTAL)
-                             : launch(linear_flash_kernel<0, 1, 1>, LinearFlashSmem<1>::TOTAL))
-            return e;
-    } else if (F == 128) {
-        if (int e = dtmem ? launch(linear_flash_kernel<8, 1>, LinearFlashSmem<1>::TOTAL) : launch(linear_flash_kernel<8, 0>, LinearFlashSmem<0>::TOTAL)) return e;
-    } else {
-        if (int e = dtmem ? launch(linear_flash_kernel<0, 1>, LinearFlashSmem<1>::TOTAL) : launch(linear_flash_kernel<0, 0>, LinearFlashSmem<0>::TOTAL)) return e;
-    }
+    int e;
+    if (R && lik == 2) e = F == 128 ? launch(linear_flash_kernel<8, 2>) : launch(linear_flash_kernel<0, 2>);
+    else if (R && lik == 3) e = F == 128 ? launch(linear_flash_kernel<8, 3>) : launch(linear_flash_kernel<0, 3>);
+    else if (R) e = F == 128 ? launch(linear_flash_kernel<8, 1>) : launch(linear_flash_kernel<0, 1>);
+    else e = F == 128 ? launch(linear_flash_kernel<8>) : launch(linear_flash_kernel<0>);
+    if (e) return e;
     BRN_LAUNCH_OK("linear_flash_kernel");
     return 0;
 }

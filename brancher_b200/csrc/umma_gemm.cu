@@ -160,8 +160,7 @@ extern "C" int brn_gemm_nt_3xtf32(const float* A, const float* B, float* D, int 
     if (int e = launch_split_tf32(A, K, M, K, Ah, Al, ld, nullptr, nullptr, 0, stream)) return e;
     if (int e = launch_split_tf32(B, K, N, K, Bh, Bl, ld, nullptr, nullptr, 0, stream)) return e;
     set_variant("tcgen05");
-    int drain = 2;
-    if (const char* env = getenv("BRN_UMMA_DRAIN")) drain = atoi(env);
+    constexpr int drain = 2;      // TMEM accumulation chain of 2 x 32 words of K between register drains (umma_gemm.cuh)
     // N tile / epilogue warps: 224 x 8 by default; BRN_GEMM_BN = 208 | 256 select the other instantiated shapes (tile-shape
     // measurements, profiles/gemm_bn_sweep.py)
     int bn = 224;

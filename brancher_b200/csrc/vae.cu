@@ -4,10 +4,10 @@
 // rows = s_local * B (decoder) or B (encoder).  All of them run on the tcgen05 3xTF32 GEMM of umma_gemm.cuh:
 //   forward   act_i   = relu(act_{i-1} . W_i^T + b_i)                  A = act_{i-1} [rows][n_in],  B = W_i   [n_out][n_in]
 //   data grad dpre_{i-1} = (dpre_i . W_i) * relu'(act_{i-1})           A = dpre_i    [rows][n_out], B = W_i^T [n_in][n_out]
-//   weight grad dW_i  = dpre_i^T . act_{i-1}                            A = dpre_i^T  [n_out][rows], B = act_{i-1}^T [n_in][rows]
+//   weight grad dW_i  = dpre_i^T . act_{i-1}                            A = dpre_i    [rows][n_out], B = act_{i-1} [rows][n_in]
 // with the bias / ReLU / Bernoulli likelihood / ReLU mask / bias-gradient column sums fused into the GEMM epilogues,
-// which write each activation (gradient) tensor in the two K-major layouts its consumers need (row-major for the next
-// layer's forward / data-gradient GEMM, transposed for the weight-gradient GEMM), already split into TF32 (hi, lo).
+// which write each activation (gradient) tensor once, row-major, as one plain fp32 matrix: the forward and data-gradient
+// GEMMs read it K-major and the weight-gradient GEMM MN-major, and both split it into TF32 (hi, lo) on the fly.
 // The K = L (latent, 2 in the example) layers -- encoder heads, sampling, first decoder layer -- are SIMT kernels.
 // Gradients are carried in "ELBO-sum units" (d sum_{s,b} elbo_sb / d .) in a zeroed scratch buffer and scaled by
 // -1/(S_total*B_total) into the caller's buffers by one final launch.
@@ -24,11 +24,10 @@ constexpr int VAE_BK = 16;          // K chunk (64-byte swizzle, 5-stage TMA rin
 constexpr int VAE_MAX_L = 16;       // latent sizes supported by the SIMT kernels
 constexpr int VAE_MAX_H0 = 1024;    // width of the first decoder layer supported by vae_dec0_bwd_kernel
 
-// [rows][n] tensor in the layouts the GEMMs consume
+// [rows][n] tensor as the GEMMs consume it
 struct VaeAct {
-    float *rm_hi, *rm_lo;     // [rows][ld]   K-major operand, K = n
-    float *t_hi, *t_lo;       // [n][ldt]     K-major operand, K = rows
-    int64_t ld, ldt;
+    float *rm_hi, *rm_lo;     // [rows][ld]   K-major operand (K = n) of the next layer, MN-major operand (K = rows) of the weight gradient
+    int64_t ld;
     int n;
 };
 
@@ -73,23 +72,13 @@ __device__ __forceinline__ float warp_colsum32(const float (&v)[32]) {
     return keep + __shfl_xor_sync(0xffffffffu, send, 1);
 }
 
-// write 4 consecutive columns of one row: TF32-split, row-major (vectorised when whole and aligned) + transposed
+// write 4 consecutive columns of one row, row-major (vectorised when whole and aligned), TF32-split
 // A NULL lo pointer means "this copy is ONE plain fp32 matrix" (the consuming GEMM splits it on the fly, SPLIT mask of
-// umma_gemm.cuh): row-major copies are always plain here, transposed copies are plain for gradient tensors.
-__device__ __forceinline__ void store_split4(const float (&v)[4], int nvalid, float* rh, float* rl, float* th, float* tl,
-                                             int64_t ldt) {
+// umma_gemm.cuh): row-major copies are always plain here.
+__device__ __forceinline__ void store_split4(const float (&v)[4], int nvalid, float* rh, float* rl) {
     float h[4], l[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) umma::split_tf32(v[j], h[j], l[j]);
-    if (th && tl) {
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-            if (j < nvalid) { th[(int64_t)j * ldt] = h[j]; tl[(int64_t)j * ldt] = l[j]; }
-    } else if (th) {
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-            if (j < nvalid) th[(int64_t)j * ldt] = v[j];
-    }
     if (!rl) {
         if (nvalid >= 4) *reinterpret_cast<float4*>(rh) = make_float4(v[0], v[1], v[2], v[3]);
         else {
@@ -108,11 +97,11 @@ __device__ __forceinline__ void store_split4(const float (&v)[4], int nvalid, fl
 }
 
 // ------------------------------------------------------------------------------------------------
-// epilogue: hidden layer forward.  out = relu(D + bias), TF32-split, both layouts.
+// epilogue: hidden layer forward.  out = relu(D + bias), row-major.
 // ------------------------------------------------------------------------------------------------
 struct EpiDense {
     struct Params {
-        const float* bias; float *rm_hi, *rm_lo, *t_hi, *t_lo; int64_t ld, ldt; int rows, cols;
+        const float* bias; float *rm_hi, *rm_lo; int64_t ld; int rows, cols;
     };
     template <int CPT>
     static __device__ __forceinline__ void finish(const Params& p, float (&r)[CPT], int row, int blk, bool, int) {
@@ -121,16 +110,13 @@ struct EpiDense {
         const int valid = min(CPT, p.cols - c0);
         float* rh = p.rm_hi + (int64_t)row * p.ld + c0;
         float* rl = p.rm_lo ? p.rm_lo + (int64_t)row * p.ld + c0 : nullptr;
-        float* th = p.t_hi ? p.t_hi + (int64_t)c0 * p.ldt + row : nullptr;      // NULL: no transposed copy (MN-major weight gradient)
-        float* tl = p.t_lo ? p.t_lo + (int64_t)c0 * p.ldt + row : nullptr;
 #pragma unroll
         for (int i = 0; i < CPT; i += 4) {
             if (i < valid) {
                 float v[4];
 #pragma unroll
                 for (int j = 0; j < 4; ++j) v[j] = (i + j < valid) ? fmaxf(r[i + j] + __ldg(p.bias + c0 + i + j), 0.f) : 0.f;
-                store_split4(v, valid - i, rh + i, rl ? rl + i : nullptr, th ? th + (int64_t)i * p.ldt : nullptr,
-                             tl ? tl + (int64_t)i * p.ldt : nullptr, p.ldt);
+                store_split4(v, valid - i, rh + i, rl ? rl + i : nullptr);
             }
         }
     }
@@ -139,12 +125,12 @@ struct EpiDense {
 // ------------------------------------------------------------------------------------------------
 // epilogue: decoder output layer + Binomial(1, logits) likelihood (distributions.py:561-575 with total_count = 1:
 // the three lgamma terms vanish):   l = D + bias ;  ll += x l - (max(l,0) + log(1 + e^-|l|)) ;  d = x - sigmoid(l)
-// d is written TF32-split in both layouts; its column sums are the output bias gradient.
+// d is written row-major; its column sums are the output bias gradient.
 // ------------------------------------------------------------------------------------------------
 struct EpiBern {
     struct Params {
         const float* bias; const float* X; int64_t ldx; int B;
-        float *rm_hi, *rm_lo, *t_hi, *t_lo; int64_t ld, ldt; int rows, cols; double* ll; float* dbias;
+        float *rm_hi, *rm_lo; int64_t ld; int rows, cols; double* ll; float* dbias;
     };
     template <int CPT>
     static __device__ __forceinline__ void finish(const Params& p, float (&r)[CPT], int row, int blk, bool, int) {
@@ -158,8 +144,6 @@ struct EpiBern {
         const float* x = p.X + (int64_t)(row_ok ? row % p.B : 0) * p.ldx + c0;
         float* rh = p.rm_hi + (int64_t)row * p.ld + c0;
         float* rl = p.rm_lo ? p.rm_lo + (int64_t)row * p.ld + c0 : nullptr;
-        float* th = p.t_hi ? p.t_hi + (int64_t)c0 * p.ldt + row : nullptr;      // NULL: no transposed copy (MN-major weight gradient)
-        float* tl = p.t_lo ? p.t_lo + (int64_t)c0 * p.ldt + row : nullptr;
         float ll = 0.f;
         if (valid == CPT && (reinterpret_cast<uintptr_t>(x) & 15) == 0) {
             // full, aligned block (the common case).  The epilogue warps were stalled on the per-element x loads 57 % of the
@@ -200,8 +184,7 @@ struct EpiBern {
                                 ll += __fmaf_rn(xv, l, -__fmaf_rn(lg, 0.6931471805599453f, fmaxf(l, 0.f)));
                                 v[j] = xv - sig;
                             }
-                            store_split4(v, 4, rh + i, rl ? rl + i : nullptr, th ? th + (int64_t)i * p.ldt : nullptr,
-                                         tl ? tl + (int64_t)i * p.ldt : nullptr, p.ldt);
+                            store_split4(v, 4, rh + i, rl ? rl + i : nullptr);
                         }
 #pragma unroll
                         for (int j = 0; j < 4; ++j) d32[hb + 4 * q + j] = v[j];
@@ -233,8 +216,7 @@ struct EpiBern {
                             v[j] = xv - sig;
                         }
                     }
-                    store_split4(v, valid - i0 - i, rh + i0 + i, rl ? rl + i0 + i : nullptr, th ? th + (int64_t)(i0 + i) * p.ldt : nullptr,
-                                 tl ? tl + (int64_t)(i0 + i) * p.ldt : nullptr, p.ldt);
+                    store_split4(v, valid - i0 - i, rh + i0 + i, rl ? rl + i0 + i : nullptr);
                 }
 #pragma unroll
                 for (int j = 0; j < 4; ++j) d32[i + j] = v[j];
@@ -250,13 +232,13 @@ struct EpiBern {
 };
 
 // ------------------------------------------------------------------------------------------------
-// epilogue: data gradient.  g = D * [mask > 0]  (mask = the hi part of the layer's ReLU output), written TF32-split in
-// both layouts (or as plain fp32 row-major when `plain` is set: the first decoder layer's SIMT backward reads that);
+// epilogue: data gradient.  g = D * [mask > 0]  (mask = the hi part of the layer's ReLU output), written row-major
+// (to `plain` when it is set: the first decoder layer's SIMT backward reads that);
 // column sums of g = the layer's bias gradient.
 // ------------------------------------------------------------------------------------------------
 struct EpiMask {
     struct Params {
-        const float* mask; int64_t ldm; float *rm_hi, *rm_lo, *t_hi, *t_lo; int64_t ld, ldt; float* plain; int64_t ldp;
+        const float* mask; int64_t ldm; float *rm_hi, *rm_lo; int64_t ld; float* plain; int64_t ldp;
         int rows, cols; float* dbias;
     };
     template <int CPT>
@@ -309,9 +291,7 @@ struct EpiMask {
                         }
                     } else {
                         store_split4(v, valid - col, p.rm_hi + (int64_t)row * p.ld + c0 + col,
-                                     p.rm_lo ? p.rm_lo + (int64_t)row * p.ld + c0 + col : nullptr,
-                                     p.t_hi ? p.t_hi + (int64_t)(c0 + col) * p.ldt + row : nullptr,
-                                     p.t_lo ? p.t_lo + (int64_t)(c0 + col) * p.ldt + row : nullptr, p.ldt);
+                                     p.rm_lo ? p.rm_lo + (int64_t)row * p.ld + c0 + col : nullptr);
                     }
                 }
 #pragma unroll
@@ -326,10 +306,8 @@ struct EpiMask {
 // N tile: 128 with SIXTEEN epilogue warps when N is a multiple of 128 (every hidden width of C5: the epilogues -- bias / ReLU /
 // mask / split stores -- are the bound of these GEMMs, and twice the warps at half the columns per thread hide their latency);
 // otherwise the narrowest instantiated width that covers N in ceil(N / 208) tiles, eight epilogue warps.
-// BRN_VAE_EW16=0 restores the round-1 choice for A/B runs.
 static int pick_bn(int N) {
-    static const bool ew16 = [] { const char* e = getenv("BRN_VAE_EW16"); return !(e && atoi(e) == 0); }();
-    if (ew16 && N % 128 == 0) return -128;
+    if (N % 128 == 0) return -128;
     const int nt = (N + 207) / 208, per = (N + nt - 1) / nt;
     return per <= 128 ? 128 : (per <= 176 ? 176 : 208);
 }
@@ -338,13 +316,9 @@ template <class Epi>
 static int launch_gemm(const float* Ah, const float* Al, int M, int64_t lda, const float* Bh, const float* Bl, int N, int64_t ldb,
                        int K, int mode, const typename Epi::Params& ep, cudaStream_t stream, bool allow_split = false) {
     switch (pick_bn(N)) {
-        // every A operand of K5 (activations, gradients; row-major or transposed) is one plain fp32 matrix: SPLIT = 1
-        case -128: {
-            // converter warps (they split the plain fp32 A tile into the TF32 pair inside the stage): 2 by default; BRN_VAE_CW=4
-            static const int cw = [] { const char* e = getenv("BRN_VAE_CW"); return e ? atoi(e) : 2; }();
-            if (cw == 4) return launch_umma_nt<128, VAE_BK, Epi, 16, 1, 4>(Ah, nullptr, M, lda, Bh, Bl, N, ldb, K, mode, 2, ep, stream, allow_split);
-            return launch_umma_nt<128, VAE_BK, Epi, 16, 1, 2>(Ah, nullptr, M, lda, Bh, Bl, N, ldb, K, mode, 2, ep, stream, allow_split);
-        }
+        // every A operand of K5 (activations, gradients) is one plain fp32 matrix: SPLIT = 1, two converter warps (they split
+        // the plain fp32 A tile into the TF32 pair inside the stage)
+        case -128: return launch_umma_nt<128, VAE_BK, Epi, 16, 1, 2>(Ah, nullptr, M, lda, Bh, Bl, N, ldb, K, mode, 2, ep, stream, allow_split);
         case 128: return launch_umma_nt<128, VAE_BK, Epi, UG_EPI_WARPS, 1, 2>(Ah, nullptr, M, lda, Bh, Bl, N, ldb, K, mode, 2, ep, stream,
                                                                            allow_split);
         case 176: return launch_umma_nt<176, VAE_BK, Epi, UG_EPI_WARPS, 1, 2>(Ah, nullptr, M, lda, Bh, Bl, N, ldb, K, mode, 2, ep, stream,
@@ -390,7 +364,7 @@ __device__ __forceinline__ float dec0_value(const float* zs, const float* __rest
 }
 
 // z = mean + eps * sd (Normal.rsample, distributions.py:122), log p(z) = sum_lat N(z; 0, 1), and the first decoder layer
-// g_0 = relu(V_0 z + c_0) written TF32-split in both layouts.  32 rows (row = s * B + b) per block.
+// g_0 = relu(V_0 z + c_0) written row-major as plain fp32.  32 rows (row = s * B + b) per block.
 __global__ void __launch_bounds__(256)
 vae_sample_dec0_kernel(const float* __restrict__ mean, const float* __restrict__ sd, const float* __restrict__ eps_in, int B, int L,
                        int R, int64_t row0_global, brn_sample_range r, uint32_t var_id, const float* __restrict__ V0,
@@ -417,20 +391,10 @@ vae_sample_dec0_kernel(const float* __restrict__ mean, const float* __restrict__
     __syncthreads();
     const float tot = block_sum(lp, red);
     if (tid == 0 && tot != 0.f) atomicAdd(lpz_acc, (double)tot);
-    for (int idx = tid; idx < 32 * h0; idx += 256) {            // row-major copy: consecutive threads -> consecutive columns
+    for (int idx = tid; idx < 32 * h0; idx += 256) {            // consecutive threads -> consecutive columns
         const int rr = idx / h0, j = idx % h0, row = r0 + rr;
         if (row < R) {
-            a0.rm_hi[(int64_t)row * a0.ld + j] = dec0_value(zs + rr * L, V0, c0, L, j);       // row-major copy: plain fp32
-        }
-    }
-    if (a0.t_hi)
-    for (int idx = tid; idx < 32 * h0; idx += 256) {            // transposed copy: consecutive threads -> consecutive rows
-        const int j = idx >> 5, rr = idx & 31, row = r0 + rr;
-        if (row < R) {
-            float hi, lo;
-            umma::split_tf32(dec0_value(zs + rr * L, V0, c0, L, j), hi, lo);
-            a0.t_hi[(int64_t)j * a0.ldt + row] = hi;
-            a0.t_lo[(int64_t)j * a0.ldt + row] = lo;
+            a0.rm_hi[(int64_t)row * a0.ld + j] = dec0_value(zs + rr * L, V0, c0, L, j);
         }
     }
 }
@@ -504,7 +468,7 @@ vae_dec0_bwd_kernel(const float* __restrict__ dpre0, int64_t ld0, const float* _
 }
 
 // backward of the encoder heads: entropy gradient, softplus chain rule, head weight / bias gradients, and the gradient
-// w.r.t. the last hidden layer's pre-activation (ReLU-masked, TF32-split, both layouts) + that layer's bias gradient.
+// w.r.t. the last hidden layer's pre-activation (ReLU-masked, row-major plain fp32) + that layer's bias gradient.
 template <int LP>
 __global__ void __launch_bounds__(256)
 vae_heads_bwd_kernel(const float* __restrict__ dmean, const float* __restrict__ dsd, const float* __restrict__ sd,
@@ -512,7 +476,6 @@ vae_heads_bwd_kernel(const float* __restrict__ dmean, const float* __restrict__ 
                      const float* __restrict__ a_lo, int64_t lda, const float* __restrict__ Wm, const float* __restrict__ Ws, int h,
                      VaeAct dpre, float* gWm, float* gWs, float* gbm, float* gbs, float* gb_last) {
     __shared__ float dm[32][LP], dsp[32][LP];
-    __shared__ float tile[8][32][33];
     const int b0 = blockIdx.x * 32, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
     for (int idx = tid; idx < 32 * LP; idx += 256) {
         const int rr = idx / LP, l = idx % LP, b = b0 + rr;
@@ -544,7 +507,6 @@ vae_heads_bwd_kernel(const float* __restrict__ dmean, const float* __restrict__ 
         float colsum = 0.f;
         for (int rr = 0; rr < 32; ++rr) {
             const int b = b0 + rr;
-            float v = 0.f;
             if (jok && b < B) {
                 const float ahi = a_hi[(int64_t)b * lda + j], a = ahi + (a_lo ? a_lo[(int64_t)b * lda + j] : 0.f);
                 float g = 0.f;
@@ -555,20 +517,11 @@ vae_heads_bwd_kernel(const float* __restrict__ dmean, const float* __restrict__ 
                     am[l] = __fmaf_rn(dm[rr][l], a, am[l]);
                     as[l] = __fmaf_rn(dsp[rr][l], a, as[l]);
                 }
-                v = ahi > 0.f ? g : 0.f;
-                dpre.rm_hi[(int64_t)b * dpre.ld + j] = v;          // gradient tensor: both copies plain fp32
+                const float v = ahi > 0.f ? g : 0.f;
+                dpre.rm_hi[(int64_t)b * dpre.ld + j] = v;
                 colsum += v;
             }
-            tile[w][rr][lane] = v;
         }
-        __syncwarp();
-        for (int i = 0; i < 32; ++i) {
-            const int jj = c0 + i, b = b0 + lane;
-            if (jj < h && b < B && dpre.t_hi) {
-                dpre.t_hi[(int64_t)jj * dpre.ldt + b] = tile[w][lane][i];
-            }
-        }
-        __syncwarp();
         if (jok) {
             atomicAdd(gb_last + j, colsum);
 #pragma unroll
@@ -629,21 +582,19 @@ struct VaeWorkspace {
             return p;
         };
         auto take = [&](size_t nfloat) { return reinterpret_cast<float*>(takeb(nfloat * sizeof(float))); };
-        // rm: ONE plain fp32 matrix (rm_lo == NULL: always the A operand of a SPLIT = 1 GEMM); t: the TF32 (hi, lo) pair for
-        // activations (B operand of the weight-gradient GEMM), one plain matrix for gradient tensors (its A operand)
-        auto act = [&](VaeAct& a, int64_t rows, int n, bool grad = false) {
-            a.n = n; a.ld = pad4l(n); a.ldt = pad4l(rows);
+        // ONE plain fp32 matrix (rm_lo == NULL): the GEMMs that read it split it on the fly (SPLIT mask of umma_gemm.cuh)
+        auto act = [&](VaeAct& a, int64_t rows, int n) {
+            a.n = n; a.ld = pad4l(n);
             a.rm_hi = take((size_t)rows * a.ld); a.rm_lo = nullptr;
-            a.t_hi = take((size_t)n * a.ldt); a.t_lo = grad ? nullptr : take((size_t)n * a.ldt);
         };
         const int64_t R = (int64_t)S * B;
         act(Xa, B, m.D);
-        for (int i = 0; i < m.n_enc; ++i) { act(enc_a[i], B, m.enc[i].n_out); act(enc_d[i], B, m.enc[i].n_out, true); }
+        for (int i = 0; i < m.n_enc; ++i) { act(enc_a[i], B, m.enc[i].n_out); act(enc_d[i], B, m.enc[i].n_out); }
         for (int i = 0; i < m.n_dec; ++i) {
             act(dec_a[i], R, m.dec[i].n_out);
-            if (i > 0) act(dec_d[i], R, m.dec[i].n_out, true);
+            if (i > 0) act(dec_d[i], R, m.dec[i].n_out);
         }
-        act(dL, R, m.D, true);
+        act(dL, R, m.D);
         ld0 = pad4l(m.dec[0].n_out);
         dpre0 = take((size_t)R * ld0);
         mean = take((size_t)B * m.L); sd = take((size_t)B * m.L); sdpre = take((size_t)B * m.L);
@@ -748,23 +699,11 @@ extern "C" int brn_vae_elbo_fwd_bwd(const float* X, int B, int64_t row0, int64_t
     BRN_CUDA_OK(cudaMemsetAsync(ws.zero_begin, 0, ws.zero_bytes, stream));
     double* acc_ll = ws.acc, *acc_lpz = ws.acc + 1, *acc_ent = ws.acc + 2;
 
-    // Weight gradients read the row-major activations / gradients MN-major (launch_umma_tn_plain): no transposed copy of any
-    // activation or gradient tensor is written (BRN_VAE_WGRAD_MN=0 restores the round-1 transposed K-major operands).
-    bool wgrad_mn = true;
-    if (const char* env = getenv("BRN_VAE_WGRAD_MN")) wgrad_mn = atoi(env) != 0;
-    if (wgrad_mn) {
-        auto drop_t = [](VaeAct& a) { a.t_hi = nullptr; a.t_lo = nullptr; };
-        drop_t(ws.Xa); drop_t(ws.dL);
-        for (int i = 0; i < m->n_enc; ++i) { drop_t(ws.enc_a[i]); drop_t(ws.enc_d[i]); }
-        for (int i = 0; i < m->n_dec; ++i) { drop_t(ws.dec_a[i]); if (i > 0) drop_t(ws.dec_d[i]); }
-    }
-    // 0. TF32-split operands: X and every weight matrix a GEMM reads, in both K-major layouts
+    // 0. operands: X as a plain row-major copy, every weight matrix a GEMM reads TF32-split in both K-major layouts
     {
         StageTimer st("vae.split_operands", stream);
         BRN_CUDA_OK(cudaMemcpy2DAsync(ws.Xa.rm_hi, ws.Xa.ld * sizeof(float), X, D * sizeof(float), D * sizeof(float), B,
                                       cudaMemcpyDeviceToDevice, stream));         // plain row-major copy with the padded pitch
-        if (!wgrad_mn)
-            if (int e = launch_split_tf32(X, D, B, D, nullptr, nullptr, ws.Xa.ld, ws.Xa.t_hi, ws.Xa.t_lo, ws.Xa.ldt, stream)) return e;
         auto wsplit = [&](const brn_dense_layer& l, VaeWeights& w) {
             return launch_split_tf32(l.W, l.n_in, l.n_out, l.n_in, w.hi, w.lo, w.ld, w.t_hi, w.t_lo, w.ldt, stream);
         };
@@ -774,7 +713,7 @@ extern "C" int brn_vae_elbo_fwd_bwd(const float* X, int B, int64_t row0, int64_t
     }
     auto dense_fwd = [&](const VaeAct& in, int64_t rows, const brn_dense_layer& l, const VaeWeights& w, VaeAct& out) {
         EpiDense::Params ep;
-        ep.bias = l.b; ep.rm_hi = out.rm_hi; ep.rm_lo = out.rm_lo; ep.t_hi = out.t_hi; ep.t_lo = out.t_lo; ep.ld = out.ld; ep.ldt = out.ldt;
+        ep.bias = l.b; ep.rm_hi = out.rm_hi; ep.rm_lo = out.rm_lo; ep.ld = out.ld;
         ep.rows = (int)rows; ep.cols = l.n_out;
         return launch_gemm<EpiDense>(in.rm_hi, in.rm_lo, (int)rows, in.ld, w.hi, w.lo, l.n_out, w.ld, l.n_in, 2, ep, stream);
     };
@@ -784,35 +723,24 @@ extern "C" int brn_vae_elbo_fwd_bwd(const float* X, int B, int64_t row0, int64_t
         EpiMask::Params ep;
         ep.mask = a_prev.rm_hi; ep.ldm = a_prev.ld;
         ep.rm_hi = dprev ? dprev->rm_hi : nullptr; ep.rm_lo = dprev ? dprev->rm_lo : nullptr;
-        ep.t_hi = dprev ? dprev->t_hi : nullptr; ep.t_lo = dprev ? dprev->t_lo : nullptr;
-        ep.ld = dprev ? dprev->ld : 0; ep.ldt = dprev ? dprev->ldt : 0; ep.plain = plain; ep.ldp = ldp;
+        ep.ld = dprev ? dprev->ld : 0; ep.plain = plain; ep.ldp = ldp;
         ep.rows = (int)rows; ep.cols = l.n_in; ep.dbias = gb_prev;
         return launch_gemm<EpiMask>(dcur.rm_hi, dcur.rm_lo, (int)rows, dcur.ld, w.t_hi, w.t_lo, l.n_in, w.ldt, l.n_out, 2, ep, stream);
     };
-    // gW = dpre^T . a_in   (K = rows: few output tiles, so the K range is split over the SMs with atomic partial sums)
+    // gW = dpre^T . a_in, read MN-major from the row-major tensors (launch_umma_tn_plain: no transposed copies)
+    // (K = rows: few output tiles, so the K range is split over the SMs with atomic partial sums)
     auto weight_grad = [&](const VaeAct& dcur, const VaeAct& a_in, int64_t rows, const brn_dense_layer& l, float* gW) {
         EpiStore::Params ep;
-        if (wgrad_mn) {
-            constexpr int cpt = 64;        // columns per epilogue thread of every variant below
-            ep.out = gW; ep.rows = l.n_out; ep.row_stride = l.n_in; ep.col_stride = 1; ep.blk_stride = cpt; ep.blk_valid = cpt;
-            ep.col_limit = l.n_in; ep.total_blks = (l.n_in + cpt - 1) / cpt;
-            // N tile 256 with sixteen epilogue and eight converter warps where the layer's input width allows it (measured at C5:
-            // 1.745 ms per evaluation against 1.78 with 128-column tiles); BRN_VAE_WGRAD_TILE = 0 | 1 | 2 forces a variant
-            static const int tile = [] { const char* e = getenv("BRN_VAE_WGRAD_TILE"); return e ? atoi(e) : 2; }();
-            if (tile == 1)
-                return launch_umma_tn_plain<128, VAE_BK, EpiStore, UG_EPI_WARPS, 8>(dcur.rm_hi, l.n_out, dcur.ld, a_in.rm_hi, l.n_in, a_in.ld,
-                                                                                    (int)rows, 0, 2, ep, stream, true);
-            if (tile == 2 && l.n_in % 256 == 0)
-                return launch_umma_tn_plain<256, VAE_BK, EpiStore, 16, 8>(dcur.rm_hi, l.n_out, dcur.ld, a_in.rm_hi, l.n_in, a_in.ld,
-                                                                          (int)rows, 0, 2, ep, stream, true);
-            return launch_umma_tn_plain<128, VAE_BK, EpiStore, UG_EPI_WARPS, 4>(dcur.rm_hi, l.n_out, dcur.ld, a_in.rm_hi, l.n_in, a_in.ld,
-                                                                                (int)rows, 0, 2, ep, stream, true);
-        }
-        const int tile = pick_bn(l.n_in), bn = tile < 0 ? -tile : tile, cpt = bn / (tile < 0 ? 4 : 2);      // columns per epilogue thread
+        constexpr int cpt = 64;        // columns per epilogue thread of both variants below
         ep.out = gW; ep.rows = l.n_out; ep.row_stride = l.n_in; ep.col_stride = 1; ep.blk_stride = cpt; ep.blk_valid = cpt;
         ep.col_limit = l.n_in; ep.total_blks = (l.n_in + cpt - 1) / cpt;
-        return launch_gemm<EpiStore>(dcur.t_hi, dcur.t_lo, l.n_out, dcur.ldt, a_in.t_hi, a_in.t_lo, l.n_in, a_in.ldt, (int)rows, 0, ep,
-                                     stream, true);
+        // N tile 256 with sixteen epilogue and eight converter warps where the layer's input width allows it (measured at C5:
+        // 1.745 ms per evaluation against 1.78 with 128-column tiles)
+        if (l.n_in % 256 == 0)
+            return launch_umma_tn_plain<256, VAE_BK, EpiStore, 16, 8>(dcur.rm_hi, l.n_out, dcur.ld, a_in.rm_hi, l.n_in, a_in.ld,
+                                                                      (int)rows, 0, 2, ep, stream, true);
+        return launch_umma_tn_plain<128, VAE_BK, EpiStore, UG_EPI_WARPS, 4>(dcur.rm_hi, l.n_out, dcur.ld, a_in.rm_hi, l.n_in, a_in.ld,
+                                                                            (int)rows, 0, 2, ep, stream, true);
     };
 
     // 1. encoder forward
@@ -846,7 +774,7 @@ extern "C" int brn_vae_elbo_fwd_bwd(const float* X, int B, int64_t row0, int64_t
         const VaeAct& in = ws.dec_a[m->n_dec - 1];
         EpiBern::Params ep;
         ep.bias = m->dec_out.b; ep.X = X; ep.ldx = D; ep.B = B;
-        ep.rm_hi = ws.dL.rm_hi; ep.rm_lo = ws.dL.rm_lo; ep.t_hi = ws.dL.t_hi; ep.t_lo = ws.dL.t_lo; ep.ld = ws.dL.ld; ep.ldt = ws.dL.ldt;
+        ep.rm_hi = ws.dL.rm_hi; ep.rm_lo = ws.dL.rm_lo; ep.ld = ws.dL.ld;
         ep.rows = (int)R; ep.cols = D; ep.ll = acc_ll; ep.dbias = ws.outW.gb;
         if (int e = launch_gemm<EpiBern>(in.rm_hi, in.rm_lo, (int)R, in.ld, ws.outW.hi, ws.outW.lo, D, ws.outW.ld, m->dec_out.n_in, 2, ep,
                                          stream))

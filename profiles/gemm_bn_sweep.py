@@ -25,6 +25,6 @@ st = cu.profile_collect(); cu.profile_enable(False)
 ms, calls = st["gemm.umma"]
 ref = (A[:64].double() @ B[:512].double().T)
 err = (D[:64, :512].double() - ref).abs().max().item()
-print("BN=%s drain=%s: %.1f us per launch, %.1f TFLOP/s fp32-equivalent, max err %.2e" % (
-    os.environ.get("BRN_GEMM_BN", "224"), os.environ.get("BRN_UMMA_DRAIN", "2"), 1e3 * ms / calls,
+print("BN=%s: %.1f us per launch, %.1f TFLOP/s fp32-equivalent, max err %.2e" % (
+    os.environ.get("BRN_GEMM_BN", "224"), 1e3 * ms / calls,
     2.0 * M * N * K / (ms / calls * 1e-3) / 1e12, err))

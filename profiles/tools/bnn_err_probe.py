@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Error of the K3 CUDA path against the fp64 oracle, relative to each tensor's own scale (max |g|), for one shape.
-Run on a B200:  BRN_UMMA_DRAIN=4 BRN_BNN_MID=4 python profiles/tools/bnn_err_probe.py [B P H C S tied]"""
+Run on a B200:  python profiles/tools/bnn_err_probe.py [B P H C S tied]"""
 import os
 import sys
 
@@ -23,8 +23,8 @@ prior = None if tied else {n: (0.0, 10.0) for n in shapes}
 l64, g64 = O.bnn_elbo(X, y, params, eps, prior, dtype=torch.float64, sample_chunk=4)
 l32, g32 = O.bnn_elbo(X, y, params, eps, prior, sample_chunk=4)
 loss, grads, _ = T.run_bnn(cu, X, y, params, eps, prior)
-print("drain=%s mid=%s variant=%s  loss rel err %.2e (fp32 oracle %.2e)" % (
-    os.environ.get("BRN_UMMA_DRAIN", "-"), os.environ.get("BRN_BNN_MID", "-"), cu.last_variant(),
+print("variant=%s  loss rel err %.2e (fp32 oracle %.2e)" % (
+    cu.last_variant(),
     abs(loss - l64) / abs(l64), abs(l32 - l64) / abs(l64)))
 for k in sorted(g64):
     sc = np.abs(g64[k]).max()

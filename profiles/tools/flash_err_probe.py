@@ -1,5 +1,5 @@
-"""Probe: signed loss / gradient error of the K2 variants (staged GEMM pair, one-pass kernel with its fallbacks) against the fp64
-oracle at a C2-shaped problem.  Usage: python profiles/tools/flash_err_probe.py [N] [S]
+"""Probe: signed loss / gradient error of the K2 variants (staged GEMM pair, one-pass kernel, the latter also with y at a 4-byte
+offset, which loads the targets per lane) against the fp64 oracle at a C2-shaped problem.  Usage: python profiles/tools/flash_err_probe.py [N] [S]
 (This probe found the loss error that grew linearly with N: a per-thread fp32 running sum of the log-likelihood.)"""
 import os, sys
 import numpy as np
@@ -22,14 +22,15 @@ r = cu.sample_range(S, seed=3, offset=5)
 eps = {"weights": cu.philox_normal(F, 0, r, DEV).cpu().numpy().reshape(S, 1, F)}
 l64, g64 = O.logreg_elbo_streamed(X.numpy(), y.numpy(), params, eps, prior)
 Xd, yd = X.to(DEV), y.to(DEV)
-for env in ({"BRN_LINEAR_FLASH": "0"}, {}, {"BRN_LINEAR_DTMEM": "0"}, {"BRN_LINEAR_Y_BULK": "0"}):
-    for k in ("BRN_LINEAR_FLASH", "BRN_LINEAR_DTMEM", "BRN_LINEAR_Y_BULK"):
-        os.environ.pop(k, None)
+y_off = torch.empty(N + 1, device=DEV)[1:]
+y_off.copy_(yd)
+for env, yt in (({"BRN_LINEAR_FLASH": "0"}, yd), ({}, yd), ({}, y_off)):
+    os.environ.pop("BRN_LINEAR_FLASH", None)
     os.environ.update(env)
     w = cu.MeanFieldVar(torch.tensor(params["weights"][0], device=DEV), torch.tensor(params["weights"][1], device=DEV), var_id=0,
                         prior_loc=torch.zeros(1, F, device=DEV), prior_scale=torch.full((1, F), 0.5, device=DEV))
-    loss = cu.linear_elbo_fwd_bwd(Xd, yd, cu.BERNOULLI, w, 1, r).item()
+    loss = cu.linear_elbo_fwd_bwd(Xd, yt, cu.BERNOULLI, w, 1, r).item()
     gm = w.dmu.cpu().numpy().reshape(1, F); gs = w.drho.cpu().numpy().reshape(1, F)
-    print(env, cu.last_variant(), "loss rel err %+.3e" % ((loss - l64) / abs(l64)),
+    print(env, "y offset %d" % (yt.data_ptr() % 16), cu.last_variant(), "loss rel err %+.3e" % ((loss - l64) / abs(l64)),
           "dmu %.3e drho %.3e" % (np.abs(gm - g64["weights_loc"]).max() / np.abs(g64["weights_loc"]).max(),
                                   np.abs(gs - g64["weights_scale"]).max() / np.abs(g64["weights_scale"]).max()))

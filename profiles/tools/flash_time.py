@@ -1,5 +1,5 @@
 """Time one K2 evaluation (CUDA events around linear_elbo_fwd_bwd at the C2 shape, X re-prepared in every call) for each setting of
-an environment switch: python profiles/tools/flash_time.py [VAR=value ...], e.g. BRN_LINEAR_DTMEM=0 BRN_LINEAR_Y_BULK=0 BRN_LINEAR_FLASH=0.
+an environment switch: python profiles/tools/flash_time.py [VAR=value ...], e.g. default=1 BRN_LINEAR_FLASH=0.
 (During development the kernel had a BRN_LF_DBG mask that skipped MMAs / epilogue math / loads / barriers to find the critical path:
 profiles/r2f_flash_history.txt.)"""
 import os, sys, torch

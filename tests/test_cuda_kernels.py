@@ -23,6 +23,16 @@ def dev(a, dtype=torch.float32):
     return torch.as_tensor(np.asarray(a), dtype=dtype).to(DEV).contiguous()
 
 
+def dev_offset(a, dtype=torch.float32):
+    """a on the device as a contiguous view whose data starts 4 bytes past an allocation (not 16-byte aligned)"""
+    t = dev(a, dtype)
+    buf = torch.empty(t.numel() + 1, dtype=dtype, device=DEV)
+    out = buf[1:].view(t.shape)
+    out.copy_(t)
+    assert out.data_ptr() % 16 == 4
+    return out
+
+
 def make_vars(cu, params, eps, names, prior=None, shapes=None):
     out = []
     for i, n in enumerate(names):
@@ -149,11 +159,12 @@ def test_bnn_philox_mode_and_shard_invariance(cu):
 
 
 # ---------------------------------------------------------------------------------------------
-def run_linear(cu, X, y, params, eps, lik, C, prior=None, r=None):
+def run_linear(cu, X, y, params, eps, lik, C, prior=None, r=None, x_offset=False, y_offset=False):
+    """x_offset / y_offset: pass X / y at a 4-byte offset from a 16-byte boundary"""
     S = eps["weights"].shape[0] if eps is not None else r.s_local
     (w,) = make_vars(cu, params, eps, ["weights"], prior)
-    yd = dev(y, torch.float32 if lik == cu.BERNOULLI else torch.int32)
-    loss = cu.linear_elbo_fwd_bwd(dev(X), yd, lik, w, C, r or cu.sample_range(S))
+    yd = (dev_offset if y_offset else dev)(y, torch.float32 if lik == cu.BERNOULLI else torch.int32)
+    loss = cu.linear_elbo_fwd_bwd((dev_offset if x_offset else dev)(X), yd, lik, w, C, r or cu.sample_range(S))
     return loss.item(), grads_of([w], ["weights"], params)
 
 
@@ -203,14 +214,13 @@ def test_linear_random_shapes(cu, N, F, C, S, lik):
 
 @pytest.mark.parametrize("N,F,S,tied", [(1, 4, 1, True), (300, 8, 5, False), (1000, 128, 70, False), (5000, 128, 300, True),
                                          (20000, 64, 130, False)])
-@pytest.mark.parametrize("split_a", ["7", "0", "1", "5"])
-def test_linear_tcgen05_variant(cu, monkeypatch, N, F, S, tied, split_a):
-    """K2 on the tensor cores: logits GEMM with the Bernoulli likelihood fused in its epilogue + K-split gradient GEMM.
-    split_a = 1 (default): d^T crosses HBM as plain fp32 and converter warps split it inside the gradient GEMM;
-    0: the epilogue writes the TF32 (hi, lo) pair."""
+@pytest.mark.parametrize("x_offset", [False, True])
+def test_linear_tcgen05_variant(cu, monkeypatch, N, F, S, tied, x_offset):
+    """K2 on the tensor cores: logits GEMM with the Bernoulli likelihood fused in its epilogue + K-split gradient GEMM; d^T
+    crosses HBM as plain fp32 and converter warps split it inside the gradient GEMM.  A 16-byte aligned X is read in place
+    by the logits GEMM (its converter warps split it); X at a 4-byte offset is split into a (hi, lo) pair first."""
     from oracle import elbo_oracle as O
     monkeypatch.setenv("BRN_LINEAR_VARIANT", "tcgen05")
-    monkeypatch.setenv("BRN_LINEAR_SPLIT_A", split_a)
     monkeypatch.setenv("BRN_LINEAR_FLASH", "0")           # the staged GEMM pair (the one-pass kernel has its own test below)
     rng = np.random.RandomState(N + F + S)
     X = rng.randn(N, F).astype("f4")
@@ -220,25 +230,22 @@ def test_linear_tcgen05_variant(cu, monkeypatch, N, F, S, tied, split_a):
     prior = None if tied else {"weights": (0.0, 0.5)}
     o32 = O.logreg_elbo(X, y, params, eps, prior, row_chunk=4096)
     o64 = O.logreg_elbo(X, y, params, eps, prior, dtype=torch.float64, row_chunk=4096)
-    loss, grads = run_linear(cu, X, y, params, eps, cu.BERNOULLI, 1, prior)
+    loss, grads = run_linear(cu, X, y, params, eps, cu.BERNOULLI, 1, prior, x_offset=x_offset)
     assert cu.last_variant() == "tcgen05"
-    check_against_oracle(loss, grads, o32, o64, "linear tcgen05 N=%d F=%d S=%d" % (N, F, S))
+    check_against_oracle(loss, grads, o32, o64, "linear tcgen05 N=%d F=%d S=%d x_offset=%s" % (N, F, S, x_offset))
 
 
 @pytest.mark.parametrize("N,F,S,tied", [(1, 16, 1, True), (63, 32, 3, False), (64, 16, 128, False), (777, 48, 129, True),
                                          (1000, 128, 70, False), (5000, 128, 300, True), (20000, 64, 130, False),
                                          (130001, 96, 200, False), (9473, 112, 1000, True)])
-@pytest.mark.parametrize("mode", ["default", "y_ldg", "d_smem"])
+@pytest.mark.parametrize("mode", ["default", "y_ldg"])
 def test_linear_flash_variant(cu, monkeypatch, N, F, S, tied, mode):
-    """K2 in one pass over X (linear_flash.cuh): logits MMA -> Bernoulli likelihood -> d through shared memory -> gradient
+    """K2 in one pass over X (linear_flash.cuh): logits MMA -> Bernoulli likelihood -> d tile in tensor memory -> gradient
     MMA, fp16 (hi, lo) operand pairs.  Ragged row blocks, ragged vector tiles, one and two 64-feature boxes, more row
-    groups than row blocks.  Modes: the default (d tile in tensor memory, targets through shared memory) and the two fallbacks."""
+    groups than row blocks.  Modes: the default (16-byte aligned y: the targets ride along with the X block through shared
+    memory) and y_ldg (y at a 4-byte offset: targets loaded per lane and broadcast with shuffles)."""
     from oracle import elbo_oracle as O
     monkeypatch.setenv("BRN_LINEAR_VARIANT", "tcgen05")
-    if mode == "y_ldg":          # targets loaded per lane + shuffles instead of riding along with the X block (the unaligned-y path)
-        monkeypatch.setenv("BRN_LINEAR_Y_BULK", "0")
-    if mode == "d_smem":         # d tile through shared memory instead of tensor memory
-        monkeypatch.setenv("BRN_LINEAR_DTMEM", "0")
     rng = np.random.RandomState(N + F + S)
     X = (rng.randn(N, F) * (1 + 3 * rng.rand(1, F))).astype("f4")
     y = rng.randint(0, 2, size=N)
@@ -247,9 +254,9 @@ def test_linear_flash_variant(cu, monkeypatch, N, F, S, tied, mode):
     prior = None if tied else {"weights": (0.0, 0.5)}
     o32 = O.logreg_elbo(X, y, params, eps, prior, row_chunk=4096)
     o64 = O.logreg_elbo(X, y, params, eps, prior, dtype=torch.float64, row_chunk=4096)
-    loss, grads = run_linear(cu, X, y, params, eps, cu.BERNOULLI, 1, prior)
+    loss, grads = run_linear(cu, X, y, params, eps, cu.BERNOULLI, 1, prior, y_offset=mode == "y_ldg")
     assert cu.last_variant() == "tcgen05-flash"
-    check_against_oracle(loss, grads, o32, o64, "linear flash N=%d F=%d S=%d" % (N, F, S))
+    check_against_oracle(loss, grads, o32, o64, "linear flash N=%d F=%d S=%d %s" % (N, F, S, mode))
 
 
 def test_linear_prepared_x(cu, monkeypatch):
@@ -341,13 +348,10 @@ def test_linear_empty_rows(cu):
                                        (257, 130, 97, 16, 5), (1024, 784, 100, 10, 4), (40, 33, 21, 3, 1),
                                        (130, 37, 5, 2, 4)])
 @pytest.mark.parametrize("tied", [True, False])
-@pytest.mark.parametrize("mid", ["5", "4"])
-def test_bnn_tcgen05_variant(cu, monkeypatch, B, P, H, C, S, tied, mid):
-    """mid = 5 (default): the mid stage fused into the forward GEMM's epilogue and the sample-axis reduction into the
-    backward GEMM's; 4: staged pipeline (forward GEMM -> mid kernel on mma.sync 3xTF32 -> backward GEMM -> statistics)."""
+def test_bnn_tcgen05_variant(cu, monkeypatch, B, P, H, C, S, tied):
+    """forward GEMM -> mid kernel on mma.sync 3xTF32 -> backward GEMM -> statistics."""
     from oracle import elbo_oracle as O
     monkeypatch.setenv("BRN_BNN_VARIANT", "tcgen05")
-    monkeypatch.setenv("BRN_BNN_MID", mid)
     X, y, params, eps, shapes = random_bnn(B * 3 + H, B, P, H, C, S)
     prior = None if tied else {n: (0.0, 10.0) for n in shapes}
     o32 = O.bnn_elbo(X, y, params, eps, prior)
@@ -416,13 +420,11 @@ def test_bnn_predict_matches_forward_oracle(cu, monkeypatch, B, P, H, C, S, vari
 
 
 @pytest.mark.parametrize("act", ["relu", "sigmoid"])
-@pytest.mark.parametrize("mid", ["4", "5"])
-def test_bnn_tcgen05_activations(cu, monkeypatch, act, mid):
-    """relu / sigmoid hidden units through the tensor-core variant (staged and fused pipelines) vs the fp64 oracle.  Relu: the
-    rows whose pre-activations come within 1e-5 (relative) of the kink are left out of the statement (see the C5 test)."""
+def test_bnn_tcgen05_activations(cu, monkeypatch, act):
+    """relu / sigmoid hidden units through the tensor-core variant vs the fp64 oracle.  Relu: the rows whose pre-activations
+    come within 1e-5 (relative) of the kink are left out of the statement (see the C5 test)."""
     from oracle import elbo_oracle as O
     monkeypatch.setenv("BRN_BNN_VARIANT", "tcgen05")
-    monkeypatch.setenv("BRN_BNN_MID", mid)
     B, P, H, C, S = 200, 64, 100, 7, 4
     X, y, params, eps, shapes = random_bnn(41, B, P, H, C, S)
     if act == "relu":          # keep every pre-activation away from zero: shift the biases by the sign of the pre-activation mean
@@ -435,4 +437,4 @@ def test_bnn_tcgen05_activations(cu, monkeypatch, act, mid):
     o64 = O.bnn_elbo(X, y, params, eps, None, dtype=torch.float64, activation=act)
     loss, grads, _ = run_bnn(cu, X, y, params, eps, None, activation=act)
     assert cu.last_variant() == "tcgen05"
-    check_against_oracle(loss, grads, o32, o64, "bnn tcgen05 %s mid=%s" % (act, mid))
+    check_against_oracle(loss, grads, o32, o64, "bnn tcgen05 %s" % act)

@@ -8,32 +8,30 @@ import numpy as np
 import pytest
 import torch
 
-from test_vae_coverage_cuda import CASES, CASE, CHILD_CASES, CHILD_SETTINGS, TRANSPOSED, case_inputs, tail_split_case
+from test_vae_coverage_cuda import CASES, CASE, case_inputs, tail_split_case
 
 SMS = 148              # B200
 VAE_BK = 16            # vae.cu:23, K chunk of every K5 GEMM
 UG_BM = 128            # umma_gemm.cuh:21, M tile
 
 
-def pick_bn(N, ew16=True):
-    """N tile of the forward, data-gradient, output and K-major weight-gradient GEMMs (vae.cu:330-335): -128 is the 128-wide
-    tile with sixteen epilogue warps"""
-    if ew16 and N % 128 == 0:
+def pick_bn(N):
+    """N tile of the forward, data-gradient and output GEMMs (vae.cu:309-313): -128 is the 128-wide tile with sixteen
+    epilogue warps"""
+    if N % 128 == 0:
         return -128
     nt = (N + 207) // 208
     per = (N + nt - 1) // nt
     return 128 if per <= 128 else (176 if per <= 176 else 208)
 
 
-def wgrad_tile(n_in, tile_env=2):
-    """N tile of the MN-major weight-gradient GEMM (vae.cu:801-809; BRN_VAE_WGRAD_TILE, default 2)"""
-    if tile_env == 1:
-        return 128
-    return 256 if tile_env == 2 and n_in % 256 == 0 else 128
+def wgrad_tile(n_in):
+    """N tile of the MN-major weight-gradient GEMM (vae.cu:739-743)"""
+    return 256 if n_in % 256 == 0 else 128
 
 
 def umma_regime(BN, M, N, K, sms, BK=VAE_BK):
-    """umma_plan with allow_split (umma_gemm.cuh:479-497): "tail" when the T = U % grid units of a last, at most half full
+    """umma_plan with allow_split (umma_gemm.cuh:462-481): "tail" when the T = U % grid units of a last, at most half full
     round are K-split, "all" when every unit is K-split over sms / U CTAs, otherwise "none"."""
     m_tiles, n_tiles, k_chunks = -(-M // UG_BM), -(-N // BN), -(-K // BK)
     U = m_tiles * n_tiles
@@ -47,48 +45,48 @@ def umma_regime(BN, M, N, K, sms, BK=VAE_BK):
 
 
 def simt_lp(L):
-    """template LP of vae_dec0_bwd_kernel and vae_heads_bwd_kernel (vae.cu:877-880, 893-896)"""
+    """template LP of vae_dec0_bwd_kernel and vae_heads_bwd_kernel (vae.cu:805-808, 821-824)"""
     return 2 if L <= 2 else 4 if L <= 4 else 8 if L <= 8 else 16
 
 
 def simt_jpt(h0):
-    """template JPT of vae_dec0_bwd_kernel (vae.cu:716-717)"""
+    """template JPT of vae_dec0_bwd_kernel (vae.cu:667-668)"""
     return 2 if h0 <= 512 else 4
 
 
-def vae_gemms(c, sms=SMS, wgrad_mn=True, ew16=True, tile_env=2):
+def vae_gemms(c, sms=SMS):
     """(role, layer, tile, regime) of every GEMM brn_vae_elbo_fwd_bwd launches for case `c`, in launch order.
-    Roles: forward (vae.cu:822-825, 844-845), output (:851), data_grad and wgrad (:859-870, 899-905).  The weight gradient is
-    the MN-major GEMM on wgrad_tile (:795-809) or, with BRN_VAE_WGRAD_MN=0, the K-major one on pick_bn (:811-815); both
-    allow the K split.  The forward, output and data-gradient GEMMs run in mode 2, which never splits."""
+    Roles: forward (vae.cu:750-753, 772-773), output (:779), data_grad and wgrad (:787-798, 827-833).  The weight gradient is
+    the MN-major GEMM on wgrad_tile (:732-744), which allows the K split.  The forward, output and data-gradient GEMMs run
+    in mode 2, which never splits."""
     B, D, R = c["B"], c["D"], c["S"] * c["B"]
     he, hd = list(c["h_enc"]), list(c["h_dec"])
     out = []
 
     def wgrad(name, n_out, n_in, rows):
-        tile = wgrad_tile(n_in, tile_env) if wgrad_mn else pick_bn(n_in, ew16)
+        tile = wgrad_tile(n_in)
         out.append(("wgrad", name, tile, umma_regime(abs(tile), n_out, n_in, rows, sms)))
 
     for i, n in enumerate(he):
-        out.append(("forward", "enc.%d" % i, pick_bn(n, ew16), None))
+        out.append(("forward", "enc.%d" % i, pick_bn(n), None))
     for i in range(1, len(hd)):
-        out.append(("forward", "dec.%d" % i, pick_bn(hd[i], ew16), None))
-    out.append(("output", "dec.out", pick_bn(D, ew16), None))
+        out.append(("forward", "dec.%d" % i, pick_bn(hd[i]), None))
+    out.append(("output", "dec.out", pick_bn(D), None))
     for i in range(len(hd), 0, -1):
         n_out = D if i == len(hd) else hd[i]
         wgrad("dec.out" if i == len(hd) else "dec.%d" % i, n_out, hd[i - 1], R)
-        out.append(("data_grad", "dec.out" if i == len(hd) else "dec.%d" % i, pick_bn(hd[i - 1], ew16), None))
+        out.append(("data_grad", "dec.out" if i == len(hd) else "dec.%d" % i, pick_bn(hd[i - 1]), None))
     for i in range(len(he) - 1, -1, -1):
         wgrad("enc.%d" % i, he[i], D if i == 0 else he[i - 1], B)
         if i > 0:
-            out.append(("data_grad", "enc.%d" % i, pick_bn(he[i - 1], ew16), None))
+            out.append(("data_grad", "enc.%d" % i, pick_bn(he[i - 1]), None))
     return out
 
 
-def branches(c, sms=SMS, **kw):
+def branches(c, sms=SMS):
     """the set of branch labels case `c` reaches"""
     got = set()
-    for role, _, tile, regime in vae_gemms(c, sms, **kw):
+    for role, _, tile, regime in vae_gemms(c, sms):
         got.add("%s tile %d" % (role, tile))
         if regime:
             got.add("%s split %s" % (role, regime))
@@ -104,10 +102,10 @@ REQUIRED = (GEMM_TILES + ["wgrad tile 256", "wgrad tile 128", "wgrad split none"
             ["%s depth %d" % (side, n) for side in ("encoder", "decoder") for n in (1, 6)])
 
 
-def reached(cases, **kw):
+def reached(cases):
     where = {}
     for c in cases:
-        for b in branches(c, **kw):
+        for b in branches(c):
             where.setdefault(b, []).append(c["name"])
     return where
 
@@ -123,31 +121,6 @@ def test_case_table_reaches_every_branch():
     assert len(CASES) == len(CASE), "case names must be unique"
 
 
-def test_transposed_subset_reaches_the_wide_tiles():
-    """BRN_VAE_WGRAD_MN=0 runs the K-major weight gradients on pick_bn's tiles: the subset reaches -128, 176 and 208 there and
-    in every other GEMM role, L = 16, and a K split"""
-    where = reached([CASE[n] for n in TRANSPOSED], wgrad_mn=False)
-    need = ["%s tile %d" % (role, t) for role in ("forward", "data_grad", "output", "wgrad") for t in (-128, 176, 208)]
-    need += ["L 16", "wgrad split all"]
-    missing = [b for b in need if b not in where]
-    assert not missing, missing
-
-
-def test_child_settings_change_the_selection():
-    """each function-static setting changes a GEMM the child cases launch, so its child process tests something"""
-    cases = [CASE[n] for n in CHILD_CASES]
-    base = [g for c in cases for g in vae_gemms(c)]
-    for var, value in CHILD_SETTINGS:
-        if var == "BRN_VAE_EW16":
-            alt = [g for c in cases for g in vae_gemms(c, ew16=False)]
-            assert alt != base and -128 not in [g[2] for g in alt]
-        elif var == "BRN_VAE_CW":          # the 4-converter-warp variant exists for the -128 tile only (vae.cu:342-347)
-            assert any(g[2] == -128 and g[0] != "wgrad" for g in base)
-        else:
-            alt = [g for c in cases for g in vae_gemms(c, tile_env=int(value))]
-            assert any(g[2] == 256 for g in base) and all(g[2] != 256 for g in alt if g[0] == "wgrad")
-
-
 def test_tail_split_case_reaches_the_tail_regime():
     for sms in (SMS, 132, 160, 170):
         c = tail_split_case(sms)
@@ -160,7 +133,6 @@ def test_mirror_spot_values():
     """values worked out by hand from vae.cu / umma_gemm.cuh"""
     assert [pick_bn(n) for n in (1, 128, 150, 176, 200, 208, 209, 250, 256, 300, 500, 513, 1000, 2000)] == \
         [128, -128, 176, 176, 208, 208, 128, 128, -128, 176, 176, 176, 208, 208]
-    assert [pick_bn(n, ew16=False) for n in (256, 512, 1024)] == [128, 176, 208]
     assert umma_regime(128, 2000, 1200, 400, 148) == "tail"          # U = 160, T = 12, 25 K chunks >= 24
     assert umma_regime(128, 2000, 1200, 368, 148) == "none"          # 23 K chunks
     assert umma_regime(256, 784, 1024, 308, 148) == "all"            # U = 28, 20 K chunks >= 10

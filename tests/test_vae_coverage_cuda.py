@@ -1,26 +1,15 @@
-"""K5 (brn_vae_elbo_fwd_bwd) on every tile width, latent size, depth, K-split regime and operand layout its host code can
-select, against the fp32 / fp64 oracle.
+"""K5 (brn_vae_elbo_fwd_bwd) on every tile width, latent size, depth and K-split regime its host code can select, against
+the fp32 / fp64 oracle.
 
 `CASES` is a plain list: tests/test_vae_coverage.py walks it through a mirror of the host-side selections of vae.cu and
 umma_gemm.cuh and fails (on the CPU) when an edit of the table leaves a branch unreached.
 
 ReLU kinks: a unit whose pre-activation lies within rounding error of zero is switched on by one correct fp32 evaluation and
 off by another (see test_c5_vae_full_config).  Each case therefore draws more data rows than it runs, and keeps the first B
-rows whose every ReLU pre-activation is at least 4e-6 (relative to its own terms) away from the kink in the fp64 forward pass.
-
-Run as a script (`python test_vae_coverage_cuda.py IN.npz... -- OUT_DIR`), the file evaluates saved inputs in a fresh process,
-so that the selections vae.cu fixes at its first call in a process (BRN_VAE_EW16, BRN_VAE_CW, BRN_VAE_WGRAD_TILE) can be
-tested."""
-import os
-import subprocess
-import sys
-
+rows whose every ReLU pre-activation is at least 4e-6 (relative to its own terms) away from the kink in the fp64 forward pass."""
 import numpy as np
 import pytest
 import torch
-
-HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(HERE)
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -32,7 +21,7 @@ def tail_split_case(sms, S=8, B=50):
 
     That GEMM is M = D (output width) by N = 1200 (last decoder width: the 128-wide MN-major tile, 10 n-tiles) over
     K = S * B rows.  D = 128 m - 48 for the smallest m with U = 10 m > sms units, T = U % sms tail units, 2 T <= sms and
-    ceil(K / 16) >= 2 (sms // T) K chunks (umma_gemm.cuh:486).  148 SMs: D = 2000, U = 160, T = 12."""
+    ceil(K / 16) >= 2 (sms // T) K chunks (umma_gemm.cuh:470).  148 SMs: D = 2000, U = 160, T = 12."""
     k_chunks = (S * B + 15) // 16
     m = sms // 10 + 1
     while True:
@@ -58,12 +47,6 @@ CASES = [
     dict(name="D300_h1024enc", B=9, D=300, L=2, h_enc=(1024, 150), h_dec=(64,), S=7, seed=110),
 ]
 CASE = {c["name"]: c for c in CASES}
-
-# BRN_VAE_WGRAD_MN=0 (transposed K-major operands, read on every call): the 176, 208 and -128 tiles and L = 16
-TRANSPOSED = ["w176_B1", "deep6", "h1024_L9", "out256", "D1_L16", "D300_h1024enc"]
-# selections fixed at the first call in a process: one child process per setting, each on CHILD_CASES
-CHILD_SETTINGS = [("BRN_VAE_EW16", "0"), ("BRN_VAE_CW", "4"), ("BRN_VAE_WGRAD_TILE", "0"), ("BRN_VAE_WGRAD_TILE", "1")]
-CHILD_CASES = ["h513_L8", "h1024_L9", "D300_h1024enc"]
 
 
 @pytest.fixture(scope="module")
@@ -156,17 +139,6 @@ def test_vae_tail_split_regime_on_this_device(cu):
     check("tail_split for %d SMs" % sms, loss, grads, *oracles(X, enc, dec, eps, row_chunk=c["row_chunk"]))
 
 
-@pytest.mark.parametrize("name", TRANSPOSED)
-def test_vae_coverage_transposed_layouts(cu, monkeypatch, name):
-    """BRN_VAE_WGRAD_MN=0: transposed K-major copies of every activation and gradient, the K-major weight-gradient GEMM on
-    pick_bn's tiles, the transposed stores of store_split4 / vae_sample_dec0_kernel / vae_heads_bwd_kernel and the transposed
-    TF32 split of X"""
-    monkeypatch.setenv("BRN_VAE_WGRAD_MN", "0")
-    X, enc, dec, eps, kept, o32, o64 = prepared(name)
-    loss, grads = run_cuda(cu, X, enc, dec, eps)
-    check("%s WGRAD_MN=0" % name, loss, grads, o32, o64)
-
-
 @pytest.mark.parametrize("sd_offset", [1e-3, 1.0])
 def test_vae_sd_offset(cu, sd_offset):
     """the encoder's sd = softplus(W_sd h + b_sd) + sd_offset with the model's offset, not the example's 0.1"""
@@ -185,72 +157,6 @@ def test_vae_saturated_logits(cu):
     assert frac > 0.5 and 60 < top < 120, (frac, top)
     loss, grads = run_cuda(cu, X, enc, dec, eps)
     check("saturated logits (%.0f %% with |l| > 30)" % (100 * frac), loss, grads, *oracles(X, enc, dec, eps))
-
-
-def pack(X, enc, dec, eps):
-    d = {"X": X, "eps": eps}
-    for side, net in (("enc", enc), ("dec", dec)):
-        for k, v in net.items():
-            if isinstance(v, list):
-                for i, a in enumerate(v):
-                    d["%s.%s.%d" % (side, k, i)] = a
-            else:
-                d["%s.%s" % (side, k)] = v
-    return d
-
-
-def unpack(z):
-    nets = {"enc": {"W": [], "b": []}, "dec": {"W": [], "b": []}}
-    for k in z.files:
-        if k in ("X", "eps"):
-            continue
-        side, rest = k.split(".", 1)
-        if rest[:2] in ("W.", "b."):
-            nets[side][rest[0]].append((int(rest[2:]), z[k]))
-        else:
-            nets[side][rest] = z[k]
-    for net in nets.values():
-        for wb in ("W", "b"):
-            net[wb] = [a for _, a in sorted(net[wb], key=lambda t: t[0])]
-    return z["X"], nets["enc"], nets["dec"], z["eps"]
-
-
-def child_main(inputs, out_dir):
-    """evaluate each saved case once on cuda:0; write loss and gradients to OUT_DIR/<basename of the input>"""
-    sys.path[:0] = [ROOT, HERE]
-    from brancher_b200 import _cuda as cu
-    cu.lib()
-    for path in inputs:
-        with np.load(path) as z:
-            X, enc, dec, eps = unpack(z)
-        loss, grads = run_cuda(cu, X, enc, dec, eps)
-        np.savez(os.path.join(out_dir, os.path.basename(path)), loss=np.float64(loss), **grads)
-    torch.cuda.synchronize()
-
-
-@pytest.mark.parametrize("var,value", CHILD_SETTINGS)
-def test_vae_function_static_selection(tmp_path, var, value):
-    """BRN_VAE_EW16=0 (no 16-epilogue-warp tile), BRN_VAE_CW=4 (four converter warps) and BRN_VAE_WGRAD_TILE=0|1 (the
-    128-wide weight-gradient tiles) are read once per process: a child process evaluates CHILD_CASES under each"""
-    inputs = []
-    for name in CHILD_CASES:
-        X, enc, dec, eps = prepared(name)[:4]
-        p = str(tmp_path / ("%s.npz" % name))
-        np.savez(p, **pack(X, enc, dec, eps))
-        inputs.append(p)
-    out_dir = tmp_path / "out"
-    out_dir.mkdir()
-    env = dict(os.environ, **{var: value})
-    cmd = [sys.executable] + (["-s"] if sys.flags.no_user_site else []) + [os.path.abspath(__file__)] + inputs + ["--", str(out_dir)]
-    res = subprocess.run(cmd, env=env, cwd=ROOT, capture_output=True, text=True, timeout=600)
-    assert res.returncode == 0, "child (%s=%s) exited with %d:\n%s\n%s" % (var, value, res.returncode, res.stdout[-4000:],
-                                                                         res.stderr[-4000:])
-    for name in CHILD_CASES:
-        o32, o64 = prepared(name)[5:]
-        with np.load(str(out_dir / ("%s.npz" % name))) as z:
-            grads = {k: z[k] for k in z.files if k != "loss"}
-            loss = float(z["loss"])
-        check("%s %s=%s" % (name, var, value), loss, grads, o32, o64)
 
 
 def test_vae_zero_local_samples_leave_outputs_untouched(cu):
@@ -316,8 +222,3 @@ def test_vae_rejects_seven_hidden_layers(cu):
     _, enc, dec, _ = V.random_vae(126, 8, 10, 2, (6,) * 7, (6,), 1)
     with pytest.raises(cu.BrancherCudaError):
         V.make_net(cu, enc, dec)
-
-
-if __name__ == "__main__":
-    sep = sys.argv.index("--")
-    child_main(sys.argv[1:sep], sys.argv[sep + 1])
