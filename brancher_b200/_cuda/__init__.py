@@ -12,7 +12,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libbrancher_cuda.so")
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 _lib = None
 
@@ -104,6 +104,13 @@ SYMBOLS = {
     "brn_bnn_elbo_fwd_bwd_act": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p] + [ctypes.c_int] * 5 +
                                  [ctypes.POINTER(MFVar), ctypes.POINTER(SampleRange), ctypes.c_void_p, ctypes.c_size_t,
                                   ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]),
+    "brn_bnn_deep_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int] * 3 + [ctypes.c_void_p, ctypes.c_int, ctypes.c_int]),
+    "brn_bnn_deep_elbo_fwd_bwd": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p] + [ctypes.c_int] * 3 +
+                                  [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(MFVar), ctypes.POINTER(SampleRange),
+                                   ctypes.c_void_p, ctypes.c_size_t, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]),
+    "brn_bnn_deep_predict": (ctypes.c_int, [ctypes.c_void_p] + [ctypes.c_int] * 3 +
+                             [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(MFVar), ctypes.POINTER(SampleRange),
+                              ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     "brn_linear_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int]),
     "brn_linear_elbo_fwd_bwd": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int64,
                                                ctypes.c_int, ctypes.c_int, ctypes.POINTER(MFVar),
@@ -372,6 +379,53 @@ def bnn_predict(X, vars4, r, labels=True, probs=True, activation="tanh"):
     pm = torch.zeros((B, C), dtype=torch.float32, device=dev) if probs else None
     _check(lib().brn_bnn_predict(_ptr(X, what="X"), B, P, H, C, ACTIVATIONS[activation], arr, ctypes.byref(r), ws.data_ptr(), ws.numel(), _ptr(logits),
                                  _ptr(lab, torch.int32), _ptr(pm), _stream(dev)), "brn_bnn_predict")
+    return logits, lab, pm
+
+
+def _deep_shape(X, vars_, activations):
+    """(B, P, H array, act array, C) of a deep BNN: vars_ = MeanFieldVar for (W1, b1, W2, b2, ..., W_out, b_out)."""
+    B, P = X.shape
+    n_hidden = len(vars_) // 2 - 1
+    if len(vars_) % 2 or len(activations) != n_hidden:
+        raise BrancherCudaError("deep BNN: %d variables and %d activations do not describe a network" % (len(vars_), len(activations)))
+    H = (ctypes.c_int * max(n_hidden, 1))(*[v.numel for v in vars_[1:-2:2]])
+    act = (ctypes.c_int * max(n_hidden, 1))(*[ACTIVATIONS[a] for a in activations])
+    return B, P, n_hidden, H, act, vars_[-1].numel
+
+
+def bnn_deep_elbo_fwd_bwd(X, y, vars_, r, activations, with_prior=True, loss=None, data_ready=None):
+    """K3 with 2..4 hidden layers.  X [B,P] fp32, y [B] int32, vars_ = MeanFieldVar for (weights1 [H1,P], b1 [H1],
+    weights2 [H2,H1], b2 [H2], ..., weights_out [C,H_L], b_out [C]); activations: one of "tanh" / "relu" / "sigmoid" per
+    hidden layer.  data_ready as for bnn_elbo_fwd_bwd."""
+    dev = X.device
+    B, P, n_hidden, H, act, C = _deep_shape(X, vars_, activations)
+    loss = torch.zeros(1, dtype=torch.float64, device=dev) if loss is None else loss
+    for v in vars_:
+        _check_eps(v, r)
+    nbytes = lib().brn_bnn_deep_workspace_bytes(B, P, n_hidden, H, C, r.s_local)
+    ws = _workspace(dev, nbytes)
+    arr = (MFVar * len(vars_))(*[v.struct() for v in vars_])
+    if data_ready is not None:
+        lib().brn_set_data_ready_event(ctypes.c_void_p(data_ready.cuda_event))
+    _check(lib().brn_bnn_deep_elbo_fwd_bwd(_ptr(X, what="X"), _ptr(y, torch.int32, "y"), B, P, n_hidden, H, act, C, arr,
+                                           ctypes.byref(r), ws.data_ptr(), ws.numel(), int(with_prior), _ptr(loss, torch.float64),
+                                           _stream(dev)), "brn_bnn_deep_elbo_fwd_bwd")
+    return loss
+
+
+def bnn_deep_predict(X, vars_, r, activations, labels=True, probs=True):
+    """Posterior-predictive pass of a deep BNN (as bnn_predict): (logits [s_local,B,C], labels int32 [s_local,B] or None,
+    probs_mean [B,C] or None)."""
+    dev = X.device
+    B, P, n_hidden, H, act, C = _deep_shape(X, vars_, activations)
+    nbytes = lib().brn_bnn_deep_workspace_bytes(B, P, n_hidden, H, C, r.s_local)
+    ws = _workspace(dev, nbytes)
+    arr = (MFVar * len(vars_))(*[v.struct() for v in vars_])
+    logits = torch.empty((r.s_local, B, C), dtype=torch.float32, device=dev)
+    lab = torch.empty((r.s_local, B), dtype=torch.int32, device=dev) if labels else None
+    pm = torch.zeros((B, C), dtype=torch.float32, device=dev) if probs else None
+    _check(lib().brn_bnn_deep_predict(_ptr(X, what="X"), B, P, n_hidden, H, act, C, arr, ctypes.byref(r), ws.data_ptr(), ws.numel(),
+                                      _ptr(logits), _ptr(lab, torch.int32), _ptr(pm), _stream(dev)), "brn_bnn_deep_predict")
     return logits, lab, pm
 
 

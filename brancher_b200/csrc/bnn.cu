@@ -596,3 +596,5 @@ extern "C" int brn_bnn_predict(const float* X, int B, int P, int H, int C, int a
     BRN_LAUNCH_OK("bnn_predict_kernel");
     return 0;
 }
+
+#include "bnn_deep.cuh"

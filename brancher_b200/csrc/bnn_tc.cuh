@@ -549,99 +549,128 @@ struct BnnTcWorkspace {
     }
 };
 
+// Layer-1 pieces of the tcgen05 variant, shared by the two-layer evaluation below and the deep networks (bnn_deep.cuh).
+// Sampling-stage part for W1 (vars w1): operand bounds (scal[SC_W2] from w2), noise + W1_s split into the forward GEMM's
+// fp16 pairs, finite padding of the odd tail sample block.
+static int bnn_tc_sample_w1(const brn_mf_var& w1, const brn_mf_var& w2, int H, int P, int64_t ldw, const brn_sample_range* r,
+                            const BnnTcWorkspace& ws, float* ws_eps, cudaStream_t stream) {
+    constexpr int HP = BNN_UMMA_HP, NS = BNN_UMMA_NSAMP;
+    const int S = r->s_local;
+    const int64_t n1 = (int64_t)H * P, n2 = w2.numel;
+    BRN_CUDA_OK(cudaMemsetAsync(ws.scal, 0, sizeof(float) * SC_SLOTS, stream));
+    // operand bounds (device scalars): injected noise is not bounded a priori
+    if (w1.eps) if (int e = launch_absmax(w1.eps, (int64_t)S * n1, ws.scal + SC_EPS, stream)) return e;
+    if (w2.eps) if (int e = launch_absmax(w2.eps, (int64_t)S * n2, ws.scal + SC_EPS, stream)) return e;
+    bnn_bounds_kernel<<<(unsigned)std::min<int64_t>((n1 + n2 + 255) / 256, 296), 256, 0, stream>>>(
+        w1.mu, w1.rho, n1, w2.mu, w2.rho, n2, ws.scal);
+    BRN_LAUNCH_OK("bnn_bounds_kernel");
+    const bool fast = (P % 4 == 0) && ((uintptr_t)w1.mu % 16 == 0) && ((uintptr_t)w1.rho % 16 == 0) &&
+                      (!w1.eps || ((uintptr_t)w1.eps % 16 == 0));
+    if (fast) {
+        constexpr int SG = 8;
+        dim3 grid((unsigned)((n1 / 4 + 255) / 256), (unsigned)((S + SG - 1) / SG));
+        sample_w1_group_kernel<SG><<<grid, 256, 0, stream>>>(w1.mu, w1.rho, w1.eps, n1, ws_eps, ldw, ws.Wh, ws.Wl, H, P, HP, ws.ldP,
+                                                             *r, w1.var_id, ws.scal);
+        BRN_LAUNCH_OK("sample_w1_group_kernel");
+    } else {
+        if (w1.eps)
+            BRN_CUDA_OK(cudaMemcpy2DAsync(ws_eps, ldw * sizeof(float), w1.eps, n1 * sizeof(float), n1 * sizeof(float), S,
+                                          cudaMemcpyDeviceToDevice, stream));
+        else if (int e = launch_philox_fill(ws_eps, ldw, n1, w1.var_id, *r, stream)) return e;
+        dim3 grid((P + 255) / 256, H, S);
+        sample_w1_generic_kernel<<<grid, 256, 0, stream>>>(w1.mu, w1.rho, ws_eps, ldw, ws.Wh, ws.Wl, H, P, HP, ws.ldP, ws.scal);
+        BRN_LAUNCH_OK("sample_w1_generic_kernel");
+    }
+    if (S % NS) {   // the odd tail tile reads one more sample block: keep it finite
+        BRN_CUDA_OK(cudaMemsetAsync(ws.Wh + (size_t)S * HP * ws.ldP, 0, sizeof(__half) * HP * ws.ldP, stream));
+        BRN_CUDA_OK(cudaMemsetAsync(ws.Wl + (size_t)S * HP * ws.ldP, 0, sizeof(__half) * HP * ws.ldP, stream));
+        BRN_CUDA_OK(cudaMemsetAsync(ws.dph + (size_t)S * HP * ws.ldB, 0, sizeof(__half) * HP * ws.ldB, stream));
+        BRN_CUDA_OK(cudaMemsetAsync(ws.dpl + (size_t)S * HP * ws.ldB, 0, sizeof(__half) * HP * ws.ldB, stream));
+    }
+    return 0;
+}
+
+// first read of the minibatch: X's bound and its fp16 pairs (row-major for the forward GEMM, transposed for the backward)
+static int bnn_tc_split_x(const float* X, int B, int P, const BnnTcWorkspace& ws, cudaStream_t stream) {
+    if (int e = wait_data_ready(stream)) return e;
+    if (int e = launch_absmax(X, (int64_t)B * P, ws.scal + SC_X, stream)) return e;
+    dim3 grid((B + 31) / 32, (P + 31) / 32), block(32, 8);
+    split_f16_kernel<<<grid, block, 0, stream>>>(X, P, B, P, ws.Xh, ws.Xl, ws.ldP, ws.Xth, ws.Xtl, ws.ldB, ws.scal);
+    BRN_LAUNCH_OK("split_f16_kernel");
+    return 0;
+}
+
+// TMEM accumulation chain = 2 x 32 words = 128 fp16 elements of K between register drains (umma_gemm.cuh): the error
+// of the evaluation grows with the chain (max gradient error / scale at the C3 shape: 0.9e-6 / 1.1e-6 / 1.3e-6 /
+// 2.3e-6 for 1 / 2 / 4 / 8, profiles/tools/bnn_err_probe.py) -- 128 elements is the chain length round 1 settled on.
+// The backward GEMM's accumulator is the per-sample weight gradient, summed over 256 samples afterwards: its chain
+// may be twice as long (measured: no change of the parity margins, 8 us per evaluation).
+constexpr int BNN_UMMA_DRAIN = 2, BNN_UMMA_DRAIN_BWD = 4;
+
+// pre_s^T [S][H][B] = (X . W1_s^T)^T, coalesced across the warp's rows b
+static int bnn_tc_gemm_fwd(int B, int P, int H, int S, const BnnTcWorkspace& ws, float* ws_pre, cudaStream_t stream) {
+    constexpr int BN = BNN_UMMA_HP * BNN_UMMA_NSAMP;
+    EpiStore::Params ep;
+    ep.out = ws_pre; ep.rows = B; ep.row_stride = 1; ep.col_stride = B; ep.blk_stride = (int64_t)B * H;
+    ep.blk_valid = H; ep.col_limit = 0; ep.total_blks = S;
+    ep.bound_a = ws.scal + SC_X; ep.bound_b = ws.scal + SC_W1; ep.bound_b_mult = 1.f;
+    return launch_umma_nt_kind<BN, BNN_UMMA_BK, EpiStore, 8, 0, 4, 1>(ws.Xh, ws.Xl, B, ws.ldP, ws.Wh, ws.Wl, S * BNN_UMMA_HP, ws.ldP, P, 0,
+                                                                        BNN_UMMA_DRAIN, ep, stream);
+}
+
+// dW1_s[h][p] = D[p, (s, h)] = (dpre_s^T X)[h][p] from the fp16 pairs ws.dph / ws.dpl, which were scaled by
+// p2_scale(dpre_mult * *dpre_bound)
+static int bnn_tc_gemm_bwd(int B, int P, int H, int S, int64_t ldw, const BnnTcWorkspace& ws, float* ws_dW1, const float* dpre_bound,
+                           float dpre_mult, cudaStream_t stream) {
+    constexpr int NS = BNN_UMMA_NSAMP, BN = BNN_UMMA_HP * NS;
+    // K-split tail (see UnitIter): the dW1 blocks of the samples in the split n-tiles take atomic partial sums
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const UmmaSplitPlan plan = umma_plan<BN, 2 * BNN_UMMA_BK>(P, S * BNN_UMMA_HP, B, sms, true);
+    if (plan.first_split_ntile >= 0) {
+        const int s_first = plan.first_split_ntile * NS;
+        if (s_first < S)
+            BRN_CUDA_OK(cudaMemset2DAsync(ws_dW1 + (size_t)s_first * ldw, ldw * sizeof(float), 0, (size_t)H * P * sizeof(float),
+                                          S - s_first, stream));
+    }
+    EpiStore::Params ep;
+    ep.out = ws_dW1; ep.rows = P; ep.row_stride = 1; ep.col_stride = P; ep.blk_stride = ldw;
+    ep.blk_valid = H; ep.col_limit = 0; ep.total_blks = S;
+    ep.bound_a = ws.scal + SC_X; ep.bound_b = dpre_bound; ep.bound_b_mult = dpre_mult;
+    return launch_umma_nt_kind<BN, BNN_UMMA_BK, EpiStore, 8, 0, 4, 1>(ws.Xth, ws.Xtl, P, ws.ldB, ws.dph, ws.dpl, S * BNN_UMMA_HP, ws.ldB, B,
+                                                                        0, BNN_UMMA_DRAIN_BWD, ep, stream, true);
+}
+
 // The tcgen05 variant of brn_bnn_elbo_fwd_bwd: sampler -> forward GEMM -> mid kernel -> backward GEMM -> statistics.
 // forward_only (brn_bnn_predict) stops after the forward GEMM.
 static int bnn_tc_eval(const float* X, const int32_t* y, const BnnLayout& L, const brn_mf_var vars[4], const brn_sample_range* r,
                        const BnnTcWorkspace& ws, float* ws_eps, float* ws_W, float* ws_dW, float* ws_pre, float* ws_stats,
                        int with_prior, double* loss, cudaStream_t stream, bool forward_only = false) {
-    constexpr int HP = BNN_UMMA_HP, NS = BNN_UMMA_NSAMP, BN = HP * NS;
-    // TMEM accumulation chain = 2 x 32 words = 128 fp16 elements of K between register drains (umma_gemm.cuh): the error
-    // of the evaluation grows with the chain (max gradient error / scale at the C3 shape: 0.9e-6 / 1.1e-6 / 1.3e-6 /
-    // 2.3e-6 for 1 / 2 / 4 / 8, profiles/tools/bnn_err_probe.py) -- 128 elements is the chain length round 1 settled on.
-    // The backward GEMM's accumulator is the per-sample weight gradient, summed over 256 samples afterwards: its chain
-    // may be twice as long (measured: no change of the parity margins, 8 us per evaluation).
-    constexpr int drain = 2, drain_bwd = 4;
     const int B = L.B, P = L.P, H = L.H, S = r->s_local;
-    const int64_t numels[4] = {(int64_t)H * P, H, (int64_t)L.C * H, L.C};
     const int64_t offs[4] = {L.oW1, L.ob1, L.oW2, L.ob2};
     const float inv_S = 1.0f / (float)r->s_total;
     {
         StageTimer st("bnn.sample_weights", stream);
-        BRN_CUDA_OK(cudaMemsetAsync(ws.scal, 0, sizeof(float) * SC_SLOTS, stream));
-        // operand bounds (device scalars): injected noise is not bounded a priori
-        if (vars[0].eps) if (int e = launch_absmax(vars[0].eps, (int64_t)S * numels[0], ws.scal + SC_EPS, stream)) return e;
-        if (vars[2].eps) if (int e = launch_absmax(vars[2].eps, (int64_t)S * numels[2], ws.scal + SC_EPS, stream)) return e;
-        bnn_bounds_kernel<<<(unsigned)std::min<int64_t>((numels[0] + numels[2] + 255) / 256, 296), 256, 0, stream>>>(
-            vars[0].mu, vars[0].rho, numels[0], vars[2].mu, vars[2].rho, numels[2], ws.scal);
-        BRN_LAUNCH_OK("bnn_bounds_kernel");
-        const bool fast = (P % 4 == 0) && ((uintptr_t)vars[0].mu % 16 == 0) && ((uintptr_t)vars[0].rho % 16 == 0) &&
-                          (!vars[0].eps || ((uintptr_t)vars[0].eps % 16 == 0));
-        if (fast) {
-            constexpr int SG = 8;
-            dim3 grid((unsigned)(((int64_t)H * P / 4 + 255) / 256), (unsigned)((S + SG - 1) / SG));
-            sample_w1_group_kernel<SG><<<grid, 256, 0, stream>>>(vars[0].mu, vars[0].rho, vars[0].eps, numels[0], ws_eps + offs[0], L.ldw,
-                                                                 ws.Wh, ws.Wl, H, P, HP, ws.ldP, *r, vars[0].var_id, ws.scal);
-            BRN_LAUNCH_OK("sample_w1_group_kernel");
-        } else {
-            if (vars[0].eps)
-                BRN_CUDA_OK(cudaMemcpy2DAsync(ws_eps + offs[0], L.ldw * sizeof(float), vars[0].eps, numels[0] * sizeof(float),
-                                              numels[0] * sizeof(float), S, cudaMemcpyDeviceToDevice, stream));
-            else if (int e = launch_philox_fill(ws_eps + offs[0], L.ldw, numels[0], vars[0].var_id, *r, stream)) return e;
-            dim3 grid((P + 255) / 256, H, S);
-            sample_w1_generic_kernel<<<grid, 256, 0, stream>>>(vars[0].mu, vars[0].rho, ws_eps + offs[0], L.ldw, ws.Wh, ws.Wl, H, P, HP,
-                                                               ws.ldP, ws.scal);
-            BRN_LAUNCH_OK("sample_w1_generic_kernel");
-        }
-        if (S % NS) {   // the odd tail tile reads one more sample block: keep it finite
-            BRN_CUDA_OK(cudaMemsetAsync(ws.Wh + (size_t)S * HP * ws.ldP, 0, sizeof(__half) * HP * ws.ldP, stream));
-            BRN_CUDA_OK(cudaMemsetAsync(ws.Wl + (size_t)S * HP * ws.ldP, 0, sizeof(__half) * HP * ws.ldP, stream));
-            BRN_CUDA_OK(cudaMemsetAsync(ws.dph + (size_t)S * HP * ws.ldB, 0, sizeof(__half) * HP * ws.ldB, stream));
-            BRN_CUDA_OK(cudaMemsetAsync(ws.dpl + (size_t)S * HP * ws.ldB, 0, sizeof(__half) * HP * ws.ldB, stream));
-        }
+        if (int e = bnn_tc_sample_w1(vars[0], vars[2], H, P, L.ldw, r, ws, ws_eps + offs[0], stream)) return e;
         // small variables: noise, sampled values, and zeroed per-sample gradient slots (accumulated into by the mid stage)
         if (int e = launch_sample_multi(vars + 1, offs + 1, 3, ws_eps, ws_W, L.ldw, *r, stream, ws_dW)) return e;
         // first read of the minibatch: everything above overlaps a host->device copy announced by brn_set_data_ready_event
-        if (int e = wait_data_ready(stream)) return e;
-        if (int e = launch_absmax(X, (int64_t)B * P, ws.scal + SC_X, stream)) return e;
-        dim3 grid((B + 31) / 32, (P + 31) / 32), block(32, 8);
-        split_f16_kernel<<<grid, block, 0, stream>>>(X, P, B, P, ws.Xh, ws.Xl, ws.ldP, ws.Xth, ws.Xtl, ws.ldB, ws.scal);
-        BRN_LAUNCH_OK("split_f16_kernel");
+        if (int e = bnn_tc_split_x(X, B, P, ws, stream)) return e;
     }
     {
         StageTimer st("bnn.gemm_fwd", stream);
-        EpiStore::Params ep;      // pre^T: [S][H][B], coalesced across the warp's rows b
-        ep.out = ws_pre; ep.rows = B; ep.row_stride = 1; ep.col_stride = B; ep.blk_stride = (int64_t)B * H;
-        ep.blk_valid = H; ep.col_limit = 0; ep.total_blks = S;
-        ep.bound_a = ws.scal + SC_X; ep.bound_b = ws.scal + SC_W1; ep.bound_b_mult = 1.f;
-        if (int e = launch_umma_nt_kind<BN, BNN_UMMA_BK, EpiStore, 8, 0, 4, 1>(ws.Xh, ws.Xl, B, ws.ldP, ws.Wh, ws.Wl, S * HP, ws.ldP, P, 0,
-                                                                               drain, ep, stream))
-            return e;
+        if (int e = bnn_tc_gemm_fwd(B, P, H, S, ws, ws_pre, stream)) return e;
     }
     if (forward_only) return 0;          // brn_bnn_predict: pre^T [S][H][B] is all it needs
     {
         StageTimer st("bnn.mid", stream);
-        if (int e = launch_mid4<HP>(ws_pre, ws_W, ws_dW, y, L, S, inv_S, loss, ws.dph, ws.dpl, ws.ldB, ws.scal, stream)) return e;
+        if (int e = launch_mid4<BNN_UMMA_HP>(ws_pre, ws_W, ws_dW, y, L, S, inv_S, loss, ws.dph, ws.dpl, ws.ldB, ws.scal, stream)) return e;
     }
     {
         StageTimer st("bnn.gemm_bwd", stream);
-        // K-split tail (see UnitIter): the dW1 blocks of the samples in the split n-tiles take atomic partial sums
-        int dev = 0, sms = 148;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        const UmmaSplitPlan plan = umma_plan<BN, 2 * BNN_UMMA_BK>(P, S * HP, B, sms, true);
-        if (plan.first_split_ntile >= 0) {
-            const int s_first = plan.first_split_ntile * NS;
-            if (s_first < S)
-                BRN_CUDA_OK(cudaMemset2DAsync(ws_dW + (size_t)s_first * L.ldw + L.oW1, L.ldw * sizeof(float), 0,
-                                              (size_t)H * P * sizeof(float), S - s_first, stream));
-        }
-        EpiStore::Params ep;      // dW1_s[h][p] = D[p, (s, h)]
-        ep.out = ws_dW + L.oW1; ep.rows = P; ep.row_stride = 1; ep.col_stride = P; ep.blk_stride = L.ldw;
-        ep.blk_valid = H; ep.col_limit = 0; ep.total_blks = S;
-        ep.bound_a = ws.scal + SC_X; ep.bound_b = ws.scal + SC_W2; ep.bound_b_mult = 2.f;
-        if (int e = launch_umma_nt_kind<BN, BNN_UMMA_BK, EpiStore, 8, 0, 4, 1>(ws.Xth, ws.Xtl, P, ws.ldB, ws.dph, ws.dpl, S * HP, ws.ldB, B,
-                                                                               0, drain_bwd, ep, stream, true))
-            return e;
+        // dpre = (W2^T da) act'(h) with sum_c |da_c| <= 2 and |act'| <= 1:  |dpre| <= 2 scal[SC_W2]
+        if (int e = bnn_tc_gemm_bwd(B, P, H, S, L.ldw, ws, ws_dW + L.oW1, ws.scal + SC_W2, 2.f, stream)) return e;
     }
     StageTimer st5("bnn.reduce_finalize", stream);
     return launch_mf_reduce_finalize_multi(vars, offs, 4, L.numel, ws_eps, L.ldw, ws_dW, L.ldw, ws_stats, *r, with_prior, loss, stream, 0);

@@ -11,7 +11,9 @@ Families
   LinearPlan  K2  observed Binomial(1)/Bernoulli/Categorical with logits = BF.matmul(W, x), W mean-field Normal
   LinregPlan  K2g observed Normal / Cauchy / Laplace(BF.matmul(W, x), sigma), W [1, F] mean-field Normal, sigma constant or a
               LogNormal latent
-  BNNPlan     K3  observed Categorical with logits = BF.matmul(W2, BF.tanh(BF.matmul(W1, x) + b1)) + b2
+  BNNPlan     K3  observed Categorical with logits = BF.matmul(W_out, h_L) + b_out, h_l = act_l(BF.matmul(W_l, h_{l-1}) + b_l),
+              h_0 = x, act_l in {BF.tanh, BF.relu, BF.sigmoid}: one hidden layer (brn_bnn_*, any width) or 2..4 hidden layers
+              of width <= 128 (brn_bnn_deep_*); every weight and bias a mean-field Normal latent
   ParticlePlan / WvgdPlan  K4 / K6  particle ensembles (SVGD, MAP, WVGD) of the K2 graph, or of the K2g graph at a constant
               noise scale
 Unrecognised graphs raise `UnsupportedModelError` -- there is no eager / CPU fallback for the ELBO.
@@ -321,15 +323,22 @@ class LinregPlan(Plan):
 class BNNPlan(Plan):
     family = "bnn (K3)"
 
-    def __init__(self, joint, posterior, k, specs, x_var, activation="tanh"):
+    def __init__(self, joint, posterior, k, layers, x_var):
+        """layers: [(weights spec, bias spec, activation of the layer's output)] from the input layer outward; the last one is
+        the output layer (activation None).  Two layers (one hidden) run on brn_bnn_*, more on brn_bnn_deep_*."""
         super().__init__(joint, posterior)
-        self.k, self.x_var, self.activation = k, x_var, activation
-        self.latents = specs          # weights1, b1, weights2, b2
+        self.k, self.x_var, self.layers = k, x_var, layers
+        self.latents = [spec for W, b, _ in layers for spec in (W, b)]          # weights1, b1, weights2, b2, ...
+        self.activations = [act for _, _, act in layers[:-1]]
+        if len(self.activations) > 1:
+            self.family = "bnn (K3, %d hidden layers)" % len(self.activations)
 
     def _launch(self, cu, mvars, r, empirical, loss=None):
         X = _data_matrix(empirical[self.x_var], "x")
         y = empirical[self.k].reshape(-1).to(torch.int32).contiguous()
-        return cu.bnn_elbo_fwd_bwd(X, y, mvars, r, loss=loss, activation=self.activation)
+        if len(self.activations) == 1:
+            return cu.bnn_elbo_fwd_bwd(X, y, mvars, r, loss=loss, activation=self.activations[0])
+        return cu.bnn_deep_elbo_fwd_bwd(X, y, mvars, r, self.activations, loss=loss)
 
     def predict(self, X, number_samples):
         """Batched posterior-predictive pass (SURVEY 8(f)3; replaces the per-image loop around
@@ -343,7 +352,10 @@ class BNNPlan(Plan):
         X = X.reshape(-1, int(np.prod(self.latents[0].shape[1:]))).contiguous()
         r = cu.sample_range(number_samples, seed=config.seed, offset=config.next_offset())
         mvars = [spec.make(cu, i, None) for i, spec in enumerate(self.latents)]
-        logits, labels, probs = cu.bnn_predict(X, mvars, r, activation=self.activation)
+        if len(self.activations) == 1:
+            logits, labels, probs = cu.bnn_predict(X, mvars, r, activation=self.activations[0])
+        else:
+            logits, labels, probs = cu.bnn_deep_predict(X, mvars, r, self.activations)
         return {"logits": logits, "samples": labels, "probs": probs, "sample_range": r}
 
 
@@ -401,25 +413,70 @@ def _lower_dense(joint, posterior):
                 raise UnsupportedModelError("Binomial/Bernoulli logistic regression needs weights of shape [1, F]")
             return LinearPlan(joint, posterior, k, ws, x, cu.CATEGORICAL if kind == "categorical" else cu.BERNOULLI, C)
 
-    # K3: logits = matmul(W2, act(matmul(W1, x) + b1)) + b2, act in {tanh, relu, sigmoid}
+    # K3: logits = matmul(W_out, h_L) + b_out, h_l = act(matmul(W_l, h_{l-1}) + b_l), h_0 = x
     if kind == "categorical":
-        for outer, b2e in _commutative_add(logits):
-            b2 = _var(b2e)
-            if not (_is_call(outer, "matmul", 2) and b2 in latents):
-                continue
-            W2, hid = _var(outer.args[0]), outer.args[1]
-            act = next((a for a in ("tanh", "relu", "sigmoid") if _is_call(hid, a, 1)), None)
-            if not (W2 in latents and act is not None):
-                continue
-            for inner, b1e in _commutative_add(hid.args[0]):
-                b1 = _var(b1e)
-                if not (_is_call(inner, "matmul", 2) and b1 in latents):
-                    continue
-                W1, x = _var(inner.args[0]), _var(inner.args[1])
-                if W1 in latents and _is_data(x) and len({W1, b1, W2, b2}) == 4 and len(latents) == 4:
-                    return BNNPlan(joint, posterior, k, [spec(W1), spec(b1), spec(W2), spec(b2)], x, activation=act)
+        mlp = _match_mlp(logits, latents)
+        if mlp is not None and len(mlp[1]) > 1:        # one layer (no hidden layer) is softmax regression with a bias: not K3
+            return _bnn_plan(joint, posterior, k, latents, spec, *mlp)
     raise UnsupportedModelError("model graph is not recognised by any fused kernel family "
                                 "(linear K2, bnn K3); likelihood link: %s" % k.partial_links["logits"].string)
+
+
+BNN_ACTIVATIONS = ("tanh", "relu", "sigmoid")
+BNN_DEEP_MAX_HIDDEN, BNN_DEEP_MAX_WIDTH, BNN_MAX_CLASSES = 4, 128, 16
+
+
+def _match_mlp(e, latents, inner=False):
+    """e = matmul(W, h) + b (either order of the sum) with W, b latents and h the data or act(<the same form>): returns
+    (x, layers), layers = [(W, b, activation applied to the layer's input)] from the input layer outward (None for the first),
+    or None.  A latent matmul without a bias where a layer is expected raises (`inner`: e sits inside an activation)."""
+    for mm, be in _commutative_add(e):
+        b, W = _var(be), _var(mm.args[0]) if _is_call(mm, "matmul", 2) else None
+        if not (W in latents and b in latents):
+            continue
+        h = mm.args[1]
+        if _is_data(_var(h)):
+            return _var(h), [(W, b, None)]
+        act = next((a for a in BNN_ACTIVATIONS if _is_call(h, a, 1)), None)
+        sub = _match_mlp(h.args[0], latents, inner=True) if act is not None else None
+        if sub is not None:
+            return sub[0], sub[1] + [(W, b, act)]
+    if _is_call(e, "matmul", 2) and _var(e.args[0]) in latents:
+        h = e.args[1]
+        if (inner and _is_data(_var(h))) or any(_is_call(h, a, 1) for a in BNN_ACTIVATIONS):
+            raise UnsupportedModelError("bnn family: the layer BF.matmul(%s, ...) has no bias; every layer of the network needs a "
+                                        "Normal bias latent (BF.matmul(W, h) + b)" % _var(e.args[0]).name)
+    return None
+
+
+def _bnn_plan(joint, posterior, k, latents, spec, x, layers):
+    """BNNPlan of a matched network (x, layers from _match_mlp), or UnsupportedModelError with the reason."""
+    n_hidden = len(layers) - 1
+    variables = [v for W, b, _ in layers for v in (W, b)]
+    if len(set(variables)) != len(variables):
+        raise UnsupportedModelError("bnn family: a latent appears in more than one layer (%s)" % ", ".join(v.name for v in variables))
+    others = [v.name for v in latents if v not in variables]
+    if others:
+        raise UnsupportedModelError("bnn family: latent(s) %s are neither weights nor biases of the network" % ", ".join(sorted(others)))
+    if n_hidden > BNN_DEEP_MAX_HIDDEN:
+        raise UnsupportedModelError("bnn family: %d hidden layers; at most %d are lowered" % (n_hidden, BNN_DEEP_MAX_HIDDEN))
+    specs = [(spec(W), spec(b)) for W, b, _ in layers]
+    if n_hidden > 1:
+        for l, (ws, bs) in enumerate(specs):
+            what = "hidden layer %d" % (l + 1) if l < n_hidden else "output layer"
+            if len(ws.shape) != 2 or int(np.prod(bs.shape)) != ws.shape[0]:
+                raise UnsupportedModelError("bnn family, %s: weights %s of shape %s and bias %s of shape %s do not form a layer"
+                                            % (what, ws.name, ws.shape, bs.name, bs.shape))
+            if l > 0 and ws.shape[1] != specs[l - 1][0].shape[0]:
+                raise UnsupportedModelError("bnn family, %s: weights %s take %d inputs, the layer below has %d units"
+                                            % (what, ws.name, ws.shape[1], specs[l - 1][0].shape[0]))
+            if l < n_hidden and ws.shape[0] > BNN_DEEP_MAX_WIDTH:
+                raise UnsupportedModelError("bnn family, %s: width %d; networks with more than one hidden layer are lowered for "
+                                            "widths up to %d" % (what, ws.shape[0], BNN_DEEP_MAX_WIDTH))
+        if specs[-1][0].shape[0] > BNN_MAX_CLASSES:
+            raise UnsupportedModelError("bnn family: %d classes; at most %d are lowered" % (specs[-1][0].shape[0], BNN_MAX_CLASSES))
+    acts = [layers[l + 1][2] for l in range(n_hidden)] + [None]
+    return BNNPlan(joint, posterior, k, [(ws, bs, a) for (ws, bs), a in zip(specs, acts)], x)
 
 
 REGRESSION_KINDS = {"normal": "Normal", "cauchy": "Cauchy", "laplace": "Laplace"}

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define BRN_ABI_VERSION 5
+#define BRN_ABI_VERSION 6
 
 /* One mean-field Normal variational variable  q(w) = N(mu, softplus(rho))  together with the Normal
  * prior p(w) = N(prior_loc, prior_scale) of the same name.
@@ -124,6 +124,26 @@ int brn_bnn_elbo_fwd_bwd_act(const float* X, const int32_t* y, int B, int P, int
 int brn_bnn_predict(const float* X, int B, int P, int H, int C, int activation, const brn_mf_var vars[4],
                     const brn_sample_range* r, void* workspace, size_t workspace_bytes, float* logits, int32_t* labels,
                     float* probs_mean, void* stream);
+
+/* K3 with 2 <= n_hidden <= 4 hidden layers (BNNs deeper than the two-layer network above):
+ *   h_1 = act[0](W1_s x + b1_s),  h_l = act[l-1](W_l,s h_{l-1} + b_l,s) for l = 2..n_hidden,  logits = W_out,s h_L + b_out,s
+ * with a Categorical(logits) likelihood over B observed rows, exactly the accumulation contract of brn_bnn_elbo_fwd_bwd_act.
+ * vars [2*n_hidden + 2] = (W1 [H[0], P], b1 [H[0]], W2 [H[1], H[0]], b2 [H[1]], ..., W_out [C, H[L-1]], b_out [C]); the Philox
+ * var_id of each is its position in this list by convention.  act[l] in {BRN_ACT_TANH, BRN_ACT_RELU, BRN_ACT_SIGMOID}.
+ * Limits: 1 <= H[l] <= 128, 1 <= C <= 16.  n_hidden == 1 is rejected: that network is brn_bnn_elbo_fwd_bwd_act /
+ * brn_bnn_predict.  The layer-1 GEMMs are those of the two-layer network (tcgen05 when 88 < H[0] <= 104, else SIMT; the same
+ * BRN_BNN_VARIANT override); the layers in between run on the tensor cores with fp32-equivalent accuracy.  s_local == 0
+ * leaves every output untouched.  The data-ready event of brn_set_data_ready_event is honoured as by brn_bnn_elbo_fwd_bwd.
+ * brn_bnn_deep_workspace_bytes returns 0 for a shape outside the limits.
+ * brn_bnn_deep_predict: the posterior-predictive pass of brn_bnn_predict for this network (logits [S_local, B, C], optional
+ * labels and probs_mean, same conventions). */
+size_t brn_bnn_deep_workspace_bytes(int B, int P, int n_hidden, const int* H, int C, int s_local);
+int brn_bnn_deep_elbo_fwd_bwd(const float* X, const int32_t* y, int B, int P, int n_hidden, const int* H, const int* act, int C,
+                              const brn_mf_var* vars, const brn_sample_range* r, void* workspace, size_t workspace_bytes,
+                              int with_prior, double* loss, void* stream);
+int brn_bnn_deep_predict(const float* X, int B, int P, int n_hidden, const int* H, const int* act, int C, const brn_mf_var* vars,
+                         const brn_sample_range* r, void* workspace, size_t workspace_bytes, float* logits, int32_t* labels,
+                         float* probs_mean, void* stream);
 
 /* K2 -- (multi-class) Bayesian logistic regression: logits_sbc = sum_f W_scf X_bf, W ~ q mean-field [C,F];
  *   likelihood 0: Bernoulli / Binomial(total_count=1, logits) with y float {0,1}  (C == 1)
