@@ -125,9 +125,7 @@ extern "C" int brn_allreduce_oneshot(const float* src, float* out, int64_t n, fl
     unsigned int* status = ticket + 1;
     unsigned int* arrive = reinterpret_cast<unsigned int*>(state_dev + 2);
     // the grid is a pure function of n (the arrival counter assumes the same grid on every call of a given state)
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = device_sm_count();
     const unsigned grid = (unsigned)std::min<int64_t>((n / 4 + 255) / 256 + 1, sms);
     allreduce_oneshot_kernel<<<grid, 256, 0, stream>>>(src, out, bufs_dev, flags_dev, rank, world, n, epoch, arrive, ticket, status,
                                                        loss_inout);

@@ -429,19 +429,14 @@ struct BnnWorkspace {
     BnnTcWorkspace tc;
     size_t bytes;
     BnnWorkspace(void* base, const BnnLayout& L, int S) {
-        size_t off = 0;
-        auto take = [&](size_t nfloat) {
-            float* p = base ? reinterpret_cast<float*>(reinterpret_cast<char*>(base) + off) : nullptr;
-            off += (nfloat * sizeof(float) + 255) / 256 * 256;
-            return p;
-        };
+        WorkspaceCarver take(base);
         eps = take((size_t)S * L.ldw);
         W = take((size_t)S * L.ldw);
         dW = take((size_t)S * L.ldw);
         pre = take((size_t)S * L.B * L.H);
         stats = take(4 * (size_t)L.ldw);
         tc.carve(take, L, S);
-        bytes = off;
+        bytes = take.off;
     }
 };
 
@@ -469,8 +464,7 @@ extern "C" int brn_bnn_elbo_fwd_bwd_act(const float* X, const int32_t* y, int B,
     BRN_CHECK_ARG(activation >= 0 && activation <= 2, "brn_bnn_elbo_fwd_bwd: unknown activation %d", activation);
     BRN_CHECK_ARG(B > 0 && P > 0 && H > 0 && C > 0, "brn_bnn_elbo_fwd_bwd: bad shape B=%d P=%d H=%d C=%d", B, P, H, C);
     BRN_CHECK_ARG(C <= BNN_MAXC, "brn_bnn_elbo_fwd_bwd: C=%d exceeds the supported maximum %d", C, BNN_MAXC);
-    BRN_CHECK_ARG(r->s_local >= 0 && r->s_total > 0 && r->s0 >= 0 && r->s0 + r->s_local <= r->s_total,
-                  "bad sample range s0=%d s_local=%d s_total=%d", r->s0, r->s_local, r->s_total);
+    if (int e = check_sample_range(*r)) return e;
     BnnLayout L(B, P, H, C, activation);
     const int64_t numels[4] = {(int64_t)H * P, H, (int64_t)C * H, C};
     const int64_t offs[4] = {L.oW1, L.ob1, L.oW2, L.ob2};
@@ -554,8 +548,7 @@ extern "C" int brn_bnn_predict(const float* X, int B, int P, int H, int C, int a
     BRN_CHECK_ARG(activation >= 0 && activation <= 2, "brn_bnn_predict: unknown activation %d", activation);
     BRN_CHECK_ARG(X && vars && r && logits, "brn_bnn_predict: NULL pointer");
     BRN_CHECK_ARG(B > 0 && P > 0 && H > 0 && C > 0 && C <= BNN_MAXC, "brn_bnn_predict: bad shape B=%d P=%d H=%d C=%d", B, P, H, C);
-    BRN_CHECK_ARG(r->s_local >= 0 && r->s_total > 0 && r->s0 >= 0 && r->s0 + r->s_local <= r->s_total,
-                  "bad sample range s0=%d s_local=%d s_total=%d", r->s0, r->s_local, r->s_total);
+    if (int e = check_sample_range(*r)) return e;
     BnnLayout L(B, P, H, C, activation);
     const int64_t numels[4] = {(int64_t)H * P, H, (int64_t)C * H, C};
     const int64_t offs[4] = {L.oW1, L.ob1, L.oW2, L.ob2};

@@ -319,12 +319,7 @@ struct DeepWorkspace {
     BnnTcWorkspace tc;
     size_t bytes;
     DeepWorkspace(void* base, const DeepLayout& D, int S) {
-        size_t off = 0;
-        auto take = [&](size_t nfloat) {
-            float* p = base ? reinterpret_cast<float*>(reinterpret_cast<char*>(base) + off) : nullptr;
-            off += (nfloat * sizeof(float) + 255) / 256 * 256;
-            return p;
-        };
+        WorkspaceCarver take(base);
         eps = take((size_t)S * D.ldw);
         W = take((size_t)S * D.ldw);
         dW = take((size_t)S * D.ldw);
@@ -334,7 +329,7 @@ struct DeepWorkspace {
             h[l] = l + 1 < D.L ? take((size_t)S * D.B * D.H[l]) : nullptr;
         }
         tc.carve(take, BnnLayout(D.B, D.P, D.H[0], D.C), S);
-        bytes = off;
+        bytes = take.off;
     }
 };
 
@@ -415,8 +410,7 @@ static int deep_check(const char* fn, const float* X, int B, int P, int n_hidden
         BRN_CHECK_ARG(H[l] > 0 && H[l] <= DEEP_MAXH, "%s: hidden width H[%d]=%d outside [1, %d]", fn, l, H[l], DEEP_MAXH);
         BRN_CHECK_ARG(act[l] >= 0 && act[l] <= 2, "%s: unknown activation act[%d]=%d", fn, l, act[l]);
     }
-    BRN_CHECK_ARG(r->s_local >= 0 && r->s_total > 0 && r->s0 >= 0 && r->s0 + r->s_local <= r->s_total,
-                  "bad sample range s0=%d s_local=%d s_total=%d", r->s0, r->s_local, r->s_total);
+    if (int e = check_sample_range(*r)) return e;
     const DeepLayout D(B, P, n_hidden, H, act, C);
     for (int v = 0; v < D.nvars(); ++v) {
         BRN_CHECK_ARG(vars[v].numel == D.n[v], "vars[%d].numel=%lld, expected %lld", v, (long long)vars[v].numel, (long long)D.n[v]);

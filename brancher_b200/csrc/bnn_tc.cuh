@@ -624,9 +624,7 @@ static int bnn_tc_gemm_bwd(int B, int P, int H, int S, int64_t ldw, const BnnTcW
                            float dpre_mult, cudaStream_t stream) {
     constexpr int NS = BNN_UMMA_NSAMP, BN = BNN_UMMA_HP * NS;
     // K-split tail (see UnitIter): the dW1 blocks of the samples in the split n-tiles take atomic partial sums
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = device_sm_count();
     const UmmaSplitPlan plan = umma_plan<BN, 2 * BNN_UMMA_BK>(P, S * BNN_UMMA_HP, B, sms, true);
     if (plan.first_split_ntile >= 0) {
         const int s_first = plan.first_split_ntile * NS;

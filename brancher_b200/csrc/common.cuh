@@ -45,6 +45,33 @@ void count_launch(int n);
         brn::count_launch(1);                                                                \
     } while (0)
 
+// SM count of the current device, read on every call (the caller may switch devices between calls)
+inline int device_sm_count() {
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    return sms;
+}
+
+// Cuts a workspace into consecutive pieces, each rounded up to 256 bytes.  With base == NULL it only counts: `off` is then
+// the number of bytes the same sequence of requests needs.
+struct WorkspaceCarver {
+    void* base; size_t off = 0;
+    explicit WorkspaceCarver(void* b) : base(b) {}
+    char* bytes(size_t n) {
+        char* p = base ? static_cast<char*>(base) + off : nullptr;
+        off += (n + 255) / 256 * 256;
+        return p;
+    }
+    float* operator()(size_t nfloat) { return reinterpret_cast<float*>(bytes(nfloat * sizeof(float))); }
+};
+
+inline int check_sample_range(const brn_sample_range& r) {
+    BRN_CHECK_ARG(r.s_local >= 0 && r.s_total > 0 && r.s0 >= 0 && r.s0 + r.s_local <= r.s_total,
+                  "bad sample range s0=%d s_local=%d s_total=%d", r.s0, r.s_local, r.s_total);
+    return 0;
+}
+
 // ---------------------------------------------------------------------------------------------
 // Philox4x32-10 (Salmon et al. 2011).  key = seed, counter = (i/4, global sample, var_id, offset).
 // One call -> 4 x u32 -> 4 standard normals (two Box-Muller pairs), element i uses lane i%4.

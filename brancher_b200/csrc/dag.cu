@@ -301,8 +301,7 @@ extern "C" int brn_dag_elbo_fwd_bwd(const brn_dag_op* ops, int n_ops, int n_slot
     BRN_CHECK_ARG(n_params == 0 || (params && dparams), "brn_dag_elbo_fwd_bwd: NULL parameter pointer");
     BRN_CHECK_ARG(n_rows >= 1 && n_cols >= 0 && (n_cols == 0 || data), "brn_dag_elbo_fwd_bwd: bad data block rows=%d cols=%d", n_rows,
                   n_cols);
-    BRN_CHECK_ARG(r->s_local >= 0 && r->s_total > 0 && r->s0 >= 0 && r->s0 + r->s_local <= r->s_total,
-                  "bad sample range s0=%d s_local=%d s_total=%d", r->s0, r->s_local, r->s_total);
+    if (int e = check_sample_range(*r)) return e;
     if (r->s_local == 0) return 0;
     set_variant("simt");
     StageTimer st("dag.fused", stream);

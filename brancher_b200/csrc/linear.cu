@@ -11,12 +11,17 @@
 // scheduled together) and nothing of size S x N ever reaches memory.
 #include "meanfield.cuh"
 #include "umma_gemm.cuh"
+#include <optional>
 #include <stdlib.h>
 
 namespace brn {
 
 constexpr int LN_T = 128;            // tile edge (rows, columns, max features)
 constexpr int LN_LD = LN_T + 4;      // smem leading dimension (keeps float4 alignment)
+
+// Likelihood codes of brn_linear_* (include/brancher_cuda.h); brn_linreg_* continue them with BRN_LINREG_NORMAL / _CAUCHY /
+// _LAPLACE.  The LIK template argument of linear_fused_kernel and linear_flash_kernel takes these codes.
+constexpr int LIN_BERNOULLI = 0, LIN_CATEGORICAL = 1;
 
 struct LinearArgs {
     const float* X; const void* y; int64_t N; int F, C, S;
@@ -28,8 +33,9 @@ struct LinearArgs {
     double* ll_cols2;                // LIK == 3: [S] += sum z^2 / (1 + z^2)
 };
 
-// 0: Bernoulli/Binomial(1) with float y, 1: Categorical with int32 labels, 2: Gaussian residuals with float y (C == 1): d = r =
-// y - l and ll_cols[s] += sum r^2 (loss unused; the noise scale is applied per sample afterwards, linreg_finish_kernel),
+// LIK, the likelihood code of the C ABI: 0: Bernoulli/Binomial(1) with float y, 1: Categorical with int32 labels, 2: Gaussian
+// residuals with float y (C == 1): d = r = y - l and ll_cols[s] += sum r^2 (loss unused; the noise scale is applied per sample
+// afterwards, linreg_finish_kernel),
 // 3: Cauchy residuals (C == 1): z = r / sigma_s, d = z / (1 + z^2), ll_cols[s] += sum log1p(z^2), ll_cols2[s] += sum z^2/(1 + z^2),
 // 4: Laplace residuals (C == 1): d = sign(r), ll_cols[s] += sum |r|  (3, 4: loss unused, finished by linreg_finish_kernel)
 template <int LIK>
@@ -72,7 +78,7 @@ __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
         isg[j] = 1.f;
-        if (LIK == 3) {
+        if (LIK == BRN_LINREG_CAUCHY) {
             const int col = (j < 4 ? tx * 4 + j : 64 + tx * 4 + (j - 4));
             if (col < ncols && j0 + col < J) isg[j] = 1.f / a.sigma[j0 + col];
         }
@@ -100,7 +106,7 @@ __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
         if (t < LN_T) {
             float v = 0.f;
             if (r0 + t < a.N) {
-                if (LIK != 1) v = reinterpret_cast<const float*>(a.y)[r0 + t];
+                if (LIK != LIN_CATEGORICAL) v = reinterpret_cast<const float*>(a.y)[r0 + t];
                 else v = __int_as_float(reinterpret_cast<const int32_t*>(a.y)[r0 + t]);
             }
             ys[t] = v;
@@ -137,7 +143,7 @@ __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
 
         // ---- phase 2: log-likelihood and d ll / d logit
         float ll_tile = 0.f;
-        if (LIK == 2) {
+        if (LIK != LIN_CATEGORICAL) {
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
                 int row = (i < 4 ? ty * 4 + i : 64 + ty * 4 + (i - 4));
@@ -148,56 +154,27 @@ __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
                 for (int j = 0; j < 8; ++j) {
                     int col = (j < 4 ? tx * 4 + j : 64 + tx * 4 + (j - 4));
                     bool ok = rv && col < ncols && (j0 + col) < J;
-                    d[j] = ok ? yv - acc[i][j] : 0.f;
-                    if (a.ll_cols) llc[j] += (double)(d[j] * d[j]);
-                }
-                *reinterpret_cast<float4*>(&Ls[row][tx * 4]) = make_float4(d[0], d[1], d[2], d[3]);
-                *reinterpret_cast<float4*>(&Ls[row][64 + tx * 4]) = make_float4(d[4], d[5], d[6], d[7]);
-            }
-            __syncthreads();
-        } else if (LIK == 3 || LIK == 4) {
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                int row = (i < 4 ? ty * 4 + i : 64 + ty * 4 + (i - 4));
-                bool rv = r0 + row < a.N;
-                float yv = ys[row];
-                float d[8];
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    int col = (j < 4 ? tx * 4 + j : 64 + tx * 4 + (j - 4));
-                    bool ok = rv && col < ncols && (j0 + col) < J;
-                    const float r = ok ? yv - acc[i][j] : 0.f;
-                    if (LIK == 3) {
+                    if constexpr (LIK == BRN_LINREG_NORMAL) {
+                        d[j] = ok ? yv - acc[i][j] : 0.f;
+                        if (a.ll_cols) llc[j] += (double)(d[j] * d[j]);
+                    } else if constexpr (LIK == BRN_LINREG_CAUCHY) {
+                        const float r = ok ? yv - acc[i][j] : 0.f;
                         const float z = r * isg[j], z2 = z * z, iq = 1.f / (1.f + z2);
                         d[j] = z * iq;
                         llc[j] += (double)log1pf(z2);
                         if (z2 != 0.f) atomicAdd(&llcol_s[col], (double)(z2 * iq));      // sixteen threads share a column
-                    } else {
+                    } else if constexpr (LIK == BRN_LINREG_LAPLACE) {
+                        const float r = ok ? yv - acc[i][j] : 0.f;
                         d[j] = r > 0.f ? 1.f : (r < 0.f ? -1.f : 0.f);      // sign(0) = 0, as torch's abs gradient
                         llc[j] += (double)fabsf(r);
+                    } else {
+                        float l = acc[i][j];
+                        float sp = log1pexpf(l);
+                        const float lv = ok ? __fmaf_rn(yv, l, -sp) : 0.f;
+                        ll_tile += lv;
+                        if (a.ll_cols) llc[j] += (double)lv;
+                        d[j] = ok ? yv - sigmoidf(l) : 0.f;
                     }
-                }
-                *reinterpret_cast<float4*>(&Ls[row][tx * 4]) = make_float4(d[0], d[1], d[2], d[3]);
-                *reinterpret_cast<float4*>(&Ls[row][64 + tx * 4]) = make_float4(d[4], d[5], d[6], d[7]);
-            }
-            __syncthreads();
-        } else if (LIK == 0) {
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                int row = (i < 4 ? ty * 4 + i : 64 + ty * 4 + (i - 4));
-                bool rv = r0 + row < a.N;
-                float yv = ys[row];
-                float d[8];
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    int col = (j < 4 ? tx * 4 + j : 64 + tx * 4 + (j - 4));
-                    bool ok = rv && col < ncols && (j0 + col) < J;
-                    float l = acc[i][j];
-                    float sp = log1pexpf(l);
-                    const float lv = ok ? __fmaf_rn(yv, l, -sp) : 0.f;
-                    ll_tile += lv;
-                    if (a.ll_cols) llc[j] += (double)lv;
-                    d[j] = ok ? yv - sigmoidf(l) : 0.f;
                 }
                 *reinterpret_cast<float4*>(&Ls[row][tx * 4]) = make_float4(d[0], d[1], d[2], d[3]);
                 *reinterpret_cast<float4*>(&Ls[row][64 + tx * 4]) = make_float4(d[4], d[5], d[6], d[7]);
@@ -263,13 +240,13 @@ __global__ void __launch_bounds__(256, 1) linear_fused_kernel(LinearArgs a) {
 
     // ---- flush
     if (a.ll_cols) {
-        if (LIK != 1) {
+        if (LIK != LIN_CATEGORICAL) {
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
                 const int col = (j < 4 ? tx * 4 + j : 64 + tx * 4 + (j - 4));
                 if (col < ncols && j0 + col < J && llc[j] != 0.0) atomicAdd(&a.ll_cols[j0 + col], llc[j]);
             }
-            if (LIK == 3) {
+            if (LIK == BRN_LINREG_CAUCHY) {
                 __syncthreads();
                 if (t < ncols && j0 + t < J && llcol_s[t] != 0.0) atomicAdd(&a.ll_cols2[j0 + t], llcol_s[t]);
             }
@@ -309,9 +286,24 @@ static int linear_tc_chunk_rows(int S, int sms) {
     return mt * 128;
 }
 
+// dW[i] = sum_j part[j * stride + i]
+__global__ void sum_slices_kernel(const float* __restrict__ part, int slices, int64_t stride, int64_t n, float* __restrict__ out) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    float acc = 0.f;
+    for (int j = 0; j < slices; ++j) acc += part[(int64_t)j * stride + i];
+    out[i] = acc;
+}
+
 }  // namespace brn
 #include "linear_flash.cuh"
 namespace brn {
+
+static int check_prepared_x(const char* fn, const void* px, int64_t N, int F) {
+    BRN_CHECK_ARG(!px || (linear_prepared_x_bytes(N, F) > 0 && (reinterpret_cast<uintptr_t>(px) & 255) == 0),
+                  "%s: a prepared X does not exist for N=%lld F=%d, or px is not 256-byte aligned", fn, (long long)N, F);
+    return 0;
+}
 
 // TF32-split operands and scratch of the tcgen05 variant (Bernoulli, C == 1); S = weight vectors (MC samples or particles)
 struct LinearTcBuffers {
@@ -343,21 +335,11 @@ struct LinearTcBuffers {
     }
 };
 
-struct WorkspaceCarver {
-    void* base; size_t off = 0;
-    explicit WorkspaceCarver(void* b) : base(b) {}
-    float* operator()(size_t nfloat) {
-        float* p = base ? reinterpret_cast<float*>(reinterpret_cast<char*>(base) + off) : nullptr;
-        off += (nfloat * sizeof(float) + 255) / 256 * 256;
-        return p;
-    }
-};
-
 struct LinearWorkspace {
     float *eps, *W, *dW, *stats;
     LinearTcBuffers tc;
     size_t bytes;
-    LinearWorkspace(void* base, int64_t numel, int S, int64_t N = 0, int F = 0, bool use_tc = false, int sms = 148) {
+    LinearWorkspace(void* base, int64_t numel, int S, int64_t N, int F, bool use_tc, int sms) {
         WorkspaceCarver take(base);
         eps = take((size_t)S * numel);
         W = take((size_t)S * numel);
@@ -368,15 +350,6 @@ struct LinearWorkspace {
         bytes = take.off;
     }
 };
-
-// dW[i] = sum_j part[j * stride + i]
-__global__ void sum_slices_kernel(const float* __restrict__ part, int slices, int64_t stride, int64_t n, float* __restrict__ out) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    float acc = 0.f;
-    for (int j = 0; j < slices; ++j) acc += part[(int64_t)j * stride + i];
-    out[i] = acc;
-}
 
 // particles: G = -(d ll / d theta) - d log N(theta; a, b) / d theta ; loss += sum -log N(theta; a, b)
 __global__ void __launch_bounds__(256)
@@ -399,11 +372,15 @@ particles_prior_kernel(const float* __restrict__ theta, const float* __restrict_
     if (threadIdx.x == 0 && prior_loc) atomicAdd(loss, tot);
 }
 
+// the shapes the staged tcgen05 pair takes (with the Bernoulli likelihood): what BRN_LINEAR_VARIANT=tcgen05 forces, and what
+// the workspace is sized for
+static bool linear_tc_shape(int64_t N, int F, int C, int S) { return C == 1 && F % 4 == 0 && F <= LT_BN2 && N >= 1 && S >= 1; }
+
 static bool linear_use_tc(int likelihood, int64_t N, int F, int C, int S) {
-    bool tc = likelihood == 0 && C == 1 && F % 4 == 0 && F <= LT_BN2 && N >= 4096 && S >= 64;
+    bool tc = likelihood == LIN_BERNOULLI && linear_tc_shape(N, F, C, S) && N >= 4096 && S >= 64;
     if (const char* env = getenv("BRN_LINEAR_VARIANT")) {
         if (!strcmp(env, "simt")) tc = false;
-        else if (!strcmp(env, "tcgen05")) tc = likelihood == 0 && C == 1 && F % 4 == 0 && F <= LT_BN2 && N >= 1 && S >= 1;
+        else if (!strcmp(env, "tcgen05")) tc = likelihood == LIN_BERNOULLI && linear_tc_shape(N, F, C, S);
     }
     return tc;
 }
@@ -421,32 +398,25 @@ static int launch_linear_fused(const float* X, const void* y, int likelihood, in
     const int spc = LN_T / C;
     const int col_tiles = (S + spc - 1) / spc;
     a.n_row_tiles = (N + LN_T - 1) / LN_T;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    int64_t groups = sms / col_tiles;
+    int64_t groups = device_sm_count() / col_tiles;
     if (groups < 1) groups = 1;
     if (groups > a.n_row_tiles) groups = a.n_row_tiles;
     a.tiles_per_group = (int)((a.n_row_tiles + groups - 1) / groups);
     groups = (a.n_row_tiles + a.tiles_per_group - 1) / a.tiles_per_group;
     const size_t smem = sizeof(float) * (3 * LN_T * LN_LD + LN_T);
     dim3 grid(col_tiles, (unsigned)groups);
-    if (likelihood == 0) {
-        BRN_CUDA_OK(cudaFuncSetAttribute(linear_fused_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        linear_fused_kernel<0><<<grid, 256, smem, stream>>>(a);
-    } else if (likelihood == 2) {
-        BRN_CUDA_OK(cudaFuncSetAttribute(linear_fused_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        linear_fused_kernel<2><<<grid, 256, smem, stream>>>(a);
-    } else if (likelihood == 3) {
-        BRN_CUDA_OK(cudaFuncSetAttribute(linear_fused_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        linear_fused_kernel<3><<<grid, 256, smem, stream>>>(a);
-    } else if (likelihood == 4) {
-        BRN_CUDA_OK(cudaFuncSetAttribute(linear_fused_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        linear_fused_kernel<4><<<grid, 256, smem, stream>>>(a);
-    } else {
-        BRN_CUDA_OK(cudaFuncSetAttribute(linear_fused_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        linear_fused_kernel<1><<<grid, 256, smem, stream>>>(a);
-    }
+    auto launch = [&](auto kern) -> int {
+        BRN_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kern<<<grid, 256, smem, stream>>>(a);
+        return 0;
+    };
+    int e;
+    if (likelihood == LIN_BERNOULLI) e = launch(linear_fused_kernel<LIN_BERNOULLI>);
+    else if (likelihood == BRN_LINREG_NORMAL) e = launch(linear_fused_kernel<BRN_LINREG_NORMAL>);
+    else if (likelihood == BRN_LINREG_CAUCHY) e = launch(linear_fused_kernel<BRN_LINREG_CAUCHY>);
+    else if (likelihood == BRN_LINREG_LAPLACE) e = launch(linear_fused_kernel<BRN_LINREG_LAPLACE>);
+    else e = launch(linear_fused_kernel<LIN_CATEGORICAL>);
+    if (e) return e;
     BRN_LAUNCH_OK("linear_fused_kernel");
     return 0;
 }
@@ -462,11 +432,8 @@ static int launch_linear_tc(const float* X, const float* y, int64_t N, int F, in
         // one pass over X: logits MMA -> likelihood -> d through shared memory -> gradient MMA (linear_flash.cuh)
         set_variant("tcgen05-flash");
         StageTimer st2(stage_fused, stream);
-        if (int e = launch_linear_flash(X, px, y, N, F, S, W, dW, loss_scale, loss, b.flash, stream)) return e;
-        const int64_t tot = (int64_t)S * F;
-        sum_slices_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(b.flash.part, b.flash.groups, tot, tot, dW);
-        BRN_LAUNCH_OK("sum_slices_kernel");
-        return 0;
+        return launch_linear_flash(LIN_BERNOULLI, X, px, y, N, F, S, W, dW, loss_scale, loss, nullptr, nullptr, nullptr, b.flash,
+                                   stream);
     }
     constexpr int drain = 2;
     // Operands that cross HBM once are kept as ONE fp32 matrix and split into TF32 (hi, lo) inside the GEMMs by converter warps
@@ -518,13 +485,10 @@ static int launch_linear_tc(const float* X, const float* y, int64_t N, int F, in
 
 extern "C" size_t brn_linear_particles_workspace_bytes(int64_t N, int F, int C, int n) {
     if (N < 0 || F <= 0 || C <= 0 || n < 0) return 0;
-    if (!(C == 1 && F % 4 == 0 && F <= LT_BN2 && N >= 1 && n >= 1)) return 0;      // only the tcgen05 variant needs scratch
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (!linear_tc_shape(N, F, C, n)) return 0;      // only the tcgen05 variant needs scratch
     WorkspaceCarver take(nullptr);
     LinearTcBuffers b;
-    b.carve(take, n, N, F, sms);
+    b.carve(take, n, N, F, device_sm_count());
     return take.off;
 }
 
@@ -537,8 +501,9 @@ extern "C" int brn_linear_particles_loss_grad(const float* X, const void* y, int
                   (long long)N, F, C, n);
     BRN_CHECK_ARG(N == 0 || (X && y), "brn_linear_particles_loss_grad: NULL data pointer");
     BRN_CHECK_ARG(F <= LN_T && C <= LN_T, "brn_linear_particles_loss_grad: F=%d / C=%d exceed the supported maximum %d", F, C, LN_T);
-    BRN_CHECK_ARG(likelihood == 0 || likelihood == 1, "brn_linear_particles_loss_grad: unknown likelihood %d", likelihood);
-    BRN_CHECK_ARG(likelihood == 1 || C == 1, "Bernoulli/Binomial likelihood needs C == 1 (got %d)", C);
+    BRN_CHECK_ARG(likelihood == LIN_BERNOULLI || likelihood == LIN_CATEGORICAL, "brn_linear_particles_loss_grad: unknown likelihood %d",
+                  likelihood);
+    BRN_CHECK_ARG(likelihood == LIN_CATEGORICAL || C == 1, "Bernoulli/Binomial likelihood needs C == 1 (got %d)", C);
     BRN_CHECK_ARG((prior_loc == nullptr) == (prior_scale == nullptr), "prior_loc and prior_scale must both be given or both NULL");
     if (n == 0) return 0;
     // tcgen05 variant (the K2 GEMM pair with the particles as the weight vectors) when the caller provides scratch
@@ -546,12 +511,9 @@ extern "C" int brn_linear_particles_loss_grad(const float* X, const void* y, int
     set_variant(use_tc ? "tcgen05" : "simt");
     const int64_t numel = (int64_t)C * F, total = numel * n;
     if (use_tc) {
-        int dev = 0, sms = 148;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
         WorkspaceCarver take(workspace);
         LinearTcBuffers b;
-        b.carve(take, n, N, F, sms);
+        b.carve(take, n, N, F, device_sm_count());
         BRN_CHECK_ARG(workspace_bytes >= take.off, "workspace too small: %zu < %zu", workspace_bytes, take.off);
         if (int e = launch_linear_tc(X, reinterpret_cast<const float*>(y), N, F, n, theta, G, -1.0f, loss, b,
                                      "particles.split_operands", "particles.loglik_grad", stream))
@@ -578,8 +540,9 @@ extern "C" int brn_linear_vectors_loglik_grad(const float* X, const void* y, int
                   (long long)N, F, C, n);
     BRN_CHECK_ARG(N == 0 || (X && y), "brn_linear_vectors_loglik_grad: NULL data pointer");
     BRN_CHECK_ARG(F <= LN_T && C <= LN_T, "brn_linear_vectors_loglik_grad: F=%d / C=%d exceed the supported maximum %d", F, C, LN_T);
-    BRN_CHECK_ARG(likelihood == 0 || likelihood == 1, "brn_linear_vectors_loglik_grad: unknown likelihood %d", likelihood);
-    BRN_CHECK_ARG(likelihood == 1 || C == 1, "Bernoulli/Binomial likelihood needs C == 1 (got %d)", C);
+    BRN_CHECK_ARG(likelihood == LIN_BERNOULLI || likelihood == LIN_CATEGORICAL, "brn_linear_vectors_loglik_grad: unknown likelihood %d",
+                  likelihood);
+    BRN_CHECK_ARG(likelihood == LIN_CATEGORICAL || C == 1, "Bernoulli/Binomial likelihood needs C == 1 (got %d)", C);
     if (n == 0) return 0;
     set_variant("simt");
     const int64_t total = (int64_t)C * F * n;
@@ -600,11 +563,7 @@ extern "C" int brn_linear_vectors_loglik_grad(const float* X, const void* y, int
 extern "C" size_t brn_linear_workspace_bytes(int64_t N, int F, int C, int s_local) {
     if (N < 0 || F <= 0 || C <= 0 || s_local < 0) return 0;
     // sized for the larger of the two variants (the likelihood is not known here): tcgen05 buffers whenever C == 1
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const bool tc = C == 1 && F % 4 == 0 && F <= LT_BN2 && N >= 1 && s_local >= 1;
-    return LinearWorkspace(nullptr, (int64_t)C * F, s_local, N, F, tc, sms).bytes;
+    return LinearWorkspace(nullptr, (int64_t)C * F, s_local, N, F, linear_tc_shape(N, F, C, s_local), device_sm_count()).bytes;
 }
 
 extern "C" size_t brn_linear_prepared_x_bytes(int64_t N, int F) { return linear_prepared_x_bytes(N, F); }
@@ -629,28 +588,23 @@ extern "C" int brn_linear_elbo_fwd_bwd_px(const float* X, const void* px, const 
                                           const brn_mf_var* w, const brn_sample_range* r, void* workspace,
                                           size_t workspace_bytes, int with_prior, double* loss, void* stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
-    BRN_CHECK_ARG(!px || (linear_prepared_x_bytes(N, F) > 0 && (reinterpret_cast<uintptr_t>(px) & 255) == 0),
-                  "brn_linear_elbo_fwd_bwd_px: a prepared X does not exist for N=%lld F=%d, or px is not 256-byte aligned", (long long)N, F);
+    if (int e = check_prepared_x("brn_linear_elbo_fwd_bwd_px", px, N, F)) return e;
     BRN_CHECK_ARG(w && r && loss, "brn_linear_elbo_fwd_bwd: NULL pointer");
     BRN_CHECK_ARG(N >= 0 && F > 0 && C > 0, "brn_linear_elbo_fwd_bwd: bad shape N=%lld F=%d C=%d", (long long)N, F, C);
     BRN_CHECK_ARG(N == 0 || (X && y), "brn_linear_elbo_fwd_bwd: NULL data pointer");
     BRN_CHECK_ARG(F <= LN_T, "brn_linear_elbo_fwd_bwd: F=%d exceeds the supported maximum %d", F, LN_T);
     BRN_CHECK_ARG(C <= LN_T, "brn_linear_elbo_fwd_bwd: C=%d exceeds the supported maximum %d", C, LN_T);
-    BRN_CHECK_ARG(likelihood == 0 || likelihood == 1, "brn_linear_elbo_fwd_bwd: unknown likelihood %d", likelihood);
-    BRN_CHECK_ARG(likelihood == 1 || C == 1, "Bernoulli/Binomial likelihood needs C == 1 (got %d)", C);
-    BRN_CHECK_ARG(r->s_local >= 0 && r->s_total > 0 && r->s0 >= 0 && r->s0 + r->s_local <= r->s_total,
-                  "bad sample range s0=%d s_local=%d s_total=%d", r->s0, r->s_local, r->s_total);
+    BRN_CHECK_ARG(likelihood == LIN_BERNOULLI || likelihood == LIN_CATEGORICAL, "brn_linear_elbo_fwd_bwd: unknown likelihood %d", likelihood);
+    BRN_CHECK_ARG(likelihood == LIN_CATEGORICAL || C == 1, "Bernoulli/Binomial likelihood needs C == 1 (got %d)", C);
+    if (int e = check_sample_range(*r)) return e;
     const int64_t numel = (int64_t)C * F;
     BRN_CHECK_ARG(w->numel == numel, "w->numel=%lld, expected C*F=%lld", (long long)w->numel, (long long)numel);
     BRN_CHECK_ARG(w->mu && w->rho && w->dmu && w->drho, "w: NULL parameter pointer");
     BRN_CHECK_ARG(!with_prior || w->tied || (w->prior_loc && w->prior_scale), "prior_loc/prior_scale required when not tied");
     const int S = r->s_local;
     if (S == 0) return 0;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const bool use_tc = linear_use_tc(likelihood, N, F, C, S);
-    LinearWorkspace ws(workspace, numel, S, N, F, use_tc, sms);
+    LinearWorkspace ws(workspace, numel, S, N, F, use_tc, device_sm_count());
     BRN_CHECK_ARG(workspace && workspace_bytes >= ws.bytes, "workspace too small: %zu < %zu", workspace_bytes, ws.bytes);
     set_variant(use_tc ? "tcgen05" : "simt");
 
@@ -686,19 +640,13 @@ extern "C" int brn_linear_elbo_fwd_bwd_px(const float* X, const void* px, const 
 // ---------------------------------------------------------------------------------------------
 namespace brn {
 
-struct LinregWorkspace {
-    float *eps, *W, *dW, *stats;
+// What the X pass of S weight vectors (linreg_x_pass) reads and writes besides the vectors and their gradient
+struct LinregXPassBuffers {
     double* R;                 // [S] sums of squared residuals (Cauchy: of log1p(z^2); Laplace: of |r|)
-    float* sigma;              // [S] noise scale per sample
+    float* sigma;              // [S] noise scale per vector
     double* T;                 // [S] Cauchy: sums of z^2 / (1 + z^2)
     LinearFlashBuffers flash;
-    size_t bytes;
-    LinregWorkspace(void* base, int S, int64_t N, int F, bool flash_path, int sms) {
-        WorkspaceCarver take(base);
-        eps = take((size_t)S * F);
-        W = take((size_t)S * F);
-        dW = take((size_t)S * F);
-        stats = take(4 * (size_t)((F + 3) / 4 * 4));
+    void carve(WorkspaceCarver& take, int S, int64_t N, int F, bool flash_path, int sms) {
         R = reinterpret_cast<double*>(take(2 * (size_t)S));
         sigma = take((size_t)S);
         T = reinterpret_cast<double*>(take(2 * (size_t)S));
@@ -708,6 +656,20 @@ struct LinregWorkspace {
             flash.Xh = reinterpret_cast<__half*>(take(((size_t)N * F + 1) / 2));
             flash.Xl = reinterpret_cast<__half*>(take(((size_t)N * F + 1) / 2));
         }
+    }
+};
+
+struct LinregWorkspace {
+    float *eps, *W, *dW, *stats;
+    LinregXPassBuffers x;
+    size_t bytes;
+    LinregWorkspace(void* base, int S, int64_t N, int F, bool flash_path, int sms) {
+        WorkspaceCarver take(base);
+        eps = take((size_t)S * F);
+        W = take((size_t)S * F);
+        dW = take((size_t)S * F);
+        stats = take(4 * (size_t)((F + 3) / 4 * 4));
+        x.carve(take, S, N, F, flash_path, sms);
         bytes = take.off;
     }
 };
@@ -826,26 +788,6 @@ linreg_finish_kernel(float* __restrict__ dW, const double* __restrict__ R, const
 // The finisher of n weight vectors (particles, or WVGD's draws) at a fixed noise scale: one thread per element (k, f) of G,
 // G_k *= the likelihood's scale (G may be NULL); the thread of f == 0 computes ll_k in fp64 and writes ll[k] (ll != NULL) or adds
 // -ll_k to *loss.  No 1/S factor: particle losses are sums over the particles.
-struct LinregVectorsWorkspace {
-    double *R, *T;
-    float* sigma;
-    LinearFlashBuffers flash;
-    size_t bytes;
-    LinregVectorsWorkspace(void* base, int n, int64_t N, int F, bool flash_path, int sms) {
-        WorkspaceCarver take(base);
-        R = reinterpret_cast<double*>(take(2 * (size_t)n));
-        T = reinterpret_cast<double*>(take(2 * (size_t)n));
-        sigma = take((size_t)n);
-        flash = LinearFlashBuffers();
-        if (flash_path) {
-            flash.carve(take, n, F, sms);
-            flash.Xh = reinterpret_cast<__half*>(take(((size_t)N * F + 1) / 2));
-            flash.Xl = reinterpret_cast<__half*>(take(((size_t)N * F + 1) / 2));
-        }
-        bytes = take.off;
-    }
-};
-
 __global__ void __launch_bounds__(256)
 linreg_vectors_finish_kernel(float* __restrict__ G, const double* __restrict__ R, const double* __restrict__ T,
                              const float* __restrict__ sig, int lik, int F, int64_t N, int n, double* __restrict__ ll,
@@ -872,13 +814,23 @@ linreg_vectors_finish_kernel(float* __restrict__ G, const double* __restrict__ R
 
 }  // namespace brn
 
+// The X pass of the regression likelihood for S weight vectors W [S][F] at the noise scales b.sigma: zeroes the sums b.R (and b.T
+// for Cauchy), then runs the one-pass kernel, or linear_fused_kernel on a zeroed G.  G leaves holding + d ll / d W before the
+// noise scale is applied (linreg_grad_scale); with G == NULL only the sums are formed.
+static int linreg_x_pass(const LinregXPassBuffers& b, int likelihood, bool use_flash, const float* X, const void* px, const float* y,
+                         int64_t N, int F, const float* W, int S, float* G, cudaStream_t stream) {
+    BRN_CUDA_OK(cudaMemsetAsync(b.R, 0, sizeof(double) * (size_t)S, stream));
+    if (likelihood == BRN_LINREG_CAUCHY) BRN_CUDA_OK(cudaMemsetAsync(b.T, 0, sizeof(double) * (size_t)S, stream));
+    if (use_flash) return launch_linear_flash(likelihood, X, px, y, N, F, S, W, G, 0.f, nullptr, b.R, b.sigma, b.T, b.flash, stream);
+    if (G) BRN_CUDA_OK(cudaMemsetAsync(G, 0, sizeof(float) * (size_t)S * F, stream));      // the finishers read G even when N == 0
+    if (N == 0) return 0;
+    return launch_linear_fused(X, y, likelihood, N, F, 1, S, W, G, 0.f, nullptr, stream, b.R, b.sigma, b.T);
+}
+
 extern "C" size_t brn_linreg_workspace_bytes(int64_t N, int F, int s_local) {
     if (N < 0 || F <= 0 || s_local < 0) return 0;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     // sized for the one-pass kernel whenever a call of this shape may take it (X's alignment is not known here)
-    return LinregWorkspace(nullptr, s_local, N, F, linreg_use_flash(nullptr, N, F, s_local), sms).bytes;
+    return LinregWorkspace(nullptr, s_local, N, F, linreg_use_flash(nullptr, N, F, s_local), device_sm_count()).bytes;
 }
 
 extern "C" int brn_linreg_elbo_fwd_bwd(const float* X, const void* px, const float* y, int64_t N, int F, const brn_mf_var* w,
@@ -900,12 +852,10 @@ extern "C" int brn_linreg_elbo_fwd_bwd_lik(const float* X, const void* px, const
     BRN_CHECK_ARG(N >= 0 && F > 0, "brn_linreg_elbo_fwd_bwd: bad shape N=%lld F=%d", (long long)N, F);
     BRN_CHECK_ARG(N == 0 || (X && y), "brn_linreg_elbo_fwd_bwd: NULL data pointer");
     BRN_CHECK_ARG(F <= LN_T, "brn_linreg_elbo_fwd_bwd: F=%d exceeds the supported maximum %d", F, LN_T);
-    BRN_CHECK_ARG(!px || (linear_prepared_x_bytes(N, F) > 0 && (reinterpret_cast<uintptr_t>(px) & 255) == 0),
-                  "brn_linreg_elbo_fwd_bwd: a prepared X does not exist for N=%lld F=%d, or px is not 256-byte aligned", (long long)N, F);
+    if (int e = check_prepared_x("brn_linreg_elbo_fwd_bwd", px, N, F)) return e;
     BRN_CHECK_ARG((nu == nullptr) != (noise_scale == nullptr),
                   "brn_linreg_elbo_fwd_bwd: give exactly one of nu (LogNormal noise latent) and noise_scale (fixed noise)");
-    BRN_CHECK_ARG(r->s_local >= 0 && r->s_total > 0 && r->s0 >= 0 && r->s0 + r->s_local <= r->s_total,
-                  "bad sample range s0=%d s_local=%d s_total=%d", r->s0, r->s_local, r->s_total);
+    if (int e = check_sample_range(*r)) return e;
     BRN_CHECK_ARG(w->numel == F, "w->numel=%lld, expected F=%d", (long long)w->numel, F);
     BRN_CHECK_ARG(w->mu && w->rho && w->dmu && w->drho, "w: NULL parameter pointer");
     BRN_CHECK_ARG(!with_prior || w->tied || (w->prior_loc && w->prior_scale), "w: prior_loc/prior_scale required when not tied");
@@ -916,11 +866,8 @@ extern "C" int brn_linreg_elbo_fwd_bwd_lik(const float* X, const void* px, const
     }
     const int S = r->s_local;
     if (S == 0) return 0;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const bool use_flash = N > 0 && linreg_use_flash(X, N, F, S);
-    LinregWorkspace ws(workspace, S, N, F, use_flash, sms);
+    LinregWorkspace ws(workspace, S, N, F, use_flash, device_sm_count());
     BRN_CHECK_ARG(workspace && workspace_bytes >= ws.bytes, "workspace too small: %zu < %zu", workspace_bytes, ws.bytes);
     set_variant(use_flash ? "tcgen05-flash" : "simt");
 
@@ -932,31 +879,20 @@ extern "C" int brn_linreg_elbo_fwd_bwd_lik(const float* X, const void* px, const
             eps = ws.eps;
         }
         if (int e = launch_sample_weights(w->mu, w->rho, eps, F, ws.W, F, F, S, stream)) return e;
-        BRN_CUDA_OK(cudaMemsetAsync(ws.R, 0, sizeof(double) * (size_t)S, stream));
-        if (likelihood == BRN_LINREG_CAUCHY) BRN_CUDA_OK(cudaMemsetAsync(ws.T, 0, sizeof(double) * (size_t)S, stream));
-        if (!use_flash) BRN_CUDA_OK(cudaMemsetAsync(ws.dW, 0, sizeof(float) * (size_t)S * F, stream));
-        linreg_sigma_kernel<<<(unsigned)((S + 255) / 256), 256, 0, stream>>>(ws.sigma, nu ? *nu : brn_mf_var{}, nu != nullptr, noise_scale,
-                                                                            *r);
+        linreg_sigma_kernel<<<(unsigned)((S + 255) / 256), 256, 0, stream>>>(ws.x.sigma, nu ? *nu : brn_mf_var{}, nu != nullptr,
+                                                                            noise_scale, *r);
         BRN_LAUNCH_OK("linreg_sigma_kernel");
     }
-    // likelihood codes of the one-pass kernel's LIK (1 Gaussian, 2 Cauchy, 3 Laplace) and of linear_fused_kernel (2, 3, 4)
-    const int lik_flash = likelihood - BRN_LINREG_NORMAL + 1, lik_simt = likelihood - BRN_LINREG_NORMAL + 2;
-    if (use_flash) {
-        StageTimer st("linreg.fused", stream);
-        if (int e = launch_linear_flash(X, px, y, N, F, S, ws.W, ws.dW, 0.f, nullptr, ws.flash, stream, ws.R, lik_flash, ws.sigma, ws.T))
-            return e;
-        const int64_t tot = (int64_t)S * F;
-        sum_slices_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(ws.flash.part, ws.flash.groups, tot, tot, ws.dW);
-        BRN_LAUNCH_OK("sum_slices_kernel");
-    } else if (N > 0) {
-        StageTimer st("linreg.fused", stream);
-        if (int e = launch_linear_fused(X, y, lik_simt, N, F, 1, S, ws.W, ws.dW, 0.f, nullptr, stream, ws.R, ws.sigma, ws.T)) return e;
+    {
+        std::optional<StageTimer> st;       // N == 0 only zeroes the sums and dW: no X pass to time
+        if (N > 0) st.emplace("linreg.fused", stream);
+        if (int e = linreg_x_pass(ws.x, likelihood, use_flash, X, px, y, N, F, ws.W, S, ws.dW, stream)) return e;
     }
     {
         StageTimer st("linreg.finish", stream);
         const int64_t tot = (int64_t)S * F;
         brn_mf_var nv = nu ? *nu : brn_mf_var{};
-        linreg_finish_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(ws.dW, ws.R, ws.T, ws.sigma, likelihood, F, N, nv,
+        linreg_finish_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(ws.dW, ws.x.R, ws.x.T, ws.x.sigma, likelihood, F, N, nv,
                                                                               nu != nullptr, *r, with_prior, loss);
         BRN_LAUNCH_OK("linreg_finish_kernel");
     }
@@ -978,56 +914,38 @@ static int linreg_vectors_check(const char* fn, const float* X, const void* px, 
     BRN_CHECK_ARG(N >= 0 && F > 0 && n >= 0, "%s: bad shape N=%lld F=%d n=%d", fn, (long long)N, F, n);
     BRN_CHECK_ARG(N == 0 || (X && y), "%s: NULL data pointer", fn);
     BRN_CHECK_ARG(F <= LN_T, "%s: F=%d exceeds the supported maximum %d", fn, F, LN_T);
-    BRN_CHECK_ARG(!px || (linear_prepared_x_bytes(N, F) > 0 && (reinterpret_cast<uintptr_t>(px) & 255) == 0),
-                  "%s: a prepared X does not exist for N=%lld F=%d, or px is not 256-byte aligned", fn, (long long)N, F);
-    return 0;
+    return check_prepared_x(fn, px, N, F);
 }
 
 static int linreg_vectors_run(const float* X, const void* px, const float* y, int likelihood, int64_t N, int F, const float* V, int n,
                               const float* noise_scale, float* G, double* ll, double* loss, void* workspace, size_t workspace_bytes,
                               const char* stage, cudaStream_t stream) {
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const bool use_flash = N > 0 && linreg_use_flash(X, N, F, n);
-    LinregVectorsWorkspace ws(workspace, n, N, F, use_flash, sms);
-    BRN_CHECK_ARG(workspace && workspace_bytes >= ws.bytes, "workspace too small: %zu < %zu", workspace_bytes, ws.bytes);
+    WorkspaceCarver take(workspace);
+    LinregXPassBuffers b;
+    b.carve(take, n, N, F, use_flash, device_sm_count());
+    BRN_CHECK_ARG(workspace && workspace_bytes >= take.off, "workspace too small: %zu < %zu", workspace_bytes, take.off);
     set_variant(use_flash ? "tcgen05-flash" : "simt");
     const int64_t tot = (int64_t)n * F;
     StageTimer st(stage, stream);
-    BRN_CUDA_OK(cudaMemsetAsync(ws.R, 0, sizeof(double) * (size_t)n, stream));
-    if (likelihood == BRN_LINREG_CAUCHY) BRN_CUDA_OK(cudaMemsetAsync(ws.T, 0, sizeof(double) * (size_t)n, stream));
     brn_sample_range r{};
     r.s_local = n;
     r.s_total = n;
-    linreg_sigma_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(ws.sigma, brn_mf_var{}, 0, noise_scale, r);
+    linreg_sigma_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(b.sigma, brn_mf_var{}, 0, noise_scale, r);
     BRN_LAUNCH_OK("linreg_sigma_kernel");
-    const int lik_flash = likelihood - BRN_LINREG_NORMAL + 1, lik_simt = likelihood - BRN_LINREG_NORMAL + 2;
-    if (use_flash) {
-        if (int e = launch_linear_flash(X, px, y, N, F, n, V, G, 0.f, nullptr, ws.flash, stream, ws.R, lik_flash, ws.sigma, ws.T))
-            return e;
-        if (G) {
-            sum_slices_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(ws.flash.part, ws.flash.groups, tot, tot, G);
-            BRN_LAUNCH_OK("sum_slices_kernel");
-        }
-    } else {
-        if (G) BRN_CUDA_OK(cudaMemsetAsync(G, 0, sizeof(float) * (size_t)tot, stream));
-        if (N > 0)
-            if (int e = launch_linear_fused(X, y, lik_simt, N, F, 1, n, V, G, 0.f, nullptr, stream, ws.R, ws.sigma, ws.T)) return e;
-    }
-    linreg_vectors_finish_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(G, ws.R, ws.T, ws.sigma, likelihood, F, N, n, ll,
-                                                                                  loss);
+    if (int e = linreg_x_pass(b, likelihood, use_flash, X, px, y, N, F, V, n, G, stream)) return e;
+    linreg_vectors_finish_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(G, b.R, b.T, b.sigma, likelihood, F, N, n, ll, loss);
     BRN_LAUNCH_OK("linreg_vectors_finish_kernel");
     return 0;
 }
 
 extern "C" size_t brn_linreg_vectors_workspace_bytes(int64_t N, int F, int n) {
     if (N < 0 || F <= 0 || n < 0) return 0;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     // sized for the one-pass kernel whenever a call of this shape may take it (X's alignment is not known here)
-    return LinregVectorsWorkspace(nullptr, n, N, F, N > 0 && linreg_use_flash(nullptr, N, F, n), sms).bytes;
+    WorkspaceCarver take(nullptr);
+    LinregXPassBuffers b;
+    b.carve(take, n, N, F, N > 0 && linreg_use_flash(nullptr, N, F, n), device_sm_count());
+    return take.off;
 }
 
 extern "C" int brn_linreg_particles_loss_grad(const float* X, const void* px, const float* y, int likelihood, int64_t N, int F,

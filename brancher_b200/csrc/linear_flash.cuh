@@ -135,10 +135,11 @@ __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.
 // The d tile (A operand of the gradient MMA) lives in tensor memory (64 columns: hi pair words, lo pair words): the epilogue
 // thread that owns TMEM lane s writes row s with tcgen05.st -- no shared-memory round trip, no generic -> async proxy fence,
 // half the shared-memory operand reads of the gradient MMA.
-// LIK: 0 = Bernoulli (d = y - sigmoid(l), loss += loss_scale * sum ll), 1 = Gaussian residuals (d = r = y - l, R[s] += sum r^2;
-// the noise scale is applied afterwards, per vector, by the caller), 2 = Cauchy (z = r / sigma_s, d = z / (1 + z^2),
-// R[s] += sum log1p(z^2), T[s] += sum z^2 / (1 + z^2)), 3 = Laplace (d = sign(r), R[s] += sum |r|; sigma applied afterwards).
-template <int KS1, int LIK = 0>
+// LIK, the likelihood code of the C ABI: LIN_BERNOULLI (d = y - sigmoid(l), loss += loss_scale * sum ll), BRN_LINREG_NORMAL
+// (Gaussian residuals: d = r = y - l, R[s] += sum r^2; the noise scale is applied afterwards, per vector, by the caller),
+// BRN_LINREG_CAUCHY (z = r / sigma_s, d = z / (1 + z^2), R[s] += sum log1p(z^2), T[s] += sum z^2 / (1 + z^2)),
+// BRN_LINREG_LAPLACE (d = sign(r), R[s] += sum |r|; sigma applied afterwards).
+template <int KS1, int LIK>
 __global__ void __launch_bounds__(LF_THREADS, 1)
 linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_constant__ CUtensorMap tmWl,
                     const __grid_constant__ CUtensorMap tmXh, const __grid_constant__ CUtensorMap tmXl, LinearFlashParams p) {
@@ -306,10 +307,10 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
         const int n_chains = (my_blocks + LF_D2_CHAIN - 1) / LF_D2_CHAIN;
         // Gaussian: d = r * r_scale with r_scale = p2_scale(max|y| + F max|W| max|X|) >= 2^13 / max|r|: |d| < 2^14 fits fp16
         float r_scale = 0.f;
-        if constexpr (LIK == 1) r_scale = p2_scale(*p.scal_y + (float)F * *p.scal_w * *p.scal_x);
+        if constexpr (LIK == BRN_LINREG_NORMAL) r_scale = p2_scale(*p.scal_y + (float)F * *p.scal_w * *p.scal_x);
         // Cauchy: lane s owns vector s, so 1 / sigma_s is one register, loaded once
         float inv_sig = 1.f;
-        if constexpr (LIK == 2) inv_sig = s_ok ? 1.f / p.sigma[s_glob] : 1.f;
+        if constexpr (LIK == BRN_LINREG_CAUCHY) inv_sig = s_ok ? 1.f / p.sigma[s_glob] : 1.f;
         double ll2_total = 0.0;     // Cauchy: sum of z^2 / (1 + z^2)
         const uint64_t c2 = f2_pack(inv1 * 1.4426950408889634f, inv1 * 1.4426950408889634f);
         const uint64_t one2 = f2_pack(1.f, 1.f), ms2 = f2_pack(-LF_D_SCALE, -LF_D_SCALE), mone2 = f2_pack(-1.f, -1.f);
@@ -344,7 +345,7 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
             uint32_t dh_w[LF_EROWS / 2], dl_w[LF_EROWS / 2];
             float ll;                                  // Bernoulli: sum of the block's log-likelihoods; Gaussian: sum of r^2
                                                        // Cauchy: sum of log1p(z^2); Laplace: sum of |r|
-            if constexpr (LIK == 0) {
+            if constexpr (LIK == LIN_BERNOULLI) {
                 const float ys_lane = y_raw * LF_D_SCALE;
                 // Per element, with raw accumulator L (logit l = L * inv1), e = exp(-|l|), sig = sigmoid(l):
                 //   d * S = y S - S sig;   ll = y l - max(l, 0) - ln(1 + e)
@@ -413,7 +414,7 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
                 asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg0) : "f"(pr0));
                 asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg1) : "f"(pr1));
                 ll = inv1 * ((ay0 + ay1) * (1.f / LF_D_SCALE) - acc_mx) - 0.6931471805599453f * (lg0 + lg1);
-            } else if constexpr (LIK == 2) {
+            } else if constexpr (LIK == BRN_LINREG_CAUCHY) {
                 // Cauchy, per element: r = y - L inv1, z = r / sigma_s, q = 1 + z^2 and ONE rcp: d = z / q lies in [-1/2, 1/2] and
                 // goes out at 2^14 (the fp16 pair cannot overflow), z^2 / q adds to T.  log1p(z^2) = ln 2 (e + log2 m) with
                 // q = 2^e m, m in [1, 2): the biased exponents add as integers and ONE lg2 per 16 elements takes the product of
@@ -474,7 +475,7 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
                 // every one of the 32 factors carries the exponent bias 127, padding rows (q = 1) included
                 ll = 0.6931471805599453f * ((float)((int)esum - 127 * LF_EROWS) + (lg0 + lg1));
                 ll2_total += (double)acc_t;
-            } else if constexpr (LIK == 3) {
+            } else if constexpr (LIK == BRN_LINREG_LAPLACE) {
                 // Laplace, per element: r = y - L inv1, d = sign(r) (sign(0) = 0, as torch's abs gradient), exact in fp16 at 2^13
                 // with a zero lo word; |r| adds to A.  No MUFU op.  Rows past the end of a ragged last block get r = 0: d = 0.
                 const uint64_t mi2 = f2_pack(-inv1, -inv1);
@@ -569,18 +570,18 @@ linear_flash_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
         while ((int)chain < n_chains) drain();
         // this CTA's share of + d ll / d W for vector s_glob, features 32 part .. + 31
         if (s_ok) {
-            constexpr float d_scale = LIK == 2 ? 2.f * LF_D_SCALE : LF_D_SCALE;      // Cauchy: |d| <= 1/2 goes out at 2^14
-            const float inv2 = 1.f / ((LIK == 1 ? r_scale : d_scale) * p2_scale(*p.scal_x));
+            constexpr float d_scale = LIK == BRN_LINREG_CAUCHY ? 2.f * LF_D_SCALE : LF_D_SCALE;      // Cauchy: |d| <= 1/2 goes out at 2^14
+            const float inv2 = 1.f / ((LIK == BRN_LINREG_NORMAL ? r_scale : d_scale) * p2_scale(*p.scal_x));
             float* o = p.part + (int64_t)g * p.part_stride + (int64_t)s_glob * F + part * LF_EFEAT;
 #pragma unroll
             for (int c = 0; c < LF_EFEAT; c += 4)
                 if (part * LF_EFEAT + c < F)
                     *reinterpret_cast<float4*>(o + c) = make_float4(r2[c] * inv2, r2[c + 1] * inv2, r2[c + 2] * inv2, r2[c + 3] * inv2);
         }
-        if constexpr (LIK != 0) {
+        if constexpr (LIK != LIN_BERNOULLI) {
             // lane s owns vector s: the two epilogue groups and two row halves of this CTA and every row group add to R[s]
             if (s_ok && ll_total != 0.0) atomicAdd(p.R + s_glob, ll_total);
-            if constexpr (LIK == 2)
+            if constexpr (LIK == BRN_LINREG_CAUCHY)
                 if (s_ok && ll2_total != 0.0) atomicAdd(p.T + s_glob, ll2_total);
         } else {
         double tot = s_ok ? ll_total : 0.0;      // vectors past S are zero rows of the W tile: their terms are not part of the sum
@@ -693,16 +694,18 @@ static int launch_prepare_x(const float* X, int64_t N, int F, float* bound, __ha
     return 0;
 }
 
-// dW [S][F] = + d ll / d W, loss += loss_scale * sum ll for S weight vectors W [S][F] over N rows (Bernoulli, C == 1).
+// The likelihood lik (LIN_BERNOULLI or BRN_LINREG_*) of N rows for S weight vectors W [S][F] in one pass over X.  The per-row-group
+// partials of + d ll / d W go to b.part and, when dW != NULL, their sum to dW [S][F].
+//   LIN_BERNOULLI       loss += loss_scale * sum ll  (R, sigma, T unused)
+//   BRN_LINREG_NORMAL   + d ll / d W is G_s = sum_b r_sb x_b with r_sb = y_b - w_s . x_b, and R[s] += sum_b r_sb^2 (loss unused)
+//   BRN_LINREG_CAUCHY   with the noise scales sigma [S]: G_s = sum_b z/(1 + z^2) x_b, z = r_sb / sigma_s, R[s] += sum_b log1p(z^2),
+//                       T[s] += sum_b z^2/(1 + z^2)
+//   BRN_LINREG_LAPLACE  G_s = sum_b sign(r_sb) x_b, R[s] += sum_b |r_sb|
 // px: a prepared X (the caller keeps it while X does not change: a training loop over fixed data then reads X once per
 // evaluation, as fp16 pairs, instead of three times), or NULL: X is split into the workspace on every call.
-// R != NULL selects a regression epilogue, lik (the LIK codes of linear_flash_kernel): 1 = Gaussian, the per-slice partials of
-// G_s = sum_b r_sb x_b, r_sb = y_b - w_s . x_b, go to b.part and R[s] += sum_b r_sb^2 (loss is unused); 2 = Cauchy, with the
-// noise scales sigma [S]: G_s = sum_b z/(1 + z^2) x_b, z = r_sb / sigma_s, R[s] += sum_b log1p(z^2), T[s] += sum_b z^2/(1 + z^2);
-// 3 = Laplace: G_s = sum_b sign(r_sb) x_b, R[s] += sum_b |r_sb|.
-static int launch_linear_flash(const float* X, const void* px, const float* y, int64_t N, int F, int S, const float* W, float* dW,
-                               float loss_scale, double* loss, const LinearFlashBuffers& b, cudaStream_t stream,
-                               double* R = nullptr, int lik = 1, const float* sigma = nullptr, double* T = nullptr) {
+static int launch_linear_flash(int lik, const float* X, const void* px, const float* y, int64_t N, int F, int S, const float* W,
+                               float* dW, float loss_scale, double* loss, double* R, const float* sigma, double* T,
+                               const LinearFlashBuffers& b, cudaStream_t stream) {
     BRN_CUDA_OK(cudaMemsetAsync(b.scal, 0, 64 * sizeof(float), stream));
     lf_absmax_kernel<<<(unsigned)std::min<int64_t>(((int64_t)S * F / 4 + 255) / 256 + 1, 148), 256, 0, stream>>>(W, (int64_t)S * F, b.scal);
     BRN_LAUNCH_OK("lf_absmax_kernel");
@@ -716,7 +719,7 @@ static int launch_linear_flash(const float* X, const void* px, const float* y, i
     } else if (int e = launch_prepare_x(X, N, F, b.scal + 1, b.Xh, b.Xl, stream)) {
         return e;
     }
-    if (R && lik == 1) {
+    if (lik == BRN_LINREG_NORMAL) {
         lf_absmax_kernel<<<(unsigned)std::min<int64_t>((N / 4 + 255) / 256 + 1, 148), 256, 0, stream>>>(y, N, b.scal + 2);
         BRN_LAUNCH_OK("lf_absmax_kernel");
     }
@@ -732,18 +735,25 @@ static int launch_linear_flash(const float* X, const void* px, const float* y, i
     p.sigma = sigma; p.T = T;
     p.y_bulk = (reinterpret_cast<uintptr_t>(y) & 15) == 0;
     dim3 grid(b.tiles, b.groups);
-    auto launch = [&](auto kern) -> int {
+    auto launch = [&](auto lik_c) -> int {
+        constexpr int LIK = decltype(lik_c)::value;
+        auto kern = F == 128 ? linear_flash_kernel<8, LIK> : linear_flash_kernel<0, LIK>;
         BRN_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, LinearFlashSmem::TOTAL));
         kern<<<grid, LF_THREADS, LinearFlashSmem::TOTAL, stream>>>(tWh, tWl, tXh, tXl, p);
         return 0;
     };
     int e;
-    if (R && lik == 2) e = F == 128 ? launch(linear_flash_kernel<8, 2>) : launch(linear_flash_kernel<0, 2>);
-    else if (R && lik == 3) e = F == 128 ? launch(linear_flash_kernel<8, 3>) : launch(linear_flash_kernel<0, 3>);
-    else if (R) e = F == 128 ? launch(linear_flash_kernel<8, 1>) : launch(linear_flash_kernel<0, 1>);
-    else e = F == 128 ? launch(linear_flash_kernel<8>) : launch(linear_flash_kernel<0>);
+    if (lik == BRN_LINREG_NORMAL) e = launch(std::integral_constant<int, BRN_LINREG_NORMAL>{});
+    else if (lik == BRN_LINREG_CAUCHY) e = launch(std::integral_constant<int, BRN_LINREG_CAUCHY>{});
+    else if (lik == BRN_LINREG_LAPLACE) e = launch(std::integral_constant<int, BRN_LINREG_LAPLACE>{});
+    else e = launch(std::integral_constant<int, LIN_BERNOULLI>{});
     if (e) return e;
     BRN_LAUNCH_OK("linear_flash_kernel");
+    if (dW) {
+        const int64_t tot = (int64_t)S * F;
+        sum_slices_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, stream>>>(b.part, b.groups, tot, tot, dW);
+        BRN_LAUNCH_OK("sum_slices_kernel");
+    }
     return 0;
 }
 

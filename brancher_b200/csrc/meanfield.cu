@@ -498,9 +498,7 @@ using namespace brn;
 
 static int check_range(const brn_sample_range* r) {
     BRN_CHECK_ARG(r != nullptr, "sample range is NULL");
-    BRN_CHECK_ARG(r->s_local >= 0 && r->s_total > 0 && r->s0 >= 0 && r->s0 + r->s_local <= r->s_total,
-                  "bad sample range s0=%d s_local=%d s_total=%d", r->s0, r->s_local, r->s_total);
-    return 0;
+    return check_sample_range(*r);
 }
 
 extern "C" int brn_philox_normal_fill(float* out, int64_t numel, uint32_t var_id, const brn_sample_range* r,

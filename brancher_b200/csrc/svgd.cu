@@ -426,26 +426,21 @@ struct SvgdWorkspace {
     // d2_rows: rows of D2 kept (n for the replicated evaluation, the rank's shard for the sharded one)
     SvgdWorkspace(void* base, int n, int d, int d2_rows = -1) {
         if (d2_rows < 0) d2_rows = n;
-        size_t off = 0;
-        auto take = [&](size_t nbytes) {
-            char* p = base ? reinterpret_cast<char*>(base) + off : nullptr;
-            off += (nbytes + 255) / 256 * 256;
-            return p;
-        };
-        D2 = reinterpret_cast<float*>(take(sizeof(float) * (size_t)(d2_rows > 0 ? d2_rows : 1) * n));
-        hist_off = off;
-        hist = reinterpret_cast<unsigned int*>(take(sizeof(unsigned int) * 4096));
-        st_off = off;
-        st = reinterpret_cast<SelectState*>(take(sizeof(SelectState)));
+        WorkspaceCarver take(base);
+        D2 = take((size_t)(d2_rows > 0 ? d2_rows : 1) * n);
+        hist_off = take.off;
+        hist = reinterpret_cast<unsigned int*>(take.bytes(sizeof(unsigned int) * 4096));
+        st_off = take.off;
+        st = reinterpret_cast<SelectState*>(take.bytes(sizeof(SelectState)));
         // tensor-core variant: theta (hi, lo) [n][ldd], |theta|^2 [n], V^T (hi, lo) [d + 1][ldn]
         ldd = (d + 3) / 4 * 4;
         ldn = (n + 3) / 4 * 4;
-        th_hi = reinterpret_cast<float*>(take(sizeof(float) * (size_t)n * ldd));
-        th_lo = reinterpret_cast<float*>(take(sizeof(float) * (size_t)n * ldd));
-        sq = reinterpret_cast<float*>(take(sizeof(float) * (size_t)n));
-        vt_hi = reinterpret_cast<float*>(take(sizeof(float) * (size_t)(d + 1) * ldn));
-        vt_lo = reinterpret_cast<float*>(take(sizeof(float) * (size_t)(d + 1) * ldn));
-        bytes = off;
+        th_hi = take((size_t)n * ldd);
+        th_lo = take((size_t)n * ldd);
+        sq = take((size_t)n);
+        vt_hi = take((size_t)(d + 1) * ldn);
+        vt_lo = take((size_t)(d + 1) * ldn);
+        bytes = take.off;
     }
 };
 
@@ -479,9 +474,7 @@ extern "C" int brn_svgd_direction(const float* theta, const float* grad, int n, 
         }
     }
     set_variant(use_tc ? "tcgen05" : "simt");
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = device_sm_count();
     {
         StageTimer st("svgd.pairwise_d2", stream);
         if (use_tc) {
@@ -589,9 +582,7 @@ extern "C" int brn_svgd_sharded_phase(const float* theta, const float* grad, int
     SvgdWorkspace ws(workspace, n, d, rows);
     BRN_CHECK_ARG(workspace && workspace_bytes >= ws.bytes, "workspace too small: %zu < %zu", workspace_bytes, ws.bytes);
     set_variant("tcgen05");
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = device_sm_count();
     const unsigned long long m = (unsigned long long)n * (unsigned long long)(n - 1) / 2ull;
     const unsigned long long k1 = (m - 1ull) / 2ull, k2 = m / 2ull;
     int64_t hblocks = ((int64_t)rows * n + 255) / 256;

@@ -499,9 +499,7 @@ inline int launch_umma_nt_kind(const void* Ah, const void* Al, int M, int64_t ld
     if (int e = mk(&tBl, (SPLIT & 2) ? Bh : Bl, N, K, ldb, BN)) return e;        // SPLIT & 2: unused
     const int m_tiles = (M + UG_BM - 1) / UG_BM, n_tiles = (N + BN - 1) / BN, k_chunks = (K + BK * KE - 1) / (BK * KE);
     drain_chunks = drain_chunks * 32 / BK;        // `drain_chunks` is given in units of 32 words of K
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = device_sm_count();
     int grid, split_T = 0, full_units = m_tiles * n_tiles;
     if (mode == 0 || mode == 2) {
         const UmmaSplitPlan pl = umma_plan<BN, BK * KE>(M, N, K, sms, allow_split && mode == 0);
@@ -540,9 +538,7 @@ inline int launch_umma_tn_plain(const float* A, int M, int64_t lda, const float*
     if (int e = make_tmap_2d_f32(&tB, B, K, N, ldb, BK, 32, true)) return e;
     const int m_tiles = (M + UG_BM - 1) / UG_BM, n_tiles = (N + BN - 1) / BN, k_chunks = (K + BK - 1) / BK;
     drain_chunks = drain_chunks * 32 / BK;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = device_sm_count();
     const UmmaSplitPlan pl = umma_plan<BN, BK>(M, N, K, sms, allow_split && mode == 0);
     if (drain_chunks < 1) drain_chunks = 2 * 32 / BK;
     auto kern = umma_nt_3xtf32_kernel<BN, BK, Epi, EW, 3, CW, 0, 1>;

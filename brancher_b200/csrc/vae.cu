@@ -575,13 +575,7 @@ struct VaeWorkspace {
     size_t bytes;
 
     VaeWorkspace(void* base, const brn_vae_model& m, int B, int S) {
-        size_t off = 0;
-        auto takeb = [&](size_t nbytes) {
-            char* p = base ? reinterpret_cast<char*>(base) + off : nullptr;
-            off += (nbytes + 255) / 256 * 256;
-            return p;
-        };
-        auto take = [&](size_t nfloat) { return reinterpret_cast<float*>(takeb(nfloat * sizeof(float))); };
+        WorkspaceCarver take(base);
         // ONE plain fp32 matrix (rm_lo == NULL): the GEMMs that read it split it on the fly (SPLIT mask of umma_gemm.cuh)
         auto act = [&](VaeAct& a, int64_t rows, int n) {
             a.n = n; a.ld = pad4l(n);
@@ -613,7 +607,7 @@ struct VaeWorkspace {
         wsplit(meanW, m.enc_mean, false);
         wsplit(sdW, m.enc_sd, false);
         // zeroed region: scratch gradients (flat), dmean/dsd, scalar accumulators
-        const size_t zb = off;
+        const size_t zb = take.off;
         int64_t g = 0;
         auto gslot = [&](VaeWeights& w, const brn_dense_layer& l) {
             w.offW = g; g += pad4l((int64_t)l.n_out * l.n_in);
@@ -626,14 +620,14 @@ struct VaeWorkspace {
         grads_numel = g;
         grads = take((size_t)g);
         dmean = take((size_t)B * m.L); dsd = take((size_t)B * m.L);
-        acc = reinterpret_cast<double*>(takeb(4 * sizeof(double)));
+        acc = reinterpret_cast<double*>(take.bytes(4 * sizeof(double)));
         zero_begin = base ? reinterpret_cast<char*>(base) + zb : nullptr;
-        zero_bytes = off - zb;
+        zero_bytes = take.off - zb;
         auto gptr = [&](VaeWeights& w) { w.gW = grads ? grads + w.offW : nullptr; w.gb = grads ? grads + w.offb : nullptr; };
         for (int i = 0; i < m.n_enc; ++i) gptr(encW[i]);
         for (int i = 0; i < m.n_dec; ++i) gptr(decW[i]);
         gptr(outW); gptr(meanW); gptr(sdW);
-        bytes = off;
+        bytes = take.off;
     }
 };
 
@@ -687,8 +681,7 @@ extern "C" int brn_vae_elbo_fwd_bwd(const float* X, int B, int64_t row0, int64_t
     if (int e = validate(m)) return e;
     BRN_CHECK_ARG(B > 0 && row0 >= 0 && row0 + B <= B_total, "brn_vae_elbo_fwd_bwd: bad row range row0=%lld B=%d B_total=%lld",
                   (long long)row0, B, (long long)B_total);
-    BRN_CHECK_ARG(r->s_local >= 0 && r->s_total > 0 && r->s0 >= 0 && r->s0 + r->s_local <= r->s_total,
-                  "bad sample range s0=%d s_local=%d s_total=%d", r->s0, r->s_local, r->s_total);
+    if (int e = check_sample_range(*r)) return e;
     const int S = r->s_local, L = m->L, D = m->D;
     if (S == 0) return 0;
     const int64_t R = (int64_t)S * B;
